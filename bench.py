@@ -1,8 +1,9 @@
 #!/usr/bin/env python
-"""Benchmark of the Fiksi solve path on B200 (contract: see the task's bench section).
+"""Benchmark of the Fiksi solve path on B200.
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K ...  # reference arm: CPU restatement
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results to DIR/<name>.npy
 
 Workload: BASELINE.json configs[1] — 65,536 randomly perturbed 20-point rigid distance trusses
 (40 free variables, 37 point-point-distance rows) per GPU, one sketch per warp, solved to the
@@ -89,7 +90,29 @@ def cpu_reference_run(n_sample, threads, first=0):
     v, p, scale = w.prepare()
     op, keep = oracle.make_problem(v[0], w.kind, w.idx, p[0], w.free_vars, w.rows)
     x, rep, secs = oracle.lm_solve_batch_uniform(op, v, p, threads=threads)
-    return n_sample / secs, secs, rep
+    return n_sample / secs, secs, x, rep
+
+
+def solve_outputs(prefix, x, rep):
+    """What a caller of a batched solve receives, as float64 arrays: the solved free variables and every report field
+    (the counters are exact in float64; the 64-bit trace hash goes as its two 32-bit halves)."""
+    import numpy as np
+    out = {prefix + "x": np.array(x, dtype=np.float64)}
+    for k in ("exit_reason", "outer_iters", "factorizations", "accepted", "ssr", "lambda"):
+        out[prefix + k] = rep[k].astype(np.float64)
+    out[prefix + "trace_hash_hi"] = (rep["trace_hash"] >> np.uint64(32)).astype(np.float64)
+    out[prefix + "trace_hash_lo"] = (rep["trace_hash"] & np.uint64(0xFFFFFFFF)).astype(np.float64)
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > 64 << 20:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs, more than 64 MB")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_reference(args, rank, world):
@@ -99,9 +122,11 @@ def run_reference(args, rank, world):
     n_sample = N_PER_GPU  # the same 65,536 sketches per step as our arm (one step is ~0.3 s on 16 host cores)
     times = []
     for k in range(args.warmup + args.steps):
-        rate, secs, rep = cpu_reference_run(n_sample, threads, first=k * n_sample)
+        rate, secs, x, rep = cpu_reference_run(n_sample, threads, first=k * n_sample)
         if k >= args.warmup:
             times.append(secs)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, solve_outputs("", x, rep))
     total = sum(times)
     value = n_sample * len(times) / total
     line = {
@@ -151,7 +176,13 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extras", action="store_true", help="skip the assembly / FP64 side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float64, rank 0's sketches): x and "
+                         "the report fields of the device-resident solve (of the CPU restatement with --impl reference), "
+                         "and the same of the streamed end-to-end call as e2e_*")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -219,9 +250,10 @@ def main():
     gpu_launches = plan.launches - launches0
     plan.download_ptr(hout.data_ptr(), hrep.data_ptr(), stream)
     torch.cuda.synchronize()
-    rep = hrep.numpy().view(fk.REPORT_DTYPE).reshape(-1)
+    rep = hrep.numpy().view(fk.REPORT_DTYPE).reshape(-1).copy()  # the host buffers are reused by the measurements below
+    outputs = solve_outputs("", hout.numpy(), rep) if args.dump_outputs else {}
     solved = float(np.mean(rep["ssr"] < 1e-8))
-    fact = float(rep["factorizations"].sum())  # (the host buffers are reused by the measurements below)
+    fact = float(rep["factorizations"].sum())
 
     # ---- end-to-end through the host-buffer C-ABI calls ------------------------------------------------------
     # (1) the System::solve-level call: RAW variables in, scale + seeded perturbation + LM + write-back on the device,
@@ -236,7 +268,7 @@ def main():
 
     def e2e_prepared():
         topo.batch_solve_into(local_rank, n, hv.data_ptr(), hp.data_ptr(), hout.data_ptr(), hrep.data_ptr())
-    e2e_steps = max(3, args.steps)
+    e2e_steps = args.steps
     e2e_secs = []
     for fn in (e2e_system, e2e_prepared):
         for _ in range(2):
@@ -271,6 +303,9 @@ def main():
     topo.batch_system_solve_wait(prev, local_rank)
     barrier()
     e2e_stream_s = time.perf_counter() - t0
+    if args.dump_outputs:
+        last_out, last_rep = outs[(e2e_steps - 1) & 1]
+        outputs.update(solve_outputs("e2e_", last_out.numpy(), last_rep.numpy().view(fk.REPORT_DTYPE).reshape(-1)))
     streamed_same = bool(np.array_equal(hout2.numpy(), hout.numpy()) and np.array_equal(hrep2.numpy(), hrep.numpy()))
     rep_sys = hrep.numpy().view(fk.REPORT_DTYPE).reshape(-1).copy()
     e2e_system()
@@ -422,7 +457,7 @@ def main():
             cores = os.cpu_count() or 1
             n_cpu, passes, secs = 65536, 0, 0.0
             while passes < 8 and secs * cores < 12.0:  # 10-30 s of CPU work: whole steps of the same workload
-                _, s1, _ = cpu_reference_run(n_cpu, cores, first=passes * n_cpu)
+                _, s1, _, _ = cpu_reference_run(n_cpu, cores, first=passes * n_cpu)
                 secs += s1
                 passes += 1
             rate = n_cpu * passes / secs
@@ -431,6 +466,8 @@ def main():
                                               f"{secs:.1f} s wall = {secs * cores:.0f} core-seconds"}
         else:
             line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": 0, "kind": "port", "sample": "skipped (--no-extras)"}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -9,7 +9,8 @@ reference-cost mode is checked by tests/test_oracle_fast_mode.py) and the script
 
   tests/golden/large_<case>.json   sizes, sha256 of the augmented CSC pattern / COLAMD permutation /
                                    etree / R pattern, the accept-reject trace, exit, counts, ssr, lambda
-  tests/golden/large_<case>_x.npy  the converged free variables (float64)
+  tests/golden/large_<case>_x.npy  the converged free variables (float64); above X_FULL_MAX variables a
+                                   seeded sample of them, described by the JSON's "x_sample"
 
 The inputs come from fiksi_b200.workloads generators (pure numpy, deterministic), so the GPU tests
 rebuild them from the case name.  lattice400x250 needs ~35 GB of RAM and a few hours on one core.
@@ -27,7 +28,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import oracle  # noqa: E402
-from large_cases import build_case  # noqa: E402
+from large_cases import X_FULL_MAX, X_SAMPLE_SIZE, build_case, x_sample_indices  # noqa: E402
 
 
 def sha(a):
@@ -58,6 +59,10 @@ def main():
             meta["oracle_lm_seconds"] = round(time.time() - t0, 1)
         meta["trace"] = trace
         meta["report"] = {k: (float(v).hex() if isinstance(v, float) else int(v)) for k, v in rep.items()}
+        if len(x) > X_FULL_MAX:
+            # the tests normalise by the largest coordinate of the whole solution, so it is kept beside the sample
+            meta["x_sample"] = {"size": X_SAMPLE_SIZE, "seed": 0, "max_abs": float(np.max(np.abs(x))).hex()}
+            x = x[x_sample_indices(len(x), X_SAMPLE_SIZE, 0)]
         np.save(os.path.join(here, f"large_{case}_x.npy"), x)
         with open(os.path.join(here, f"large_{case}.json"), "w") as f:
             json.dump(meta, f, indent=1, sort_keys=True)

@@ -4,6 +4,16 @@ import numpy as np
 
 from fiksi_b200 import workloads as wl
 
+# Golden coordinate files stay well under 1 MB: a case with more than X_FULL_MAX free variables (512 KB)
+# stores a seeded sample of X_SAMPLE_SIZE of them.
+X_FULL_MAX = 65536
+X_SAMPLE_SIZE = 16384
+
+
+def x_sample_indices(n_free, size, seed):
+    """Sorted indices of the converged coordinates that a sampled golden stores."""
+    return np.sort(np.random.default_rng(seed).choice(n_free, size=size, replace=False))
+
 
 def irregular_graph(n_pts, seed=11, ties=4, window=400, extent=100.0, noise=0.01):
     """Random points in sweep order, every point tied to its `ties` nearest earlier points inside a window

@@ -10,6 +10,7 @@ import pytest
 
 import scenarios as sc
 from fiksi_b200 import workloads as wl
+from large_cases import X_FULL_MAX
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 
@@ -83,5 +84,11 @@ def test_golden_fixtures_are_consistent():
     for f in metas:
         meta = json.load(open(os.path.join(g, f)))
         x = np.load(os.path.join(g, f[:-5] + "_x.npy"))
-        assert x.shape == (meta["n_free"],) and np.all(np.isfinite(x))
+        if "x_sample" in meta:
+            assert meta["n_free"] > X_FULL_MAX and x.shape == (meta["x_sample"]["size"],)
+            assert np.max(np.abs(x)) <= float.fromhex(meta["x_sample"]["max_abs"])
+        else:
+            assert x.shape == (meta["n_free"],)
+        assert x.dtype == np.float64 and np.all(np.isfinite(x))
+        assert os.path.getsize(os.path.join(g, f[:-5] + "_x.npy")) < 1 << 20
         assert len(meta["trace"]) == meta["report"]["factorizations"]

@@ -6,6 +6,7 @@
 #include <cstdlib>
 #include <atomic>
 #include <cstring>
+#include <functional>
 #include <list>
 #include <map>
 #include <memory>
@@ -48,6 +49,44 @@ int usable_devices() {
         return 0;
     }
     return n;
+}
+
+// Device arguments of the entry points.  Multi-device calls: n_gpus <= 0 or more than are visible means all visible devices.
+int clamp_gpus(int& n_gpus) {
+    const int ndev = usable_devices();
+    if (ndev == 0) return fail(FK_ERR_NO_DEVICE, "no CUDA device visible; fiksi_b200 has no CPU fallback");
+    if (n_gpus <= 0 || n_gpus > ndev) n_gpus = ndev;
+    return FK_OK;
+}
+int check_device(int device) {
+    int ndev = 0;
+    const int rc = clamp_gpus(ndev);
+    if (rc != FK_OK) return rc;
+    return device >= 0 && device < ndev ? FK_OK : fail(FK_ERR_INVALID, "device index out of range");
+}
+
+// Runs fn(device, lo, hi) on contiguous shares [lo, hi) of n items, one host thread per device, and returns the first failure
+// in device order.  n_gpus == 1: the calling thread on its current device (one process per GPU keeps the device it chose).
+template <class Fn>
+int shard_over_devices(int n_gpus, uint32_t n, const Fn& fn) {
+    if (n_gpus == 1) {
+        int cur = 0;
+        if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
+        return fn(cur, 0u, n);
+    }
+    std::vector<int> rcs(n_gpus, FK_OK);
+    std::vector<std::string> errs(n_gpus);  // (g_error is per thread)
+    std::vector<std::thread> pool;
+    for (int g = 0; g < n_gpus; g++) {
+        const uint32_t lo = (uint32_t)((uint64_t)n * g / n_gpus), hi = (uint32_t)((uint64_t)n * (g + 1) / n_gpus);
+        pool.emplace_back([&, g, lo, hi] {
+            if (hi > lo && (rcs[g] = fn(g, lo, hi)) != FK_OK) errs[g] = g_error;
+        });
+    }
+    for (auto& th : pool) th.join();
+    for (int g = 0; g < n_gpus; g++)
+        if (rcs[g] != FK_OK) return fail(rcs[g], errs[g]);
+    return FK_OK;
 }
 
 // Packs the topology tables into one device allocation and fills the DevProgram view.
@@ -136,7 +175,7 @@ int upload_program(const fk::Topology& t, int device, DeviceProgram& out) {
 }  // namespace
 
 struct fk_batch_plan;
-// Per-device staging pipeline of fk_batch_solve: kStreams plans + streams, reused across calls.
+// Per-device staging pipeline of the host-buffer batch calls: kStreams plans + streams, reused across calls.
 struct DevicePipeline {
 // (eight chunks in flight: a chunk's kernel lasts one LM solve however small the chunk is, so with three the copies of
 // small chunks could not keep the device busy; bench truss end to end 56.2 -> 59.0 M sketches/s with 16 chunks.  Swept on
@@ -157,8 +196,8 @@ struct DevicePipeline {
     unsigned char* small_d = nullptr;
     cudaStream_t small_stream = nullptr;
     cudaEvent_t shared_param_ev = nullptr;  // fk_batch_system_solve with one parameter row for all sketches: its upload, once per call
-    // fk_batch_system_solve_begin / _wait: up to two calls in flight.  A call's token picks (by parity) the events recorded behind its
-    // last chunk on every stream and its copy of the shared parameter row.
+    // Every call on the chunk pipeline takes a token.  Its parity picks the call's copy of the shared parameter row and the events
+    // recorded behind its last chunk on every stream (the _begin / _wait halves: up to two calls in flight).
     uint64_t next_token = 1;
     cudaEvent_t done_ev[2][kStreams] = {};
     double* d_shared_param[2] = {nullptr, nullptr};
@@ -449,7 +488,7 @@ static int single_pass_plan_for(fk_topology* topo, const std::vector<fk_topology
 }
 
 static int single_pass_device_range(fk_topology* topo, const std::vector<fk_topology*>& subs, int device, uint32_t lo, uint32_t hi,
-                                    double* vars, const double* param, fk_report* reports, std::string* err) {
+                                    double* vars, const double* param, fk_report* reports) {
     const fk::Topology& t = topo->t;
     const size_t steps = subs.size();
     uint32_t max_free = 1;
@@ -461,7 +500,6 @@ static int single_pass_device_range(fk_topology* topo, const std::vector<fk_topo
     auto done = [&](int code) {
         if (stream) cudaStreamDestroy(stream);
         cudaFree(d_vars); cudaFree(d_params); cudaFree(d_out); cudaFree(d_rep); cudaFree(d_rep_t);
-        if (code != FK_OK && err) *err = g_error;
         return code;
     };
 #define SP_CU(call)                                              \
@@ -514,32 +552,15 @@ int fk_batch_solve_single_pass(const fk_topology* topo_c, uint32_t n, double* va
     if (rc != FK_OK) return rc;
     if (n_steps) *n_steps = (uint32_t)subs->size();
     if (n == 0) return FK_OK;
-    const int ndev = usable_devices();
-    if (ndev == 0) return fail(FK_ERR_NO_DEVICE, "no CUDA device visible; fiksi_b200 has no CPU fallback");
-    if (n_gpus <= 0 || n_gpus > ndev) n_gpus = ndev;
-    if (n_gpus == 1) {
-        int cur = 0;
-        if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
-        return single_pass_device_range(topo, *subs, cur, 0, n, vars, param, reports, nullptr);
-    }
-    std::vector<int> rcs(n_gpus, FK_OK);
-    std::vector<std::string> errs(n_gpus);
-    std::vector<std::thread> pool;
-    for (int g = 0; g < n_gpus; g++) {
-        const uint32_t lo = (uint32_t)((uint64_t)n * g / n_gpus), hi = (uint32_t)((uint64_t)n * (g + 1) / n_gpus);
-        pool.emplace_back([=, &rcs, &errs]() {
-            if (hi > lo) rcs[g] = single_pass_device_range(topo, *subs, g, lo, hi, vars, param, reports, &errs[g]);
-        });
-    }
-    for (auto& th : pool) th.join();
-    for (int g = 0; g < n_gpus; g++)
-        if (rcs[g] != FK_OK) return fail(rcs[g], errs[g]);
-    return FK_OK;
+    if ((rc = clamp_gpus(n_gpus)) != FK_OK) return rc;
+    return shard_over_devices(n_gpus, n, [&](int device, uint32_t lo, uint32_t hi) {
+        return single_pass_device_range(topo, *subs, device, lo, hi, vars, param, reports);
+    });
 }
 
 // ---- L-BFGS on a uniform batch -------------------------------------------------------------------
 static int run_device_range(fk_topology* topo, int device, uint32_t lo, uint32_t hi, const double* vars, const double* param,
-                            double* free_out, fk_report* reports, std::string* err, int optimizer = 0, uint64_t* token = nullptr);
+                            double* free_out, fk_report* reports, int optimizer = 0, uint64_t* token = nullptr);
 
 int fk_batch_solve_lbfgs(const fk_topology* topo_c, int device, uint32_t n, const double* vars, const double* param, double* free_out,
                          fk_report* reports) {
@@ -547,20 +568,18 @@ int fk_batch_solve_lbfgs(const fk_topology* topo_c, int device, uint32_t n, cons
     if (n == 0) return FK_OK;
     if (!vars || !free_out || !reports || (!param && topo_c->t.n_expr)) return fail(FK_ERR_INVALID, "null buffer");
     if (topo_c->t.path != 0) return fail(FK_ERR_TOO_LARGE, "L-BFGS is built for the shared-memory tile paths only");
-    const int ndev = usable_devices();
-    if (ndev == 0) return fail(FK_ERR_NO_DEVICE, "no CUDA device visible; fiksi_b200 has no CPU fallback");
-    if (device < 0 || device >= ndev) return fail(FK_ERR_INVALID, "device index out of range");
+    const int rc = check_device(device);
+    if (rc != FK_OK) return rc;
     // same pooled plans / streams / pinned staging as the LM entry (no allocation per call)
-    return run_device_range(const_cast<fk_topology*>(topo_c), device, 0, n, vars, param, free_out, reports, nullptr, 1);
+    return run_device_range(const_cast<fk_topology*>(topo_c), device, 0, n, vars, param, free_out, reports, 1);
 }
 
 // ---- System::analyze on a batch -----------------------------------------------------------------
 int fk_batch_analyze(const fk_topology* topo_c, int device, uint32_t n, const double* vars, const double* param, uint8_t* independent) {
     fk_topology* topo = const_cast<fk_topology*>(topo_c);
     if (!topo || (n && (!vars || !independent || (!param && topo->t.n_expr)))) return fail(FK_ERR_INVALID, "null argument");
-    const int ndev = usable_devices();
-    if (ndev == 0) return fail(FK_ERR_NO_DEVICE, "no CUDA device visible; fiksi_b200 has no CPU fallback");
-    if (device < 0 || device >= ndev) return fail(FK_ERR_INVALID, "device index out of range");
+    const int rc = check_device(device);
+    if (rc != FK_OK) return rc;
     const fk::Topology& t = topo->t;
     if (n == 0 || t.n_expr == 0) return FK_OK;
     AnalyzePool* pool;
@@ -611,9 +630,8 @@ int fk_batch_analyze(const fk_topology* topo_c, int device, uint32_t n, const do
 int fk_batch_plan_create(const fk_topology* topo_c, uint32_t capacity, int device, fk_batch_plan** out) {
     fk_topology* topo = const_cast<fk_topology*>(topo_c);
     if (!topo || !out || capacity == 0) return fail(FK_ERR_INVALID, "null topology / zero capacity");
-    int ndev = usable_devices();
-    if (ndev == 0) return fail(FK_ERR_NO_DEVICE, "no CUDA device visible; fiksi_b200 has no CPU fallback");
-    if (device < 0 || device >= ndev) return fail(FK_ERR_INVALID, "device index out of range");
+    int rc = check_device(device);
+    if (rc != FK_OK) return rc;
     if (topo->t.path == 2)
         return fail(FK_ERR_TOO_LARGE, "topology needs the global sparse path; use fk_lm_solve");
     CU(cudaSetDevice(device));
@@ -622,7 +640,7 @@ int fk_batch_plan_create(const fk_topology* topo_c, uint32_t capacity, int devic
     if (prop.major != 10) return fail(FK_ERR_NO_DEVICE, "device is not sm_100 class; kernels are built for sm_100a only");
     std::unique_ptr<fk_batch_plan> p(new fk_batch_plan());
     p->topo = topo; p->device = device; p->capacity = capacity;
-    int rc = topo->program_for(device, &p->prog, &p->full);
+    rc = topo->program_for(device, &p->prog, &p->full);
     if (rc != FK_OK) return rc;
     const fk::Topology& t = topo->t;
     CU(cudaMalloc(&p->d_vars, sizeof(double) * std::max<size_t>(1, (size_t)capacity * t.n_vars)));
@@ -766,12 +784,20 @@ void fk_host_free(void* p) {
     if (p) cudaFreeHost(p);
 }
 
-// Chunk of the host-buffer pipelines: about an eighth of the request (copies of one chunk overlap the kernels of the
-// others), at least 2,048 sketches, and whole waves of the sketch-per-thread kernel when that is the kernel in use.
-static uint32_t pipeline_chunk(fk_topology* topo, int device, uint32_t total, uint32_t n_chunks) {
+// ---- host-buffer batch: shard by sketch over the devices, pipeline chunks per device ----------------
+// Chunk of the host-buffer pipeline: about 1/n_chunks of the request (FK_E2E_CHUNKS overrides n_chunks; copies of one chunk
+// overlap the kernels of the others), at least 2,048 sketches, and with `waves` whole waves of the sketch-per-thread kernel when
+// that is the kernel in use.
+static uint32_t pipeline_chunk(fk_topology* topo, int device, uint32_t total, uint32_t n_chunks, bool waves) {
+    static const uint32_t env_chunks = [] {
+        const char* e = std::getenv("FK_E2E_CHUNKS");  // tuning knob
+        const int v = e ? std::atoi(e) : 0;
+        return (uint32_t)(v >= 1 && v <= 256 ? v : 0);
+    }();
+    if (env_chunks) n_chunks = env_chunks;
     uint32_t chunk = std::min(total, std::max<uint32_t>(2048, (total + n_chunks - 1) / n_chunks));
     const fk::DevProgram* prog = nullptr;
-    if (topo->program_for(device, &prog) == FK_OK && fk::batch_lm_uses_sketch_kernel(*prog, total)) {
+    if (waves && topo->program_for(device, &prog) == FK_OK && fk::batch_lm_uses_sketch_kernel(*prog, total)) {
         static int sms[64] = {0};
         if (device >= 0 && device < 64 && sms[device] == 0) {
             int v = 0;
@@ -783,7 +809,99 @@ static uint32_t pipeline_chunk(fk_topology* topo, int device, uint32_t total, ui
     return chunk;
 }
 
-// ---- host-buffer batch: shard by sketch over the devices, pipeline chunks per device ----------------
+// The chunk pipeline of one (topology, device), shared by every host-buffer batch call on it.  Sketches [lo, hi) go in chunks of
+// `chunk` over FK_E2E_STREAMS streams (default: all kStreams), each stream with its own pooled plan, which is reused only after its
+// previous chunk has drained.  `prologue` (optional) runs once under the pipeline's lock before the first chunk, with the call's
+// token slot and the number of streams in use.  `enqueue` enqueues the upload, kernels and download of one chunk on the plan's
+// stream and calls mark() after the upload and after the kernels (the FK_E2E_TRACE timeline).
+// token == nullptr: returns when the results are in the caller's buffers.  Otherwise it returns once every chunk is enqueued (the
+// host still waits, chunk by chunk, for a free plan) and *token names the call for fk_batch_system_solve_wait.  On an error it
+// first drains every stream, so that no copy into the caller's buffers is still running when it returns.
+using PipelinePrologue = std::function<int(DevicePipeline& pl, int slot, uint32_t use_streams)>;
+using PipelineChunk = std::function<int(fk_batch_plan* p, cudaStream_t st, uint32_t at, uint32_t cnt, const std::function<void()>& mark)>;
+static int run_pipeline(fk_topology* topo, int device, uint32_t lo, uint32_t hi, uint32_t chunk, uint64_t* token,
+                        const PipelinePrologue& prologue, const PipelineChunk& enqueue) {
+    constexpr uint32_t kStreams = DevicePipeline::kStreams;
+    static const uint32_t use_streams = [] {
+        const char* e = std::getenv("FK_E2E_STREAMS");  // tuning knob: chunks in flight (at most kStreams)
+        const int v = e ? std::atoi(e) : 0;
+        return (uint32_t)(v >= 1 && v <= (int)kStreams ? v : (int)kStreams);
+    }();
+    // FK_E2E_TRACE=1 (debug): CUDA-event timeline of the chunks of every call to stderr (upload done / kernel done / download done)
+    static const bool trace = std::getenv("FK_E2E_TRACE") != nullptr;
+    CU(cudaSetDevice(device));
+    DevicePipeline* pl = topo->pipeline_for(device);
+    std::lock_guard<std::mutex> lock(pl->mu);
+    int rc = FK_OK;
+    if (pl->chunk < chunk) {
+        pl->release();
+        for (uint32_t s = 0; s < kStreams && rc == FK_OK; s++) {
+            rc = fk_batch_plan_create(topo, chunk, device, &pl->plans[s]);
+            if (rc == FK_OK && cudaStreamCreateWithFlags(&pl->streams[s], cudaStreamNonBlocking) != cudaSuccess)
+                rc = fail(FK_ERR_CUDA, "cudaStreamCreate failed");
+        }
+        if (rc != FK_OK) {
+            pl->release();
+            return rc;
+        }
+        pl->chunk = chunk;
+    }
+    const uint64_t my_token = pl->next_token++;
+    const int slot = (int)(my_token & 1u);
+    uint32_t s = 0;
+    std::vector<cudaEvent_t> tev;
+    cudaEvent_t t_start = nullptr;
+    const std::function<void()> mark = [&] {
+        if (!trace) return;
+        cudaEvent_t ev;
+        cudaEventCreate(&ev);
+        cudaEventRecord(ev, pl->streams[s]);
+        tev.push_back(ev);
+    };
+    if (trace) {
+        cudaEventCreate(&t_start);
+        cudaEventRecord(t_start, pl->streams[0]);
+    }
+    if (prologue) rc = prologue(*pl, slot, use_streams);
+    for (uint32_t at = lo; at < hi && rc == FK_OK; at += chunk, s = (s + 1) % use_streams) {
+        const cudaError_t e = cudaStreamSynchronize(pl->streams[s]);
+        if (e != cudaSuccess) {
+            rc = cuda_fail(e, "cudaStreamSynchronize");
+            break;
+        }
+        rc = enqueue(pl->plans[s], pl->streams[s], at, std::min(chunk, hi - at), mark);
+        mark();
+    }
+    auto record_done = [&]() -> int {  // the _begin half: events behind the call's last chunk on every stream
+        for (uint32_t k = 0; k < kStreams; k++) {
+            if (!pl->done_ev[slot][k]) CU(cudaEventCreateWithFlags(&pl->done_ev[slot][k], cudaEventDisableTiming));
+            CU(cudaEventRecord(pl->done_ev[slot][k], pl->streams[k]));
+        }
+        return FK_OK;
+    };
+    if (rc == FK_OK && token && !trace && (rc = record_done()) == FK_OK) {
+        *token = my_token;
+        return FK_OK;
+    }
+    for (uint32_t k = 0; k < kStreams; k++) {
+        const cudaError_t e = cudaStreamSynchronize(pl->streams[k]);
+        if (e != cudaSuccess && rc == FK_OK) rc = cuda_fail(e, "batch kernel / copy failed");
+    }
+    if (rc == FK_OK && token) *token = my_token;  // (tracing: the call has completed; waiting for it is a no-op)
+    if (trace) {
+        for (size_t c = 0; c + 2 < tev.size(); c += 3) {
+            float a = 0, b = 0, d = 0;
+            cudaEventElapsedTime(&a, t_start, tev[c]);
+            cudaEventElapsedTime(&b, t_start, tev[c + 1]);
+            cudaEventElapsedTime(&d, t_start, tev[c + 2]);
+            fprintf(stderr, "[e2e trace] chunk %2zu: upload done %7.1f us, kernel done %7.1f us, download done %7.1f us\n", c / 3, a * 1e3f, b * 1e3f, d * 1e3f);
+        }
+        for (cudaEvent_t ev : tev) cudaEventDestroy(ev);
+        cudaEventDestroy(t_start);
+    }
+    return rc;
+}
+
 static int launch_optimizer(const fk::DevProgram& prog, const DeviceProgram& full, int optimizer, uint32_t n, const double* vars,
                             const double* params, double* out, fk_report* reps, cudaStream_t st) {
     if (optimizer == 1) return fk::launch_batch_lbfgs(prog, full.jcolptr, full.jrow, n, vars, params, out, reps, st);
@@ -792,36 +910,26 @@ static int launch_optimizer(const fk::DevProgram& prog, const DeviceProgram& ful
 
 // Small request (one sketch, a handful): the caller's (pageable) arrays go through ONE pinned staging block -- one
 // copy in, the kernel, one copy out, one synchronisation -- instead of four pageable copies on the chunk pipeline.
-// (Enqueue and finish are separate so that a caller can overlap host work with the request.)
-struct SmallRequest {
-    DevicePipeline* pl = nullptr;
-    std::unique_lock<std::mutex> lock;  // the pipeline's staging block is ours until finish()
-    size_t in_al = 0, out_x = 0, out_r = 0;
-};
 static bool small_fits(const fk::Topology& t, uint32_t total) {
     const size_t in_v = sizeof(double) * (size_t)total * t.n_vars, in_p = sizeof(double) * (size_t)total * t.n_expr;
     const size_t out_x = sizeof(double) * (size_t)total * t.n_free, out_r = sizeof(fk_report) * (size_t)total;
     return ((in_v + in_p + 15) & ~size_t(15)) + out_x + out_r <= DevicePipeline::kSmallBytes;
 }
-static int small_enqueue(fk_topology* topo, int device, uint32_t lo, uint32_t hi, const double* vars, const double* param, int optimizer,
-                         SmallRequest& rq, std::string* err) {
+static int small_solve(fk_topology* topo, int device, uint32_t lo, uint32_t hi, const double* vars, const double* param,
+                       double* free_out, fk_report* reports, int optimizer) {
     const fk::Topology& t = topo->t;
     const uint32_t total = hi - lo;
     DevicePipeline* pl = topo->pipeline_for(device);
-    rq.lock = std::unique_lock<std::mutex>(pl->mu);
-    rq.pl = pl;
+    std::lock_guard<std::mutex> lock(pl->mu);  // the pipeline's staging block is ours until the results are copied out
     const size_t in_v = sizeof(double) * (size_t)total * t.n_vars, in_p = sizeof(double) * (size_t)total * t.n_expr;
-    rq.out_x = sizeof(double) * (size_t)total * t.n_free;
-    rq.out_r = sizeof(fk_report) * (size_t)total;
-    rq.in_al = (in_v + in_p + 15) & ~size_t(15);
+    const size_t out_x = sizeof(double) * (size_t)total * t.n_free, out_r = sizeof(fk_report) * (size_t)total;
+    const size_t in_al = (in_v + in_p + 15) & ~size_t(15);
     const fk::DevProgram* prog = nullptr;
     const DeviceProgram* full = nullptr;
     int rc = topo->program_for(device, &prog, &full);
-    auto give_up = [&](int code) { if (err) *err = g_error; rq.lock.unlock(); rq.pl = nullptr; return code; };
-    if (rc != FK_OK) return give_up(rc);
-    auto bad = [&](cudaError_t e, const char* what) { return give_up(cuda_fail(e, what)); };
+    if (rc != FK_OK) return rc;
     cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) return bad(e, "cudaSetDevice");
+    if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
     if (!pl->small_h || !pl->small_d || !pl->small_stream) {
         // all three or none: a half-initialised block would poison every later call on this topology
         if (pl->small_h) cudaFreeHost(pl->small_h);
@@ -829,14 +937,14 @@ static int small_enqueue(fk_topology* topo, int device, uint32_t lo, uint32_t hi
         if (pl->small_stream) cudaStreamDestroy(pl->small_stream);
         pl->small_h = pl->small_d = nullptr;
         pl->small_stream = nullptr;
-        if ((e = cudaMallocHost((void**)&pl->small_h, DevicePipeline::kSmallBytes)) != cudaSuccess) { pl->small_h = nullptr; return bad(e, "cudaMallocHost"); }
+        if ((e = cudaMallocHost((void**)&pl->small_h, DevicePipeline::kSmallBytes)) != cudaSuccess) { pl->small_h = nullptr; return cuda_fail(e, "cudaMallocHost"); }
         if ((e = cudaMalloc((void**)&pl->small_d, DevicePipeline::kSmallBytes)) != cudaSuccess) {
             cudaFreeHost(pl->small_h); pl->small_h = pl->small_d = nullptr;
-            return bad(e, "cudaMalloc");
+            return cuda_fail(e, "cudaMalloc");
         }
         if ((e = cudaStreamCreateWithFlags(&pl->small_stream, cudaStreamNonBlocking)) != cudaSuccess) {
             cudaFreeHost(pl->small_h); cudaFree(pl->small_d); pl->small_h = pl->small_d = nullptr; pl->small_stream = nullptr;
-            return bad(e, "cudaStreamCreate");
+            return cuda_fail(e, "cudaStreamCreate");
         }
     }
     std::memcpy(pl->small_h, vars + (size_t)lo * t.n_vars, in_v);
@@ -849,125 +957,40 @@ static int small_enqueue(fk_topology* topo, int device, uint32_t lo, uint32_t hi
         int dev = 0, ok = 0;
         return cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&ok, cudaDevAttrCanUseHostPointerForRegisteredMem, dev) == cudaSuccess && ok != 0;
     }();
-    const bool zero_copy = !no_zero_copy && can_map && rq.in_al + rq.out_x + rq.out_r <= 8 * 1024;
+    const bool zero_copy = !no_zero_copy && can_map && in_al + out_x + out_r <= 8 * 1024;
     unsigned char* base = zero_copy ? pl->small_h : pl->small_d;
-    if (!zero_copy && (e = cudaMemcpyAsync(pl->small_d, pl->small_h, in_v + in_p, cudaMemcpyHostToDevice, pl->small_stream)) != cudaSuccess) return bad(e, "cudaMemcpyAsync");
+    if (!zero_copy && (e = cudaMemcpyAsync(pl->small_d, pl->small_h, in_v + in_p, cudaMemcpyHostToDevice, pl->small_stream)) != cudaSuccess) return cuda_fail(e, "cudaMemcpyAsync");
     const int le = launch_optimizer(*prog, *full, optimizer, total, (const double*)base, (const double*)(base + in_v),
-                                    (double*)(base + rq.in_al), (fk_report*)(base + rq.in_al + rq.out_x), pl->small_stream);
-    if (le == (int)cudaErrorInvalidConfiguration && optimizer == 1) { fail(FK_ERR_TOO_LARGE, "the L-BFGS state of one sketch does not fit the tile path"); return give_up(FK_ERR_TOO_LARGE); }
-    if (le != 0) return bad((cudaError_t)le, "launch batched solve kernel");
-    if (!zero_copy && (e = cudaMemcpyAsync(pl->small_h + rq.in_al, pl->small_d + rq.in_al, rq.out_x + rq.out_r, cudaMemcpyDeviceToHost, pl->small_stream)) != cudaSuccess) return bad(e, "cudaMemcpyAsync");
+                                    (double*)(base + in_al), (fk_report*)(base + in_al + out_x), pl->small_stream);
+    if (le == (int)cudaErrorInvalidConfiguration && optimizer == 1) return fail(FK_ERR_TOO_LARGE, "the L-BFGS state of one sketch does not fit the tile path");
+    if (le != 0) return cuda_fail((cudaError_t)le, "launch batched solve kernel");
+    if (!zero_copy && (e = cudaMemcpyAsync(pl->small_h + in_al, pl->small_d + in_al, out_x + out_r, cudaMemcpyDeviceToHost, pl->small_stream)) != cudaSuccess) return cuda_fail(e, "cudaMemcpyAsync");
+    if ((e = cudaStreamSynchronize(pl->small_stream)) != cudaSuccess) return cuda_fail(e, "batch kernel / copy failed");
+    std::memcpy(free_out + (size_t)lo * t.n_free, pl->small_h + in_al, out_x);
+    if (reports) std::memcpy(reports + lo, pl->small_h + in_al + out_x, out_r);
     return FK_OK;
 }
-static int small_finish(const fk::Topology& t, uint32_t lo, SmallRequest& rq, double* free_out, fk_report* reports, std::string* err) {
-    if (!rq.pl) return FK_OK;
-    DevicePipeline* pl = rq.pl;
-    int rc = FK_OK;
-    const cudaError_t e = cudaStreamSynchronize(pl->small_stream);
-    if (e != cudaSuccess) {
-        rc = cuda_fail(e, "batch kernel / copy failed");
-        if (err) *err = g_error;
-    } else {
-        std::memcpy(free_out + (size_t)lo * t.n_free, pl->small_h + rq.in_al, rq.out_x);
-        if (reports) std::memcpy(reports + lo, pl->small_h + rq.in_al + rq.out_x, rq.out_r);
-    }
-    rq.lock.unlock();
-    rq.pl = nullptr;
-    return rc;
-}
 
-// token != nullptr: return once every chunk is enqueued; *token names the call for fk_batch_solve_device_wait (0: already complete).
+// Sketches [lo, hi) of a uniform batch on one device: a small request through the staging block, anything larger through the
+// chunk pipeline.  optimizer 1: L-BFGS.  token: see run_pipeline; the caller sets *token = 0, which is what a small request
+// (complete when it returns) leaves there.
 static int run_device_range(fk_topology* topo, int device, uint32_t lo, uint32_t hi, const double* vars, const double* param,
-                            double* free_out, fk_report* reports, std::string* err, int optimizer, uint64_t* token) {
+                            double* free_out, fk_report* reports, int optimizer, uint64_t* token) {
+    if (hi == lo) return FK_OK;
     const fk::Topology& t = topo->t;
-    const uint32_t total = hi - lo;
-    if (token) *token = 0;
-    if (total == 0) return FK_OK;
-    if (small_fits(t, total)) {
-        SmallRequest rq;
-        int rc = small_enqueue(topo, device, lo, hi, vars, param, optimizer, rq, err);
-        if (rc == FK_OK) rc = small_finish(t, lo, rq, free_out, reports, err);
-        return rc;
-    }
-    DevicePipeline* pl = topo->pipeline_for(device);
-    std::lock_guard<std::mutex> lock(pl->mu);
-    constexpr uint32_t kStreams = DevicePipeline::kStreams;
-    // chunks small enough to overlap H2D / kernel / D2H, large enough to fill the machine
-    static const uint32_t n_chunks = [] {
-        const char* e = std::getenv("FK_E2E_CHUNKS");  // tuning knob
-        const int v = e ? std::atoi(e) : 0;
-        return (uint32_t)(v >= 1 && v <= 256 ? v : 8);
-    }();
-    uint32_t chunk = optimizer == 0 ? pipeline_chunk(topo, device, total, n_chunks)
-                                    : std::min(total, std::max<uint32_t>(2048, (total + n_chunks - 1) / n_chunks));
-    int rc = FK_OK;
-    if (pl->chunk < chunk) {
-        pl->release();
-        for (uint32_t s = 0; s < kStreams && rc == FK_OK; s++) {
-            rc = fk_batch_plan_create(topo, chunk, device, &pl->plans[s]);
-            if (rc == FK_OK && cudaStreamCreateWithFlags(&pl->streams[s], cudaStreamNonBlocking) != cudaSuccess)
-                rc = fail(FK_ERR_CUDA, "cudaStreamCreate failed");
-        }
-        if (rc == FK_OK) pl->chunk = chunk;
-        else pl->release();
-    } else {
-        if (pl->chunk < total) chunk = std::min(chunk, pl->chunk);  // (plans sized by an earlier, smaller request)
-    }
-    // FK_E2E_TRACE=1 (debug): CUDA-event timeline of the chunks of one call to stderr (upload done / kernel done / download done)
-    static const bool trace = std::getenv("FK_E2E_TRACE") != nullptr;
-    std::vector<cudaEvent_t> tev;
-    cudaEvent_t t_start = nullptr;
-    auto stamp = [&](cudaStream_t st) {
-        if (!trace) return;
-        cudaEvent_t ev;
-        cudaEventCreate(&ev);
-        cudaEventRecord(ev, st);
-        tev.push_back(ev);
-    };
-    if (trace) {
-        cudaEventCreate(&t_start);
-        cudaEventRecord(t_start, pl->streams[0]);
-    }
-    uint32_t s = 0;
-    for (uint32_t at = lo; at < hi && rc == FK_OK; at += chunk, s = (s + 1) % kStreams) {
-        uint32_t cnt = std::min(chunk, hi - at);
-        // a plan's buffers are reused only after its previous chunk has fully drained
-        if (cudaStreamSynchronize(pl->streams[s]) != cudaSuccess) { rc = fail(FK_ERR_CUDA, "stream sync failed"); break; }
-        rc = fk_batch_plan_upload(pl->plans[s], cnt, vars + (size_t)at * t.n_vars, param ? param + (size_t)at * t.n_expr : nullptr, pl->streams[s]);
-        stamp(pl->streams[s]);
-        if (rc == FK_OK) rc = optimizer == 1 ? fk_batch_plan_run_lbfgs(pl->plans[s], pl->streams[s]) : fk_batch_plan_run(pl->plans[s], pl->streams[s]);
-        stamp(pl->streams[s]);
-        if (rc == FK_OK) rc = fk_batch_plan_download(pl->plans[s], free_out + (size_t)at * t.n_free, reports ? reports + at : nullptr, pl->streams[s]);
-        stamp(pl->streams[s]);
-    }
-    if (token && !trace && rc == FK_OK) {
-        const uint64_t my_token = pl->next_token++;
-        const int slot = (int)(my_token & 1u);
-        for (uint32_t k = 0; k < kStreams; k++) {
-            if (!pl->streams[k]) continue;
-            if (!pl->done_ev[slot][k] && cudaEventCreateWithFlags(&pl->done_ev[slot][k], cudaEventDisableTiming) != cudaSuccess)
-                return fail(FK_ERR_CUDA, "cudaEventCreate failed");
-            if (cudaEventRecord(pl->done_ev[slot][k], pl->streams[k]) != cudaSuccess) return fail(FK_ERR_CUDA, "cudaEventRecord failed");
-        }
-        *token = my_token;
-        return FK_OK;
-    }
-    for (uint32_t k = 0; k < kStreams; k++)
-        if (pl->streams[k] && cudaStreamSynchronize(pl->streams[k]) != cudaSuccess && rc == FK_OK)
-            rc = cuda_fail(cudaGetLastError(), "batch kernel / copy failed");
-    if (trace) {
-        for (size_t c = 0; c + 2 < tev.size(); c += 3) {
-            float a = 0, b = 0, d = 0;
-            cudaEventElapsedTime(&a, t_start, tev[c]);
-            cudaEventElapsedTime(&b, t_start, tev[c + 1]);
-            cudaEventElapsedTime(&d, t_start, tev[c + 2]);
-            fprintf(stderr, "[e2e trace] chunk %2zu: upload done %7.1f us, kernel done %7.1f us, download done %7.1f us\n", c / 3, a * 1e3f, b * 1e3f, d * 1e3f);
-        }
-        for (cudaEvent_t ev : tev) cudaEventDestroy(ev);
-        cudaEventDestroy(t_start);
-    }
-    if (rc != FK_OK && err) *err = g_error;
-    return rc;
+    if (small_fits(t, hi - lo)) return small_solve(topo, device, lo, hi, vars, param, free_out, reports, optimizer);
+    // (the L-BFGS kernel is not the sketch-per-thread kernel: its chunks are not rounded to that kernel's waves)
+    const uint32_t chunk = pipeline_chunk(topo, device, hi - lo, 8, optimizer == 0);
+    return run_pipeline(topo, device, lo, hi, chunk, token, nullptr,
+                        [&](fk_batch_plan* p, cudaStream_t st, uint32_t at, uint32_t cnt, const std::function<void()>& mark) {
+                            int rc = fk_batch_plan_upload(p, cnt, vars + (size_t)at * t.n_vars, param ? param + (size_t)at * t.n_expr : nullptr, st);
+                            if (rc != FK_OK) return rc;
+                            mark();
+                            rc = optimizer == 1 ? fk_batch_plan_run_lbfgs(p, st) : fk_batch_plan_run(p, st);
+                            if (rc != FK_OK) return rc;
+                            mark();
+                            return fk_batch_plan_download(p, free_out + (size_t)at * t.n_free, reports ? reports + at : nullptr, st);
+                        });
 }
 
 // ---- System::solve level batch: scale, perturbation and write-back on the device -----------------------------
@@ -1015,11 +1038,9 @@ static int prepare_tables_for(fk_topology* topo, int device, const fk_prepare_op
     return FK_OK;
 }
 
-// token == nullptr: the call returns when the results are in the caller's buffers.  Otherwise it returns once every chunk is
-// enqueued (the host still waits, chunk by chunk, for a free plan: at most kStreams chunks are in flight) and *token names the
-// call for fk_batch_system_solve_wait.
-static int system_solve_enqueue(const fk_topology* topo_c, int device, uint32_t n, const double* raw_vars, const double* raw_param,
-                                const fk_prepare_opts* opts, double* free_out, double* scales_out, fk_report* reports, uint64_t* token) {
+// fk_batch_system_solve, and its _begin half with a token.
+static int batch_system_solve(const fk_topology* topo_c, int device, uint32_t n, const double* raw_vars, const double* raw_param,
+                              const fk_prepare_opts* opts, double* free_out, double* scales_out, fk_report* reports, uint64_t* token) {
     fk_topology* topo = const_cast<fk_topology*>(topo_c);
     if (!topo || !opts) return fail(FK_ERR_INVALID, "null argument");
     if (token) *token = 0;
@@ -1027,89 +1048,49 @@ static int system_solve_enqueue(const fk_topology* topo_c, int device, uint32_t 
     const fk::Topology& t = topo->t;
     if (!raw_vars || !free_out || (!raw_param && t.n_expr)) return fail(FK_ERR_INVALID, "null buffer");
     if (t.path == 2) return fail(FK_ERR_TOO_LARGE, "topology needs the global sparse path; use fk_system_solve");
-    const int ndev = usable_devices();
-    if (ndev == 0) return fail(FK_ERR_NO_DEVICE, "no CUDA device visible; fiksi_b200 has no CPU fallback");
-    if (device < 0 || device >= ndev) return fail(FK_ERR_INVALID, "device index out of range");
-    PrepareTables* pt = nullptr;
-    int rc = prepare_tables_for(topo, device, *opts, &pt);
+    int rc = check_device(device);
     if (rc != FK_OK) return rc;
+    PrepareTables* pt = nullptr;
+    if ((rc = prepare_tables_for(topo, device, *opts, &pt)) != FK_OK) return rc;
     const bool shared = (opts->flags & FK_PREP_SHARED_PARAM) != 0;
-    DevicePipeline* pl = topo->pipeline_for(device);
-    std::lock_guard<std::mutex> lock(pl->mu);
-    constexpr uint32_t kStreams = DevicePipeline::kStreams;
-    static const uint32_t n_chunks = [] {
-        const char* e = std::getenv("FK_E2E_CHUNKS");  // tuning knob
-        const int v = e ? std::atoi(e) : 0;
-        return (uint32_t)(v >= 1 && v <= 256 ? v : 16);
-    }();
-    uint32_t chunk = pipeline_chunk(topo, device, n, n_chunks);
-    if (pl->chunk < chunk) {
-        pl->release();
-        for (uint32_t s = 0; s < kStreams && rc == FK_OK; s++) {
-            rc = fk_batch_plan_create(topo, chunk, device, &pl->plans[s]);
-            if (rc == FK_OK && cudaStreamCreateWithFlags(&pl->streams[s], cudaStreamNonBlocking) != cudaSuccess) rc = fail(FK_ERR_CUDA, "cudaStreamCreate failed");
-        }
-        if (rc == FK_OK) pl->chunk = chunk;
-        else { pl->release(); return rc; }
-    }
-    CU(cudaSetDevice(device));
-    for (uint32_t s = 0; s < kStreams; s++) {  // unscaled input / scale buffers of the plans, on first use
-        fk_batch_plan* p = pl->plans[s];
-        if (!p->d_raw_vars) CU(cudaMalloc(&p->d_raw_vars, sizeof(double) * std::max<size_t>(1, (size_t)p->capacity * t.n_vars)));
-        if (!p->d_raw_param) CU(cudaMalloc(&p->d_raw_param, sizeof(double) * std::max<size_t>(1, (size_t)p->capacity * t.n_expr)));
-        if (!p->d_scales) CU(cudaMalloc(&p->d_scales, sizeof(double) * p->capacity));
-    }
     static const bool no_fuse = std::getenv("FK_NO_FUSED_PREPARE") != nullptr;  // A/B knob
-    static const uint32_t use_streams = [] {
-        const char* e = std::getenv("FK_E2E_STREAMS");  // tuning knob: chunks in flight (at most kStreams)
-        const int v = e ? std::atoi(e) : 0;
-        return (uint32_t)(v >= 1 && v <= (int)DevicePipeline::kStreams ? v : (int)DevicePipeline::kStreams);
-    }();
-    // FK_E2E_TRACE=1 (debug): CUDA-event timeline of the chunks of one call to stderr (upload done / kernel done / download done)
-    static const bool trace = std::getenv("FK_E2E_TRACE") != nullptr;
-    std::vector<cudaEvent_t> tev;
-    cudaEvent_t t_start = nullptr;
-    if (trace) {
-        cudaEventCreate(&t_start);
-        cudaEventRecord(t_start, pl->streams[0]);
-    }
-    // One parameter row for all sketches: uploaded once per call, every stream waits for it (a 300-byte copy per chunk kept the
-    // H2D engine ~10 us per chunk, which the first chunks of a call -- the ones the device is waiting for -- paid in full).
-    const uint64_t my_token = pl->next_token++;
-    const int slot = (int)(my_token & 1u);
     const double* d_shared_param = nullptr;
-    if (shared && t.n_expr) {
-        if (!pl->shared_param_ev) CU(cudaEventCreateWithFlags(&pl->shared_param_ev, cudaEventDisableTiming));
-        if (pl->shared_param_cap < t.n_expr) {  // (two rows: the kernels of the previous call may still read theirs)
-            for (int a = 0; a < 2; a++) {
-                if (pl->d_shared_param[a]) CU(cudaFree(pl->d_shared_param[a]));
-                pl->d_shared_param[a] = nullptr;
-                CU(cudaMalloc(&pl->d_shared_param[a], sizeof(double) * t.n_expr));
-            }
-            pl->shared_param_cap = t.n_expr;
+    auto prologue = [&](DevicePipeline& pl, int slot, uint32_t use_streams) -> int {
+        for (fk_batch_plan* p : pl.plans) {  // unscaled input / scale buffers of the plans, on first use
+            if (!p->d_raw_vars) CU(cudaMalloc(&p->d_raw_vars, sizeof(double) * std::max<size_t>(1, (size_t)p->capacity * t.n_vars)));
+            if (!p->d_raw_param) CU(cudaMalloc(&p->d_raw_param, sizeof(double) * std::max<size_t>(1, (size_t)p->capacity * t.n_expr)));
+            if (!p->d_scales) CU(cudaMalloc(&p->d_scales, sizeof(double) * p->capacity));
         }
-        d_shared_param = pl->d_shared_param[slot];
-        CU(cudaMemcpyAsync(pl->d_shared_param[slot], raw_param, sizeof(double) * t.n_expr, cudaMemcpyHostToDevice, pl->streams[0]));
-        CU(cudaEventRecord(pl->shared_param_ev, pl->streams[0]));
-        for (uint32_t k = 1; k < use_streams; k++) CU(cudaStreamWaitEvent(pl->streams[k], pl->shared_param_ev, 0));
-    }
+        if (!shared || !t.n_expr) return FK_OK;
+        // One parameter row for all sketches: uploaded once per call, every stream waits for it (a 300-byte copy per chunk kept the
+        // H2D engine ~10 us per chunk, which the first chunks of a call -- the ones the device is waiting for -- paid in full).
+        if (!pl.shared_param_ev) CU(cudaEventCreateWithFlags(&pl.shared_param_ev, cudaEventDisableTiming));
+        if (pl.shared_param_cap < t.n_expr) {  // (two rows: the kernels of the previous call may still read theirs)
+            for (int a = 0; a < 2; a++) {
+                if (pl.d_shared_param[a]) CU(cudaFree(pl.d_shared_param[a]));
+                pl.d_shared_param[a] = nullptr;
+                CU(cudaMalloc(&pl.d_shared_param[a], sizeof(double) * t.n_expr));
+            }
+            pl.shared_param_cap = t.n_expr;
+        }
+        d_shared_param = pl.d_shared_param[slot];
+        CU(cudaMemcpyAsync(pl.d_shared_param[slot], raw_param, sizeof(double) * t.n_expr, cudaMemcpyHostToDevice, pl.streams[0]));
+        CU(cudaEventRecord(pl.shared_param_ev, pl.streams[0]));
+        for (uint32_t k = 1; k < use_streams; k++) CU(cudaStreamWaitEvent(pl.streams[k], pl.shared_param_ev, 0));
+        return FK_OK;
+    };
     // (Chunks that taper at both ends of a call -- a quarter and a half of the regular size first, halving down to 1,024 sketches at the
     // end -- bring the first kernel forward from 65 to 24 us and change nothing: 1,108 against 1,092 us per call.  The last kernel ends
     // ~1,070 us after the call started either way; the chunked kernels together take ~1,040 us where one launch over the resident
     // batch takes 905.)
-    uint32_t s = 0;
-    for (uint32_t at = 0; at < n && rc == FK_OK; at += chunk, s = (s + 1) % use_streams) {
-        const uint32_t cnt = std::min(chunk, n - at);
-        fk_batch_plan* p = pl->plans[s];
-        cudaStream_t st = pl->streams[s];
+    auto enqueue = [&](fk_batch_plan* p, cudaStream_t st, uint32_t at, uint32_t cnt, const std::function<void()>& mark) -> int {
         const bool fused = !no_fuse && fk::batch_lm_uses_sketch_kernel(*p->prog, cnt) && fk::sk_raw_fits(*p->prog->sketch_prog, shared);
-        CU(cudaStreamSynchronize(st));  // the plan's buffers are reused only after its previous chunk has drained
         p->n = cnt;
         if (t.n_vars) CU(cudaMemcpyAsync(p->d_raw_vars, raw_vars + (size_t)at * t.n_vars, sizeof(double) * (size_t)cnt * t.n_vars, cudaMemcpyHostToDevice, st));
         if (t.n_expr && !shared)
             CU(cudaMemcpyAsync(p->d_raw_param, raw_param + (size_t)at * t.n_expr, sizeof(double) * (size_t)cnt * t.n_expr, cudaMemcpyHostToDevice, st));
         const double* d_param = shared ? d_shared_param : p->d_raw_param;
-        if (trace) { cudaEvent_t ev; cudaEventCreate(&ev); cudaEventRecord(ev, st); tev.push_back(ev); }
+        mark();
         int e;
         if (fused) {  // the sketch-per-thread kernel scales, perturbs and writes back itself (SkRaw)
             fk::SkRaw raw{};
@@ -1126,47 +1107,24 @@ static int system_solve_enqueue(const fk_topology* topo_c, int device, uint32_t 
             p->launches += 3;
         }
         if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_batch_system_solve kernels");
-        if (trace) { cudaEvent_t ev; cudaEventCreate(&ev); cudaEventRecord(ev, st); tev.push_back(ev); }
+        mark();
         if (t.n_free) CU(cudaMemcpyAsync(free_out + (size_t)at * t.n_free, p->d_out, sizeof(double) * (size_t)cnt * t.n_free, cudaMemcpyDeviceToHost, st));
         if (scales_out) CU(cudaMemcpyAsync(scales_out + at, p->d_scales, sizeof(double) * cnt, cudaMemcpyDeviceToHost, st));
         if (reports) CU(cudaMemcpyAsync(reports + at, p->d_rep, sizeof(fk_report) * (size_t)cnt, cudaMemcpyDeviceToHost, st));
-        if (trace) { cudaEvent_t ev; cudaEventCreate(&ev); cudaEventRecord(ev, st); tev.push_back(ev); }
-    }
-    if (token && !trace) {
-        for (uint32_t k = 0; k < kStreams; k++) {
-            if (!pl->streams[k]) continue;
-            if (!pl->done_ev[slot][k]) CU(cudaEventCreateWithFlags(&pl->done_ev[slot][k], cudaEventDisableTiming));
-            CU(cudaEventRecord(pl->done_ev[slot][k], pl->streams[k]));
-        }
-        *token = my_token;
-        return rc;
-    }
-    for (uint32_t k = 0; k < kStreams; k++)
-        if (pl->streams[k]) CU(cudaStreamSynchronize(pl->streams[k]));
-    if (token) *token = my_token;  // (tracing: the call has completed; waiting for it is a no-op)
-    if (trace) {
-        for (size_t c = 0; c + 2 < tev.size() + 0 && c < tev.size(); c += 3) {
-            float a = 0, b = 0, d = 0;
-            cudaEventElapsedTime(&a, t_start, tev[c]);
-            cudaEventElapsedTime(&b, t_start, tev[c + 1]);
-            cudaEventElapsedTime(&d, t_start, tev[c + 2]);
-            fprintf(stderr, "[e2e trace] chunk %2zu: upload done %7.1f us, kernel done %7.1f us, download done %7.1f us\n", c / 3, a * 1e3f, b * 1e3f, d * 1e3f);
-        }
-        for (cudaEvent_t ev : tev) cudaEventDestroy(ev);
-        cudaEventDestroy(t_start);
-    }
-    return rc;
+        return FK_OK;
+    };
+    return run_pipeline(topo, device, 0, n, pipeline_chunk(topo, device, n, 16, true), token, prologue, enqueue);
 }
 
 int fk_batch_system_solve(const fk_topology* topo, int device, uint32_t n, const double* raw_vars, const double* raw_param,
                           const fk_prepare_opts* opts, double* free_out, double* scales_out, fk_report* reports) {
-    return system_solve_enqueue(topo, device, n, raw_vars, raw_param, opts, free_out, scales_out, reports, nullptr);
+    return batch_system_solve(topo, device, n, raw_vars, raw_param, opts, free_out, scales_out, reports, nullptr);
 }
 
 int fk_batch_system_solve_begin(const fk_topology* topo, int device, uint32_t n, const double* raw_vars, const double* raw_param,
                                 const fk_prepare_opts* opts, double* free_out, double* scales_out, fk_report* reports, uint64_t* token) {
     if (!token) return fail(FK_ERR_INVALID, "null token");
-    return system_solve_enqueue(topo, device, n, raw_vars, raw_param, opts, free_out, scales_out, reports, token);
+    return batch_system_solve(topo, device, n, raw_vars, raw_param, opts, free_out, scales_out, reports, token);
 }
 
 int fk_batch_system_solve_wait(const fk_topology* topo_c, int device, uint64_t token) {
@@ -1189,29 +1147,28 @@ int fk_batch_system_solve_wait(const fk_topology* topo_c, int device, uint64_t t
     return FK_OK;
 }
 
-int fk_batch_solve_device(const fk_topology* topo_c, int device, uint32_t n, const double* vars, const double* param,
-                          double* free_out, fk_report* reports) {
+// fk_batch_solve_device, and its _begin half with a token.
+static int batch_solve_device(const fk_topology* topo_c, int device, uint32_t n, const double* vars, const double* param,
+                              double* free_out, fk_report* reports, uint64_t* token) {
     fk_topology* topo = const_cast<fk_topology*>(topo_c);
     if (!topo) return fail(FK_ERR_INVALID, "null topology");
+    if (token) *token = 0;
     if (n == 0) return FK_OK;
     if (!vars || !free_out || (!param && topo->t.n_expr)) return fail(FK_ERR_INVALID, "null buffer");
-    int ndev = usable_devices();
-    if (ndev == 0) return fail(FK_ERR_NO_DEVICE, "no CUDA device visible; fiksi_b200 has no CPU fallback");
-    if (device < 0 || device >= ndev) return fail(FK_ERR_INVALID, "device index out of range");
-    return run_device_range(topo, device, 0, n, vars, param, free_out, reports, nullptr);
+    const int rc = check_device(device);
+    if (rc != FK_OK) return rc;
+    return run_device_range(topo, device, 0, n, vars, param, free_out, reports, 0, token);
 }
 
-int fk_batch_solve_device_begin(const fk_topology* topo_c, int device, uint32_t n, const double* vars, const double* param,
+int fk_batch_solve_device(const fk_topology* topo, int device, uint32_t n, const double* vars, const double* param,
+                          double* free_out, fk_report* reports) {
+    return batch_solve_device(topo, device, n, vars, param, free_out, reports, nullptr);
+}
+
+int fk_batch_solve_device_begin(const fk_topology* topo, int device, uint32_t n, const double* vars, const double* param,
                                 double* free_out, fk_report* reports, uint64_t* token) {
-    fk_topology* topo = const_cast<fk_topology*>(topo_c);
-    if (!topo || !token) return fail(FK_ERR_INVALID, "null topology / token");
-    *token = 0;
-    if (n == 0) return FK_OK;
-    if (!vars || !free_out || (!param && topo->t.n_expr)) return fail(FK_ERR_INVALID, "null buffer");
-    int ndev = usable_devices();
-    if (ndev == 0) return fail(FK_ERR_NO_DEVICE, "no CUDA device visible; fiksi_b200 has no CPU fallback");
-    if (device < 0 || device >= ndev) return fail(FK_ERR_INVALID, "device index out of range");
-    return run_device_range(topo, device, 0, n, vars, param, free_out, reports, nullptr, 0, token);
+    if (!token) return fail(FK_ERR_INVALID, "null token");
+    return batch_solve_device(topo, device, n, vars, param, free_out, reports, token);
 }
 
 int fk_batch_solve_device_wait(const fk_topology* topo, int device, uint64_t token) { return fk_batch_system_solve_wait(topo, device, token); }
@@ -1222,40 +1179,26 @@ int fk_batch_solve(const fk_topology* topo_c, uint32_t n, const double* vars, co
     if (!topo) return fail(FK_ERR_INVALID, "null topology");
     if (n == 0) return FK_OK;
     if (!vars || !free_out || (!param && topo->t.n_expr)) return fail(FK_ERR_INVALID, "null buffer");
-    int ndev = usable_devices();
-    if (ndev == 0) return fail(FK_ERR_NO_DEVICE, "no CUDA device visible; fiksi_b200 has no CPU fallback");
-    if (n_gpus <= 0 || n_gpus > ndev) n_gpus = ndev;
-    if (n_gpus == 1) {
-        int cur = 0;  // one process per GPU: honour the caller's current device
-        if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
-        return run_device_range(topo, cur, 0, n, vars, param, free_out, reports, nullptr);
-    }
-    std::vector<int> rcs(n_gpus, FK_OK);
-    std::vector<std::string> errs(n_gpus);
-    std::vector<std::thread> pool;
-    for (int g = 0; g < n_gpus; g++) {
-        uint32_t lo = (uint32_t)((uint64_t)n * g / n_gpus), hi = (uint32_t)((uint64_t)n * (g + 1) / n_gpus);
-        pool.emplace_back([=, &rcs, &errs]() { rcs[g] = run_device_range(topo, g, lo, hi, vars, param, free_out, reports, &errs[g]); });
-    }
-    for (auto& th : pool) th.join();
-    for (int g = 0; g < n_gpus; g++)
-        if (rcs[g] != FK_OK) return fail(rcs[g], errs[g]);
-    return FK_OK;
+    const int rc = clamp_gpus(n_gpus);
+    if (rc != FK_OK) return rc;
+    return shard_over_devices(n_gpus, n, [&](int device, uint32_t lo, uint32_t hi) {
+        return run_device_range(topo, device, lo, hi, vars, param, free_out, reports);
+    });
 }
 
 // ---- single system with a cached topology (any path) --------------------------------------------------
 int fk_topology_lm_solve(fk_topology* topo, const double* vars, const double* param, double* free_values,
                          fk_report* report) {
     if (!topo || !free_values || (!vars && topo->t.n_vars)) return fail(FK_ERR_INVALID, "null argument");
-    int ndev = usable_devices();
-    if (ndev == 0) return fail(FK_ERR_NO_DEVICE, "no CUDA device visible; fiksi_b200 has no CPU fallback");
     int cur = 0;
     if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
+    int rc = check_device(cur);
+    if (rc != FK_OK) return rc;
     const fk::Topology& t = topo->t;
     if (t.path == 2) {
         fk::SparseSolver* sp = nullptr;
         std::string err;
-        int rc = topo->sparse_for(cur, &sp, &err);
+        rc = topo->sparse_for(cur, &sp, &err);
         if (rc != FK_OK) return fail(rc, err);
         // the caller's free values are the starting point (== `variables` of lm.rs:21)
         if (!param && t.n_expr) return fail(FK_ERR_INVALID, "null parameter array");
@@ -1272,7 +1215,7 @@ int fk_topology_lm_solve(fk_topology* topo, const double* vars, const double* pa
     // first single-system solve, serves these calls (same operations per entry, same results; tools/lat_probe.py:
     // 144 -> 89 us on the mixed-primitive sketch).
     fk_topology* exec = topo->lanes32();
-    int rc = run_device_range(exec, cur, 0, 1, v.data(), param ? param : zero.data(), out.data(), report, nullptr);
+    rc = run_device_range(exec, cur, 0, 1, v.data(), param ? param : zero.data(), out.data(), report);
     if (rc == FK_OK && t.n_free) std::memcpy(free_values, out.data(), sizeof(double) * t.n_free);
     return rc;
 }
@@ -1280,13 +1223,14 @@ int fk_topology_lm_solve(fk_topology* topo, const double* vars, const double* pa
 int fk_topology_eval(fk_topology* topo, const double* vars, const double* param, const double* free_values,
                      double* out_r, double* out_j, int repeats, float* ms_per_eval) {
     if (!topo || !vars || !free_values) return fail(FK_ERR_INVALID, "null argument");
-    if (usable_devices() == 0) return fail(FK_ERR_NO_DEVICE, "no CUDA device visible; fiksi_b200 has no CPU fallback");
-    if (topo->t.path != 2) return fail(FK_ERR_INVALID, "fk_topology_eval serves the global sparse path; use fk_batch_plan_eval");
     int cur = 0;
     if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
+    int rc = check_device(cur);
+    if (rc != FK_OK) return rc;
+    if (topo->t.path != 2) return fail(FK_ERR_INVALID, "fk_topology_eval serves the global sparse path; use fk_batch_plan_eval");
     fk::SparseSolver* sp = nullptr;
     std::string err;
-    int rc = topo->sparse_for(cur, &sp, &err);
+    rc = topo->sparse_for(cur, &sp, &err);
     if (rc == FK_OK) {
         std::lock_guard<std::mutex> lock(topo->sparse_mu);
         rc = sp->eval_once(vars, param, free_values, out_r, out_j, repeats, ms_per_eval, &err);
@@ -1350,11 +1294,17 @@ uint64_t structural_signature(const fk_problem& p) {
     if (p.n_rows) mixb(p.rows, 4 * (size_t)p.n_rows);
     return sig;
 }
-bool same_structure(const fk::Topology& t, const fk_problem& p) {
-    return t.n_vars == p.n_vars && t.n_expr == p.n_expr && t.n_free == p.n_free && t.n_rows == p.n_rows &&
-           (!p.n_expr || (!std::memcmp(t.kind.data(), p.kind, p.n_expr) && !std::memcmp(t.idx.data(), p.idx, 16 * (size_t)p.n_expr))) &&
-           (!p.n_free || !std::memcmp(t.free_vars.data(), p.free_vars, 4 * (size_t)p.n_free)) &&
-           (!p.n_rows || !std::memcmp(t.rows.data(), p.rows, 4 * (size_t)p.n_rows));
+bool same_structure(const fk_problem& a, const fk_problem& p) {
+    return a.n_vars == p.n_vars && a.n_expr == p.n_expr && a.n_free == p.n_free && a.n_rows == p.n_rows &&
+           (!p.n_expr || (!std::memcmp(a.kind, p.kind, p.n_expr) && !std::memcmp(a.idx, p.idx, 16 * (size_t)p.n_expr))) &&
+           (!p.n_free || !std::memcmp(a.free_vars, p.free_vars, 4 * (size_t)p.n_free)) &&
+           (!p.n_rows || !std::memcmp(a.rows, p.rows, 4 * (size_t)p.n_rows));
+}
+fk_problem structure_of(const fk::Topology& t) {  // (no values: vars / param stay null)
+    fk_problem p{};
+    p.n_vars = t.n_vars; p.n_expr = t.n_expr; p.kind = t.kind.data(); p.idx = t.idx.data();
+    p.n_free = t.n_free; p.free_vars = t.free_vars.data(); p.n_rows = t.n_rows; p.rows = t.rows.data();
+    return p;
 }
 bool problem_arrays_ok(const fk_problem& p) {
     return !((p.n_vars && !p.vars) || (p.n_expr && (!p.kind || !p.idx)) || (p.n_free && !p.free_vars) || (p.n_rows && !p.rows));
@@ -1365,7 +1315,7 @@ std::shared_ptr<fk_topology> cache_lookup(uint64_t sig, const fk_problem& p) {
     std::lock_guard<std::mutex> lock(c.mu);
     auto range = c.index.equal_range(sig);
     for (auto q = range.first; q != range.second; ++q)
-        if (same_structure(q->second->topo->t, p)) {
+        if (same_structure(structure_of(q->second->topo->t), p)) {
             c.lru.splice(c.lru.begin(), c.lru, q->second);  // (list iterators stay valid)
             c.hits++;
             return c.lru.front().topo;
@@ -1511,9 +1461,7 @@ int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems, double* con
                       int n_gpus) {
     if (n == 0) return FK_OK;
     if (!problems || !free_values) return fail(FK_ERR_INVALID, "null argument");
-    const int ndev = usable_devices();
-    if (ndev == 0) return fail(FK_ERR_NO_DEVICE, "no CUDA device visible; fiksi_b200 has no CPU fallback");
-    if (n_gpus <= 0 || n_gpus > ndev) n_gpus = ndev;
+    if (const int rc = clamp_gpus(n_gpus); rc != FK_OK) return rc;
     // ---- group the problems by topology -----------------------------------------------------------------
     struct Group {
         uint64_t sig = 0;
@@ -1536,17 +1484,8 @@ int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems, double* con
         const uint64_t sig = structural_signature(*p);
         size_t gi = SIZE_MAX;
         auto range = by_sig.equal_range(sig);
-        for (auto it = range.first; it != range.second; ++it) {
-            const fk_problem& q = *problems[groups[it->second].members[0]];
-            const fk_problem& pp = *p;
-            if (q.n_vars == pp.n_vars && q.n_expr == pp.n_expr && q.n_free == pp.n_free && q.n_rows == pp.n_rows &&
-                (!pp.n_expr || (!std::memcmp(q.kind, pp.kind, pp.n_expr) && !std::memcmp(q.idx, pp.idx, 16 * (size_t)pp.n_expr))) &&
-                (!pp.n_free || !std::memcmp(q.free_vars, pp.free_vars, 4 * (size_t)pp.n_free)) &&
-                (!pp.n_rows || !std::memcmp(q.rows, pp.rows, 4 * (size_t)pp.n_rows))) {
-                gi = it->second;
-                break;
-            }
-        }
+        for (auto it = range.first; it != range.second && gi == SIZE_MAX; ++it)
+            if (same_structure(*problems[groups[it->second].members[0]], *p)) gi = it->second;
         if (gi == SIZE_MAX) {
             groups.emplace_back();
             groups.back().sig = sig;
@@ -1594,7 +1533,7 @@ int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems, double* con
     size_t rr = 0;
     int first_rc = FK_OK;
     std::string first_err;
-    auto note = [&](int rc, const std::string& e) { if (rc != FK_OK && first_rc == FK_OK) { first_rc = rc; first_err = e; } };
+    auto note = [&](int rc) { if (rc != FK_OK && first_rc == FK_OK) { first_rc = rc; first_err = g_error; } };
     // Several small groups: ONE launch of the heterogeneous kernel for all of them (one warp per system) instead of one
     // launch, two copies and a synchronisation per topology.  Groups of 64 systems and more keep the uniform batch kernels
     // (from there the sketch-per-thread kernel is the faster one).  (FK_NO_HETERO=1: A/B knob.)
@@ -1619,21 +1558,12 @@ int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems, double* con
             }
             if (!items.empty() && n_gpus > 1 && items.size() >= 64u * (size_t)n_gpus) {
                 // several devices: contiguous shares of the systems, one host thread and one launch per device
-                std::vector<int> rcs(n_gpus, FK_OK);
-                std::vector<std::string> errs(n_gpus);
-                std::vector<std::thread> pool;
-                for (int g = 0; g < n_gpus; g++)
-                    pool.emplace_back([&, g] {
-                        const size_t lo = items.size() * g / n_gpus, hi = items.size() * (g + 1) / n_gpus;
-                        std::vector<HeteroItem> part(items.begin() + lo, items.begin() + hi);
-                        rcs[g] = hetero_solve(g, topos32, part, problems, free_values, reports);
-                        if (rcs[g] != FK_OK) errs[g] = g_error;
-                    });
-                for (auto& th : pool) th.join();
-                for (int g = 0; g < n_gpus; g++) note(rcs[g], errs[g]);
+                note(shard_over_devices(n_gpus, (uint32_t)items.size(), [&](int device, uint32_t lo, uint32_t hi) {
+                    const std::vector<HeteroItem> part(items.begin() + lo, items.begin() + hi);
+                    return hetero_solve(device, topos32, part, problems, free_values, reports);
+                }));
             } else if (!items.empty()) {
-                const int rc = hetero_solve(cur, topos32, items, problems, free_values, reports);
-                if (rc != FK_OK) note(rc, g_error);
+                note(hetero_solve(cur, topos32, items, problems, free_values, reports));
             }
         }
     }
@@ -1661,20 +1591,14 @@ int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems, double* con
         const size_t cnt = gr.members.size();
         if (t.path == 2) {  // large systems: one after the other through the global sparse path
             for (uint32_t i : gr.members) {
-                int rc = fk_topology_lm_solve(gr.topo.get(), problems[i]->vars, problems[i]->param, free_values[i], reports ? &reports[i] : nullptr);
-                if (rc != FK_OK) note(rc, g_error);
+                note(fk_topology_lm_solve(gr.topo.get(), problems[i]->vars, problems[i]->param, free_values[i], reports ? &reports[i] : nullptr));
             }
             continue;
         }
-        int rc = FK_OK;
-        std::string e;
-        if (groups_to_devices || n_gpus == 1 || small_fits(t, (uint32_t)cnt)) {
-            rc = run_device_range(gr.topo.get(), gr.device, 0, (uint32_t)cnt, gr.vars.data(), gr.param.data(), gr.out.data(), gr.reps.data(), &e, 0);
-        } else {
-            rc = fk_batch_solve(gr.topo.get(), (uint32_t)cnt, gr.vars.data(), gr.param.data(), gr.out.data(), gr.reps.data(), n_gpus);
-            if (rc != FK_OK) e = g_error;
-        }
-        if (rc != FK_OK) { note(rc, e); continue; }
+        const int rc = groups_to_devices || n_gpus == 1 || small_fits(t, (uint32_t)cnt)
+            ? run_device_range(gr.topo.get(), gr.device, 0, (uint32_t)cnt, gr.vars.data(), gr.param.data(), gr.out.data(), gr.reps.data())
+            : fk_batch_solve(gr.topo.get(), (uint32_t)cnt, gr.vars.data(), gr.param.data(), gr.out.data(), gr.reps.data(), n_gpus);
+        if (rc != FK_OK) { note(rc); continue; }
         for (size_t k = 0; k < cnt; k++) {
             std::memcpy(free_values[gr.members[k]], &gr.out[k * t.n_free], sizeof(double) * t.n_free);
             if (reports) reports[gr.members[k]] = gr.reps[k];

@@ -211,8 +211,12 @@ class Topology:
         return {"available": bool(ok.value), "state_doubles": ent.value, "table_words": words.value}
 
     def batch_kernel(self, n_sketches):
-        """fk_topology_batch_kernel: 'sketch' or 'tile', the kernel a batched LM solve of this size launches."""
-        return {0: "tile", 1: "sketch", 2: "sketch_pair"}[lib().fk_topology_batch_kernel(self._h, int(n_sketches))]
+        """fk_topology_batch_kernel: the kernel a batched LM solve of this size launches: 'tile', 'sketch', 'sketch_pair', or
+        'sparse_batch' (global sparse path: one CTA per sketch over the supernodal tree)."""
+        k = lib().fk_topology_batch_kernel(self._h, int(n_sketches))
+        if k < 0:
+            check(k)
+        return {0: "tile", 1: "sketch", 2: "sketch_pair", 3: "sparse_batch"}[k]
 
     def plan(self, capacity, device=0):
         return BatchPlan(self, capacity, device)

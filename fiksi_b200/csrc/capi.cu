@@ -21,6 +21,7 @@
 #include "lm_sketch.cuh"
 #include "multifrontal.cuh"
 #include "single_pass.hpp"
+#include "sparse_batch.cuh"
 #include "sparse_path.cuh"
 #include "symbolic.hpp"
 
@@ -96,6 +97,7 @@ struct DeviceProgram {
     fk::DevProgram view{};
     const uint32_t *jcolptr = nullptr, *jrow = nullptr;  // CSC of the Jacobian (L-BFGS)
     std::unique_ptr<fk::SkProgram> sketch;               // parameter block of the sketch-per-thread LM kernel
+    std::unique_ptr<fk::SparseBatchProgram> sparse_batch;  // path 2: tables of the one-CTA-per-sketch supernodal LM kernel
     ~DeviceProgram() {
         if (buf) {
             cudaSetDevice(device);
@@ -169,6 +171,32 @@ int upload_program(const fk::Topology& t, int device, DeviceProgram& out) {
         p.tab = (const uint32_t*)(b + o_sk);
         v.sketch_prog = out.sketch.get();
     }
+    if (t.path == 2) {
+        std::string err;
+        out.sparse_batch.reset(new fk::SparseBatchProgram());
+        const int rc = out.sparse_batch->init(t, v, device, &err);
+        if (rc != FK_OK) return fail(rc, err);
+    }
+    return FK_OK;
+}
+
+// The batched LM kernel of a topology, chosen in this one place: on the global sparse path the one-CTA-per-sketch kernel
+// over the supernodal tree (workspace `ws` with room for `ws_ctas` CTAs, see alloc_lm_workspace), launch_batch_lm's
+// tile / sketch-per-thread kernels otherwise.
+int launch_lm(const DeviceProgram& full, uint32_t n, const double* vars, const double* params, double* out, fk_report* reps,
+              double* ws, uint32_t ws_ctas, cudaStream_t st) {
+    if (full.sparse_batch) return full.sparse_batch->launch(n, vars, params, out, reps, ws, ws_ctas, st);
+    return fk::launch_batch_lm(full.view, n, vars, params, out, reps, st);
+}
+
+// Workspace of launch_lm for launches of up to `capacity` sketches (nothing off the global sparse path): per-CTA workspaces
+// for min(capacity, resident CTAs) CTAs, within fk::kSbWorkspaceBytes.  Two launches that may run at the same time need two
+// workspaces.
+int alloc_lm_workspace(const DeviceProgram& full, uint32_t capacity, double** ws, uint32_t* ws_ctas) {
+    if (!full.sparse_batch) return FK_OK;
+    const uint32_t ctas = full.sparse_batch->workspace_ctas(capacity);
+    CU(cudaMalloc(ws, sizeof(double) * full.sparse_batch->workspace_doubles(ctas)));
+    *ws_ctas = ctas;
     return FK_OK;
 }
 
@@ -195,6 +223,8 @@ struct DevicePipeline {
     unsigned char* small_h = nullptr;
     unsigned char* small_d = nullptr;
     cudaStream_t small_stream = nullptr;
+    double* small_ws = nullptr;  // launch_lm workspace of the small requests (global sparse path)
+    uint32_t small_ws_ctas = 0;
     cudaEvent_t shared_param_ev = nullptr;  // fk_batch_system_solve with one parameter row for all sketches: its upload, once per call
     // Every call on the chunk pipeline takes a token.  Its parity picks the call's copy of the shared parameter row and the events
     // recorded behind its last chunk on every stream (the _begin / _wait halves: up to two calls in flight).
@@ -254,6 +284,8 @@ struct fk_topology {
     std::mutex sp_mu;                   // SinglePass plan: one sub-topology per strongly connected set
     bool sp_planned = false;
     std::vector<fk_topology*> sp_subs;
+    int sb_fit = 1;                     // path 2: FK_OK when the sparse batch kernel takes the topology (1: not yet analysed)
+    std::string sb_err;
     ~fk_topology();
 
     int sparse_for(int device, fk::SparseSolver** out, std::string* err) {
@@ -322,12 +354,14 @@ struct fk_batch_plan {
     const DeviceProgram* full = nullptr;
     double *d_vars = nullptr, *d_params = nullptr, *d_out = nullptr, *d_er = nullptr, *d_ej = nullptr;
     fk_report* d_rep = nullptr;
+    double* d_ws = nullptr;  // launch_lm workspace (global sparse path)
+    uint32_t ws_ctas = 0;
     double *d_raw_vars = nullptr, *d_raw_param = nullptr, *d_scales = nullptr;  // fk_batch_system_solve: unscaled input, scale per sketch
     uint64_t launches = 0;
     ~fk_batch_plan() {
         cudaSetDevice(device);
         cudaFree(d_vars); cudaFree(d_params); cudaFree(d_out); cudaFree(d_er); cudaFree(d_ej); cudaFree(d_rep);
-        cudaFree(d_raw_vars); cudaFree(d_raw_param); cudaFree(d_scales);
+        cudaFree(d_raw_vars); cudaFree(d_raw_param); cudaFree(d_scales); cudaFree(d_ws);
     }
 };
 
@@ -347,8 +381,11 @@ void DevicePipeline::release() {
     if (small_h) cudaFreeHost(small_h);
     if (small_d) cudaFree(small_d);
     if (small_stream) cudaStreamDestroy(small_stream);
+    if (small_ws) cudaFree(small_ws);
     small_h = small_d = nullptr;
     small_stream = nullptr;
+    small_ws = nullptr;
+    small_ws_ctas = 0;
     if (shared_param_ev) cudaEventDestroy(shared_param_ev);
     shared_param_ev = nullptr;
     for (int a = 0; a < 2; a++) {
@@ -632,8 +669,6 @@ int fk_batch_plan_create(const fk_topology* topo_c, uint32_t capacity, int devic
     if (!topo || !out || capacity == 0) return fail(FK_ERR_INVALID, "null topology / zero capacity");
     int rc = check_device(device);
     if (rc != FK_OK) return rc;
-    if (topo->t.path == 2)
-        return fail(FK_ERR_TOO_LARGE, "topology needs the global sparse path; use fk_lm_solve");
     CU(cudaSetDevice(device));
     cudaDeviceProp prop;
     CU(cudaGetDeviceProperties(&prop, device));
@@ -647,6 +682,7 @@ int fk_batch_plan_create(const fk_topology* topo_c, uint32_t capacity, int devic
     CU(cudaMalloc(&p->d_params, sizeof(double) * std::max<size_t>(1, (size_t)capacity * t.n_expr)));
     CU(cudaMalloc(&p->d_out, sizeof(double) * std::max<size_t>(1, (size_t)capacity * t.n_free)));
     CU(cudaMalloc(&p->d_rep, sizeof(fk_report) * (size_t)capacity));
+    if ((rc = alloc_lm_workspace(*p->full, capacity, &p->d_ws, &p->ws_ctas)) != FK_OK) return rc;
     *out = p.release();
     return FK_OK;
 }
@@ -667,9 +703,9 @@ int fk_batch_plan_upload(fk_batch_plan* plan, uint32_t n, const double* vars, co
 int fk_batch_plan_run(fk_batch_plan* plan, void* stream) {
     if (!plan) return fail(FK_ERR_INVALID, "null plan");
     CU(cudaSetDevice(plan->device));
-    int e = fk::launch_batch_lm(*plan->prog, plan->n, plan->d_vars, plan->d_params, plan->d_out,
-                                plan->d_rep, stream);
-    if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_batch_lm_kernel");
+    const int e = launch_lm(*plan->full, plan->n, plan->d_vars, plan->d_params, plan->d_out, plan->d_rep, plan->d_ws, plan->ws_ctas,
+                            (cudaStream_t)stream);
+    if (e != 0) return cuda_fail((cudaError_t)e, "launch batched LM kernel");
     if (plan->n) plan->launches++;
     return FK_OK;
 }
@@ -718,6 +754,7 @@ int fk_batch_plan_sync(fk_batch_plan* plan) {
 int fk_batch_plan_eval(fk_batch_plan* plan, int mode, void* stream) {
     if (!plan) return fail(FK_ERR_INVALID, "null plan");
     const fk::Topology& t = plan->topo->t;
+    if (t.path == 2) return fail(FK_ERR_TOO_LARGE, "the evaluation kernels of a batch plan serve the shared-memory paths only; use fk_topology_eval");
     CU(cudaSetDevice(plan->device));
     if (!plan->d_er) CU(cudaMalloc(&plan->d_er, sizeof(double) * std::max<size_t>(1, (size_t)plan->capacity * t.n_rows)));
     if (!plan->d_ej && mode == 0) CU(cudaMalloc(&plan->d_ej, sizeof(double) * std::max<size_t>(1, (size_t)plan->capacity * t.jac_nnz)));
@@ -760,8 +797,14 @@ int fk_topology_sketch_kernel_info(const fk_topology* topo, int* available, uint
     return FK_OK;
 }
 
-int fk_topology_batch_kernel(const fk_topology* topo, uint32_t n_sketches) {
-    if (!topo) return fail(FK_ERR_INVALID, "null topology");
+int fk_topology_batch_kernel(const fk_topology* topo_c, uint32_t n_sketches) {
+    if (!topo_c) return fail(FK_ERR_INVALID, "null topology");
+    fk_topology* topo = const_cast<fk_topology*>(topo_c);
+    if (topo->t.path == 2) {  // host analysis only (no device needed), once per topology
+        std::lock_guard<std::mutex> lock(topo->mu);
+        if (topo->sb_fit == 1) topo->sb_fit = fk::sparse_batch_fits(topo->t, nullptr, &topo->sb_err);
+        return topo->sb_fit == FK_OK ? 3 : fail(topo->sb_fit, topo->sb_err);
+    }
     const fk::Topology::SketchTables& k = topo->t.sk;
     fk::SkProgram probe{};
     probe.entries = k.entries;
@@ -902,10 +945,10 @@ static int run_pipeline(fk_topology* topo, int device, uint32_t lo, uint32_t hi,
     return rc;
 }
 
-static int launch_optimizer(const fk::DevProgram& prog, const DeviceProgram& full, int optimizer, uint32_t n, const double* vars,
-                            const double* params, double* out, fk_report* reps, cudaStream_t st) {
-    if (optimizer == 1) return fk::launch_batch_lbfgs(prog, full.jcolptr, full.jrow, n, vars, params, out, reps, st);
-    return fk::launch_batch_lm(prog, n, vars, params, out, reps, st);
+static int launch_optimizer(const DeviceProgram& full, int optimizer, uint32_t n, const double* vars, const double* params, double* out,
+                            fk_report* reps, double* ws, uint32_t ws_ctas, cudaStream_t st) {
+    if (optimizer == 1) return fk::launch_batch_lbfgs(full.view, full.jcolptr, full.jrow, n, vars, params, out, reps, st);
+    return launch_lm(full, n, vars, params, out, reps, ws, ws_ctas, st);
 }
 
 // Small request (one sketch, a handful): the caller's (pageable) arrays go through ONE pinned staging block -- one
@@ -947,21 +990,28 @@ static int small_solve(fk_topology* topo, int device, uint32_t lo, uint32_t hi, 
             return cuda_fail(e, "cudaStreamCreate");
         }
     }
+    if (full->sparse_batch && pl->small_ws_ctas < full->sparse_batch->workspace_ctas(total)) {  // grow-only
+        if (pl->small_ws) cudaFree(pl->small_ws);
+        pl->small_ws = nullptr;
+        pl->small_ws_ctas = 0;
+        if ((rc = alloc_lm_workspace(*full, total, &pl->small_ws, &pl->small_ws_ctas)) != FK_OK) return rc;
+    }
     std::memcpy(pl->small_h, vars + (size_t)lo * t.n_vars, in_v);
     if (in_p) std::memcpy(pl->small_h + in_v, param + (size_t)lo * t.n_expr, in_p);
     // A few kilobytes: the kernel reads its inputs from, and writes its results to, the pinned block itself (pinned host
     // memory is mapped into the device's address space under unified addressing; the kernel touches every input and output
-    // once) -- two DMA set-ups less on a path that is all latency.  FK_NO_ZERO_COPY=1 keeps the two copies (A/B knob).
+    // once) -- two DMA set-ups less on a path that is all latency.  FK_NO_ZERO_COPY=1 keeps the two copies (A/B knob).  Not
+    // for the sparse batch kernel: it reads the parameters and fixed variables again on every evaluation.
     static const bool no_zero_copy = std::getenv("FK_NO_ZERO_COPY") != nullptr;
     static const bool can_map = [] {
         int dev = 0, ok = 0;
         return cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&ok, cudaDevAttrCanUseHostPointerForRegisteredMem, dev) == cudaSuccess && ok != 0;
     }();
-    const bool zero_copy = !no_zero_copy && can_map && in_al + out_x + out_r <= 8 * 1024;
+    const bool zero_copy = !no_zero_copy && can_map && !full->sparse_batch && in_al + out_x + out_r <= 8 * 1024;
     unsigned char* base = zero_copy ? pl->small_h : pl->small_d;
     if (!zero_copy && (e = cudaMemcpyAsync(pl->small_d, pl->small_h, in_v + in_p, cudaMemcpyHostToDevice, pl->small_stream)) != cudaSuccess) return cuda_fail(e, "cudaMemcpyAsync");
-    const int le = launch_optimizer(*prog, *full, optimizer, total, (const double*)base, (const double*)(base + in_v),
-                                    (double*)(base + in_al), (fk_report*)(base + in_al + out_x), pl->small_stream);
+    const int le = launch_optimizer(*full, optimizer, total, (const double*)base, (const double*)(base + in_v), (double*)(base + in_al),
+                                    (fk_report*)(base + in_al + out_x), pl->small_ws, pl->small_ws_ctas, pl->small_stream);
     if (le == (int)cudaErrorInvalidConfiguration && optimizer == 1) return fail(FK_ERR_TOO_LARGE, "the L-BFGS state of one sketch does not fit the tile path");
     if (le != 0) return cuda_fail((cudaError_t)le, "launch batched solve kernel");
     if (!zero_copy && (e = cudaMemcpyAsync(pl->small_h + in_al, pl->small_d + in_al, out_x + out_r, cudaMemcpyDeviceToHost, pl->small_stream)) != cudaSuccess) return cuda_fail(e, "cudaMemcpyAsync");
@@ -1047,7 +1097,6 @@ static int batch_system_solve(const fk_topology* topo_c, int device, uint32_t n,
     if (n == 0) return FK_OK;
     const fk::Topology& t = topo->t;
     if (!raw_vars || !free_out || (!raw_param && t.n_expr)) return fail(FK_ERR_INVALID, "null buffer");
-    if (t.path == 2) return fail(FK_ERR_TOO_LARGE, "topology needs the global sparse path; use fk_system_solve");
     int rc = check_device(device);
     if (rc != FK_OK) return rc;
     PrepareTables* pt = nullptr;
@@ -1102,7 +1151,7 @@ static int batch_system_solve(const fk_topology* topo_c, int device, uint32_t n,
         } else {
             e = fk::launch_batch_prepare(cnt, t.n_vars, t.n_expr, pt->d_kind, shared, (uint32_t)pt->perturb_vars.size(), pt->d_perturb, pt->d_draws,
                                          p->d_raw_vars, d_param, p->d_vars, p->d_params, p->d_scales, st);
-            if (e == 0) e = fk::launch_batch_lm(*p->prog, cnt, p->d_vars, p->d_params, p->d_out, p->d_rep, st);
+            if (e == 0) e = launch_lm(*p->full, cnt, p->d_vars, p->d_params, p->d_out, p->d_rep, p->d_ws, p->ws_ctas, st);
             if (e == 0) e = fk::launch_batch_unscale(cnt, t.n_free, p->d_scales, p->d_out, st);
             p->launches += 3;
         }

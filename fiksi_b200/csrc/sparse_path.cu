@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "expressions.cuh"
+#include "lm_rules.cuh"
 #include "multifrontal.cuh"
 
 namespace fk {
@@ -403,7 +404,7 @@ int SparseSolver::solve(const double* vars, const double* param, double* free_va
     SP_CU(cudaMemcpyAsync(I.h_scalars, I.d_scalars, 4 * sizeof(double), cudaMemcpyDeviceToHost, st));
     SP_CU(cudaStreamSynchronize(st));
     double ssr = I.h_scalars[1];
-    if (std::isfinite(ssr) && std::fabs(ssr - 1e-8) <= 1e-8 * (8.0 * 1.1102230246251565e-16 * (double)m + 1e-13)) {
+    if (lm_initial_ssr_needs_exact(ssr, m)) {
         SP_CU(I.sumsq_exact(r, m, I.d_scalars + 1));  // the first lm.rs:110 test sits on its threshold: decide on the reference's sum
         SP_CU(cudaMemcpyAsync(I.h_scalars, I.d_scalars, 4 * sizeof(double), cudaMemcpyDeviceToHost, st));
         SP_CU(cudaStreamSynchronize(st));
@@ -456,15 +457,9 @@ int SparseSolver::solve(const double* vars, const double* param, double* free_va
         }
         double dn = I.h_scalars[0];
         double ssr_s = I.h_scalars[1];
-        {   // Decisions of lm.rs:139,151,164,110 taken on tree-reduced sums: when one of them is closer to its
-            // threshold than the tree and the reference's sequential sum can differ, redo the three sums in the
-            // reference's order and decide on those (and carry the exact ssr forward).
-            const double tol = 8.0 * 1.1102230246251565e-16 * (double)std::max(n, m) + 1e-13;
-            auto near = [&](double a, double b) { return std::fabs(a - b) <= tol * std::max(std::fabs(a), std::fabs(b)); };
-            const bool critical = fstat == 0 && std::isfinite(ssr_s) && std::isfinite(dn) &&
-                                  (near(dn, 1e-12) || near(ssr_s, ssr) || near(ssr_s, 1e-8) ||
-                                   (ssr_s < ssr && std::fabs((ssr - ssr_s) / ssr - 1e-6) <= 4.0 * tol));
-            if (critical) {
+        {   // Decisions of lm.rs:139,151,164,110 taken on tree-reduced sums (lm_rules.cuh): near a threshold, redo the
+            // three sums in the reference's order and decide on those (and carry the exact ssr forward).
+            if (lm_step_needs_exact(fstat, dn, ssr_s, ssr, n, m)) {
                 SP_CU(I.sumsq_exact(I.d_delta, n, I.d_scalars + 0));
                 SP_CU(I.sumsq_exact(rs, m, I.d_scalars + 1));
                 SP_CU(I.sumsq_exact(r, m, I.d_scalars + 3));

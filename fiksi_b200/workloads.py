@@ -145,8 +145,9 @@ def cad_mix(n_sketches, seed=0xF1C50004, first=0):
     return Workload("cad_mix", _CTL_KIND, _CTL_IDX, np.arange(11), np.arange(8), raw, param)
 
 
-def lattice(nx=400, ny=250, noise=0.02, seed=0xF1C50003):
-    """Config 3: nx*ny unit lattice, raster order; PPD to left, up, up-left neighbours."""
+def lattice(nx=400, ny=250, noise=0.02, seed=0xF1C50003, n_sketches=1, first=0):
+    """Config 3: nx*ny unit lattice, raster order; PPD to left, up, up-left neighbours.  Sketch k of a batch draws its
+    noise from splitmix64(seed + first + k) (as truss does); the default single sketch is config 3 itself."""
     pts = np.array([[x, y] for y in range(ny) for x in range(nx)], dtype=np.float64)
     kind, idx, dist = [], [], []
     for y in range(ny):
@@ -161,10 +162,11 @@ def lattice(nx=400, ny=250, noise=0.02, seed=0xF1C50003):
                 idx.append([2 * i, 2 * j, 0, 0])
                 dist.append(math.hypot(dx, dy))
     n_pts = nx * ny
-    u = uniform_pm1(splitmix64(np.array([seed], dtype=np.uint64), 2 * n_pts))
+    ids = np.arange(first, first + n_sketches, dtype=np.uint64)
+    u = uniform_pm1(splitmix64(np.uint64(seed) + ids, 2 * n_pts))
     raw = pts.reshape(1, -1) + noise * u
     return Workload(f"lattice{nx}x{ny}", kind, idx, np.arange(2 * n_pts), np.arange(len(kind)), raw,
-                    np.array(dist).reshape(1, -1))
+                    np.tile(np.array(dist), (n_sketches, 1)))
 
 
 def hinged_triangles(n_triangles, n_sketches=1):

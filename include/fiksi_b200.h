@@ -195,7 +195,12 @@ FK_API int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems,
 
 /* Uniform batch: n sketches sharing one topology.  vars[n][n_vars], param[n][n_expr] (row-major,
  * one sketch after another), free_out[n][n_free], reports[n].  This is the throughput entry
- * point for configs 2, 4 and 5. */
+ * point for configs 2, 4 and 5.  The batched entry points (this one, fk_batch_solve_device[_begin/_wait],
+ * fk_batch_system_solve[_begin/_wait] and the batch plan) also take topologies on the global sparse path
+ * (info.path == 2) whose largest supernodal front has at most 236 rows: one CTA per sketch runs the LM loop over
+ * the supernodal tree with the front in shared memory (fk_topology_batch_kernel returns 3), with the decisions of
+ * fk_topology_lm_solve.  Larger fronts: FK_ERR_TOO_LARGE naming the front order; solve such systems with
+ * fk_topology_lm_solve. */
 FK_API int fk_batch_solve(const fk_topology* topo, uint32_t n, const double* vars,
                           const double* param, double* free_out, fk_report* reports, int n_gpus);
 
@@ -239,7 +244,9 @@ FK_API int fk_batch_system_solve_begin(const fk_topology* topo, int device, uint
                                        double* scales_out, fk_report* reports, uint64_t* token);
 FK_API int fk_batch_system_solve_wait(const fk_topology* topo, int device, uint64_t token);
 
-/* Device-resident batch plan (one device; used by bench.py and by fk_batch_solve internally). */
+/* Device-resident batch plan (one device; used by bench.py and by fk_batch_solve internally).  Global sparse path
+ * topologies are taken up to the front limit of fk_batch_solve (creation fails with FK_ERR_TOO_LARGE above it); their plan
+ * also holds the kernel's workspace, one per resident CTA up to `capacity`. */
 typedef struct fk_batch_plan fk_batch_plan;
 FK_API int fk_batch_plan_create(const fk_topology* topo, uint32_t capacity, int device,
                                 fk_batch_plan** out);
@@ -276,7 +283,8 @@ FK_API int fk_topology_sketch_kernel_info(const fk_topology* topo, int* availabl
 
 /* Which kernel a batched LM solve of n_sketches sketches of this topology launches under the current
  * fk_set_lm_kernel choice: 0 tile kernel, 1 sketch-per-thread (one warp per 32 sketches), 2 sketch-per-thread in its
- * warp-pair shape (negative: error). */
+ * warp-pair shape, 3 the one-CTA-per-sketch kernel of the global sparse path (negative: error, FK_ERR_TOO_LARGE when a
+ * global sparse path topology has a front of more than 236 rows). */
 FK_API int fk_topology_batch_kernel(const fk_topology* topo, uint32_t n_sketches);
 
 /* Topology cache of fk_lm_solve / fk_lm_solve_batch / fk_system_solve*: the symbolic analysis of a flattened
@@ -300,7 +308,8 @@ FK_API void fk_host_free(void* p);
  * values scattered into the precomputed CSC pattern out_j[n][jac_nnz] (device-resident plan
  * buffers).  == Subsystem::calculate_residuals_and_sparse_jacobian, fiksi/src/subsystem.rs:126-166
  * followed by SparseColMat::from_triplet_mat.  mode 0: residuals + Jacobian (K1); mode 1:
- * residuals only (K2, subsystem.rs:93-104). */
+ * residuals only (K2, subsystem.rs:93-104).  Shared-memory paths only: FK_ERR_TOO_LARGE on a global sparse path
+ * plan (fk_topology_eval evaluates those). */
 FK_API int fk_batch_plan_eval(fk_batch_plan* plan, int mode, void* stream);
 FK_API int fk_batch_plan_eval_download(fk_batch_plan* plan, double* out_r, double* out_j, void* stream);
 

@@ -61,7 +61,7 @@ EXPORTS = [
     "fk_system_add_circle", "fk_system_fix", "fk_system_add_constraint", "fk_system_num_variables",
     "fk_system_num_constraints", "fk_system_element_variable", "fk_system_get_variables", "fk_system_set_variable",
     "fk_system_set_parameter", "fk_system_solve", "fk_system_residuals", "fk_system_num_components",
-    "fk_system_component", "fk_topology_supernodal", "fk_batch_analyze", "fk_system_analyze", "fk_batch_solve_lbfgs", "fk_batch_plan_run_lbfgs", "fk_system_solve_opts", "fk_system_single_pass_plan", "fk_system_recursive_assembly_plan", "fk_batch_solve_single_pass",
+    "fk_system_component", "fk_topology_supernodal", "fk_batch_analyze", "fk_topology_analyze_kernel", "fk_system_analyze", "fk_batch_solve_lbfgs", "fk_batch_plan_run_lbfgs", "fk_system_solve_opts", "fk_system_single_pass_plan", "fk_system_recursive_assembly_plan", "fk_batch_solve_single_pass",
     "fk_set_lm_kernel", "fk_get_lm_kernel", "fk_topology_sketch_kernel_info",
     "fk_topology_batch_kernel", "fk_batch_system_solve", "fk_batch_system_solve_begin", "fk_batch_system_solve_wait", "fk_batch_solve_device_begin", "fk_batch_solve_device_wait", "fk_topology_cache_configure", "fk_topology_cache_clear", "fk_topology_cache_stats",
 ]

@@ -218,6 +218,14 @@ class Topology:
             check(k)
         return {0: "tile", 1: "sketch", 2: "sketch_pair", 3: "sparse_batch"}[k]
 
+    def analyze_kernel(self, n_sketches):
+        """fk_topology_analyze_kernel: the kernel batch_analyze of this size launches on the current device: 'warp' (matrix
+        in shared memory), 'cta' (one CTA per sketch, matrix in global memory) or 'group' (a group of CTAs per sketch)."""
+        k = lib().fk_topology_analyze_kernel(self._h, int(n_sketches))
+        if k < 0:
+            check(k)
+        return {0: "warp", 1: "cta", 2: "group"}[k]
+
     def plan(self, capacity, device=0):
         return BatchPlan(self, capacity, device)
 

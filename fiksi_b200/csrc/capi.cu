@@ -17,6 +17,7 @@
 #include <vector>
 
 #include "../../include/fiksi_b200.h"
+#include "analyze.cuh"
 #include "lm_kernels.cuh"
 #include "lm_sketch.cuh"
 #include "multifrontal.cuh"
@@ -245,10 +246,12 @@ struct AnalyzePool {
     double *d_vars = nullptr, *d_param = nullptr;
     uint8_t* d_out = nullptr;
     uint32_t capacity = 0;
+    double* d_ws = nullptr;  // workspace of the global-memory kernels, at most fk::kAnWorkspaceBytes
+    uint64_t ws_bytes = 0;
     cudaStream_t stream = nullptr;
     ~AnalyzePool() {
         if (device >= 0) cudaSetDevice(device);
-        cudaFree(d_kind); cudaFree(d_slot); cudaFree(d_vars); cudaFree(d_param); cudaFree(d_out);
+        cudaFree(d_kind); cudaFree(d_slot); cudaFree(d_vars); cudaFree(d_param); cudaFree(d_out); cudaFree(d_ws);
         if (stream) cudaStreamDestroy(stream);
     }
 };
@@ -619,6 +622,11 @@ int fk_batch_analyze(const fk_topology* topo_c, int device, uint32_t n, const do
     if (rc != FK_OK) return rc;
     const fk::Topology& t = topo->t;
     if (n == 0 || t.n_expr == 0) return FK_OK;
+    CU(cudaSetDevice(device));
+    fk::AnalyzePlan plan;
+    std::string err;
+    const int prc = fk::choose_analyze(t.n_vars, t.n_expr, n, device, &plan, &err);  // the limit rule, before any allocation
+    if (prc != FK_OK) return fail(prc, err);
     AnalyzePool* pool;
     {
         std::lock_guard<std::mutex> lock(topo->mu);
@@ -627,7 +635,6 @@ int fk_batch_analyze(const fk_topology* topo_c, int device, uint32_t n, const do
         pool = p.get();
     }
     std::lock_guard<std::mutex> lock(pool->mu);
-    CU(cudaSetDevice(device));
     if (pool->device < 0) {  // tables: once per (topology, device)
         std::vector<uint32_t> slot_var((size_t)t.n_expr * 8, 0);
         for (uint32_t e = 0; e < t.n_expr; e++) {
@@ -652,12 +659,19 @@ int fk_batch_analyze(const fk_topology* topo_c, int device, uint32_t n, const do
         CU(cudaMalloc(&pool->d_out, (size_t)cap * t.n_expr));
         pool->capacity = cap;
     }
+    if (pool->ws_bytes < plan.workspace_bytes()) {  // grow-only, within fk::kAnWorkspaceBytes
+        cudaFree(pool->d_ws);
+        pool->d_ws = nullptr; pool->ws_bytes = 0;
+        CU(cudaMalloc(&pool->d_ws, plan.workspace_bytes()));
+        pool->ws_bytes = plan.workspace_bytes();
+    }
     CU(cudaMemcpyAsync(pool->d_vars, vars, sizeof(double) * (size_t)n * t.n_vars, cudaMemcpyHostToDevice, pool->stream));
     CU(cudaMemcpyAsync(pool->d_param, param, sizeof(double) * (size_t)n * t.n_expr, cudaMemcpyHostToDevice, pool->stream));
-    const int e = fk::launch_batch_analyze(t.n_vars, t.n_expr, pool->d_kind, pool->d_slot, n, pool->d_vars, pool->d_param, pool->d_out, pool->stream);
-    if (e == (int)cudaErrorInvalidConfiguration)
-        return fail(FK_ERR_TOO_LARGE, "the expression x variable matrix of one sketch does not fit shared memory");
-    if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_batch_analyze_kernel");
+    const int e = plan.kernel == fk::kAnWarp
+                      ? fk::launch_batch_analyze(t.n_vars, t.n_expr, pool->d_kind, pool->d_slot, n, pool->d_vars, pool->d_param, pool->d_out, pool->stream)
+                      : fk::launch_analyze(plan, t.n_vars, t.n_expr, pool->d_kind, pool->d_slot, n, pool->d_vars, pool->d_param, pool->d_out,
+                                           pool->d_ws, pool->stream);
+    if (e != 0) return cuda_fail((cudaError_t)e, plan.kernel == fk::kAnWarp ? "launch fk_batch_analyze_kernel" : "launch fk_analyze_cta_kernel");
     CU(cudaMemcpyAsync(independent, pool->d_out, (size_t)n * t.n_expr, cudaMemcpyDeviceToHost, pool->stream));
     CU(cudaStreamSynchronize(pool->stream));
     return FK_OK;
@@ -813,6 +827,19 @@ int fk_topology_batch_kernel(const fk_topology* topo_c, uint32_t n_sketches) {
     p.sketch_prog = (k.ok && fk::sk_fits(k.entries, k.tab.size())) ? &probe : nullptr;
     if (!fk::batch_lm_uses_sketch_kernel(p, n_sketches)) return 0;
     return fk::sketch_kernel_is_pair(probe, n_sketches) ? 2 : 1;
+}
+
+int fk_topology_analyze_kernel(const fk_topology* topo_c, uint32_t n_sketches) {
+    if (!topo_c) return fail(FK_ERR_INVALID, "null topology");
+    int device = 0;  // (the warp kernel and the limit rule need no device; cta / group are sized on the current one)
+    if (cudaGetDevice(&device) != cudaSuccess) {
+        cudaGetLastError();
+        device = 0;
+    }
+    fk::AnalyzePlan plan;
+    std::string err;
+    const int rc = fk::choose_analyze(topo_c->t.n_vars, topo_c->t.n_expr, n_sketches, device, &plan, &err);
+    return rc == FK_OK ? plan.kernel : fail(rc, err);
 }
 
 void* fk_host_alloc(size_t bytes) {

@@ -696,11 +696,16 @@ fk_batch_analyze_kernel(uint32_t n_vars, uint32_t n_expr, const uint8_t* __restr
     for (uint32_t r = lane; r < m; r += 32) out[(size_t)sketch * m + r] = (uint8_t)inc[r];
 }
 
+size_t batch_analyze_warp_bytes(uint32_t n_vars, uint32_t n_expr) {
+    return (((size_t)n_expr * n_vars * sizeof(double) + ((size_t)n_vars + n_expr) * sizeof(uint32_t)) + 15) & ~(size_t)15;
+}
+bool batch_analyze_warp_fits(uint32_t n_vars, uint32_t n_expr) { return batch_analyze_warp_bytes(n_vars, n_expr) <= 200 * 1024; }
+
 int launch_batch_analyze(uint32_t n_vars, uint32_t n_expr, const uint8_t* kinds, const uint32_t* slot_var, uint32_t n_sketches,
                          const double* vars, const double* params, uint8_t* out, void* stream) {
     if (n_sketches == 0 || n_expr == 0) return 0;
-    const size_t per_warp = (((size_t)n_expr * n_vars * sizeof(double) + ((size_t)n_vars + n_expr) * sizeof(uint32_t)) + 15) & ~(size_t)15;
-    if (per_warp > 200 * 1024) return (int)cudaErrorInvalidConfiguration;
+    if (!batch_analyze_warp_fits(n_vars, n_expr)) return (int)cudaErrorInvalidConfiguration;
+    const size_t per_warp = batch_analyze_warp_bytes(n_vars, n_expr);
     const uint32_t wpc = (uint32_t)std::max<size_t>(1, std::min<size_t>(kAnalyzeWarps, (200 * 1024) / per_warp));
     const size_t smem = per_warp * wpc;
     cudaError_t e = cudaFuncSetAttribute(fk_batch_analyze_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -3,6 +3,7 @@
 // LM loop of fiksi/src/solve/lm.rs:21-193 on it out of shared memory.
 #pragma once
 #include <atomic>
+#include <cstddef>
 #include <cstdint>
 
 #include "../../include/fiksi_b200.h"
@@ -64,8 +65,11 @@ int batch_lm_uses_sketch_kernel(const DevProgram& prog, uint32_t n_sketches);
 std::atomic<int>& lm_kernel_choice();
 int launch_batch_eval(const DevProgram& prog, uint32_t n_sketches, const double* vars,
                       const double* params, double* out_r, double* out_j, int mode, void* stream);
-// System::analyze on a batch: kinds[n_expr], slot_var[n_expr][8] device tables; out[n][n_expr].
-// Returns cudaErrorInvalidConfiguration when one n_expr x n_vars matrix does not fit shared memory.
+// System::analyze on a batch, one warp per sketch: kinds[n_expr], slot_var[n_expr][8] device tables; out[n][n_expr].
+// Returns cudaErrorInvalidConfiguration when one n_expr x n_vars matrix does not fit shared memory
+// (batch_analyze_warp_fits: at most 200 KiB per warp with the column order and the flags).
+size_t batch_analyze_warp_bytes(uint32_t n_vars, uint32_t n_expr);
+bool batch_analyze_warp_fits(uint32_t n_vars, uint32_t n_expr);
 int launch_batch_analyze(uint32_t n_vars, uint32_t n_expr, const uint8_t* kinds, const uint32_t* slot_var, uint32_t n_sketches,
                          const double* vars, const double* params, uint8_t* out, void* stream);
 // L-BFGS on a uniform batch (tile paths with 8 / 16 / 32 lanes only); d_jcolptr[n+1], d_jrow[jnnz]: CSC

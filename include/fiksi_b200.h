@@ -344,10 +344,19 @@ FK_API int fk_batch_plan_run_lbfgs(fk_batch_plan* plan, void* stream);
  * parameters param[n][n_expr], reduced by incremental_gauss_jordan_elimination (:33-117, epsilon 1e-8).
  * independent[n][n_expr] receives 1 for an expression that increases the rank, 0 for a dependent one
  * (the constraint owning a dependent expression is what System::analyze reports as overconstrained).
- * The topology's free set and row list are not used.  One warp per sketch on `device`; returns
- * FK_ERR_TOO_LARGE when one n_expr x n_vars matrix does not fit shared memory. */
+ * The topology's free set and row list are not used.  Kernels on `device` (fk_topology_analyze_kernel): one warp per
+ * sketch with the matrix in shared memory where it fits (at most 200 KiB with the column order and the flags); otherwise
+ * the matrix in global memory, one CTA per sketch when the batch fills the device and a cooperative group of CTAs per
+ * sketch below that.  Limit: n_vars <= 26,624 (the row being reduced is held in shared memory) and one sketch's
+ * min(n_expr, n_vars) x n_vars matrix within the 4 GiB workspace of a (topology, device), which a large sketch shares
+ * with fewer sketches in flight.  Above it, FK_ERR_TOO_LARGE with the sizes in fk_last_error(), before any allocation. */
 FK_API int fk_batch_analyze(const fk_topology* topo, int device, uint32_t n, const double* vars, const double* param,
                             uint8_t* independent);
+/* Which kernel fk_batch_analyze launches for n_sketches sketches of this topology on the current device: 0 one warp per
+ * sketch, 1 one CTA per sketch, 2 groups of CTAs per sketch; negative on error (FK_ERR_TOO_LARGE above the limit of
+ * fk_batch_analyze).  Environment FK_ANALYZE_KERNEL=warp|cta|group forces one wherever it can take the shape (tests,
+ * A/B measurements); a forced warp kernel on a matrix it cannot hold is FK_ERR_TOO_LARGE. */
+FK_API int fk_topology_analyze_kernel(const fk_topology* topo, uint32_t n_sketches);
 
 /* ---- fiksi::System mirror (host side above the solve boundary) ------------------------------- */
 /* Same operations, argument meaning and ordering rules as fiksi::System (fiksi/src/lib.rs:252-467):
@@ -410,7 +419,9 @@ FK_API int fk_system_single_pass_plan(const fk_system* s, uint32_t* sizes3, uint
                                       uint32_t* expr_ptr, uint32_t* exprs);
 FK_API int fk_system_residuals(fk_system* s, double* out /* [num_constraints] */); /* calculate_residual */
 /* == System::analyze (lib.rs:454-458): ids of the constraints that own a dependent expression, in
- * expression order, up to `cap`; *n_found receives their number. */
+ * expression order, up to `cap`; *n_found receives their number.  All variables and expressions of the system go
+ * through fk_batch_analyze as one sketch on device 0 (a group of CTAs once its matrix leaves shared memory), under
+ * the same size limit. */
 FK_API int fk_system_analyze(fk_system* s, uint32_t* constraints, uint32_t cap, uint32_t* n_found);
 FK_API uint32_t fk_system_num_components(const fk_system* s);
 FK_API int fk_system_component(const fk_system* s, uint32_t index, uint32_t* n_elements, uint32_t* elements,

@@ -4,5 +4,6 @@ The product is ``libfiksi_b200.so`` (C ABI in ``include/fiksi_b200.h``); this pa
 ctypes face used by the tests and the benchmark.
 """
 from ._lib import FiksiError, FkProblem, FkReport, REPORT_DTYPE, LIB_PATH, lib, make_problem  # noqa: F401
-from .api import BatchPlan, Topology, device_count, fp64_peak_tflops, lm_solve, lm_solve_batch  # noqa: F401
+from .api import (BatchPlan, Topology, device_count, fp64_peak_tflops, lbfgs_solve, lbfgs_solve_batch, lm_solve,  # noqa: F401
+                  lm_solve_batch)
 from .system import System  # noqa: F401

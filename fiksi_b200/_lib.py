@@ -37,6 +37,10 @@ class FkPrepareOpts(C.Structure):
                 ("seed", C.c_uint32), ("pad", C.c_uint32)]
 
 
+class FkSolvingOptions(C.Structure):
+    _fields_ = [("optimizer", C.c_uint32), ("decomposer", C.c_uint32), ("perturb", C.c_uint32), ("pad", C.c_uint32)]
+
+
 class FkTopologyInfo(C.Structure):
     _fields_ = [(n, C.c_uint32) for n in (
         "n_vars", "n_expr", "n_free", "n_rows", "jac_nnz", "aug_nnz", "r_nnz", "etree_height",
@@ -63,7 +67,8 @@ EXPORTS = [
     "fk_system_set_parameter", "fk_system_solve", "fk_system_residuals", "fk_system_num_components",
     "fk_system_component", "fk_topology_supernodal", "fk_batch_analyze", "fk_topology_analyze_kernel", "fk_system_analyze", "fk_batch_solve_lbfgs", "fk_batch_plan_run_lbfgs", "fk_system_solve_opts", "fk_system_single_pass_plan", "fk_system_recursive_assembly_plan", "fk_batch_solve_single_pass",
     "fk_set_lm_kernel", "fk_get_lm_kernel", "fk_topology_sketch_kernel_info",
-    "fk_topology_batch_kernel", "fk_batch_system_solve", "fk_batch_system_solve_begin", "fk_batch_system_solve_wait", "fk_batch_solve_device_begin", "fk_batch_solve_device_wait", "fk_topology_cache_configure", "fk_topology_cache_clear", "fk_topology_cache_stats",
+    "fk_topology_batch_kernel", "fk_topology_lbfgs_kernel", "fk_lbfgs_solve", "fk_lbfgs_solve_batch", "fk_batch_plan_run_lbfgs_global",
+    "fk_system_solve_options", "fk_batch_system_solve", "fk_batch_system_solve_begin", "fk_batch_system_solve_wait", "fk_batch_solve_device_begin", "fk_batch_solve_device_wait", "fk_topology_cache_configure", "fk_topology_cache_clear", "fk_topology_cache_stats",
 ]
 
 _lib = None

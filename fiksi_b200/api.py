@@ -226,6 +226,14 @@ class Topology:
             check(k)
         return {0: "warp", 1: "cta", 2: "group"}[k]
 
+    def lbfgs_kernel(self, n_sketches):
+        """fk_topology_lbfgs_kernel: the L-BFGS kernel the batch calls launch: 0 the tile kernel (state in shared memory),
+        1 the CTA kernel (one CTA per sketch, state in global memory; any size)."""
+        k = lib().fk_topology_lbfgs_kernel(self._h, int(n_sketches))
+        if k < 0:
+            check(k)
+        return k
+
     def plan(self, capacity, device=0):
         return BatchPlan(self, capacity, device)
 
@@ -265,6 +273,10 @@ class BatchPlan:
 
     def run_lbfgs(self, stream=0):
         check(lib().fk_batch_plan_run_lbfgs(self._h, C.c_void_p(stream)))
+
+    def run_lbfgs_global(self, stream=0):
+        """fk_batch_plan_run_lbfgs_global: L-BFGS with the CTA kernel on any plan."""
+        check(lib().fk_batch_plan_run_lbfgs_global(self._h, C.c_void_p(stream)))
 
     def download(self, free_out, reports, stream=0):
         check(lib().fk_batch_plan_download(self._h, C.c_void_p(free_out.ctypes.data if free_out is not None else 0),
@@ -346,14 +358,31 @@ def lm_solve(problem: FkProblem, free_values):
     return x, report_dict(rep)
 
 
-def lm_solve_batch(problems, free_values_list, n_gpus=1):
+def _solve_batch(fn, problems, free_values_list, n_gpus):
     n = len(problems)
-    arr = (C.POINTER(FkProblem) * n)(*[C.pointer(p) for p in problems])
+    arr = (C.POINTER(FkProblem) * max(n, 1))(*[C.pointer(p) for p in problems])
     xs = [np.array(v, dtype=np.float64) for v in free_values_list]
-    fv = (C.POINTER(C.c_double) * n)(*[ptr(x, C.c_double) for x in xs])
+    fv = (C.POINTER(C.c_double) * max(n, 1))(*[ptr(x, C.c_double) for x in xs])
     reports = np.zeros(n, dtype=REPORT_DTYPE)
-    check(lib().fk_lm_solve_batch(n, arr, fv, reports.ctypes.data_as(C.POINTER(FkReport)), n_gpus))
+    check(fn(n, arr, fv, reports.ctypes.data_as(C.POINTER(FkReport)), n_gpus))
     return xs, reports
+
+
+def lm_solve_batch(problems, free_values_list, n_gpus=1):
+    return _solve_batch(lib().fk_lm_solve_batch, problems, free_values_list, n_gpus)
+
+
+def lbfgs_solve(problem: FkProblem, free_values):
+    """== lbfgs(problem, variables) (fiksi/src/solve/lbfgs.rs:20) through fk_lbfgs_solve (any size)."""
+    x = np.array(free_values, dtype=np.float64)
+    rep = FkReport()
+    check(lib().fk_lbfgs_solve(C.byref(problem), ptr(x, C.c_double), C.byref(rep)))
+    return x, report_dict(rep)
+
+
+def lbfgs_solve_batch(problems, free_values_list, n_gpus=1):
+    """fk_lbfgs_solve_batch: problems of any structure and size, grouped by topology."""
+    return _solve_batch(lib().fk_lbfgs_solve_batch, problems, free_values_list, n_gpus)
 
 
 def report_dict(rep):

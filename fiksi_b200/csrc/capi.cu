@@ -18,6 +18,7 @@
 
 #include "../../include/fiksi_b200.h"
 #include "analyze.cuh"
+#include "lbfgs_global.cuh"
 #include "lm_kernels.cuh"
 #include "lm_sketch.cuh"
 #include "multifrontal.cuh"
@@ -98,7 +99,8 @@ struct DeviceProgram {
     fk::DevProgram view{};
     const uint32_t *jcolptr = nullptr, *jrow = nullptr;  // CSC of the Jacobian (L-BFGS)
     std::unique_ptr<fk::SkProgram> sketch;               // parameter block of the sketch-per-thread LM kernel
-    std::unique_ptr<fk::SparseBatchProgram> sparse_batch;  // path 2: tables of the one-CTA-per-sketch supernodal LM kernel
+    std::unique_ptr<fk::SparseBatchProgram> sparse_batch;  // path 2: tables of the one-CTA-per-sketch supernodal LM kernel, built
+                                                           // by the first caller that launches LM (fk_topology::program_for)
     ~DeviceProgram() {
         if (buf) {
             cudaSetDevice(device);
@@ -172,12 +174,6 @@ int upload_program(const fk::Topology& t, int device, DeviceProgram& out) {
         p.tab = (const uint32_t*)(b + o_sk);
         v.sketch_prog = out.sketch.get();
     }
-    if (t.path == 2) {
-        std::string err;
-        out.sparse_batch.reset(new fk::SparseBatchProgram());
-        const int rc = out.sparse_batch->init(t, v, device, &err);
-        if (rc != FK_OK) return fail(rc, err);
-    }
     return FK_OK;
 }
 
@@ -226,6 +222,9 @@ struct DevicePipeline {
     cudaStream_t small_stream = nullptr;
     double* small_ws = nullptr;  // launch_lm workspace of the small requests (global sparse path)
     uint32_t small_ws_ctas = 0;
+    double* small_lb_ws = nullptr;  // L-BFGS CTA kernel workspace of the small requests
+    uint32_t small_lb_ws_ctas = 0;
+    bool plans_lm = false;  // the plans were created for LM too
     cudaEvent_t shared_param_ev = nullptr;  // fk_batch_system_solve with one parameter row for all sketches: its upload, once per call
     // Every call on the chunk pipeline takes a token.  Its parity picks the call's copy of the shared parameter row and the events
     // recorded behind its last chunk on every stream (the _begin / _wait halves: up to two calls in flight).
@@ -334,7 +333,20 @@ struct fk_topology {
         return p.get();
     }
 
-    int program_for(int device, const fk::DevProgram** out, const DeviceProgram** full = nullptr) {
+    // Path 2: whether the sparse batch LM kernel takes the topology (largest front), host analysis once per topology.
+    int sb_check() {
+        std::lock_guard<std::mutex> lock(mu);
+        if (sb_fit == 1) sb_fit = fk::sparse_batch_fits(t, nullptr, &sb_err);
+        return sb_fit == FK_OK ? FK_OK : fail(sb_fit, sb_err);
+    }
+
+    // Device tables on `device`.  lm: the caller launches LM, which on the global sparse path also needs the tables of the
+    // sparse batch kernel (refused above its front limit); L-BFGS needs none of them.
+    int program_for(int device, const fk::DevProgram** out, const DeviceProgram** full = nullptr, bool lm = true) {
+        if (lm && t.path == 2) {
+            const int rc = sb_check();
+            if (rc != FK_OK) return rc;
+        }
         std::lock_guard<std::mutex> lock(mu);
         auto it = programs.find(device);
         if (it == programs.end()) {
@@ -343,8 +355,16 @@ struct fk_topology {
             if (rc != FK_OK) return rc;
             it = programs.emplace(device, std::move(p)).first;
         }
-        *out = &it->second->view;
-        if (full) *full = it->second.get();
+        DeviceProgram& p = *it->second;
+        if (lm && t.path == 2 && !p.sparse_batch) {
+            std::string err;
+            std::unique_ptr<fk::SparseBatchProgram> sb(new fk::SparseBatchProgram());
+            const int rc = sb->init(t, p.view, device, &err);
+            if (rc != FK_OK) return fail(rc, err);
+            p.sparse_batch = std::move(sb);
+        }
+        *out = &p.view;
+        if (full) *full = &p;
         return FK_OK;
     }
 };
@@ -359,12 +379,15 @@ struct fk_batch_plan {
     fk_report* d_rep = nullptr;
     double* d_ws = nullptr;  // launch_lm workspace (global sparse path)
     uint32_t ws_ctas = 0;
+    bool lm = true;          // LM may run on the plan (false: the L-BFGS calls' internal plans, which skip its tables)
+    double* d_lb_ws = nullptr;  // L-BFGS CTA kernel workspace, grown on first use
+    uint32_t lb_ws_ctas = 0;
     double *d_raw_vars = nullptr, *d_raw_param = nullptr, *d_scales = nullptr;  // fk_batch_system_solve: unscaled input, scale per sketch
     uint64_t launches = 0;
     ~fk_batch_plan() {
         cudaSetDevice(device);
         cudaFree(d_vars); cudaFree(d_params); cudaFree(d_out); cudaFree(d_er); cudaFree(d_ej); cudaFree(d_rep);
-        cudaFree(d_raw_vars); cudaFree(d_raw_param); cudaFree(d_scales); cudaFree(d_ws);
+        cudaFree(d_raw_vars); cudaFree(d_raw_param); cudaFree(d_scales); cudaFree(d_ws); cudaFree(d_lb_ws);
     }
 };
 
@@ -385,10 +408,14 @@ void DevicePipeline::release() {
     if (small_d) cudaFree(small_d);
     if (small_stream) cudaStreamDestroy(small_stream);
     if (small_ws) cudaFree(small_ws);
+    if (small_lb_ws) cudaFree(small_lb_ws);
     small_h = small_d = nullptr;
     small_stream = nullptr;
     small_ws = nullptr;
     small_ws_ctas = 0;
+    small_lb_ws = nullptr;
+    small_lb_ws_ctas = 0;
+    plans_lm = false;
     if (shared_param_ev) cudaEventDestroy(shared_param_ev);
     shared_param_ev = nullptr;
     for (int a = 0; a < 2; a++) {
@@ -602,12 +629,21 @@ int fk_batch_solve_single_pass(const fk_topology* topo_c, uint32_t n, double* va
 static int run_device_range(fk_topology* topo, int device, uint32_t lo, uint32_t hi, const double* vars, const double* param,
                             double* free_out, fk_report* reports, int optimizer = 0, uint64_t* token = nullptr);
 
+// The L-BFGS kernel of a topology, chosen in this one place: 0 the tile kernel (state in shared memory) for every topology it
+// takes, 1 the CTA kernel (state in global memory) otherwise.  Host only.
+static int choose_lbfgs(const fk_topology* topo, uint32_t n_sketches) {
+    (void)n_sketches;  // (the choice depends on the topology alone)
+    const fk::Topology& t = topo->t;
+    return t.path == 0 && fk::batch_lbfgs_tile_fits(t.n_free, t.n_rows, t.jac_nnz, t.tile) ? 0 : 1;
+}
+
 int fk_batch_solve_lbfgs(const fk_topology* topo_c, int device, uint32_t n, const double* vars, const double* param, double* free_out,
                          fk_report* reports) {
     if (!topo_c) return fail(FK_ERR_INVALID, "null topology");
     if (n == 0) return FK_OK;
     if (!vars || !free_out || !reports || (!param && topo_c->t.n_expr)) return fail(FK_ERR_INVALID, "null buffer");
     if (topo_c->t.path != 0) return fail(FK_ERR_TOO_LARGE, "L-BFGS is built for the shared-memory tile paths only");
+    if (choose_lbfgs(topo_c, n) != 0) return fail(FK_ERR_TOO_LARGE, "the L-BFGS state of one sketch does not fit the tile path");
     const int rc = check_device(device);
     if (rc != FK_OK) return rc;
     // same pooled plans / streams / pinned staging as the LM entry (no allocation per call)
@@ -678,8 +714,9 @@ int fk_batch_analyze(const fk_topology* topo_c, int device, uint32_t n, const do
 }
 
 // ---- device-resident batch plan -----------------------------------------------------------------
-int fk_batch_plan_create(const fk_topology* topo_c, uint32_t capacity, int device, fk_batch_plan** out) {
-    fk_topology* topo = const_cast<fk_topology*>(topo_c);
+// lm: LM may run on the plan.  The L-BFGS calls create their internal plans without, so that they skip the tables of the
+// sparse batch LM kernel and its front limit.
+static int plan_create(fk_topology* topo, uint32_t capacity, int device, bool lm, fk_batch_plan** out) {
     if (!topo || !out || capacity == 0) return fail(FK_ERR_INVALID, "null topology / zero capacity");
     int rc = check_device(device);
     if (rc != FK_OK) return rc;
@@ -688,17 +725,21 @@ int fk_batch_plan_create(const fk_topology* topo_c, uint32_t capacity, int devic
     CU(cudaGetDeviceProperties(&prop, device));
     if (prop.major != 10) return fail(FK_ERR_NO_DEVICE, "device is not sm_100 class; kernels are built for sm_100a only");
     std::unique_ptr<fk_batch_plan> p(new fk_batch_plan());
-    p->topo = topo; p->device = device; p->capacity = capacity;
-    rc = topo->program_for(device, &p->prog, &p->full);
+    p->topo = topo; p->device = device; p->capacity = capacity; p->lm = lm;
+    rc = topo->program_for(device, &p->prog, &p->full, lm);
     if (rc != FK_OK) return rc;
     const fk::Topology& t = topo->t;
     CU(cudaMalloc(&p->d_vars, sizeof(double) * std::max<size_t>(1, (size_t)capacity * t.n_vars)));
     CU(cudaMalloc(&p->d_params, sizeof(double) * std::max<size_t>(1, (size_t)capacity * t.n_expr)));
     CU(cudaMalloc(&p->d_out, sizeof(double) * std::max<size_t>(1, (size_t)capacity * t.n_free)));
     CU(cudaMalloc(&p->d_rep, sizeof(fk_report) * (size_t)capacity));
-    if ((rc = alloc_lm_workspace(*p->full, capacity, &p->d_ws, &p->ws_ctas)) != FK_OK) return rc;
+    if (lm && (rc = alloc_lm_workspace(*p->full, capacity, &p->d_ws, &p->ws_ctas)) != FK_OK) return rc;
     *out = p.release();
     return FK_OK;
+}
+
+int fk_batch_plan_create(const fk_topology* topo, uint32_t capacity, int device, fk_batch_plan** out) {
+    return plan_create(const_cast<fk_topology*>(topo), capacity, device, true, out);
 }
 
 void fk_batch_plan_destroy(fk_batch_plan* plan) { delete plan; }
@@ -722,6 +763,39 @@ int fk_batch_plan_run(fk_batch_plan* plan, void* stream) {
     if (e != 0) return cuda_fail((cudaError_t)e, "launch batched LM kernel");
     if (plan->n) plan->launches++;
     return FK_OK;
+}
+
+// Grow-only L-BFGS CTA workspace with room for `ctas` CTAs (*buf, *have: its current size).
+static int grow_lbfgs_workspace(const fk::DevProgram& prog, uint32_t ctas, double** buf, uint32_t* have) {
+    if (*have >= ctas) return FK_OK;
+    if (*buf) cudaFree(*buf);
+    *buf = nullptr;
+    *have = 0;
+    CU(cudaMalloc(buf, sizeof(double) * fk::lbfgs_workspace_doubles(prog, ctas)));
+    *have = ctas;
+    return FK_OK;
+}
+
+static int run_lbfgs_cta(const DeviceProgram& full, uint32_t n, const double* vars, const double* params, double* out, fk_report* reps,
+                         double** ws, uint32_t* ws_ctas, cudaStream_t st) {
+    if (n == 0) return FK_OK;
+    const uint32_t ctas = fk::lbfgs_workspace_ctas(full.view, n);
+    if (ctas == 0) return fail(FK_ERR_CUDA, "occupancy query of fk_lbfgs_cta_kernel failed");
+    const int rc = grow_lbfgs_workspace(full.view, ctas, ws, ws_ctas);
+    if (rc != FK_OK) return rc;
+    const int e = fk::launch_lbfgs_cta(full.view, full.jcolptr, full.jrow, n, vars, params, out, reps, *ws, ctas, st);
+    if (e == (int)cudaErrorInvalidConfiguration) return fail(FK_ERR_TOO_LARGE, "more than 2^24 Jacobian entries");
+    if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_lbfgs_cta_kernel");
+    return FK_OK;
+}
+
+int fk_batch_plan_run_lbfgs_global(fk_batch_plan* plan, void* stream) {
+    if (!plan) return fail(FK_ERR_INVALID, "null plan");
+    CU(cudaSetDevice(plan->device));
+    const int rc = run_lbfgs_cta(*plan->full, plan->n, plan->d_vars, plan->d_params, plan->d_out, plan->d_rep, &plan->d_lb_ws,
+                                 &plan->lb_ws_ctas, (cudaStream_t)stream);
+    if (rc == FK_OK && plan->n) plan->launches++;
+    return rc;
 }
 
 int fk_batch_plan_run_lbfgs(fk_batch_plan* plan, void* stream) {
@@ -815,9 +889,8 @@ int fk_topology_batch_kernel(const fk_topology* topo_c, uint32_t n_sketches) {
     if (!topo_c) return fail(FK_ERR_INVALID, "null topology");
     fk_topology* topo = const_cast<fk_topology*>(topo_c);
     if (topo->t.path == 2) {  // host analysis only (no device needed), once per topology
-        std::lock_guard<std::mutex> lock(topo->mu);
-        if (topo->sb_fit == 1) topo->sb_fit = fk::sparse_batch_fits(topo->t, nullptr, &topo->sb_err);
-        return topo->sb_fit == FK_OK ? 3 : fail(topo->sb_fit, topo->sb_err);
+        const int rc = topo->sb_check();
+        return rc == FK_OK ? 3 : rc;
     }
     const fk::Topology::SketchTables& k = topo->t.sk;
     fk::SkProgram probe{};
@@ -827,6 +900,11 @@ int fk_topology_batch_kernel(const fk_topology* topo_c, uint32_t n_sketches) {
     p.sketch_prog = (k.ok && fk::sk_fits(k.entries, k.tab.size())) ? &probe : nullptr;
     if (!fk::batch_lm_uses_sketch_kernel(p, n_sketches)) return 0;
     return fk::sketch_kernel_is_pair(probe, n_sketches) ? 2 : 1;
+}
+
+int fk_topology_lbfgs_kernel(const fk_topology* topo, uint32_t n_sketches) {
+    if (!topo) return fail(FK_ERR_INVALID, "null topology");
+    return choose_lbfgs(topo, n_sketches);
 }
 
 int fk_topology_analyze_kernel(const fk_topology* topo_c, uint32_t n_sketches) {
@@ -889,8 +967,9 @@ static uint32_t pipeline_chunk(fk_topology* topo, int device, uint32_t total, ui
 // first drains every stream, so that no copy into the caller's buffers is still running when it returns.
 using PipelinePrologue = std::function<int(DevicePipeline& pl, int slot, uint32_t use_streams)>;
 using PipelineChunk = std::function<int(fk_batch_plan* p, cudaStream_t st, uint32_t at, uint32_t cnt, const std::function<void()>& mark)>;
+// lm: the chunks run LM (plans made for L-BFGS only are then made again).
 static int run_pipeline(fk_topology* topo, int device, uint32_t lo, uint32_t hi, uint32_t chunk, uint64_t* token,
-                        const PipelinePrologue& prologue, const PipelineChunk& enqueue) {
+                        const PipelinePrologue& prologue, const PipelineChunk& enqueue, bool lm = true) {
     constexpr uint32_t kStreams = DevicePipeline::kStreams;
     static const uint32_t use_streams = [] {
         const char* e = std::getenv("FK_E2E_STREAMS");  // tuning knob: chunks in flight (at most kStreams)
@@ -903,10 +982,11 @@ static int run_pipeline(fk_topology* topo, int device, uint32_t lo, uint32_t hi,
     DevicePipeline* pl = topo->pipeline_for(device);
     std::lock_guard<std::mutex> lock(pl->mu);
     int rc = FK_OK;
-    if (pl->chunk < chunk) {
+    if (pl->chunk < chunk || (lm && !pl->plans_lm)) {
+        const uint32_t cap = std::max(chunk, pl->chunk);
         pl->release();
         for (uint32_t s = 0; s < kStreams && rc == FK_OK; s++) {
-            rc = fk_batch_plan_create(topo, chunk, device, &pl->plans[s]);
+            rc = plan_create(topo, cap, device, lm, &pl->plans[s]);
             if (rc == FK_OK && cudaStreamCreateWithFlags(&pl->streams[s], cudaStreamNonBlocking) != cudaSuccess)
                 rc = fail(FK_ERR_CUDA, "cudaStreamCreate failed");
         }
@@ -914,7 +994,8 @@ static int run_pipeline(fk_topology* topo, int device, uint32_t lo, uint32_t hi,
             pl->release();
             return rc;
         }
-        pl->chunk = chunk;
+        pl->chunk = cap;
+        pl->plans_lm = lm;
     }
     const uint64_t my_token = pl->next_token++;
     const int slot = (int)(my_token & 1u);
@@ -972,11 +1053,6 @@ static int run_pipeline(fk_topology* topo, int device, uint32_t lo, uint32_t hi,
     return rc;
 }
 
-static int launch_optimizer(const DeviceProgram& full, int optimizer, uint32_t n, const double* vars, const double* params, double* out,
-                            fk_report* reps, double* ws, uint32_t ws_ctas, cudaStream_t st) {
-    if (optimizer == 1) return fk::launch_batch_lbfgs(full.view, full.jcolptr, full.jrow, n, vars, params, out, reps, st);
-    return launch_lm(full, n, vars, params, out, reps, ws, ws_ctas, st);
-}
 
 // Small request (one sketch, a handful): the caller's (pageable) arrays go through ONE pinned staging block -- one
 // copy in, the kernel, one copy out, one synchronisation -- instead of four pageable copies on the chunk pipeline.
@@ -996,8 +1072,9 @@ static int small_solve(fk_topology* topo, int device, uint32_t lo, uint32_t hi, 
     const size_t in_al = (in_v + in_p + 15) & ~size_t(15);
     const fk::DevProgram* prog = nullptr;
     const DeviceProgram* full = nullptr;
-    int rc = topo->program_for(device, &prog, &full);
+    int rc = topo->program_for(device, &prog, &full, optimizer == 0);
     if (rc != FK_OK) return rc;
+    const bool lbfgs_cta = optimizer == 1 && choose_lbfgs(topo, total) == 1;
     cudaError_t e = cudaSetDevice(device);
     if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
     if (!pl->small_h || !pl->small_d || !pl->small_stream) {
@@ -1017,7 +1094,7 @@ static int small_solve(fk_topology* topo, int device, uint32_t lo, uint32_t hi, 
             return cuda_fail(e, "cudaStreamCreate");
         }
     }
-    if (full->sparse_batch && pl->small_ws_ctas < full->sparse_batch->workspace_ctas(total)) {  // grow-only
+    if (optimizer == 0 && full->sparse_batch && pl->small_ws_ctas < full->sparse_batch->workspace_ctas(total)) {  // grow-only
         if (pl->small_ws) cudaFree(pl->small_ws);
         pl->small_ws = nullptr;
         pl->small_ws_ctas = 0;
@@ -1028,19 +1105,27 @@ static int small_solve(fk_topology* topo, int device, uint32_t lo, uint32_t hi, 
     // A few kilobytes: the kernel reads its inputs from, and writes its results to, the pinned block itself (pinned host
     // memory is mapped into the device's address space under unified addressing; the kernel touches every input and output
     // once) -- two DMA set-ups less on a path that is all latency.  FK_NO_ZERO_COPY=1 keeps the two copies (A/B knob).  Not
-    // for the sparse batch kernel: it reads the parameters and fixed variables again on every evaluation.
+    // for the sparse batch LM kernel or the L-BFGS kernels: they read the parameters and fixed variables again on every
+    // evaluation.
     static const bool no_zero_copy = std::getenv("FK_NO_ZERO_COPY") != nullptr;
     static const bool can_map = [] {
         int dev = 0, ok = 0;
         return cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&ok, cudaDevAttrCanUseHostPointerForRegisteredMem, dev) == cudaSuccess && ok != 0;
     }();
-    const bool zero_copy = !no_zero_copy && can_map && !full->sparse_batch && in_al + out_x + out_r <= 8 * 1024;
+    const bool zero_copy = !no_zero_copy && can_map && optimizer == 0 && !full->sparse_batch && in_al + out_x + out_r <= 8 * 1024;
     unsigned char* base = zero_copy ? pl->small_h : pl->small_d;
     if (!zero_copy && (e = cudaMemcpyAsync(pl->small_d, pl->small_h, in_v + in_p, cudaMemcpyHostToDevice, pl->small_stream)) != cudaSuccess) return cuda_fail(e, "cudaMemcpyAsync");
-    const int le = launch_optimizer(*full, optimizer, total, (const double*)base, (const double*)(base + in_v), (double*)(base + in_al),
-                                    (fk_report*)(base + in_al + out_x), pl->small_ws, pl->small_ws_ctas, pl->small_stream);
-    if (le == (int)cudaErrorInvalidConfiguration && optimizer == 1) return fail(FK_ERR_TOO_LARGE, "the L-BFGS state of one sketch does not fit the tile path");
-    if (le != 0) return cuda_fail((cudaError_t)le, "launch batched solve kernel");
+    const double *d_vars = (const double*)base, *d_param = (const double*)(base + in_v);
+    double* d_out = (double*)(base + in_al);
+    fk_report* d_rep = (fk_report*)(base + in_al + out_x);
+    if (lbfgs_cta) {
+        if ((rc = run_lbfgs_cta(*full, total, d_vars, d_param, d_out, d_rep, &pl->small_lb_ws, &pl->small_lb_ws_ctas, pl->small_stream)) != FK_OK)
+            return rc;
+    } else {
+        const int le = optimizer == 1 ? fk::launch_batch_lbfgs(full->view, full->jcolptr, full->jrow, total, d_vars, d_param, d_out, d_rep, pl->small_stream)
+                                      : launch_lm(*full, total, d_vars, d_param, d_out, d_rep, pl->small_ws, pl->small_ws_ctas, pl->small_stream);
+        if (le != 0) return cuda_fail((cudaError_t)le, optimizer == 1 ? "launch fk_batch_lbfgs_kernel" : "launch batched solve kernel");
+    }
     if (!zero_copy && (e = cudaMemcpyAsync(pl->small_h + in_al, pl->small_d + in_al, out_x + out_r, cudaMemcpyDeviceToHost, pl->small_stream)) != cudaSuccess) return cuda_fail(e, "cudaMemcpyAsync");
     if ((e = cudaStreamSynchronize(pl->small_stream)) != cudaSuccess) return cuda_fail(e, "batch kernel / copy failed");
     std::memcpy(free_out + (size_t)lo * t.n_free, pl->small_h + in_al, out_x);
@@ -1049,8 +1134,8 @@ static int small_solve(fk_topology* topo, int device, uint32_t lo, uint32_t hi, 
 }
 
 // Sketches [lo, hi) of a uniform batch on one device: a small request through the staging block, anything larger through the
-// chunk pipeline.  optimizer 1: L-BFGS.  token: see run_pipeline; the caller sets *token = 0, which is what a small request
-// (complete when it returns) leaves there.
+// chunk pipeline.  optimizer 1: L-BFGS with the kernel of choose_lbfgs.  token: see run_pipeline; the caller sets *token = 0,
+// which is what a small request (complete when it returns) leaves there.
 static int run_device_range(fk_topology* topo, int device, uint32_t lo, uint32_t hi, const double* vars, const double* param,
                             double* free_out, fk_report* reports, int optimizer, uint64_t* token) {
     if (hi == lo) return FK_OK;
@@ -1058,16 +1143,18 @@ static int run_device_range(fk_topology* topo, int device, uint32_t lo, uint32_t
     if (small_fits(t, hi - lo)) return small_solve(topo, device, lo, hi, vars, param, free_out, reports, optimizer);
     // (the L-BFGS kernel is not the sketch-per-thread kernel: its chunks are not rounded to that kernel's waves)
     const uint32_t chunk = pipeline_chunk(topo, device, hi - lo, 8, optimizer == 0);
+    const bool lbfgs_cta = optimizer == 1 && choose_lbfgs(topo, hi - lo) == 1;
     return run_pipeline(topo, device, lo, hi, chunk, token, nullptr,
                         [&](fk_batch_plan* p, cudaStream_t st, uint32_t at, uint32_t cnt, const std::function<void()>& mark) {
                             int rc = fk_batch_plan_upload(p, cnt, vars + (size_t)at * t.n_vars, param ? param + (size_t)at * t.n_expr : nullptr, st);
                             if (rc != FK_OK) return rc;
                             mark();
-                            rc = optimizer == 1 ? fk_batch_plan_run_lbfgs(p, st) : fk_batch_plan_run(p, st);
+                            rc = optimizer == 0 ? fk_batch_plan_run(p, st) : lbfgs_cta ? fk_batch_plan_run_lbfgs_global(p, st) : fk_batch_plan_run_lbfgs(p, st);
                             if (rc != FK_OK) return rc;
                             mark();
                             return fk_batch_plan_download(p, free_out + (size_t)at * t.n_free, reports ? reports + at : nullptr, st);
-                        });
+                        },
+                        optimizer == 0);
 }
 
 // ---- System::solve level batch: scale, perturbation and write-back on the device -----------------------------
@@ -1249,6 +1336,14 @@ int fk_batch_solve_device_begin(const fk_topology* topo, int device, uint32_t n,
 
 int fk_batch_solve_device_wait(const fk_topology* topo, int device, uint64_t token) { return fk_batch_system_solve_wait(topo, device, token); }
 
+// n sketches of one topology over n_gpus devices: contiguous shares, one host thread per device (fk_batch_solve).
+static int solve_sharded(fk_topology* topo, uint32_t n, const double* vars, const double* param, double* free_out, fk_report* reports,
+                         int n_gpus, int optimizer) {
+    return shard_over_devices(n_gpus, n, [&](int device, uint32_t lo, uint32_t hi) {
+        return run_device_range(topo, device, lo, hi, vars, param, free_out, reports, optimizer);
+    });
+}
+
 int fk_batch_solve(const fk_topology* topo_c, uint32_t n, const double* vars, const double* param, double* free_out,
                    fk_report* reports, int n_gpus) {
     fk_topology* topo = const_cast<fk_topology*>(topo_c);
@@ -1257,9 +1352,7 @@ int fk_batch_solve(const fk_topology* topo_c, uint32_t n, const double* vars, co
     if (!vars || !free_out || (!param && topo->t.n_expr)) return fail(FK_ERR_INVALID, "null buffer");
     const int rc = clamp_gpus(n_gpus);
     if (rc != FK_OK) return rc;
-    return shard_over_devices(n_gpus, n, [&](int device, uint32_t lo, uint32_t hi) {
-        return run_device_range(topo, device, lo, hi, vars, param, free_out, reports);
-    });
+    return solve_sharded(topo, n, vars, param, free_out, reports, n_gpus, 0);
 }
 
 // ---- single system with a cached topology (any path) --------------------------------------------------
@@ -1533,25 +1626,21 @@ static int hetero_solve(int device, const std::vector<fk_topology*>& topos32, co
     return FK_OK;
 }
 
-int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems, double* const* free_values, fk_report* reports,
-                      int n_gpus) {
-    if (n == 0) return FK_OK;
-    if (!problems || !free_values) return fail(FK_ERR_INVALID, "null argument");
-    if (const int rc = clamp_gpus(n_gpus); rc != FK_OK) return rc;
+// The problems of a batch call, grouped by structure: one topology per group, from the cache or analysed on host threads.
+struct BatchGroup {
+    uint64_t sig = 0;
+    std::shared_ptr<fk_topology> topo;
+    std::vector<uint32_t> members;
+    int rc = FK_OK;
+    std::string err;
+    // staging of the group's uniform batch
+    std::vector<double> vars, param, out;
+    std::vector<fk_report> reps;
+    int device = 0;
+    bool done = false;  // solved by the heterogeneous launch
+};
+static int group_by_topology(uint32_t n, const fk_problem* const* problems, double* const* free_values, std::vector<BatchGroup>& groups) {
     // ---- group the problems by topology -----------------------------------------------------------------
-    struct Group {
-        uint64_t sig = 0;
-        std::shared_ptr<fk_topology> topo;
-        std::vector<uint32_t> members;
-        int rc = FK_OK;
-        std::string err;
-        // staging of the group's uniform batch
-        std::vector<double> vars, param, out;
-        std::vector<fk_report> reps;
-        int device = 0;
-        bool done = false;  // solved by the heterogeneous launch
-    };
-    std::vector<Group> groups;
     std::multimap<uint64_t, size_t> by_sig;
     for (uint32_t i = 0; i < n; i++) {
         const fk_problem* p = problems[i];
@@ -1601,6 +1690,40 @@ int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems, double* con
             cache_insert(groups[g].sig, groups[g].topo);
         }
     }
+    return FK_OK;
+}
+
+// The group's members as one uniform batch (their free values written into their variable rows; no parameters: zeros).
+static void stage_group(BatchGroup& gr, const fk_problem* const* problems, double* const* free_values) {
+    const fk::Topology& t = gr.topo->t;
+    const size_t cnt = gr.members.size();
+    gr.vars.resize(cnt * t.n_vars); gr.param.resize(cnt * std::max<uint32_t>(t.n_expr, 1)); gr.out.resize(cnt * std::max<uint32_t>(t.n_free, 1));
+    gr.reps.resize(cnt);
+    for (size_t k = 0; k < cnt; k++) {
+        const fk_problem* p = problems[gr.members[k]];
+        if (t.n_vars) std::memcpy(&gr.vars[k * t.n_vars], p->vars, sizeof(double) * t.n_vars);
+        for (uint32_t f = 0; f < t.n_free; f++) gr.vars[k * t.n_vars + t.free_vars[f]] = free_values[gr.members[k]][f];
+        if (t.n_expr) {
+            if (p->param) std::memcpy(&gr.param[k * t.n_expr], p->param, sizeof(double) * t.n_expr);
+            else std::fill(gr.param.begin() + k * t.n_expr, gr.param.begin() + (k + 1) * t.n_expr, 0.0);
+        }
+    }
+}
+static void unstage_group(const BatchGroup& gr, double* const* free_values, fk_report* reports) {
+    const fk::Topology& t = gr.topo->t;
+    for (size_t k = 0; k < gr.members.size(); k++) {
+        std::memcpy(free_values[gr.members[k]], &gr.out[k * t.n_free], sizeof(double) * t.n_free);
+        if (reports) reports[gr.members[k]] = gr.reps[k];
+    }
+}
+
+int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems, double* const* free_values, fk_report* reports,
+                      int n_gpus) {
+    if (n == 0) return FK_OK;
+    if (!problems || !free_values) return fail(FK_ERR_INVALID, "null argument");
+    if (const int rc = clamp_gpus(n_gpus); rc != FK_OK) return rc;
+    std::vector<BatchGroup> groups;
+    if (const int rc = group_by_topology(n, problems, free_values, groups); rc != FK_OK) return rc;
     int cur = 0;
     if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
     // ---- solve.  With several devices and at least as many groups, whole groups go to devices round robin; otherwise
@@ -1625,7 +1748,7 @@ int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems, double* con
             std::vector<fk_topology*> topos32;
             std::vector<HeteroItem> items;
             for (size_t q = 0; q < small.size(); q++) {
-                Group& gr = groups[small[q]];
+                BatchGroup& gr = groups[small[q]];
                 fk_topology* t32 = gr.topo->lanes32();
                 if (t32->t.tile != 32) continue;  // no 32-lane tables (FK_NO_LATENCY_TWIN): the group keeps the uniform kernel
                 for (uint32_t i : gr.members) items.push_back({(uint32_t)topos32.size(), i});
@@ -1643,25 +1766,12 @@ int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems, double* con
             }
         }
     }
-    for (Group& gr : groups) {
-        if (gr.done) continue;
-        const fk::Topology& t = gr.topo->t;
-        const size_t cnt = gr.members.size();
-        if (t.path == 2) continue;  // large systems below
-        gr.vars.resize(cnt * t.n_vars); gr.param.resize(cnt * std::max<uint32_t>(t.n_expr, 1)); gr.out.resize(cnt * std::max<uint32_t>(t.n_free, 1));
-        gr.reps.resize(cnt);
-        for (size_t k = 0; k < cnt; k++) {
-            const fk_problem* p = problems[gr.members[k]];
-            if (t.n_vars) std::memcpy(&gr.vars[k * t.n_vars], p->vars, sizeof(double) * t.n_vars);
-            for (uint32_t f = 0; f < t.n_free; f++) gr.vars[k * t.n_vars + t.free_vars[f]] = free_values[gr.members[k]][f];
-            if (t.n_expr) {
-                if (p->param) std::memcpy(&gr.param[k * t.n_expr], p->param, sizeof(double) * t.n_expr);
-                else std::fill(gr.param.begin() + k * t.n_expr, gr.param.begin() + (k + 1) * t.n_expr, 0.0);
-            }
-        }
+    for (BatchGroup& gr : groups) {
+        if (gr.done || gr.topo->t.path == 2) continue;  // (large systems below)
+        stage_group(gr, problems, free_values);
         gr.device = groups_to_devices ? (int)(rr++ % (size_t)n_gpus) : cur;
     }
-    for (Group& gr : groups) {
+    for (BatchGroup& gr : groups) {
         if (gr.done) continue;
         const fk::Topology& t = gr.topo->t;
         const size_t cnt = gr.members.size();
@@ -1673,15 +1783,48 @@ int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems, double* con
         }
         const int rc = groups_to_devices || n_gpus == 1 || small_fits(t, (uint32_t)cnt)
             ? run_device_range(gr.topo.get(), gr.device, 0, (uint32_t)cnt, gr.vars.data(), gr.param.data(), gr.out.data(), gr.reps.data())
-            : fk_batch_solve(gr.topo.get(), (uint32_t)cnt, gr.vars.data(), gr.param.data(), gr.out.data(), gr.reps.data(), n_gpus);
+            : solve_sharded(gr.topo.get(), (uint32_t)cnt, gr.vars.data(), gr.param.data(), gr.out.data(), gr.reps.data(), n_gpus, 0);
         if (rc != FK_OK) { note(rc); continue; }
-        for (size_t k = 0; k < cnt; k++) {
-            std::memcpy(free_values[gr.members[k]], &gr.out[k * t.n_free], sizeof(double) * t.n_free);
-            if (reports) reports[gr.members[k]] = gr.reps[k];
-        }
+        unstage_group(gr, free_values, reports);
     }
     if (cudaSetDevice(cur) != cudaSuccess) cudaGetLastError();
     return first_rc == FK_OK ? FK_OK : fail(first_rc, first_err);
+}
+
+int fk_lbfgs_solve_batch(uint32_t n, const fk_problem* const* problems, double* const* free_values, fk_report* reports, int n_gpus) {
+    if (n == 0) return FK_OK;
+    if (!problems || !free_values) return fail(FK_ERR_INVALID, "null argument");
+    if (const int rc = clamp_gpus(n_gpus); rc != FK_OK) return rc;
+    std::vector<BatchGroup> groups;
+    if (const int rc = group_by_topology(n, problems, free_values, groups); rc != FK_OK) return rc;
+    int cur = 0;
+    if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
+    // With several devices and at least as many groups, whole groups go to devices round robin; otherwise every large group
+    // is sharded by sketch over the devices.
+    const bool groups_to_devices = n_gpus > 1 && groups.size() >= (size_t)n_gpus;
+    size_t rr = 0;
+    int first_rc = FK_OK;
+    std::string first_err;
+    for (BatchGroup& gr : groups) {
+        stage_group(gr, problems, free_values);
+        gr.device = groups_to_devices ? (int)(rr++ % (size_t)n_gpus) : cur;
+        const uint32_t cnt = (uint32_t)gr.members.size();
+        const int rc = groups_to_devices || n_gpus == 1 || small_fits(gr.topo->t, cnt)
+            ? run_device_range(gr.topo.get(), gr.device, 0, cnt, gr.vars.data(), gr.param.data(), gr.out.data(), gr.reps.data(), 1)
+            : solve_sharded(gr.topo.get(), cnt, gr.vars.data(), gr.param.data(), gr.out.data(), gr.reps.data(), n_gpus, 1);
+        if (rc == FK_OK) unstage_group(gr, free_values, reports);
+        else if (first_rc == FK_OK) { first_rc = rc; first_err = g_error; }
+        std::vector<double>().swap(gr.vars);  // (large systems: one group's staging at a time)
+        std::vector<double>().swap(gr.out);
+    }
+    if (cudaSetDevice(cur) != cudaSuccess) cudaGetLastError();
+    return first_rc == FK_OK ? FK_OK : fail(first_rc, first_err);
+}
+
+int fk_lbfgs_solve(const fk_problem* problem, double* free_values, fk_report* report) {
+    const fk_problem* ps[1] = {problem};
+    double* fv[1] = {free_values};
+    return fk_lbfgs_solve_batch(1, ps, fv, report, 1);
 }
 
 int fk_lm_solve(const fk_problem* problem, double* free_values, fk_report* report) {

@@ -15,12 +15,11 @@
 #include <cstdlib>
 
 #include "expressions.cuh"
+#include "lbfgs_core.cuh"
 #include "lm_kernels.cuh"
 #include "lm_sketch.cuh"
 
 namespace fk {
-
-constexpr uint32_t kNop = 0xFFFFFFFFu;
 
 template <int TILE>
 struct TileOps {
@@ -717,42 +716,9 @@ int launch_batch_analyze(uint32_t n_vars, uint32_t n_expr, const uint8_t* kinds,
 }
 
 // ---- L-BFGS (SURVEY 8f-3): fiksi/src/solve/lbfgs.rs on one tile per sketch -------------------------------
-// Same tile layout as the LM kernel (TILE lanes per sketch, state in shared memory), the reference's
-// control flow line by line: two-loop recursion with a history of 5 (lbfgs.rs:77-143), Hager-Zhang
-// line search (mod hager_zhang, :218-506) and the three exits (:53-56, :177-182).  Every scalar that
-// steers the control flow (dot products, sums of squares) is accumulated sequentially in index order
-// by every lane, exactly as the reference's iterator sums do, so the decisions are the oracle's.
-// The dense row-major Jacobian of the reference is kept in its sparse CSC form; the dense path's
-// "assign per slot" rule (expressions.rs:1003-1007) is honoured by eval_row_assign.
-struct LbfgsTables {
-    const uint32_t* jcolptr;  // [n+1] CSC of the Jacobian without damping rows
-    const uint32_t* jrow;     // [jnnz]
-};
-
-template <int KIND>
-__device__ __forceinline__ void eval_row_assign(const DevProgram& P, uint32_t row, const double* xfree, const double* __restrict__ vars,
-                                                const double* __restrict__ params, double* rdst, double* jdst) {
-    const uint32_t hdr = __ldg(P.row_hdr + row);
-    if (hdr == kNop) return;
-    const int kind = KIND >= 0 ? KIND : (int)(hdr & 0xFFu);
-    const int a = dev::arity_of(kind);
-    uint2 sl[8];
-    double v[8], g[8];
-#pragma unroll
-    for (int s = 0; s < 8; s++) {
-        v[s] = 0.0;
-        sl[s] = make_uint2(kNop, kNop);
-        if (s < a) {
-            sl[s] = __ldg(P.row_slots + row * 8 + s);
-            v[s] = (int32_t)sl[s].x >= 0 ? xfree[sl[s].x] : __ldg(vars + (sl[s].x & 0x7FFFFFFFu));
-        }
-    }
-    rdst[row] = dev::eval_expression(kind, v, __ldg(params + (hdr >> 8)), g);
-#pragma unroll
-    for (int s = 0; s < 8; s++)
-        if (s < a && sl[s].y != kNop) jdst[sl[s].y & 0xFFFFFFu] = g[s];  // assignment: the later slot wins
-}
-
+// Same tile layout as the LM kernel (TILE lanes per sketch, state in shared memory); the control flow is
+// lbfgs_solve (lbfgs_core.cuh).  Every lane computes each sequential sum itself, which keeps the control flow
+// uniform across the tile without a broadcast.
 __device__ __forceinline__ double dot_seq(const double* a, const double* b, uint32_t n) {
     double s = 0.0;
 #pragma unroll 4
@@ -760,7 +726,34 @@ __device__ __forceinline__ double dot_seq(const double* a, const double* b, uint
     return s;
 }
 
-struct HzParam { double p, phi, dphi; };
+template <int TILE, int KIND>
+struct TileLbfgsOps {
+    const DevProgram& P;
+    const LbfgsTables& T;
+    const double* vars;
+    const double* params;
+    int lane;
+    unsigned msk;
+    __device__ void sync() const { if (TILE > 1) TileOps<TILE>::sync(msk); }
+    __device__ bool leader() const { return lane == 0; }
+    template <class F>
+    __device__ void each(uint32_t cnt, F f) const {
+        for (uint32_t i = lane; i < cnt; i += TILE) f(i);
+    }
+    __device__ double dot(const double* a, const double* b, uint32_t k) const { return dot_seq(a, b, k); }
+    __device__ void dot2(const double* a1, const double* b1, uint32_t k1, const double* a2, const double* b2, uint32_t k2, double* o1,
+                         double* o2) const {
+        *o1 = dot_seq(a1, b1, k1);
+        *o2 = dot_seq(a2, b2, k2);
+    }
+    // residuals + Jacobian + gradient at `pt` (== Eval::calculate_phi without the phi / dphi sums)
+    __device__ void evaluate(const double* pt, const LbfgsVecs& s) const {
+        for (uint32_t rd = 0; rd < P.eval_rounds; rd++) eval_row_assign<KIND>(P, rd * TILE + lane, pt, vars, params, s.r, s.J);
+        sync();
+        for (uint32_t c = lane; c < P.n; c += TILE) s.g[c] = lbfgs_grad_col(T, s.J, s.r, c);
+        sync();
+    }
+};
 
 template <int TILE, int KIND>
 __global__ void __launch_bounds__(128)
@@ -773,217 +766,49 @@ fk_batch_lbfgs_kernel(const DevProgram P, const LbfgsTables T, uint32_t n_sketch
     const int lane = threadIdx.x % TILE;
     const uint32_t sketch = blockIdx.x * tiles_per_cta + tile_id;
     if (sketch >= n_sketches) return;
-    const unsigned msk = TileOps<TILE>::mask();
     const uint32_t n = P.n, m = P.m;
-    double* x = smem + (size_t)tile_id * stride_doubles;
-    double* xs = x + n;
-    double* g = xs + n;
-    double* dir = g + n;
-    double* sh = dir + n;        // [5][n]
-    double* yh = sh + 5 * n;     // [5][n]
-    double* r = yh + 5 * n;      // [m]
-    double* J = r + m;           // [jnnz]
-    double* rho = J + P.jnnz;    // [5]
-    double* alpha = rho + 5;     // [5]
+    LbfgsVecs s;
+    s.x = smem + (size_t)tile_id * stride_doubles;
+    s.xs = s.x + n;
+    s.g = s.xs + n;
+    s.dir = s.g + n;
+    s.sh = s.dir + n;        // [5][n]
+    s.yh = s.sh + 5 * n;     // [5][n]
+    s.r = s.yh + 5 * n;      // [m]
+    s.J = s.r + m;           // [jnnz]
+    s.rho = s.J + P.jnnz;    // [5]
+    s.alpha = s.rho + 5;     // [5]
     const double* vars = vars_all + (size_t)sketch * P.n_vars;
-    const double* params = params_all + (size_t)sketch * P.n_expr;
-    auto sync = [&] { if (TILE > 1) TileOps<TILE>::sync(msk); };
+    TileLbfgsOps<TILE, KIND> ops{P, T, vars, params_all + (size_t)sketch * P.n_expr, lane, TileOps<TILE>::mask()};
+    lbfgs_solve(ops, P, vars, s, free_out + (size_t)sketch * n, reports + sketch);
+}
 
-    uint32_t evaluations = 0;
-    // residuals + Jacobian + gradient at `pt` (== Eval::calculate_phi without the phi / dphi sums)
-    auto evaluate = [&](const double* pt) {
-        for (uint32_t rd = 0; rd < P.eval_rounds; rd++) eval_row_assign<KIND>(P, rd * TILE + lane, pt, vars, params, r, J);
-        sync();
-        for (uint32_t c = lane; c < n; c += TILE) {  // lbfgs.rs:201-212: rows ascending, from 0.0
-            double acc = 0.0;
-            for (uint32_t q = __ldg(T.jcolptr + c); q < __ldg(T.jcolptr + c + 1); q++) acc += J[q] * r[__ldg(T.jrow + q)];
-            g[c] = acc;
-        }
-        sync();
-        evaluations++;
-    };
+// Shared memory of one CTA of the tile kernel, and how many sketches it holds; 0 when the topology does not take the
+// tile kernel (lanes other than 4 / 8 / 16 / 32, or the state of a warp's sketches above 220 KiB).
+static size_t lbfgs_tile_smem(uint32_t n, uint32_t m, uint32_t jnnz, uint32_t tile, int* tiles_per_cta) {
+    if (tile != 4 && tile != 8 && tile != 16 && tile != 32) return 0;
+    const uint32_t stride = lbfgs_smem_doubles(n, m, jnnz) | 1u;
+    const size_t bytes_per_sketch = (size_t)stride * sizeof(double);
+    const int tiles_per_warp = 32 / (int)tile;
+    int warps = 4;
+    while (warps > 1 && bytes_per_sketch * tiles_per_warp * warps > 72 * 1024) warps >>= 1;
+    *tiles_per_cta = tiles_per_warp * warps;
+    const size_t smem = bytes_per_sketch * *tiles_per_cta;
+    return smem > 220 * 1024 ? 0 : smem;
+}
 
-    for (uint32_t i = lane; i < n; i += TILE) x[i] = __ldg(vars + __ldg(P.free_vars + i));
-    for (uint32_t i = lane; i < P.jnnz; i += TILE) J[i] = 0.0;
-    // The histories start as zeros (lbfgs.rs:66-72) and the reference READS not-yet-written slots during
-    // the first five iterations (slot (k + i) % 5 for i < min(k, 5), :84-85): they must be zero here too.
-    for (uint32_t i = lane; i < 10 * n; i += TILE) sh[i] = 0.0;  // sh and yh are contiguous
-    for (uint32_t i = lane; i < 10; i += TILE) rho[i] = 0.0;     // rho and alpha are contiguous
-    sync();
-    evaluate(x);
-    double prev = sum_squares_seq(r, m);
-    uint32_t exit_reason = 3, iterations = 0;
-    uint64_t trace = 0;
-    double last_step = 0.0, ssr = prev;
-    bool run = !(prev < 1e-4);
-    if (!run) exit_reason = 0;
-
-    for (uint32_t k = 0; run && k < 100; k++) {
-        const uint32_t hl = k < 5 ? k : 5;
-        for (uint32_t j = lane; j < n; j += TILE) dir[j] = g[j];
-        sync();
-        for (uint32_t ii = hl; ii-- > 0;) {  // lbfgs.rs:83-99
-            const uint32_t h = (k + ii) % 5;
-            const double a_i = rho[h] * dot_seq(sh + h * n, dir, n);
-            sync();
-            if (lane == 0) alpha[ii] = a_i;
-            for (uint32_t j = lane; j < n; j += TILE) dir[j] -= a_i * yh[h * n + j];
-            sync();
-        }
-        if (k > 0) {  // :101-121
-            const uint32_t hp = (k - 1) % 5;
-            const double sdy = dot_seq(sh + hp * n, yh + hp * n, n), ydy = dot_seq(yh + hp * n, yh + hp * n, n);
-            if (ydy > 0.0) {
-                const double scale = sdy / ydy;
-                sync();
-                for (uint32_t j = lane; j < n; j += TILE) dir[j] *= scale;
-                sync();
-            }
-        }
-        for (uint32_t ii = 0; ii < hl; ii++) {  // :123-139
-            const uint32_t h = (k + ii) % 5;
-            const double beta = rho[h] * dot_seq(yh + h * n, dir, n);
-            const double coef = alpha[ii] - beta;
-            sync();
-            for (uint32_t j = lane; j < n; j += TILE) dir[j] += sh[h * n + j] * coef;
-            sync();
-        }
-        const uint32_t h = k % 5;
-        for (uint32_t j = lane; j < n; j += TILE) {
-            dir[j] *= -1.0;          // :141-143
-            yh[h * n + j] = g[j];    // :149-150
-            xs[j] = x[j];
-        }
-        sync();
-
-        // ---- hager_zhang::line_search (:461-506) --------------------------------------------------------
-        const double phi0 = prev, dphi0 = dot_seq(g, dir, n);
-        const uint32_t evals_before = evaluations;
-        bool guard = false;
-        auto calculate_phi = [&](double p) -> HzParam {  // :270-286
-            sync();
-            for (uint32_t j = lane; j < n; j += TILE) xs[j] = x[j] + p * dir[j];
-            sync();
-            evaluate(xs);
-            HzParam out;
-            out.p = p;
-            out.phi = sum_squares_seq(r, m);
-            out.dphi = dot_seq(g, dir, n);
-#ifdef FK_LBFGS_DEBUG
-            if (sketch == 0 && lane == 0) printf("gpu k=%u p=%a phi=%a dphi=%a\n", k, p, out.phi, out.dphi);
-#endif
-            return out;
-        };
-        auto secant = [](HzParam a, HzParam b) { return (a.p * b.dphi - b.p * a.dphi) / (b.dphi - a.dphi); };
-        auto wolfe = [&](HzParam c) {  // :307-322
-            if ((c.phi <= phi0 + c.p * (1e-4 * dphi0)) && (c.dphi >= 0.9 * dphi0)) return true;
-            if (c.phi <= phi0 + 1e-6 && (2.0 * 1e-4 - 1.0) * dphi0 >= c.dphi && c.dphi >= 0.9 * dphi0) return true;
-            return false;
-        };
-        auto update = [&](HzParam a, HzParam b, HzParam c, HzParam& oa, HzParam& ob) {  // :325-353
-            if (c.p < a.p || c.p > b.p) { oa = a; ob = b; return; }
-            if (c.dphi >= 0.0) { oa = a; ob = c; return; }
-            if (c.phi <= phi0 + 1e-6) { oa = c; ob = b; return; }
-            HzParam aa = a, bb = c;
-            for (int it = 0;; it++) {
-                if (it >= 200) { guard = true; oa = aa; ob = bb; return; }
-                const HzParam d = calculate_phi((1.0 - 0.5) * aa.p + 0.5 * bb.p);
-                if (d.dphi >= 0.0) { oa = aa; ob = d; return; }
-                else if (d.phi <= phi0 + 1e-6) aa = d;
-                else bb = d;
-            }
-        };
-        HzParam res = calculate_phi(1.0);  // :447-452
-        if (!wolfe(res)) {
-            HzParam a{0.0, phi0, dphi0};
-            HzParam b = calculate_phi(5.0);  // bracket, :401-410
-            HzParam c = res;
-            bool found = false;
-            for (int it = 0; it < 100 && !found && !guard; it++) {  // search, :414-443
-                // secant2, :360-398
-                HzParam a_, b_;
-                bool have = false;
-                HzParam cc = calculate_phi(secant(a, b));
-                if (wolfe(cc)) { res = cc; found = true; break; }
-                update(a, b, cc, a_, b_);
-                if (guard) break;
-                if (cc.p == b_.p) {
-                    const HzParam c2 = calculate_phi(secant(b, b_));
-                    if (wolfe(c2)) { res = c2; found = true; break; }
-                    HzParam na, nb;
-                    update(a_, b_, c2, na, nb);
-                    a_ = na; b_ = nb;
-                    have = true;
-                } else if (cc.p == a_.p) {
-                    const HzParam c2 = calculate_phi(secant(a, a_));
-                    if (wolfe(c2)) { res = c2; found = true; break; }
-                    HzParam na, nb;
-                    update(a_, b_, c2, na, nb);
-                    a_ = na; b_ = nb;
-                    have = true;
-                }
-                (void)have;
-                if (guard) break;
-                if (b_.p - a_.p > 0.66 * (b.p - a.p)) {
-                    c = calculate_phi(0.5 * (a.p + b.p));
-                    if (wolfe(c)) { res = c; found = true; break; }
-                    HzParam na, nb;
-                    update(a, b, c, na, nb);
-                    a = na; b = nb;
-                } else {
-                    a = a_; b = b_;
-                }
-            }
-            if (!found) res = calculate_phi(c.p);  // :440-442
-        }
-        sync();
-        for (uint32_t j = lane; j < n; j += TILE) x[j] = xs[j];  // :169
-        iterations++;
-        trace = trace * 31ull + (uint64_t)(evaluations - evals_before);
-        last_step = res.p;
-        ssr = res.phi;
-        if (guard) { exit_reason = 4; break; }
-        for (uint32_t j = lane; j < n; j += TILE) {  // :171-180
-            const double sv = res.p * dir[j];
-            sh[h * n + j] = sv;
-            yh[h * n + j] = g[j] - yh[h * n + j];
-        }
-        sync();
-        const double sdy = dot_seq(sh + h * n, yh + h * n, n);
-        if (lane == 0) rho[h] = 1.0 / sdy;
-        sync();
-        if (fabs(prev - res.phi) < 1e-10) { exit_reason = 1; break; }
-        if (res.phi < 1e-6) { exit_reason = 2; break; }
-        prev = res.phi;
-    }
-
-    sync();
-    double* out = free_out + (size_t)sketch * n;
-    for (uint32_t i = lane; i < n; i += TILE) out[i] = x[i];
-    if (lane == 0) {
-        fk_report rep;
-        rep.exit_reason = exit_reason;
-        rep.outer_iters = iterations;
-        rep.factorizations = evaluations;
-        rep.accepted = iterations;
-        rep.ssr = ssr;
-        rep.lambda = last_step;
-        rep.trace_hash = trace;
-        reports[sketch] = rep;
-    }
+bool batch_lbfgs_tile_fits(uint32_t n, uint32_t m, uint32_t jnnz, uint32_t tile) {
+    int tiles_per_cta = 0;
+    return lbfgs_tile_smem(n, m, jnnz, tile, &tiles_per_cta) != 0;
 }
 
 template <int TILE, int KIND>
 static int launch_lbfgs_t(const DevProgram& prog, const LbfgsTables& T, uint32_t n_sketches, const double* vars, const double* params,
                           double* free_out, fk_report* reports, cudaStream_t stream) {
+    int tiles_per_cta = 0;
+    const size_t smem = lbfgs_tile_smem(prog.n, prog.m, prog.jnnz, TILE, &tiles_per_cta);
+    if (smem == 0) return (int)cudaErrorInvalidConfiguration;
     const uint32_t stride = lbfgs_smem_doubles(prog.n, prog.m, prog.jnnz) | 1u;
-    const size_t bytes_per_sketch = (size_t)stride * sizeof(double);
-    const int tiles_per_warp = 32 / TILE;
-    int warps = 4;
-    while (warps > 1 && bytes_per_sketch * tiles_per_warp * warps > 72 * 1024) warps >>= 1;
-    const int tiles_per_cta = tiles_per_warp * warps;
-    const size_t smem = bytes_per_sketch * tiles_per_cta;
-    if (smem > 220 * 1024) return (int)cudaErrorInvalidConfiguration;
     cudaError_t e = cudaFuncSetAttribute(fk_batch_lbfgs_kernel<TILE, KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     const uint32_t grid = (n_sketches + tiles_per_cta - 1) / tiles_per_cta;

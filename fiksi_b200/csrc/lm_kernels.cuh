@@ -72,8 +72,10 @@ size_t batch_analyze_warp_bytes(uint32_t n_vars, uint32_t n_expr);
 bool batch_analyze_warp_fits(uint32_t n_vars, uint32_t n_expr);
 int launch_batch_analyze(uint32_t n_vars, uint32_t n_expr, const uint8_t* kinds, const uint32_t* slot_var, uint32_t n_sketches,
                          const double* vars, const double* params, uint8_t* out, void* stream);
-// L-BFGS on a uniform batch (tile paths with 8 / 16 / 32 lanes only); d_jcolptr[n+1], d_jrow[jnnz]: CSC
+// L-BFGS on a uniform batch (tile paths with 4 / 8 / 16 / 32 lanes only); d_jcolptr[n+1], d_jrow[jnnz]: CSC
 // of the Jacobian.  Returns cudaErrorInvalidConfiguration when the topology does not take a tile path.
+// batch_lbfgs_tile_fits: whether it takes a topology with these sizes and lanes (host only).
+bool batch_lbfgs_tile_fits(uint32_t n, uint32_t m, uint32_t jnnz, uint32_t tile);
 int launch_batch_lbfgs(const DevProgram& prog, const uint32_t* d_jcolptr, const uint32_t* d_jrow, uint32_t n_sketches, const double* vars,
                        const double* params, double* free_out, fk_report* reports, void* stream);
 // SinglePass (fiksi/src/assemble/mod.rs:201-208): writes the solved free values of one set back into the

@@ -251,134 +251,13 @@ int fk_system_set_parameter(fk_system* s, uint32_t constraint, double value) {
     return FK_OK;
 }
 
-// == System::solve(SolvingOptions { optimizer: LevenbergMarquardt, decomposer: None, perturb })
-// (lib.rs:464, assemble/mod.rs:46-167).  reports: one per solved component in component order, up
-// to `cap`; *n_solved receives the number of components solved.
-int fk_system_solve(fk_system* s, int perturb, fk_report* reports, uint32_t cap, uint32_t* n_solved) {
-    if (!s) return FK_ERR_INVALID;
-    if (n_solved) *n_solved = 0;
-    const size_t nv = s->vars.size();
-    // assemble/mod.rs:32-44,58-79: RMS of all variables and of the distance parameters (sequential sums)
-    double sum = 0.0;
-    size_t cnt = 0;
-    for (double v : s->vars) { sum += v * v; cnt++; }
-    for (size_t e = 0; e < s->kind.size(); e++)
-        if (s->kind[e] == FK_POINT_POINT_DISTANCE || s->kind[e] == FK_POINT_LINE_DISTANCE) { sum += s->param[e] * s->param[e]; cnt++; }
-    const double scale = std::sqrt(sum / (double)cnt);
-    const double recip = 1.0 / scale;
-    std::vector<double> vt(nv);
-    for (size_t i = 0; i < nv; i++) vt[i] = s->vars[i] * recip;
-    std::vector<double> pt(s->param);
-    for (size_t e = 0; e < pt.size(); e++)
-        if (s->kind[e] == FK_POINT_POINT_DISTANCE || s->kind[e] == FK_POINT_LINE_DISTANCE) pt[e] = recip * s->param[e];
+}  // extern "C"
 
-    // One compact problem per non-empty component: the referenced variables are renumbered
-    // locally (ascending, so x/y of a point stay adjacent), which also lets components of the same
-    // shape share one topology inside fk_lm_solve_batch.
-    struct Local {
-        std::vector<double> vars, param, x;
-        std::vector<uint8_t> kind;
-        std::vector<uint32_t> idx, free_local, rows, free_global;
-        fk_problem prob;
-    };
-    std::vector<std::unique_ptr<Local>> locals;
-    Lcg rng{42};  // assemble/mod.rs:47: one generator per solve, consumed by the components in order
-    for (const fk_system::Comp& c : s->comps) {
-        if (c.elements.empty()) continue;  // assemble/mod.rs:87-89
-        std::set<uint32_t> free_set;
-        for (uint32_t e : c.elements) {
-            uint32_t v[4];
-            int n = s->element_vars(e, v);
-            for (int k = 0; k < n; k++)
-                if (!s->fixed[v[k]]) free_set.insert(v[k]);
-        }
-        if (perturb) {  // assemble/mod.rs:113-124
-            for (uint32_t fv : free_set) {
-                const double r1 = rng.next();
-                const double r2 = rng.next();
-                vt[fv] += vt[fv] * (1.0 / 8196.0) * r1 + (1.0 / 65568.0) * r2;
-            }
-        }
-        std::unique_ptr<Local> L(new Local());
-        std::vector<uint32_t> exprs;
-        for (uint32_t ci : c.constraints)
-            for (uint8_t k = 0; k < s->constrs[ci].n_expr; k++) exprs.push_back(s->constrs[ci].first_expr + k);
-        std::set<uint32_t> used(free_set.begin(), free_set.end());
-        for (uint32_t e : exprs) {
-            uint32_t sv[8];
-            int a = fk::expand_slots(s->kind[e], &s->idx[4 * (size_t)e], sv);
-            for (int k = 0; k < a; k++) used.insert(sv[k]);
-        }
-        std::map<uint32_t, uint32_t> local;
-        for (uint32_t g : used) {
-            local.emplace(g, (uint32_t)L->vars.size());
-            L->vars.push_back(vt[g]);  // values as of now: later components have not been perturbed yet
-        }
-        for (uint32_t g : free_set) {
-            L->free_global.push_back(g);
-            L->free_local.push_back(local[g]);
-            L->x.push_back(vt[g]);
-        }
-        static const int stored[FK_NUM_KINDS] = {2, 2, 3, 3, 3, 3, 4, 4, 4, 4, 4, 3, 3};
-        for (uint32_t e : exprs) {
-            L->rows.push_back((uint32_t)L->kind.size());
-            L->kind.push_back(s->kind[e]);
-            L->param.push_back(pt[e]);
-            for (int q = 0; q < 4; q++) L->idx.push_back(q < stored[s->kind[e]] ? local[s->idx[4 * (size_t)e + q]] : 0);
-        }
-        fk_problem& p = L->prob;
-        p.n_vars = (uint32_t)L->vars.size(); p.vars = L->vars.data();
-        p.n_expr = (uint32_t)L->kind.size(); p.kind = L->kind.data(); p.idx = L->idx.data(); p.param = L->param.data();
-        p.n_free = (uint32_t)L->free_local.size(); p.free_vars = L->free_local.data();
-        p.n_rows = (uint32_t)L->rows.size(); p.rows = L->rows.data();
-        locals.push_back(std::move(L));
-    }
-    if (locals.empty()) return FK_OK;
-    std::vector<const fk_problem*> probs;
-    std::vector<double*> xs;
-    for (auto& L : locals) {
-        probs.push_back(&L->prob);
-        xs.push_back(L->x.data());
-    }
-    std::vector<fk_report> reps(locals.size());
-    int rc = fk_lm_solve_batch((uint32_t)locals.size(), probs.data(), xs.data(), reps.data(), 1);
-    if (rc != FK_OK) return rc;
-    // assemble/mod.rs:161-166
-    for (auto& L : locals)
-        for (size_t k = 0; k < L->free_global.size(); k++) s->vars[L->free_global[k]] = scale * L->x[k];
-    for (size_t k = 0; k < locals.size() && reports && k < cap; k++) reports[k] = reps[k];
-    if (n_solved) *n_solved = (uint32_t)locals.size();
-    return FK_OK;
-}
-
-// ---- Decomposer::SinglePass (SURVEY 8f-1) ------------------------------------------------------------
 namespace {
 
-// The equation graph of lib.rs:262,395,434.
-void equation_graph(const fk_system* s, std::vector<std::vector<uint32_t>>& var_exprs, std::vector<std::vector<uint32_t>>& expr_vars) {
-    var_exprs.assign(s->vars.size(), {});
-    expr_vars.assign(s->kind.size(), {});
-    for (uint32_t e = 0; e < s->kind.size(); e++) {
-        uint32_t sv[8];
-        const int a = fk::expand_slots(s->kind[e], &s->idx[4 * (size_t)e], sv);
-        expr_vars[e].assign(sv, sv + a);
-        for (int k = 0; k < a; k++) var_exprs[sv[k]].push_back(e);
-    }
-}
-
-std::vector<uint32_t> component_free_variables(const fk_system* s, const fk_system::Comp& c) {
-    std::set<uint32_t> free_set;
-    for (uint32_t e : c.elements) {
-        uint32_t v[4];
-        const int n = s->element_vars(e, v);
-        for (int k = 0; k < n; k++)
-            if (!s->fixed[v[k]]) free_set.insert(v[k]);
-    }
-    return std::vector<uint32_t>(free_set.begin(), free_set.end());
-}
-
 // One compact fk_problem: `free_sorted` free, `exprs` as rows (in that order), every other referenced
-// variable fixed at its current value in `vt`.
+// variable fixed at its current value in `vt`.  Referenced variables are renumbered ascending, so x/y of a point
+// stay adjacent, and sub-problems of the same shape share one topology inside the batch calls.
 struct LocalProblem {
     std::vector<double> vars, param, x;
     std::vector<uint8_t> kind;
@@ -415,6 +294,119 @@ void build_local(const fk_system* s, const std::vector<double>& vt, const std::v
     p.n_expr = (uint32_t)L.kind.size(); p.kind = L.kind.data(); p.idx = L.idx.data(); p.param = L.param.data();
     p.n_free = (uint32_t)L.free_local.size(); p.free_vars = L.free_local.data();
     p.n_rows = (uint32_t)L.rows.size(); p.rows = L.rows.data();
+}
+
+struct PreparedSystem {
+    double scale = 1.0;
+    std::vector<std::unique_ptr<LocalProblem>> locals;  // one per non-empty component, in component order
+};
+
+// assemble/mod.rs:32-124: scale, seeded perturbation and the per-component problems.
+void prepare_components(const fk_system* s, int perturb, PreparedSystem& out) {
+    const size_t nv = s->vars.size();
+    // assemble/mod.rs:32-44,58-79: RMS of all variables and of the distance parameters (sequential sums)
+    double sum = 0.0;
+    size_t cnt = 0;
+    for (double v : s->vars) { sum += v * v; cnt++; }
+    for (size_t e = 0; e < s->kind.size(); e++)
+        if (s->kind[e] == FK_POINT_POINT_DISTANCE || s->kind[e] == FK_POINT_LINE_DISTANCE) { sum += s->param[e] * s->param[e]; cnt++; }
+    const double scale = out.scale = std::sqrt(sum / (double)cnt);
+    const double recip = 1.0 / scale;
+    std::vector<double> vt(nv);
+    for (size_t i = 0; i < nv; i++) vt[i] = s->vars[i] * recip;
+    std::vector<double> pt(s->param);
+    for (size_t e = 0; e < pt.size(); e++)
+        if (s->kind[e] == FK_POINT_POINT_DISTANCE || s->kind[e] == FK_POINT_LINE_DISTANCE) pt[e] = recip * s->param[e];
+    Lcg rng{42};  // assemble/mod.rs:47: one generator per solve, consumed by the components in order
+    for (const fk_system::Comp& c : s->comps) {
+        if (c.elements.empty()) continue;  // assemble/mod.rs:87-89
+        std::set<uint32_t> free_set;
+        for (uint32_t e : c.elements) {
+            uint32_t v[4];
+            int n = s->element_vars(e, v);
+            for (int k = 0; k < n; k++)
+                if (!s->fixed[v[k]]) free_set.insert(v[k]);
+        }
+        if (perturb) {  // assemble/mod.rs:113-124
+            for (uint32_t fv : free_set) {
+                const double r1 = rng.next();
+                const double r2 = rng.next();
+                vt[fv] += vt[fv] * (1.0 / 8196.0) * r1 + (1.0 / 65568.0) * r2;
+            }
+        }
+        std::vector<uint32_t> exprs;
+        for (uint32_t ci : c.constraints)
+            for (uint8_t k = 0; k < s->constrs[ci].n_expr; k++) exprs.push_back(s->constrs[ci].first_expr + k);
+        std::unique_ptr<LocalProblem> L(new LocalProblem());
+        // (values as of now: later components have not been perturbed yet)
+        build_local(s, vt, pt, std::vector<uint32_t>(free_set.begin(), free_set.end()), exprs, *L);
+        out.locals.push_back(std::move(L));
+    }
+}
+
+// == System::solve(SolvingOptions { optimizer, decomposer: None, perturb }) (lib.rs:464, assemble/mod.rs:46-167): every
+// component in one batch call of the optimizer (0 LM, 1 L-BFGS, assemble/mod.rs:148-158).
+int solve_components(fk_system* s, int optimizer, int perturb, fk_report* reports, uint32_t cap, uint32_t* n_solved) {
+    if (n_solved) *n_solved = 0;
+    PreparedSystem ps;
+    prepare_components(s, perturb, ps);
+    std::vector<std::unique_ptr<LocalProblem>>& locals = ps.locals;
+    if (locals.empty()) return FK_OK;
+    std::vector<const fk_problem*> probs;
+    std::vector<double*> xs;
+    for (auto& L : locals) {
+        probs.push_back(&L->prob);
+        xs.push_back(L->x.data());
+    }
+    std::vector<fk_report> reps(locals.size());
+    const uint32_t n = (uint32_t)locals.size();
+    int rc = optimizer == 1 ? fk_lbfgs_solve_batch(n, probs.data(), xs.data(), reps.data(), 1)
+                            : fk_lm_solve_batch(n, probs.data(), xs.data(), reps.data(), 1);
+    if (rc != FK_OK) return rc;
+    // assemble/mod.rs:161-166
+    for (auto& L : locals)
+        for (size_t k = 0; k < L->free_global.size(); k++) s->vars[L->free_global[k]] = ps.scale * L->x[k];
+    for (size_t k = 0; k < locals.size() && reports && k < cap; k++) reports[k] = reps[k];
+    if (n_solved) *n_solved = n;
+    return FK_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+// == System::solve(SolvingOptions { optimizer: LevenbergMarquardt, decomposer: None, perturb })
+// (lib.rs:464, assemble/mod.rs:46-167).  reports: one per solved component in component order, up
+// to `cap`; *n_solved receives the number of components solved.
+int fk_system_solve(fk_system* s, int perturb, fk_report* reports, uint32_t cap, uint32_t* n_solved) {
+    if (!s) return FK_ERR_INVALID;
+    return solve_components(s, 0, perturb, reports, cap, n_solved);
+}
+
+// ---- Decomposer::SinglePass (SURVEY 8f-1) ------------------------------------------------------------
+namespace {
+
+// The equation graph of lib.rs:262,395,434.
+void equation_graph(const fk_system* s, std::vector<std::vector<uint32_t>>& var_exprs, std::vector<std::vector<uint32_t>>& expr_vars) {
+    var_exprs.assign(s->vars.size(), {});
+    expr_vars.assign(s->kind.size(), {});
+    for (uint32_t e = 0; e < s->kind.size(); e++) {
+        uint32_t sv[8];
+        const int a = fk::expand_slots(s->kind[e], &s->idx[4 * (size_t)e], sv);
+        expr_vars[e].assign(sv, sv + a);
+        for (int k = 0; k < a; k++) var_exprs[sv[k]].push_back(e);
+    }
+}
+
+std::vector<uint32_t> component_free_variables(const fk_system* s, const fk_system::Comp& c) {
+    std::set<uint32_t> free_set;
+    for (uint32_t e : c.elements) {
+        uint32_t v[4];
+        const int n = s->element_vars(e, v);
+        for (int k = 0; k < n; k++)
+            if (!s->fixed[v[k]]) free_set.insert(v[k]);
+    }
+    return std::vector<uint32_t>(free_set.begin(), free_set.end());
 }
 
 }  // namespace
@@ -702,6 +694,14 @@ int fk_system_solve_opts(fk_system* s, int decomposer, int perturb, fk_report* r
     }
     if (n_solved) *n_solved = solved;
     return FK_OK;
+}
+
+// == System::solve(options).  The reference dispatches on the optimizer only under Decomposer::None (assemble/mod.rs:148-158);
+// SinglePass and RecursiveAssembly call levenberg_marquardt directly (:191, :224) whatever the optimizer.
+int fk_system_solve_options(fk_system* s, const fk_solving_options* opts, fk_report* reports, uint32_t cap, uint32_t* n_solved) {
+    if (!s || !opts || opts->optimizer > 1 || opts->decomposer > 2 || opts->perturb > 1 || opts->pad != 0) return FK_ERR_INVALID;
+    if (opts->optimizer == 1 && opts->decomposer == 0) return solve_components(s, 1, (int)opts->perturb, reports, cap, n_solved);
+    return fk_system_solve_opts(s, (int)opts->decomposer, (int)opts->perturb, reports, cap, n_solved);
 }
 
 // The recombination plan of all components as one stream of 32-bit words (host only, no device): per step

@@ -7,9 +7,10 @@ import ctypes as C
 
 import numpy as np
 
-from ._lib import FkReport, REPORT_DTYPE, check, lib, ptr
+from ._lib import FkReport, FkSolvingOptions, REPORT_DTYPE, check, lib, ptr
 
 _BAD = 0xFFFFFFFF
+_OPTIMIZERS = {"lm": 0, "lbfgs": 1}
 
 
 class System:
@@ -65,29 +66,29 @@ class System:
         v = self.variables
         return float(v[i]), float(v[i + 1])
 
-    def solve(self, perturb=True):
-        """System::solve(SolvingOptions::DEFAULT) (perturb=True) on the GPU."""
-        cap = max(1, lib().fk_system_num_components(self._h))
-        reps = np.zeros(cap, dtype=REPORT_DTYPE)
+    def _solve(self, decomposer, perturb, optimizer, cap):
+        if optimizer not in _OPTIMIZERS:
+            raise ValueError(f"optimizer must be 'lm' or 'lbfgs', not {optimizer!r}")
+        opts = FkSolvingOptions(_OPTIMIZERS[optimizer], decomposer, int(bool(perturb)), 0)
+        reps = np.zeros(max(1, cap), dtype=REPORT_DTYPE)
         n = C.c_uint32(0)
-        check(lib().fk_system_solve(self._h, int(perturb), reps.ctypes.data_as(C.POINTER(FkReport)), cap, C.byref(n)))
+        check(lib().fk_system_solve_options(self._h, C.byref(opts), reps.ctypes.data_as(C.POINTER(FkReport)), len(reps), C.byref(n)))
         self._reports = reps[:n.value]
 
-    def solve_single_pass(self, perturb=True):
-        """System::solve with Decomposer::SinglePass (assemble/mod.rs:169-210) on the GPU."""
-        cap = max(1, len(self.single_pass_plan()))
-        reps = np.zeros(cap, dtype=REPORT_DTYPE)
-        n = C.c_uint32(0)
-        check(lib().fk_system_solve_opts(self._h, 1, int(perturb), reps.ctypes.data_as(C.POINTER(FkReport)), cap, C.byref(n)))
-        self._reports = reps[:n.value]
+    def solve(self, perturb=True, optimizer="lm"):
+        """System::solve(SolvingOptions { optimizer, decomposer: None, perturb }) on the GPU; optimizer 'lm'
+        (LevenbergMarquardt, the default) or 'lbfgs' (LBfgs)."""
+        self._solve(0, perturb, optimizer, lib().fk_system_num_components(self._h))
 
-    def solve_recursive_assembly(self, perturb=True):
-        """System::solve with Decomposer::RecursiveAssembly (assemble/mod.rs:212-277) on the GPU."""
-        cap = max(1, self.recursive_assembly_plan()[0])
-        reps = np.zeros(cap, dtype=REPORT_DTYPE)
-        n = C.c_uint32(0)
-        check(lib().fk_system_solve_opts(self._h, 2, int(perturb), reps.ctypes.data_as(C.POINTER(FkReport)), cap, C.byref(n)))
-        self._reports = reps[:n.value]
+    def solve_single_pass(self, perturb=True, optimizer="lm"):
+        """System::solve with Decomposer::SinglePass (assemble/mod.rs:169-210) on the GPU.  The reference runs LM here
+        whatever the optimizer (assemble/mod.rs:191)."""
+        self._solve(1, perturb, optimizer, len(self.single_pass_plan()))
+
+    def solve_recursive_assembly(self, perturb=True, optimizer="lm"):
+        """System::solve with Decomposer::RecursiveAssembly (assemble/mod.rs:212-277) on the GPU.  The reference runs LM
+        here whatever the optimizer (assemble/mod.rs:224)."""
+        self._solve(2, perturb, optimizer, self.recursive_assembly_plan()[0])
 
     def recursive_assembly_plan(self):
         """(number of steps, serialised plan words) of fk_system_recursive_assembly_plan (host only)."""

@@ -331,11 +331,25 @@ FK_API int fk_batch_solve_single_pass(const fk_topology* topo, uint32_t n, doubl
  * iterations, 4 guard (the reference's unbounded bisection loop, :338-351, would not return);
  * outer_iters = line searches, factorizations = residual+Jacobian evaluations, ssr, lambda = last step
  * size, trace_hash = h*31 + evaluations per line search.  Shared-memory tile paths only
- * (FK_ERR_TOO_LARGE otherwise). */
+ * (FK_ERR_TOO_LARGE otherwise); fk_lbfgs_solve_batch takes systems of every size. */
 FK_API int fk_batch_solve_lbfgs(const fk_topology* topo, int device, uint32_t n, const double* vars, const double* param,
                                 double* free_out, fk_report* reports);
-/* Same on the resident sketches of a batch plan (fk_batch_plan_upload / _download around it). */
+/* Same on the resident sketches of a batch plan (fk_batch_plan_upload / _download around it).  Tile paths only, as
+ * fk_batch_solve_lbfgs; fk_batch_plan_run_lbfgs_global runs any plan. */
 FK_API int fk_batch_plan_run_lbfgs(fk_batch_plan* plan, void* stream);
+/* Same with the CTA kernel on any plan: one CTA of 256 threads per sketch, the sketch's L-BFGS state in global memory,
+ * bit-identical to the tile kernel.  The plan grows its workspace on first use (at most 1 GiB: a large system gets
+ * fewer CTAs in flight) and frees it with the plan. */
+FK_API int fk_batch_plan_run_lbfgs_global(fk_batch_plan* plan, void* stream);
+/* L-BFGS kernel the batch calls use for a topology: 0 the tile kernel (every topology fk_batch_solve_lbfgs takes),
+ * 1 the CTA kernel (every other topology; no size limit but device memory).  Host only. */
+FK_API int fk_topology_lbfgs_kernel(const fk_topology* topo, uint32_t n_sketches);
+/* The L-BFGS counterparts of fk_lm_solve / fk_lm_solve_batch, for systems of every size: problems grouped by structure
+ * through the topology cache, one launch per group (the kernel of fk_topology_lbfgs_kernel), groups placed on or
+ * sharded over n_gpus devices as fk_lm_solve_batch does.  Reports as fk_batch_solve_lbfgs. */
+FK_API int fk_lbfgs_solve(const fk_problem* problem, double* free_values, fk_report* report);
+FK_API int fk_lbfgs_solve_batch(uint32_t n, const fk_problem* const* problems, double* const* free_values, fk_report* reports,
+                                int n_gpus);
 
 /* ---- System::analyze: over-constraint detection (SURVEY 8f-2) -------------------------------------- */
 /* == find_overconstraints (fiksi/src/analyze/numerical/mod.rs:123-163) for n sketches sharing one
@@ -407,6 +421,18 @@ FK_API int fk_system_solve(fk_system* s, int perturb, fk_report* reports, uint32
  * (assemble/mod.rs:282-590: cluster poses + the step's elements, FK_POSE_POINT_X/Y rows) solved by the GPU LM,
  * owned points moved with their cluster's pose afterwards).  reports: one per solved sub-problem, up to `cap`. */
 FK_API int fk_system_solve_opts(fk_system* s, int decomposer, int perturb, fk_report* reports, uint32_t cap, uint32_t* n_solved);
+/* SolvingOptions (lib.rs:205-237).  optimizer 0: LevenbergMarquardt, 1: LBfgs; decomposer as fk_system_solve_opts;
+ * perturb 0 / 1; pad must be 0. */
+typedef struct fk_solving_options {
+    uint32_t optimizer, decomposer, perturb, pad;
+} fk_solving_options;
+/* == System::solve(options).  optimizer 0 is fk_system_solve_opts(decomposer).  optimizer 1 with Decomposer::None: the
+ * scale, seeded perturbation and per-component problems of fk_system_solve, every component solved by L-BFGS in one
+ * fk_lbfgs_solve_batch call, write-back as assemble/mod.rs:161-166; reports as fk_batch_solve_lbfgs.  The reference
+ * dispatches on the optimizer only under Decomposer::None (assemble/mod.rs:148-158): SinglePass and RecursiveAssembly
+ * call levenberg_marquardt directly (:191, :224), so optimizer 1 with decomposer 1 or 2 runs LM, identically to
+ * optimizer 0.  Any other value: FK_ERR_INVALID. */
+FK_API int fk_system_solve_options(fk_system* s, const fk_solving_options* opts, fk_report* reports, uint32_t cap, uint32_t* n_solved);
 /* Host-only probe of the RecursiveAssembly plan (no device needed) as a stream of 32-bit words: per step
  * n_constraints, constraints..., n_elements, elements..., n_free, free elements..., then the maps on_frontiers,
  * owned_elements, frontier_elements (recursive_assembly.rs:75-114) as n_keys and per key (ascending) key, n,

@@ -69,6 +69,7 @@ EXPORTS = [
     "fk_set_lm_kernel", "fk_get_lm_kernel", "fk_topology_sketch_kernel_info",
     "fk_topology_batch_kernel", "fk_topology_lbfgs_kernel", "fk_lbfgs_solve", "fk_lbfgs_solve_batch", "fk_batch_plan_run_lbfgs_global",
     "fk_system_solve_options", "fk_batch_system_solve", "fk_batch_system_solve_begin", "fk_batch_system_solve_wait", "fk_batch_solve_device_begin", "fk_batch_solve_device_wait", "fk_topology_cache_configure", "fk_topology_cache_clear", "fk_topology_cache_stats",
+    "fk_system_batch_solve", "fk_system_batch_layout",
 ]
 
 _lib = None

@@ -26,6 +26,7 @@
 #include "sparse_batch.cuh"
 #include "sparse_path.cuh"
 #include "symbolic.hpp"
+#include "system_batch.cuh"
 
 namespace {
 
@@ -1834,3 +1835,291 @@ int fk_lm_solve(const fk_problem* problem, double* free_values, fk_report* repor
 }
 
 }  // extern "C"
+
+// ---- fk_system_batch_solve: System::solve over n variants of one drawing -------------------------------------------
+namespace fk {
+
+int system_batch_fail(int code, const std::string& msg) { return fail(code, msg); }
+
+// The buffers of one device: the structures' batch plans (capacity chunk * multiplicity), the chunk's raw input and output
+// rows, and the index tables of the two kernels, all on one stream.
+struct SystemBatchDevice {
+    std::mutex mu;
+    int device = -1;
+    bool ready = false;          // tables uploaded
+    cudaStream_t stream = nullptr;
+    uint32_t chunk = 0;          // variants the buffers hold
+    bool lm = false;             // the plans were made for LM (which on the global sparse path needs the sparse batch tables)
+    std::vector<fk_batch_plan*> plans;
+    void* d_tables = nullptr;    // kinds, expression -> constraint, draws, slot / expression tables, scatter tables, descriptors
+    const uint8_t* d_kind = nullptr;
+    const uint32_t *d_expr_con = nullptr, *d_var_struct = nullptr, *d_var_off = nullptr, *d_comp_struct = nullptr, *d_comp_member = nullptr;
+    const double* d_draws = nullptr;
+    SbStructure* d_desc = nullptr;
+    std::vector<SbStructure> desc;  // (host copy; the buffer pointers change with the plans)
+    double *d_raw_vars = nullptr, *d_raw_param = nullptr, *d_tmpl_vars = nullptr, *d_tmpl_param = nullptr, *d_scales = nullptr, *d_vars_out = nullptr;
+    fk_report* d_rep_out = nullptr;
+    void release_buffers() {
+        for (fk_batch_plan* p : plans) delete p;
+        plans.clear();
+        cudaFree(d_raw_vars); cudaFree(d_raw_param); cudaFree(d_scales); cudaFree(d_vars_out); cudaFree(d_rep_out);
+        d_raw_vars = d_raw_param = d_scales = d_vars_out = nullptr;
+        d_rep_out = nullptr;
+        chunk = 0;
+    }
+    ~SystemBatchDevice() {
+        if (device < 0) return;
+        cudaSetDevice(device);
+        release_buffers();
+        cudaFree(d_tables); cudaFree(d_desc); cudaFree(d_tmpl_vars); cudaFree(d_tmpl_param);
+        if (stream) cudaStreamDestroy(stream);
+    }
+};
+
+struct SystemBatch {
+    SystemBatchLayout L;
+    struct Structure {
+        std::shared_ptr<fk_topology> topo;
+        std::vector<uint32_t> members;                 // component indices
+        std::vector<uint32_t> slot_var, slot_draw, expr;  // [mult][nv], [mult][nv], [mult][ne]
+    };
+    std::vector<Structure> st;
+    std::vector<uint32_t> comp_struct, comp_member;  // per component
+    std::vector<uint32_t> var_struct, var_off;       // per system variable: structure solving it (kSbNone: none), offset in the variant's block
+    std::mutex mu;
+    std::map<int, std::unique_ptr<SystemBatchDevice>> devices;
+};
+
+int system_batch_create(SystemBatchLayout&& layout, const std::vector<const fk_problem*>& problems, std::shared_ptr<SystemBatch>* out) {
+    std::shared_ptr<SystemBatch> b = std::make_shared<SystemBatch>();
+    b->L = std::move(layout);
+    const SystemBatchLayout& L = b->L;
+    const uint32_t nc = (uint32_t)problems.size();
+    std::vector<BatchGroup> groups;
+    if (nc) {
+        static double dummy = 0.0;  // (group_by_topology checks the free-value pointers; nothing is written through them)
+        std::vector<double*> fv(nc, &dummy);
+        const int rc = group_by_topology(nc, problems.data(), fv.data(), groups);
+        if (rc != FK_OK) return rc;
+    }
+    b->comp_struct.assign(nc, kSbNone);
+    b->comp_member.assign(nc, 0);
+    b->var_struct.assign(L.n_vars, kSbNone);
+    b->var_off.assign(L.n_vars, 0);
+    for (BatchGroup& g : groups) {
+        SystemBatch::Structure S;
+        S.topo = g.topo;
+        S.members = g.members;
+        const uint32_t si = (uint32_t)b->st.size(), nf = g.topo->t.n_free;
+        for (uint32_t m = 0; m < S.members.size(); m++) {
+            const SystemBatchLayout::Component& c = L.comps[S.members[m]];
+            S.slot_var.insert(S.slot_var.end(), c.slot_var.begin(), c.slot_var.end());
+            S.slot_draw.insert(S.slot_draw.end(), c.slot_draw.begin(), c.slot_draw.end());
+            S.expr.insert(S.expr.end(), c.expr.begin(), c.expr.end());
+            b->comp_struct[S.members[m]] = si;
+            b->comp_member[S.members[m]] = m;
+            for (uint32_t f = 0; f < c.free_var.size(); f++) {
+                b->var_struct[c.free_var[f]] = si;
+                b->var_off[c.free_var[f]] = m * nf + f;
+            }
+        }
+        b->st.push_back(std::move(S));
+    }
+    *out = std::move(b);
+    return FK_OK;
+}
+
+void system_batch_layout(const SystemBatch& b, uint32_t* n_components, uint32_t* n_structures, std::vector<uint32_t>* multiplicity) {
+    if (n_components) *n_components = (uint32_t)b.L.comps.size();
+    if (n_structures) *n_structures = (uint32_t)b.st.size();
+    if (multiplicity) {
+        multiplicity->clear();
+        for (const SystemBatch::Structure& S : b.st) multiplicity->push_back((uint32_t)S.members.size());
+    }
+}
+
+// Variants per chunk: the chunk's buffers within about 1 GiB of device memory (FK_SYSTEM_BATCH_CHUNK=n overrides), at least one.
+static uint32_t system_batch_chunk(const SystemBatch& b, uint32_t n, uint32_t n_reports) {
+    static const uint32_t env = [] {
+        const char* e = std::getenv("FK_SYSTEM_BATCH_CHUNK");  // test knob
+        const long v = e ? std::atol(e) : 0;
+        return (uint32_t)(v >= 1 && v <= (long)UINT32_MAX ? v : 0);
+    }();
+    uint64_t bytes = sizeof(double) * (2ull * b.L.n_vars + b.L.n_constraints + 1) + sizeof(fk_report) * (uint64_t)n_reports;
+    uint64_t max_mult = 1;
+    for (const SystemBatch::Structure& S : b.st) {
+        const fk::Topology& t = S.topo->t;
+        bytes += S.members.size() * (sizeof(double) * ((uint64_t)t.n_vars + t.n_expr + t.n_free) + sizeof(fk_report));
+        max_mult = std::max<uint64_t>(max_mult, S.members.size());
+    }
+    uint64_t chunk = env ? env : std::max<uint64_t>(1, (1ull << 30) / bytes);
+    chunk = std::min<uint64_t>(chunk, std::max<uint64_t>(1, (uint64_t)INT32_MAX / max_mult));  // sketches per launch stay in range
+    return (uint32_t)std::min<uint64_t>(chunk, n);
+}
+
+static SystemBatchDevice* system_batch_device_slot(SystemBatch& b, int device) {
+    std::lock_guard<std::mutex> lock(b.mu);
+    auto& p = b.devices[device];
+    if (!p) p.reset(new SystemBatchDevice());
+    return p.get();
+}
+
+// Tables once per device; plans and chunk buffers grow with the chunk (and are made again when LM follows L-BFGS).  The caller
+// holds d->mu.
+static int system_batch_device(SystemBatch& b, SystemBatchDevice* d, int device, uint32_t chunk, uint32_t n_reports, bool lm) {
+    CU(cudaSetDevice(device));
+    const SystemBatchLayout& L = b.L;
+    const uint32_t n_expr = (uint32_t)L.kind.size(), ns = (uint32_t)b.st.size(), nc = (uint32_t)L.comps.size();
+    if (!d->ready) {
+        d->device = device;
+        if (!d->stream) CU(cudaStreamCreateWithFlags(&d->stream, cudaStreamNonBlocking));
+        cudaFree(d->d_tables); cudaFree(d->d_desc); cudaFree(d->d_tmpl_vars); cudaFree(d->d_tmpl_param);  // (an earlier attempt's)
+        d->d_tables = nullptr; d->d_desc = nullptr; d->d_tmpl_vars = d->d_tmpl_param = nullptr;
+        struct Item { const void* src; size_t bytes; size_t at; };
+        std::vector<Item> items;
+        size_t off = 0;
+        auto add = [&](const auto& vec) {
+            using T = typename std::decay<decltype(vec)>::type::value_type;
+            const size_t at = reserve<T>(off, vec.size());
+            items.push_back({vec.data(), vec.size() * sizeof(T), at});
+            return at;
+        };
+        const size_t o_kind = add(L.kind), o_con = add(L.expr_constraint), o_draws = add(L.draws), o_vs = add(b.var_struct), o_vo = add(b.var_off),
+                     o_cs = add(b.comp_struct), o_cm = add(b.comp_member);
+        std::vector<size_t> o_sv(ns), o_sd(ns), o_ex(ns);
+        for (uint32_t s = 0; s < ns; s++) {
+            o_sv[s] = add(b.st[s].slot_var);
+            o_sd[s] = add(b.st[s].slot_draw);
+            o_ex[s] = add(b.st[s].expr);
+        }
+        std::vector<unsigned char> host(off + 16, 0);
+        for (const Item& it : items)
+            if (it.bytes) std::memcpy(host.data() + it.at, it.src, it.bytes);
+        CU(cudaMalloc(&d->d_tables, host.size()));
+        CU(cudaMemcpyAsync(d->d_tables, host.data(), host.size(), cudaMemcpyHostToDevice, d->stream));
+        CU(cudaStreamSynchronize(d->stream));  // (host leaves scope)
+        unsigned char* t = (unsigned char*)d->d_tables;
+        d->d_kind = t + o_kind;
+        d->d_expr_con = (const uint32_t*)(t + o_con);
+        d->d_draws = (const double*)(t + o_draws);
+        d->d_var_struct = (const uint32_t*)(t + o_vs); d->d_var_off = (const uint32_t*)(t + o_vo);
+        d->d_comp_struct = (const uint32_t*)(t + o_cs); d->d_comp_member = (const uint32_t*)(t + o_cm);
+        d->desc.assign(ns, SbStructure{});
+        for (uint32_t s = 0; s < ns; s++) {
+            const fk::Topology& tp = b.st[s].topo->t;
+            SbStructure& S = d->desc[s];
+            S.slot_var = (const uint32_t*)(t + o_sv[s]); S.slot_draw = (const uint32_t*)(t + o_sd[s]); S.expr = (const uint32_t*)(t + o_ex[s]);
+            S.nv = tp.n_vars; S.ne = tp.n_expr; S.nf = tp.n_free; S.mult = (uint32_t)b.st[s].members.size();
+        }
+        CU(cudaMalloc(&d->d_desc, sizeof(SbStructure) * std::max<uint32_t>(ns, 1)));
+        CU(cudaMalloc(&d->d_tmpl_vars, sizeof(double) * std::max<uint32_t>(L.n_vars, 1)));
+        CU(cudaMalloc(&d->d_tmpl_param, sizeof(double) * std::max<uint32_t>(n_expr, 1)));
+        d->ready = true;
+    }
+    if (d->chunk >= chunk && (d->lm || !lm) && d->plans.size() == ns) return FK_OK;
+    const uint32_t cap = std::max(chunk, d->chunk);
+    d->release_buffers();
+    for (uint32_t s = 0; s < ns; s++) {
+        fk_batch_plan* p = nullptr;
+        const int rc = plan_create(b.st[s].topo.get(), cap * (uint32_t)b.st[s].members.size(), device, lm, &p);
+        if (rc != FK_OK) {
+            d->release_buffers();
+            return rc;
+        }
+        d->plans.push_back(p);
+        SbStructure& S = d->desc[s];
+        S.vars = p->d_vars; S.params = p->d_params; S.out = p->d_out; S.reps = p->d_rep;
+    }
+    auto alloc = [&](auto** ptr, size_t count) -> int {
+        CU(cudaMalloc((void**)ptr, sizeof(**ptr) * std::max<size_t>(count, 1)));
+        return FK_OK;
+    };
+    int rc = FK_OK;
+    if ((rc = alloc(&d->d_raw_vars, (size_t)cap * L.n_vars)) != FK_OK || (rc = alloc(&d->d_raw_param, (size_t)cap * L.n_constraints)) != FK_OK ||
+        (rc = alloc(&d->d_scales, cap)) != FK_OK || (rc = alloc(&d->d_vars_out, (size_t)cap * L.n_vars)) != FK_OK ||
+        (rc = alloc(&d->d_rep_out, (size_t)cap * std::max<uint32_t>(std::min(n_reports, nc), 1))) != FK_OK) {
+        d->release_buffers();
+        return rc;
+    }
+    if (ns) CU(cudaMemcpyAsync(d->d_desc, d->desc.data(), sizeof(SbStructure) * ns, cudaMemcpyHostToDevice, d->stream));
+    CU(cudaStreamSynchronize(d->stream));  // (desc may change before a later call's copy)
+    d->chunk = cap;
+    d->lm = lm;
+    return FK_OK;
+}
+
+// Variants [lo, hi) on one device, chunk after chunk on its stream: upload, prepare + gather, one launch per structure, scatter,
+// download.
+static int system_batch_range(SystemBatch& b, const SystemBatchCall& c, int device, uint32_t lo, uint32_t hi) {
+    const SystemBatchLayout& L = b.L;
+    const uint32_t n_expr = (uint32_t)L.kind.size(), ns = (uint32_t)b.st.size(), nc = (uint32_t)L.comps.size();
+    const uint32_t n_rep = c.reports ? std::min(c.reports_per_variant, nc) : 0;
+    const uint32_t chunk = system_batch_chunk(b, hi - lo, n_rep);
+    SystemBatchDevice* d = system_batch_device_slot(b, device);
+    std::lock_guard<std::mutex> lock(d->mu);
+    int rc = system_batch_device(b, d, device, chunk, nc, c.optimizer == 0);
+    if (rc != FK_OK) return rc;
+    cudaStream_t st = d->stream;
+    auto run = [&]() -> int {
+        if (L.n_vars) CU(cudaMemcpyAsync(d->d_tmpl_vars, c.tmpl_vars, sizeof(double) * L.n_vars, cudaMemcpyHostToDevice, st));
+        if (n_expr) CU(cudaMemcpyAsync(d->d_tmpl_param, c.tmpl_param, sizeof(double) * n_expr, cudaMemcpyHostToDevice, st));
+        for (uint32_t at = lo; at < hi; at += chunk) {
+            const uint32_t cnt = std::min(chunk, hi - at);
+            const double* raw = d->d_tmpl_vars;
+            uint32_t raw_stride = 0;
+            if (c.vars) {
+                if (L.n_vars)
+                    CU(cudaMemcpyAsync(d->d_raw_vars, c.vars + (size_t)at * L.n_vars, sizeof(double) * (size_t)cnt * L.n_vars, cudaMemcpyHostToDevice, st));
+                raw = d->d_raw_vars;
+                raw_stride = L.n_vars;
+            }
+            if (c.params && L.n_constraints)
+                CU(cudaMemcpyAsync(d->d_raw_param, c.params + (size_t)at * L.n_constraints, sizeof(double) * (size_t)cnt * L.n_constraints,
+                                   cudaMemcpyHostToDevice, st));
+            int e = launch_system_batch_prepare(cnt, L.n_vars, n_expr, L.n_constraints, d->d_kind, d->d_expr_con, d->d_draws, c.perturb, raw,
+                                                raw_stride, c.params ? d->d_raw_param : nullptr, d->d_tmpl_param, ns, d->d_desc, d->d_scales, st);
+            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_batch_prepare_kernel");
+            for (uint32_t s = 0; s < ns; s++) {
+                fk_batch_plan* p = d->plans[s];
+                p->n = cnt * (uint32_t)b.st[s].members.size();
+                const int r = c.optimizer == 0                    ? fk_batch_plan_run(p, st)
+                              : choose_lbfgs(p->topo, p->n) == 1 ? fk_batch_plan_run_lbfgs_global(p, st)
+                                                                 : fk_batch_plan_run_lbfgs(p, st);
+                if (r != FK_OK) return r;
+            }
+            e = launch_system_batch_scatter(cnt, L.n_vars, raw, raw_stride, d->d_scales, d->d_var_struct, d->d_var_off, n_rep, d->d_comp_struct,
+                                            d->d_comp_member, d->d_desc, d->d_vars_out, d->d_rep_out, st);
+            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_batch_scatter_kernel");
+            if (L.n_vars)
+                CU(cudaMemcpyAsync(c.vars_out + (size_t)at * L.n_vars, d->d_vars_out, sizeof(double) * (size_t)cnt * L.n_vars, cudaMemcpyDeviceToHost, st));
+            if (n_rep)
+                CU(cudaMemcpy2DAsync(c.reports + (size_t)at * c.reports_per_variant, sizeof(fk_report) * c.reports_per_variant, d->d_rep_out,
+                                     sizeof(fk_report) * n_rep, sizeof(fk_report) * n_rep, cnt, cudaMemcpyDeviceToHost, st));
+        }
+        return FK_OK;
+    };
+    rc = run();
+    // (also after an error: no copy into the caller's buffers may still be running when the call returns)
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (rc == FK_OK && e != cudaSuccess) rc = cuda_fail(e, "fk_system_batch_solve kernels / copies");
+    return rc;
+}
+
+int system_batch_solve(SystemBatch& b, const SystemBatchCall& c) {
+    if (c.optimizer == 0)  // LM on the global sparse path: the front limit of fk_batch_solve
+        for (const SystemBatch::Structure& S : b.st)
+            if (S.topo->t.path == 2 && S.topo->sb_check() != FK_OK)
+                return fail(FK_ERR_TOO_LARGE, "component " + std::to_string(S.members[0]) + ": " + S.topo->sb_err +
+                                                  "; Optimizer::LBfgs takes systems of every size");
+    if (c.n == 0) return FK_OK;
+    int n_gpus = c.n_gpus;
+    const int rc = clamp_gpus(n_gpus);
+    if (rc != FK_OK) return rc;
+    int cur = 0;
+    if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
+    const int r = shard_over_devices(n_gpus, c.n, [&](int device, uint32_t lo, uint32_t hi) { return system_batch_range(b, c, device, lo, hi); });
+    if (cudaSetDevice(cur) != cudaSuccess) cudaGetLastError();
+    return r;
+}
+
+}  // namespace fk

@@ -18,6 +18,7 @@
 #include "lbfgs_core.cuh"
 #include "lm_kernels.cuh"
 #include "lm_sketch.cuh"
+#include "prepare.cuh"
 
 namespace fk {
 
@@ -1003,31 +1004,7 @@ fk_batch_prepare_kernel(uint32_t n_sketches, uint32_t n_vars, uint32_t n_expr, c
     if (k >= n_sketches) return;
     const double* rv = raw_vars + (size_t)k * n_vars;
     const double* rp = raw_param + (shared_param ? 0 : (size_t)k * n_expr);
-    double sum = 0.0;
-    uint32_t cnt = n_vars;
-    {
-        uint32_t i = 0;
-        for (; i + 8 <= n_vars; i += 8) {  // eight loads in flight, the additions stay in order
-            double v[8];
-#pragma unroll
-            for (int u = 0; u < 8; u++) v[u] = __ldg(rv + i + u);
-#pragma unroll
-            for (int u = 0; u < 8; u++) sum = sum + v[u] * v[u];
-        }
-        for (; i < n_vars; i++) {
-            const double v = __ldg(rv + i);
-            sum = sum + v * v;
-        }
-    }
-    for (uint32_t e = 0; e < n_expr; e++) {
-        const uint32_t kd = __ldg(kinds + e);
-        if (kd == FK_POINT_POINT_DISTANCE || kd == FK_POINT_LINE_DISTANCE) {
-            const double q = __ldg(rp + e);
-            sum = sum + q * q;
-            cnt++;
-        }
-    }
-    const double scale = sqrt(sum / (double)cnt);
+    const double scale = prepare_scale(rv, n_vars, n_expr, kinds, [&](uint32_t e) { return __ldg(rp + e); });
     const double recip = 1.0 / scale;
     double* ov = vars + (size_t)k * n_vars;
     double* op = params + (size_t)k * n_expr;
@@ -1036,16 +1013,15 @@ fk_batch_prepare_kernel(uint32_t n_sketches, uint32_t n_vars, uint32_t n_expr, c
     for (uint32_t i = 0; i < n_vars; i++) {
         double col = __ldg(rv + i) * recip;
         if (i == next) {
-            col = col + (col * (1.0 / 8196.0) * __ldg(draws + 2 * j) + (1.0 / 65568.0) * __ldg(draws + 2 * j + 1));
+            col = prepare_perturb(col, __ldg(draws + 2 * j), __ldg(draws + 2 * j + 1));
             j++;
             next = j < n_perturb ? __ldg(perturb_vars + j) : 0xFFFFFFFFu;
         }
         ov[i] = col;
     }
     for (uint32_t e = 0; e < n_expr; e++) {
-        const uint32_t kd = __ldg(kinds + e);
         const double q = __ldg(rp + e);
-        op[e] = (kd == FK_POINT_POINT_DISTANCE || kd == FK_POINT_LINE_DISTANCE) ? recip * q : q;
+        op[e] = prepare_is_distance(__ldg(kinds + e)) ? recip * q : q;
     }
     scales[k] = scale;
 }

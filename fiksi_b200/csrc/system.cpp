@@ -8,6 +8,7 @@
 #include <cstring>
 #include <map>
 #include <memory>
+#include <mutex>
 #include <set>
 #include <stdexcept>
 #include <string>
@@ -17,6 +18,7 @@
 #include "recursive_assembly.hpp"
 #include "single_pass.hpp"
 #include "symbolic.hpp"
+#include "system_batch.cuh"
 
 namespace {
 
@@ -62,6 +64,10 @@ struct fk_system {
     std::vector<Comp> comps;
     std::string error;
     std::unique_ptr<fk_topology, void (*)(fk_topology*)> eval_topo{nullptr, fk_topology_destroy};
+    // fk_system_batch_solve's plan (components grouped by structure, device tables): built on first use, dropped by every
+    // structural edit (elements, constraints, fix / unfix); new variable or parameter values keep it.
+    mutable std::mutex batch_mu;
+    mutable std::shared_ptr<fk::SystemBatch> batch;
 
     uint32_t new_element(uint8_t tag, uint32_t a, uint32_t b, const double* v, int nv) {
         uint32_t id = (uint32_t)elems.size();
@@ -74,6 +80,7 @@ struct fk_system {
         elems.push_back({tag, nv ? first : a, b});
         comp_of.push_back(0);
         eval_topo.reset();
+        drop_batch_plan();
         return id;
     }
     int element_vars(uint32_t e, uint32_t out[4]) const {
@@ -119,6 +126,10 @@ struct fk_system {
         comps[target - 1].elements.swap(merged.elements);
         comps[target - 1].constraints.swap(merged.constraints);
     }
+    void drop_batch_plan() {
+        std::lock_guard<std::mutex> lock(batch_mu);
+        batch.reset();
+    }
     void push_expr(uint8_t k, uint32_t i0, uint32_t i1, uint32_t i2, uint32_t i3, double p) {
         kind.push_back(k);
         idx.push_back(i0); idx.push_back(i1); idx.push_back(i2); idx.push_back(i3);
@@ -156,6 +167,7 @@ int fk_system_fix(fk_system* s, uint32_t element, int fix) {
     uint32_t v[4];
     int n = s->element_vars(element, v);
     for (int k = 0; k < n; k++) s->fixed[v[k]] = fix ? 1 : 0;
+    s->drop_batch_plan();
     return FK_OK;
 }
 
@@ -227,6 +239,7 @@ uint32_t fk_system_add_constraint(fk_system* s, int tag, const uint32_t* el, uin
     for (int k = 0; k < n_inc; k++) rec.inc[k] = inc[k];
     s->constrs.push_back(rec);
     s->eval_topo.reset();
+    s->drop_batch_plan();
     return id;
 }
 
@@ -262,6 +275,7 @@ struct LocalProblem {
     std::vector<double> vars, param, x;
     std::vector<uint8_t> kind;
     std::vector<uint32_t> idx, free_local, rows, free_global;
+    std::vector<uint32_t> slot_global;  // local variable -> system variable
     fk_problem prob;
 };
 void build_local(const fk_system* s, const std::vector<double>& vt, const std::vector<double>& pt, const std::vector<uint32_t>& free_sorted,
@@ -276,6 +290,7 @@ void build_local(const fk_system* s, const std::vector<double>& vt, const std::v
     for (uint32_t g : used) {
         local.emplace(g, (uint32_t)L.vars.size());
         L.vars.push_back(vt[g]);
+        L.slot_global.push_back(g);
     }
     for (uint32_t g : free_sorted) {
         L.free_global.push_back(g);
@@ -840,6 +855,99 @@ int fk_system_component(const fk_system* s, uint32_t ci, uint32_t* n_elements, u
     if (elements) std::copy(c.elements.begin(), c.elements.end(), elements);
     if (constraints) std::copy(c.constraints.begin(), c.constraints.end(), constraints);
     return FK_OK;
+}
+
+}  // extern "C"
+
+// ---- System::solve over n variants of one drawing ------------------------------------------------------------------
+namespace {
+
+// The drawing's batch plan: per non-empty component (component order) its LocalProblem numbering, the draws of the solve's
+// generator and, per local variable, the draw already applied at the component's snapshot -- prepare_components perturbs
+// component by component, so a variable of a later component is read unperturbed and one of an earlier component perturbed.
+int batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemBatch>* out) {
+    std::lock_guard<std::mutex> lock(s->batch_mu);
+    if (!s->batch) {
+        fk::SystemBatchLayout lay;
+        lay.n_vars = (uint32_t)s->vars.size();
+        lay.n_constraints = (uint32_t)s->constrs.size();
+        lay.kind = s->kind;
+        lay.expr_constraint.assign(s->kind.size(), fk::kSbNone);
+        for (uint32_t c = 0; c < s->constrs.size(); c++) lay.expr_constraint[s->constrs[c].first_expr] = c;  // update_parameter
+        std::vector<uint32_t> var_draw(s->vars.size(), fk::kSbNone);
+        std::vector<std::unique_ptr<LocalProblem>> locals;
+        Lcg rng{42};
+        for (const fk_system::Comp& c : s->comps) {
+            if (c.elements.empty()) continue;  // assemble/mod.rs:87-89
+            const std::vector<uint32_t> free_sorted = component_free_variables(s, c);
+            for (uint32_t fv : free_sorted) {
+                if (var_draw[fv] != fk::kSbNone) return fk::system_batch_fail(FK_ERR_INTERNAL, "a variable is free in two components");
+                var_draw[fv] = (uint32_t)(lay.draws.size() / 2);
+                lay.draws.push_back(rng.next());
+                lay.draws.push_back(rng.next());
+            }
+            std::vector<uint32_t> exprs;
+            for (uint32_t ci : c.constraints)
+                for (uint8_t k = 0; k < s->constrs[ci].n_expr; k++) exprs.push_back(s->constrs[ci].first_expr + k);
+            std::unique_ptr<LocalProblem> L(new LocalProblem());
+            build_local(s, s->vars, s->param, free_sorted, exprs, *L);
+            fk::SystemBatchLayout::Component comp;
+            comp.slot_var = L->slot_global;
+            for (uint32_t g : L->slot_global) comp.slot_draw.push_back(var_draw[g]);
+            comp.expr = exprs;
+            comp.free_var = free_sorted;
+            lay.comps.push_back(std::move(comp));
+            locals.push_back(std::move(L));
+        }
+        std::vector<const fk_problem*> probs;
+        for (const auto& L : locals) probs.push_back(&L->prob);
+        const int rc = fk::system_batch_create(std::move(lay), probs, &s->batch);
+        if (rc != FK_OK) return rc;
+    }
+    *out = s->batch;
+    return FK_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int fk_system_batch_layout(const fk_system* s, uint32_t* n_components, uint32_t* n_structures, uint32_t* multiplicity) {
+    if (!s) return fk::system_batch_fail(FK_ERR_INVALID, "null system");
+    std::shared_ptr<fk::SystemBatch> b;
+    const int rc = batch_plan_for(s, &b);
+    if (rc != FK_OK) return rc;
+    std::vector<uint32_t> mult;
+    fk::system_batch_layout(*b, n_components, n_structures, &mult);
+    if (multiplicity) std::copy(mult.begin(), mult.end(), multiplicity);
+    return FK_OK;
+}
+
+int fk_system_batch_solve(const fk_system* s, const fk_solving_options* opts, uint32_t n, const double* vars, const double* params,
+                          double* vars_out, fk_report* reports, uint32_t reports_per_variant, uint32_t* n_solved, int n_gpus) {
+    if (!s || !opts || !vars_out) return fk::system_batch_fail(FK_ERR_INVALID, "null system, options or vars_out");
+    if (opts->optimizer > 1 || opts->perturb > 1 || opts->pad != 0) return fk::system_batch_fail(FK_ERR_INVALID, "invalid solving options");
+    if (opts->decomposer != 0)
+        return fk::system_batch_fail(FK_ERR_INVALID, "fk_system_batch_solve takes Decomposer::None only (decomposer 0)");
+    std::shared_ptr<fk::SystemBatch> b;
+    int rc = batch_plan_for(s, &b);
+    if (rc != FK_OK) return rc;
+    uint32_t nc = 0;
+    fk::system_batch_layout(*b, &nc, nullptr, nullptr);
+    if (n_solved) *n_solved = nc;
+    fk::SystemBatchCall c;
+    c.optimizer = (int)opts->optimizer;
+    c.perturb = (int)opts->perturb;
+    c.n_gpus = n_gpus;
+    c.n = n;
+    c.vars = vars;
+    c.params = params;
+    c.tmpl_vars = s->vars.data();
+    c.tmpl_param = s->param.data();
+    c.vars_out = vars_out;
+    c.reports = reports;
+    c.reports_per_variant = reports_per_variant;
+    return fk::system_batch_solve(*b, c);
 }
 
 }  // extern "C"

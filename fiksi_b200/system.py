@@ -80,6 +80,47 @@ class System:
         (LevenbergMarquardt, the default) or 'lbfgs' (LBfgs)."""
         self._solve(0, perturb, optimizer, lib().fk_system_num_components(self._h))
 
+    def batch_layout(self):
+        """(solved components, distinct component structures, [components per structure]) of batch_solve's plan (host
+        only)."""
+        nc, ns = C.c_uint32(0), C.c_uint32(0)
+        check(lib().fk_system_batch_layout(self._h, C.byref(nc), C.byref(ns), None))
+        mult = np.zeros(max(ns.value, 1), np.uint32)
+        check(lib().fk_system_batch_layout(self._h, C.byref(nc), C.byref(ns), ptr(mult, C.c_uint32)))
+        return int(nc.value), int(ns.value), mult[:ns.value].tolist()
+
+    def batch_solve(self, vars=None, params=None, optimizer="lm", perturb=True, n_gpus=1, n=None):
+        """System.solve(perturb, optimizer) of n variants of this drawing in one call (fk_system_batch_solve): variant v
+        starts from variables vars[v] ([n][n_variables]) and constraint parameters params[v] ([n][n_constraints]); None
+        takes this system's own values (then `n` says how many variants).  The system itself is not modified.  Returns
+        (variables after each variant's solve [n][n_variables], reports [n][solved components] as REPORT_DTYPE)."""
+        if optimizer not in _OPTIMIZERS:
+            raise ValueError(f"optimizer must be 'lm' or 'lbfgs', not {optimizer!r}")
+        nv, ncon = lib().fk_system_num_variables(self._h), self.num_constraints()
+        def rows(a, width):
+            a = np.ascontiguousarray(a, dtype=np.float64)
+            return a.reshape(len(a) if a.ndim == 2 else -1, width)
+        if vars is not None:
+            vars = rows(vars, nv)
+        if params is not None:
+            params = rows(params, ncon)
+        sizes = {len(a) for a in (vars, params) if a is not None}
+        if n is not None:
+            sizes.add(int(n))
+        if len(sizes) != 1:
+            raise ValueError("give vars, params or n, with one number of variants")
+        count = sizes.pop()
+        n_solved = self.batch_layout()[0]
+        out = np.zeros((count, nv))
+        reps = np.zeros((count, n_solved), dtype=REPORT_DTYPE)
+        opts = FkSolvingOptions(_OPTIMIZERS[optimizer], 0, int(bool(perturb)), 0)
+        got = C.c_uint32(0)
+        check(lib().fk_system_batch_solve(
+            self._h, C.byref(opts), count, None if vars is None else ptr(vars, C.c_double),
+            None if params is None else ptr(params, C.c_double), ptr(out, C.c_double),
+            reps.ctypes.data_as(C.POINTER(FkReport)), n_solved, C.byref(got), int(n_gpus)))
+        return out, reps
+
     def solve_single_pass(self, perturb=True, optimizer="lm"):
         """System::solve with Decomposer::SinglePass (assemble/mod.rs:169-210) on the GPU.  The reference runs LM here
         whatever the optimizer (assemble/mod.rs:191)."""

@@ -221,7 +221,7 @@ FK_API int fk_batch_solve_device_wait(const fk_topology* topo, int device, uint6
  * raw_vars[n][n_vars] and raw_param ([n][n_expr], or ONE row with FK_PREP_SHARED_PARAM) in and free_out[n][n_free]
  * (UNSCALED values, i.e. what System::solve writes into system.variables), scales_out[n] (optional) and reports out.
  * Restriction: the sketch is one connected component whose problem names every variable and expression of the
- * system (the scale is a property of the whole system). */
+ * system (the scale is a property of the whole system); fk_system_batch_solve takes any drawing of the fk_system mirror. */
 enum { FK_PREP_SHARED_PARAM = 1, FK_PREP_PERTURB = 2 };
 typedef struct {
     uint32_t flags;               /* FK_PREP_* */
@@ -433,6 +433,30 @@ typedef struct fk_solving_options {
  * call levenberg_marquardt directly (:191, :224), so optimizer 1 with decomposer 1 or 2 runs LM, identically to
  * optimizer 0.  Any other value: FK_ERR_INVALID. */
 FK_API int fk_system_solve_options(fk_system* s, const fk_solving_options* opts, fk_report* reports, uint32_t cap, uint32_t* n_solved);
+/* == System::solve(options) (lib.rs:464, assemble/mod.rs:46-167) applied to n variants of the drawing `s`: variant v is `s`
+ * with every variable set to vars[v][i] (fk_system_set_variable) and every constraint parameter set to params[v][c]
+ * (fk_system_set_parameter), then solved.  vars == NULL: every variant starts from s's variables; params == NULL: from s's
+ * parameters.  vars_out[n][n_vars] receives what fk_system_get_variables would return after that solve, bit for bit what
+ * fk_system_solve_options gives on a copy of `s` with the variant's numbers (LM on the global sparse path: the decisions of
+ * that call, coordinates within the documented difference between the sparse batch kernel and the single-system path).
+ * reports[v][k] (row stride reports_per_variant, may be NULL): the report of the k-th solved component (component order, as
+ * fk_system_solve), the first reports_per_variant of them; *n_solved = solved components per variant (the same for every
+ * variant).  Only Decomposer::None: opts->decomposer != 0 is FK_ERR_INVALID.  Variants are sharded over n_gpus devices
+ * (0 == all visible) as fk_batch_solve does.  `s` is not modified.
+ * On the device: one kernel scales, perturbs and gathers every component's input rows straight into the batch buffers of its
+ * structure (components of identical shape share one topology: sketch = variant * multiplicity + member), one batched launch
+ * per structure (the kernels of fk_batch_solve / fk_lbfgs_solve_batch), one kernel writes the unscaled rows back.  The plan
+ * (components, structures, their topologies and device tables) is kept on `s` until a structural edit (an add_*, fix / unfix).
+ * Variants go in chunks whose device buffers stay within about 1 GiB (at least one variant per chunk).  Refusals come before
+ * any device work and leave vars_out untouched: FK_ERR_INVALID for bad arguments, FK_ERR_TOO_LARGE with LM when a
+ * component's largest supernodal front exceeds the 236 rows of fk_batch_solve (the message names the component and the
+ * front's order; L-BFGS takes every size). */
+FK_API int fk_system_batch_solve(const fk_system* s, const fk_solving_options* opts, uint32_t n, const double* vars,
+                                 const double* params, double* vars_out, fk_report* reports, uint32_t reports_per_variant,
+                                 uint32_t* n_solved, int n_gpus);
+/* Host-only probe of fk_system_batch_solve's plan (no device needed): solved components, distinct component structures,
+ * and the components per structure in order of first appearance (multiplicity[n_structures], may be NULL). */
+FK_API int fk_system_batch_layout(const fk_system* s, uint32_t* n_components, uint32_t* n_structures, uint32_t* multiplicity);
 /* Host-only probe of the RecursiveAssembly plan (no device needed) as a stream of 32-bit words: per step
  * n_constraints, constraints..., n_elements, elements..., n_free, free elements..., then the maps on_frontiers,
  * owned_elements, frontier_elements (recursive_assembly.rs:75-114) as n_keys and per key (ascending) key, n,

@@ -1938,13 +1938,19 @@ void system_batch_layout(const SystemBatch& b, uint32_t* n_components, uint32_t*
     }
 }
 
-// Variants per chunk: the chunk's buffers within about 1 GiB of device memory (FK_SYSTEM_BATCH_CHUNK=n overrides), at least one.
-static uint32_t system_batch_chunk(const SystemBatch& b, uint32_t n, uint32_t n_reports) {
+// FK_SYSTEM_BATCH_CHUNK=n: variants per chunk of both system batch calls (test knob), 0 when unset.
+static uint32_t system_batch_chunk_env() {
     static const uint32_t env = [] {
-        const char* e = std::getenv("FK_SYSTEM_BATCH_CHUNK");  // test knob
+        const char* e = std::getenv("FK_SYSTEM_BATCH_CHUNK");
         const long v = e ? std::atol(e) : 0;
         return (uint32_t)(v >= 1 && v <= (long)UINT32_MAX ? v : 0);
     }();
+    return env;
+}
+
+// Variants per chunk: the chunk's buffers within about 1 GiB of device memory (FK_SYSTEM_BATCH_CHUNK=n overrides), at least one.
+static uint32_t system_batch_chunk(const SystemBatch& b, uint32_t n, uint32_t n_reports) {
+    const uint32_t env = system_batch_chunk_env();
     uint64_t bytes = sizeof(double) * (2ull * b.L.n_vars + b.L.n_constraints + 1) + sizeof(fk_report) * (uint64_t)n_reports;
     uint64_t max_mult = 1;
     for (const SystemBatch::Structure& S : b.st) {
@@ -2118,6 +2124,333 @@ int system_batch_solve(SystemBatch& b, const SystemBatchCall& c) {
     int cur = 0;
     if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
     const int r = shard_over_devices(n_gpus, c.n, [&](int device, uint32_t lo, uint32_t hi) { return system_batch_range(b, c, device, lo, hi); });
+    if (cudaSetDevice(cur) != cudaSuccess) cudaGetLastError();
+    return r;
+}
+
+// ---- fk_system_batch_solve_single_pass: Decomposer::SinglePass over n variants of one drawing ---------------------------
+// The device state of fk_system_batch_solve plus the resident rows of the scaled variables (vt) and parameters (pt) that the
+// waves read and write, and the per-wave descriptors of the gather / scatter kernel.  d_desc holds the one identity structure
+// through which the prepare kernel writes vt and pt; plans are one per structure (capacity chunk * the structure's most sets
+// in one wave).
+struct SystemSpDevice : SystemBatchDevice {
+    double *d_vt = nullptr, *d_pt = nullptr;
+    const uint8_t* d_solved = nullptr;
+    const uint32_t *d_pvar = nullptr, *d_pdraw = nullptr;  // the perturbations of waves >= 1, wave after wave
+    std::vector<uint32_t> pert_off;                        // [n_waves + 1]
+    std::vector<SpGroup> groups;                           // (host copy) every wave's groups, wave after wave
+    std::vector<uint32_t> group_off;                       // [n_waves + 1]
+    SpGroup* d_groups = nullptr;
+    void release_sp_buffers() {
+        cudaFree(d_vt); cudaFree(d_pt);
+        d_vt = d_pt = nullptr;
+        release_buffers();
+    }
+    ~SystemSpDevice() {
+        if (device < 0) return;
+        cudaSetDevice(device);
+        cudaFree(d_vt); cudaFree(d_pt); cudaFree(d_groups);
+    }
+};
+
+struct SystemSpBatch {
+    SystemBatchLayout L;  // comps: the sets
+    struct Structure {
+        std::shared_ptr<fk_topology> topo;
+        std::vector<uint32_t> members;  // set indices
+        uint32_t wave_mult = 0;         // most sets of the structure in one wave: the plan's sketches per variant
+    };
+    std::vector<Structure> st;
+    std::vector<uint32_t> set_struct;
+    struct Group {  // the sets of one structure in one wave, in plan order: the tables of its SpGroup
+        uint32_t structure = 0;
+        std::vector<uint32_t> sets, slot_var, expr, free_var;
+    };
+    std::vector<std::vector<Group>> waves;
+    std::vector<std::vector<uint32_t>> wave_perturb;  // variables whose perturbation runs at the start of wave w >= 1
+    std::vector<uint8_t> solved;                      // per system variable: some set solves it
+    std::mutex mu;
+    std::map<int, std::unique_ptr<SystemSpDevice>> devices;
+};
+
+int system_sp_batch_create(SystemBatchLayout&& layout, const std::vector<const fk_problem*>& problems, std::shared_ptr<SystemSpBatch>* out) {
+    std::shared_ptr<SystemSpBatch> b = std::make_shared<SystemSpBatch>();
+    b->L = std::move(layout);
+    const SystemBatchLayout& L = b->L;
+    const uint32_t n_sets = (uint32_t)problems.size();
+    std::vector<BatchGroup> groups;
+    if (n_sets) {
+        static double dummy = 0.0;  // (group_by_topology checks the free-value pointers; nothing is written through them)
+        std::vector<double*> fv(n_sets, &dummy);
+        const int rc = group_by_topology(n_sets, problems.data(), fv.data(), groups);
+        if (rc != FK_OK) return rc;
+    }
+    b->set_struct.assign(n_sets, kSbNone);
+    for (BatchGroup& g : groups) {
+        for (uint32_t k : g.members) b->set_struct[k] = (uint32_t)b->st.size();
+        b->st.push_back({g.topo, g.members, 0});
+    }
+    b->waves.assign(L.n_waves, {});
+    b->solved.assign(L.n_vars, 0);
+    for (uint32_t k = 0; k < n_sets; k++) {
+        std::vector<SystemSpBatch::Group>& wave = b->waves[L.comp_wave[k]];
+        const uint32_t si = b->set_struct[k];
+        auto it = std::find_if(wave.begin(), wave.end(), [&](const SystemSpBatch::Group& g) { return g.structure == si; });
+        if (it == wave.end()) {
+            wave.emplace_back();
+            wave.back().structure = si;
+            it = wave.end() - 1;
+        }
+        const SystemBatchLayout::Component& c = L.comps[k];
+        it->sets.push_back(k);
+        it->slot_var.insert(it->slot_var.end(), c.slot_var.begin(), c.slot_var.end());
+        it->expr.insert(it->expr.end(), c.expr.begin(), c.expr.end());
+        it->free_var.insert(it->free_var.end(), c.free_var.begin(), c.free_var.end());
+        b->st[si].wave_mult = std::max(b->st[si].wave_mult, (uint32_t)it->sets.size());
+        for (uint32_t g : c.free_var) b->solved[g] = 1;
+    }
+    // (a perturbation scheduled behind the last wave precedes no set: nothing reads it, and vars_out keeps unsolved variables raw)
+    b->wave_perturb.assign(L.n_waves, {});
+    for (uint32_t i = 0; i < L.n_vars; i++)
+        if (L.var_wave[i] != kSbNone && L.var_wave[i] > 0 && L.var_wave[i] < L.n_waves) b->wave_perturb[L.var_wave[i]].push_back(i);
+    *out = std::move(b);
+    return FK_OK;
+}
+
+void system_sp_batch_layout(const SystemSpBatch& b, uint32_t* n_sets, uint32_t* n_waves, uint32_t* n_structures,
+                            std::vector<uint32_t>* set_wave, std::vector<uint32_t>* set_structure) {
+    if (n_sets) *n_sets = (uint32_t)b.L.comps.size();
+    if (n_waves) *n_waves = b.L.n_waves;
+    if (n_structures) *n_structures = (uint32_t)b.st.size();
+    if (set_wave) *set_wave = b.L.comp_wave;
+    if (set_structure) *set_structure = b.set_struct;
+}
+
+// Variants per chunk, as system_batch_chunk: raw, resident and output rows plus every structure's plan buffers.
+static uint32_t system_sp_chunk(const SystemSpBatch& b, uint32_t n, uint32_t n_reports) {
+    const uint32_t env = system_batch_chunk_env();
+    const uint64_t n_expr = b.L.kind.size();
+    uint64_t bytes = sizeof(double) * (3ull * b.L.n_vars + b.L.n_constraints + n_expr + 1) + sizeof(fk_report) * (uint64_t)n_reports;
+    uint64_t max_mult = 1;
+    for (const SystemSpBatch::Structure& S : b.st) {
+        const fk::Topology& t = S.topo->t;
+        bytes += S.wave_mult * (sizeof(double) * ((uint64_t)t.n_vars + t.n_expr + t.n_free) + sizeof(fk_report));
+        max_mult = std::max<uint64_t>(max_mult, S.wave_mult);
+    }
+    uint64_t chunk = env ? env : std::max<uint64_t>(1, (1ull << 30) / bytes);
+    chunk = std::min<uint64_t>(chunk, std::max<uint64_t>(1, (uint64_t)INT32_MAX / max_mult));  // sketches per launch stay in range
+    chunk = std::min<uint64_t>(chunk, std::max<uint64_t>(1, (uint64_t)UINT32_MAX / std::max<uint64_t>({1, b.L.n_vars, n_expr})));
+    return (uint32_t)std::min<uint64_t>(chunk, n);
+}
+
+static SystemSpDevice* system_sp_device_slot(SystemSpBatch& b, int device) {
+    std::lock_guard<std::mutex> lock(b.mu);
+    auto& p = b.devices[device];
+    if (!p) p.reset(new SystemSpDevice());
+    return p.get();
+}
+
+// Tables once per device; plans, buffers and descriptors grow with the chunk.  The caller holds d->mu.
+static int system_sp_device(SystemSpBatch& b, SystemSpDevice* d, int device, uint32_t chunk, uint32_t n_reports) {
+    CU(cudaSetDevice(device));
+    const SystemBatchLayout& L = b.L;
+    const uint32_t n_expr = (uint32_t)L.kind.size(), ns = (uint32_t)b.st.size(), nw = L.n_waves;
+    if (!d->ready) {
+        d->device = device;
+        if (!d->stream) CU(cudaStreamCreateWithFlags(&d->stream, cudaStreamNonBlocking));
+        cudaFree(d->d_tables); cudaFree(d->d_desc); cudaFree(d->d_tmpl_vars); cudaFree(d->d_tmpl_param); cudaFree(d->d_groups);  // (an earlier attempt's)
+        d->d_tables = nullptr; d->d_desc = nullptr; d->d_tmpl_vars = d->d_tmpl_param = nullptr; d->d_groups = nullptr;
+        // the identity structure of the prepare kernel: every variable (with its draw where the perturbation runs before any
+        // set) and every expression
+        std::vector<uint32_t> ident_var(L.n_vars), ident_draw(L.n_vars, kSbNone), ident_expr(n_expr);
+        for (uint32_t i = 0; i < L.n_vars; i++) {
+            ident_var[i] = i;
+            if (L.var_wave[i] == 0) ident_draw[i] = L.var_draw[i];
+        }
+        for (uint32_t e = 0; e < n_expr; e++) ident_expr[e] = e;
+        std::vector<uint32_t> pvar, pdraw;
+        d->pert_off.assign(1, 0);
+        for (uint32_t w = 0; w < nw; w++) {
+            for (uint32_t i : b.wave_perturb[w]) {
+                pvar.push_back(i);
+                pdraw.push_back(L.var_draw[i]);
+            }
+            d->pert_off.push_back((uint32_t)pvar.size());
+        }
+        struct Item { const void* src; size_t bytes; size_t at; };
+        std::vector<Item> items;
+        size_t off = 0;
+        auto add = [&](const auto& vec) {
+            using T = typename std::decay<decltype(vec)>::type::value_type;
+            const size_t at = reserve<T>(off, vec.size());
+            items.push_back({vec.data(), vec.size() * sizeof(T), at});
+            return at;
+        };
+        const size_t o_kind = add(L.kind), o_con = add(L.expr_constraint), o_draws = add(L.draws), o_iv = add(ident_var), o_id = add(ident_draw),
+                     o_ie = add(ident_expr), o_solved = add(b.solved), o_pv = add(pvar), o_pd = add(pdraw);
+        struct GroupAt { size_t sv, ex, fv, st; };
+        std::vector<GroupAt> at;
+        for (const auto& wave : b.waves)
+            for (const SystemSpBatch::Group& g : wave) at.push_back({add(g.slot_var), add(g.expr), add(g.free_var), add(g.sets)});
+        std::vector<unsigned char> host(off + 16, 0);
+        for (const Item& it : items)
+            if (it.bytes) std::memcpy(host.data() + it.at, it.src, it.bytes);
+        CU(cudaMalloc(&d->d_tables, host.size()));
+        CU(cudaMemcpyAsync(d->d_tables, host.data(), host.size(), cudaMemcpyHostToDevice, d->stream));
+        CU(cudaStreamSynchronize(d->stream));  // (host leaves scope)
+        unsigned char* t = (unsigned char*)d->d_tables;
+        d->d_kind = t + o_kind;
+        d->d_expr_con = (const uint32_t*)(t + o_con);
+        d->d_draws = (const double*)(t + o_draws);
+        d->d_solved = t + o_solved;
+        d->d_pvar = (const uint32_t*)(t + o_pv); d->d_pdraw = (const uint32_t*)(t + o_pd);
+        d->desc.assign(1, SbStructure{});
+        SbStructure& I = d->desc[0];
+        I.slot_var = (const uint32_t*)(t + o_iv); I.slot_draw = (const uint32_t*)(t + o_id); I.expr = (const uint32_t*)(t + o_ie);
+        I.nv = L.n_vars; I.ne = n_expr; I.nf = 0; I.mult = 1;
+        d->groups.clear();
+        d->group_off.assign(1, 0);
+        size_t q = 0;
+        for (const auto& wave : b.waves) {
+            for (const SystemSpBatch::Group& g : wave) {
+                const fk::Topology& tp = b.st[g.structure].topo->t;
+                SpGroup G{};
+                G.s.slot_var = (const uint32_t*)(t + at[q].sv); G.s.expr = (const uint32_t*)(t + at[q].ex);
+                G.free_var = (const uint32_t*)(t + at[q].fv); G.step = (const uint32_t*)(t + at[q].st);
+                G.s.nv = tp.n_vars; G.s.ne = tp.n_expr; G.s.nf = tp.n_free; G.s.mult = (uint32_t)g.sets.size();
+                d->groups.push_back(G);
+                q++;
+            }
+            d->group_off.push_back((uint32_t)d->groups.size());
+        }
+        CU(cudaMalloc(&d->d_desc, sizeof(SbStructure)));
+        CU(cudaMalloc(&d->d_groups, sizeof(SpGroup) * std::max<size_t>(d->groups.size(), 1)));
+        CU(cudaMalloc(&d->d_tmpl_vars, sizeof(double) * std::max<uint32_t>(L.n_vars, 1)));
+        CU(cudaMalloc(&d->d_tmpl_param, sizeof(double) * std::max<uint32_t>(n_expr, 1)));
+        d->ready = true;
+    }
+    if (d->chunk >= chunk && d->plans.size() == ns) return FK_OK;
+    const uint32_t cap = std::max(chunk, d->chunk);
+    d->release_sp_buffers();
+    for (uint32_t s = 0; s < ns; s++) {
+        fk_batch_plan* p = nullptr;
+        const int rc = plan_create(b.st[s].topo.get(), cap * b.st[s].wave_mult, device, true, &p);
+        if (rc != FK_OK) {
+            d->release_sp_buffers();
+            return rc;
+        }
+        d->plans.push_back(p);
+    }
+    auto alloc = [&](auto** ptr, size_t count) -> int {
+        CU(cudaMalloc((void**)ptr, sizeof(**ptr) * std::max<size_t>(count, 1)));
+        return FK_OK;
+    };
+    const uint32_t n_sets = (uint32_t)L.comps.size();
+    int rc = FK_OK;
+    if ((rc = alloc(&d->d_raw_vars, (size_t)cap * L.n_vars)) != FK_OK || (rc = alloc(&d->d_raw_param, (size_t)cap * L.n_constraints)) != FK_OK ||
+        (rc = alloc(&d->d_scales, cap)) != FK_OK || (rc = alloc(&d->d_vars_out, (size_t)cap * L.n_vars)) != FK_OK ||
+        (rc = alloc(&d->d_vt, (size_t)cap * L.n_vars)) != FK_OK || (rc = alloc(&d->d_pt, (size_t)cap * n_expr)) != FK_OK ||
+        (rc = alloc(&d->d_rep_out, (size_t)cap * std::max<uint32_t>(std::min(n_reports, n_sets), 1))) != FK_OK) {
+        d->release_sp_buffers();
+        return rc;
+    }
+    d->desc[0].vars = d->d_vt;
+    d->desc[0].params = d->d_pt;
+    {
+        size_t q = 0;
+        for (const auto& wave : b.waves)
+            for (const SystemSpBatch::Group& g : wave) {
+                const fk_batch_plan* p = d->plans[g.structure];
+                SpGroup& G = d->groups[q++];
+                G.s.vars = p->d_vars; G.s.params = p->d_params; G.s.out = p->d_out; G.s.reps = p->d_rep;
+            }
+    }
+    CU(cudaMemcpyAsync(d->d_desc, d->desc.data(), sizeof(SbStructure), cudaMemcpyHostToDevice, d->stream));
+    if (!d->groups.empty())
+        CU(cudaMemcpyAsync(d->d_groups, d->groups.data(), sizeof(SpGroup) * d->groups.size(), cudaMemcpyHostToDevice, d->stream));
+    CU(cudaStreamSynchronize(d->stream));  // (the descriptors may change before a later call's copy)
+    d->chunk = cap;
+    d->lm = true;
+    return FK_OK;
+}
+
+// Variants [lo, hi) on one device, chunk after chunk on its stream: upload; prepare (scale, the perturbations that precede every
+// set, the resident rows vt / pt); per wave one gather / scatter launch and one LM launch per structure present; a last gather /
+// scatter launch with the write-back; download.
+static int system_sp_range(SystemSpBatch& b, const SystemBatchCall& c, int device, uint32_t lo, uint32_t hi) {
+    const SystemBatchLayout& L = b.L;
+    const uint32_t n_expr = (uint32_t)L.kind.size(), nw = L.n_waves, n_sets = (uint32_t)L.comps.size();
+    const uint32_t n_rep = c.reports ? std::min(c.reports_per_variant, n_sets) : 0;
+    const uint32_t chunk = system_sp_chunk(b, hi - lo, n_rep);
+    SystemSpDevice* d = system_sp_device_slot(b, device);
+    std::lock_guard<std::mutex> lock(d->mu);
+    int rc = system_sp_device(b, d, device, chunk, n_sets);
+    if (rc != FK_OK) return rc;
+    cudaStream_t st = d->stream;
+    auto run = [&]() -> int {
+        if (L.n_vars) CU(cudaMemcpyAsync(d->d_tmpl_vars, c.tmpl_vars, sizeof(double) * L.n_vars, cudaMemcpyHostToDevice, st));
+        if (n_expr) CU(cudaMemcpyAsync(d->d_tmpl_param, c.tmpl_param, sizeof(double) * n_expr, cudaMemcpyHostToDevice, st));
+        for (uint32_t at = lo; at < hi; at += chunk) {
+            const uint32_t cnt = std::min(chunk, hi - at);
+            const double* raw = d->d_tmpl_vars;
+            uint32_t raw_stride = 0;
+            if (c.vars) {
+                if (L.n_vars)
+                    CU(cudaMemcpyAsync(d->d_raw_vars, c.vars + (size_t)at * L.n_vars, sizeof(double) * (size_t)cnt * L.n_vars, cudaMemcpyHostToDevice, st));
+                raw = d->d_raw_vars;
+                raw_stride = L.n_vars;
+            }
+            if (c.params && L.n_constraints)
+                CU(cudaMemcpyAsync(d->d_raw_param, c.params + (size_t)at * L.n_constraints, sizeof(double) * (size_t)cnt * L.n_constraints,
+                                   cudaMemcpyHostToDevice, st));
+            int e = launch_system_batch_prepare(cnt, L.n_vars, n_expr, L.n_constraints, d->d_kind, d->d_expr_con, d->d_draws, c.perturb, raw,
+                                                raw_stride, c.params ? d->d_raw_param : nullptr, d->d_tmpl_param, 1, d->d_desc, d->d_scales, st);
+            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_batch_prepare_kernel");
+            for (uint32_t w = 0; w <= nw; w++) {
+                const uint32_t s_lo = w ? d->group_off[w - 1] : 0, s_hi = w ? d->group_off[w] : 0;
+                const uint32_t g_lo = w < nw ? d->group_off[w] : 0, g_hi = w < nw ? d->group_off[w + 1] : 0;
+                const uint32_t p_lo = c.perturb && w < nw ? d->pert_off[w] : 0, p_hi = c.perturb && w < nw ? d->pert_off[w + 1] : 0;
+                e = launch_system_sp_gather_scatter(cnt, L.n_vars, n_expr, d->d_vt, d->d_pt, s_hi - s_lo, d->d_groups + s_lo, n_rep, d->d_rep_out,
+                                                    p_hi - p_lo, d->d_pvar + p_lo, d->d_pdraw + p_lo, d->d_draws, g_hi - g_lo, d->d_groups + g_lo,
+                                                    d->d_solved, raw, raw_stride, d->d_scales, w == nw ? d->d_vars_out : nullptr, st);
+                if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_sp_gather_scatter_kernel");
+                if (w == nw) break;
+                for (const SystemSpBatch::Group& g : b.waves[w]) {  // LM under SinglePass whatever the optimizer (assemble/mod.rs:191)
+                    fk_batch_plan* p = d->plans[g.structure];
+                    p->n = cnt * (uint32_t)g.sets.size();
+                    const int r = fk_batch_plan_run(p, st);
+                    if (r != FK_OK) return r;
+                }
+            }
+            if (L.n_vars)
+                CU(cudaMemcpyAsync(c.vars_out + (size_t)at * L.n_vars, d->d_vars_out, sizeof(double) * (size_t)cnt * L.n_vars, cudaMemcpyDeviceToHost, st));
+            if (n_rep)
+                CU(cudaMemcpy2DAsync(c.reports + (size_t)at * c.reports_per_variant, sizeof(fk_report) * c.reports_per_variant, d->d_rep_out,
+                                     sizeof(fk_report) * n_rep, sizeof(fk_report) * n_rep, cnt, cudaMemcpyDeviceToHost, st));
+        }
+        return FK_OK;
+    };
+    rc = run();
+    // (also after an error: no copy into the caller's buffers may still be running when the call returns)
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (rc == FK_OK && e != cudaSuccess) rc = cuda_fail(e, "fk_system_batch_solve_single_pass kernels / copies");
+    return rc;
+}
+
+int system_sp_batch_solve(SystemSpBatch& b, const SystemBatchCall& c) {
+    for (const SystemSpBatch::Structure& S : b.st)  // sets on the global sparse path: the front limit of fk_batch_solve
+        if (S.topo->t.path == 2 && S.topo->sb_check() != FK_OK) {
+            const uint32_t k = S.members[0];
+            return fail(FK_ERR_TOO_LARGE, "set " + std::to_string(k) + " (first expression " + std::to_string(b.L.comps[k].expr[0]) +
+                                              "): " + S.topo->sb_err + "; fk_system_solve_opts solves it one variant at a time");
+        }
+    if (c.n == 0) return FK_OK;
+    int n_gpus = c.n_gpus;
+    const int rc = clamp_gpus(n_gpus);
+    if (rc != FK_OK) return rc;
+    int cur = 0;
+    if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
+    const int r = shard_over_devices(n_gpus, c.n, [&](int device, uint32_t lo, uint32_t hi) { return system_sp_range(b, c, device, lo, hi); });
     if (cudaSetDevice(cur) != cudaSuccess) cudaGetLastError();
     return r;
 }

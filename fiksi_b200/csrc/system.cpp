@@ -68,6 +68,7 @@ struct fk_system {
     // structural edit (elements, constraints, fix / unfix); new variable or parameter values keep it.
     mutable std::mutex batch_mu;
     mutable std::shared_ptr<fk::SystemBatch> batch;
+    mutable std::shared_ptr<fk::SystemSpBatch> sp_batch;  // fk_system_batch_solve_single_pass's plan, kept and dropped alike
 
     uint32_t new_element(uint8_t tag, uint32_t a, uint32_t b, const double* v, int nv) {
         uint32_t id = (uint32_t)elems.size();
@@ -129,6 +130,7 @@ struct fk_system {
     void drop_batch_plan() {
         std::lock_guard<std::mutex> lock(batch_mu);
         batch.reset();
+        sp_batch.reset();
     }
     void push_expr(uint8_t k, uint32_t i0, uint32_t i1, uint32_t i2, uint32_t i3, double p) {
         kind.push_back(k);
@@ -908,6 +910,79 @@ int batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemBatch>* out) {
     return FK_OK;
 }
 
+// fk_system_batch_solve_single_pass's plan: the sets of fk_system_solve_opts(decomposer = 1) in its order, each as its
+// LocalProblem numbering, the draws of batch_plan_for, and the waves.  The host loop is a sequence of nodes: per non-empty
+// component its perturbation (reads and writes the component's free variables) followed by its sets (read their variables,
+// write their free ones).  Node b follows an earlier node a when a writes what b reads or writes, or reads what b writes; sets
+// reach across components (SinglePass plans over the equation graph of every expression), so these edges are computed, not
+// assumed.  Times: a set of wave w at 2w + 1, a perturbation at the start of wave w at 2w; every node goes to the earliest
+// time after all nodes it follows (ASAP).  The perturbation nodes count whether or not the call perturbs, so the waves do not
+// depend on it.  Any schedule that respects the edges computes the host loop's values.
+int single_pass_batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemSpBatch>* out) {
+    std::lock_guard<std::mutex> lock(s->batch_mu);
+    if (!s->sp_batch) {
+        fk::SystemBatchLayout lay;
+        lay.n_vars = (uint32_t)s->vars.size();
+        lay.n_constraints = (uint32_t)s->constrs.size();
+        lay.kind = s->kind;
+        lay.expr_constraint.assign(s->kind.size(), fk::kSbNone);
+        for (uint32_t c = 0; c < s->constrs.size(); c++) lay.expr_constraint[s->constrs[c].first_expr] = c;  // update_parameter
+        lay.var_draw.assign(s->vars.size(), fk::kSbNone);
+        lay.var_wave.assign(s->vars.size(), fk::kSbNone);
+        std::vector<int64_t> last_write(s->vars.size(), -1), last_read(s->vars.size(), -1);  // latest time of a writer / reader
+        // earliest time after every node that the node reading `reads` and writing `writes` (a subset of reads) follows
+        auto earliest = [&](const std::vector<uint32_t>& reads, const std::vector<uint32_t>& writes) {
+            int64_t t = -1;
+            for (uint32_t g : reads) t = std::max(t, last_write[g]);
+            for (uint32_t g : writes) t = std::max(t, last_read[g]);
+            return t + 1;
+        };
+        auto place = [&](const std::vector<uint32_t>& reads, const std::vector<uint32_t>& writes, int64_t time) {
+            for (uint32_t g : reads) last_read[g] = std::max(last_read[g], time);
+            for (uint32_t g : writes) last_write[g] = std::max(last_write[g], time);
+        };
+        std::vector<std::vector<uint32_t>> var_exprs, expr_vars;
+        equation_graph(s, var_exprs, expr_vars);
+        fk::SinglePassPlanner planner(var_exprs, expr_vars);
+        std::vector<std::unique_ptr<LocalProblem>> locals;
+        Lcg rng{42};
+        for (const fk_system::Comp& c : s->comps) {
+            if (c.elements.empty()) continue;  // assemble/mod.rs:87-89
+            const std::vector<uint32_t> free_sorted = component_free_variables(s, c);
+            const int64_t tp = earliest(free_sorted, free_sorted);
+            const uint32_t pw = (uint32_t)((tp + 1) / 2);  // first wave start at or after tp
+            for (uint32_t fv : free_sorted) {
+                if (lay.var_draw[fv] != fk::kSbNone) return fk::system_batch_fail(FK_ERR_INTERNAL, "a variable is free in two components");
+                lay.var_draw[fv] = (uint32_t)(lay.draws.size() / 2);
+                lay.var_wave[fv] = pw;
+                lay.draws.push_back(rng.next());
+                lay.draws.push_back(rng.next());
+            }
+            place(free_sorted, free_sorted, 2 * (int64_t)pw);
+            for (const fk::SinglePassStep& st : planner.plan(free_sorted)) {
+                std::unique_ptr<LocalProblem> L(new LocalProblem());
+                build_local(s, s->vars, s->param, st.free_variables, st.expressions, *L);
+                const uint32_t w = (uint32_t)(earliest(L->slot_global, st.free_variables) / 2);  // first set time 2w + 1 at or after it
+                place(L->slot_global, st.free_variables, 2 * (int64_t)w + 1);
+                fk::SystemBatchLayout::Component comp;
+                comp.slot_var = L->slot_global;
+                comp.expr = st.expressions;
+                comp.free_var = st.free_variables;
+                lay.comps.push_back(std::move(comp));
+                lay.comp_wave.push_back(w);
+                lay.n_waves = std::max(lay.n_waves, w + 1);
+                locals.push_back(std::move(L));
+            }
+        }
+        std::vector<const fk_problem*> probs;
+        for (const auto& L : locals) probs.push_back(&L->prob);
+        const int rc = fk::system_sp_batch_create(std::move(lay), probs, &s->sp_batch);
+        if (rc != FK_OK) return rc;
+    }
+    *out = s->sp_batch;
+    return FK_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -948,6 +1023,43 @@ int fk_system_batch_solve(const fk_system* s, const fk_solving_options* opts, ui
     c.reports = reports;
     c.reports_per_variant = reports_per_variant;
     return fk::system_batch_solve(*b, c);
+}
+
+int fk_system_single_pass_batch_layout(const fk_system* s, uint32_t* n_steps, uint32_t* n_waves, uint32_t* n_structures,
+                                       uint32_t* step_wave, uint32_t* step_structure) {
+    if (!s) return fk::system_batch_fail(FK_ERR_INVALID, "null system");
+    std::shared_ptr<fk::SystemSpBatch> b;
+    const int rc = single_pass_batch_plan_for(s, &b);
+    if (rc != FK_OK) return rc;
+    std::vector<uint32_t> set_wave, set_structure;
+    fk::system_sp_batch_layout(*b, n_steps, n_waves, n_structures, &set_wave, &set_structure);
+    if (step_wave) std::copy(set_wave.begin(), set_wave.end(), step_wave);
+    if (step_structure) std::copy(set_structure.begin(), set_structure.end(), step_structure);
+    return FK_OK;
+}
+
+int fk_system_batch_solve_single_pass(const fk_system* s, int perturb, uint32_t n, const double* vars, const double* params,
+                                      double* vars_out, fk_report* reports, uint32_t reports_per_variant, uint32_t* n_solved, int n_gpus) {
+    if (!s || !vars_out) return fk::system_batch_fail(FK_ERR_INVALID, "null system or vars_out");
+    if (perturb != 0 && perturb != 1) return fk::system_batch_fail(FK_ERR_INVALID, "perturb must be 0 or 1");
+    std::shared_ptr<fk::SystemSpBatch> b;
+    int rc = single_pass_batch_plan_for(s, &b);
+    if (rc != FK_OK) return rc;
+    uint32_t n_sets = 0;
+    fk::system_sp_batch_layout(*b, &n_sets, nullptr, nullptr, nullptr, nullptr);
+    if (n_solved) *n_solved = n_sets;
+    fk::SystemBatchCall c;
+    c.perturb = perturb;
+    c.n_gpus = n_gpus;
+    c.n = n;
+    c.vars = vars;
+    c.params = params;
+    c.tmpl_vars = s->vars.data();
+    c.tmpl_param = s->param.data();
+    c.vars_out = vars_out;
+    c.reports = reports;
+    c.reports_per_variant = reports_per_variant;
+    return fk::system_sp_batch_solve(*b, c);
 }
 
 }  // extern "C"

@@ -1,6 +1,8 @@
 // Kernels of fk_system_batch_solve (System::solve over n variants of one drawing): the scale, perturbation and gather of
 // every component's input rows into its structure's batch buffers, and the write-back of the solved components into the
 // variants' variable rows.  The arithmetic of the pre-processing is prepare.cuh's, shared with fk_batch_prepare_kernel.
+// fk_system_batch_solve_single_pass reuses the prepare kernel (one identity structure: the resident scaled rows) and moves
+// values between the waves of strongly connected sets with fk_system_sp_gather_scatter_kernel.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -92,6 +94,84 @@ fk_system_batch_scatter_kernel(uint32_t n, uint32_t n_vars, const double* __rest
         const SbStructure& S = structures[__ldg(comp_struct + k)];
         reports_out[i] = __ldg((const unsigned long long*)(S.reps + v * S.mult + __ldg(comp_member + k)) + w);
     }
+}
+
+// Between two waves of fk_system_batch_solve_single_pass.  One CTA per `vb` consecutive variants, so that the phases (scatter,
+// perturbations, gather, write-back) of a variant are ordered by __syncthreads alone.  A group's rows of variants
+// [v0, v0 + nb) are contiguous in its batch buffers (sketch = variant * mult + member): consecutive threads read the solved
+// values and write the gathered rows at consecutive addresses; the resident rows vt / pt are read and written by index.
+__global__ void __launch_bounds__(256)
+fk_system_sp_gather_scatter_kernel(uint32_t n, uint32_t vb, uint32_t n_vars, uint32_t n_expr, double* __restrict__ vt,
+                                   const double* __restrict__ pt, uint32_t n_scatter, const SpGroup* __restrict__ scatter,
+                                   uint32_t n_reports, uint64_t* __restrict__ reports_out, uint32_t n_perturb,
+                                   const uint32_t* __restrict__ perturb_var, const uint32_t* __restrict__ perturb_draw,
+                                   const double* __restrict__ draws, uint32_t n_gather, const SpGroup* __restrict__ gather,
+                                   const uint8_t* __restrict__ solved, const double* __restrict__ raw_vars, uint32_t raw_vars_stride,
+                                   const double* __restrict__ scales, double* __restrict__ vars_out) {
+    const uint32_t v0 = blockIdx.x * vb;
+    const uint32_t nb = min(vb, n - v0);
+    double* vrow = vt + (size_t)v0 * n_vars;
+    for (uint32_t g = 0; g < n_scatter; g++) {  // assemble/mod.rs:201-208: the set's solution replaces its free variables
+        const SpGroup G = scatter[g];
+        const uint32_t row = G.s.mult * G.s.nf;
+        const double* src = G.s.out + (size_t)v0 * row;
+        for (uint32_t i = threadIdx.x; i < nb * row; i += blockDim.x) {
+            const uint32_t b = i / row, r = i - b * row;
+            vrow[(size_t)b * n_vars + __ldg(G.free_var + r)] = src[i];
+        }
+        constexpr uint32_t W = sizeof(fk_report) / 8;
+        const uint32_t words = G.s.mult * W;
+        const unsigned long long* rsrc = (const unsigned long long*)(G.s.reps + (size_t)v0 * G.s.mult);
+        for (uint32_t i = threadIdx.x; i < nb * words; i += blockDim.x) {
+            const uint32_t b = i / words, r = i - b * words, m = r / W, w = r - m * W;
+            const uint32_t k = __ldg(G.step + m);
+            if (k < n_reports) reports_out[((size_t)(v0 + b) * n_reports + k) * W + w] = rsrc[i];
+        }
+    }
+    __syncthreads();
+    for (uint32_t i = threadIdx.x; i < nb * n_perturb; i += blockDim.x) {  // assemble/mod.rs:113-124, this component's turn
+        const uint32_t b = i / n_perturb, k = i - b * n_perturb;
+        const uint32_t d = __ldg(perturb_draw + k);
+        double& x = vrow[(size_t)b * n_vars + __ldg(perturb_var + k)];
+        x = prepare_perturb(x, __ldg(draws + 2 * (size_t)d), __ldg(draws + 2 * (size_t)d + 1));
+    }
+    __syncthreads();
+    for (uint32_t g = 0; g < n_gather; g++) {
+        const SpGroup G = gather[g];
+        const uint32_t row = G.s.mult * G.s.nv, prow = G.s.mult * G.s.ne;
+        double* ov = G.s.vars + (size_t)v0 * row;
+        for (uint32_t i = threadIdx.x; i < nb * row; i += blockDim.x) {
+            const uint32_t b = i / row, r = i - b * row;
+            ov[i] = vrow[(size_t)b * n_vars + __ldg(G.s.slot_var + r)];
+        }
+        double* op = G.s.params + (size_t)v0 * prow;
+        const double* prow_src = pt + (size_t)v0 * n_expr;
+        for (uint32_t i = threadIdx.x; i < nb * prow; i += blockDim.x) {
+            const uint32_t b = i / prow, r = i - b * prow;
+            op[i] = __ldg(prow_src + (size_t)b * n_expr + __ldg(G.s.expr + r));
+        }
+    }
+    if (!vars_out) return;
+    for (uint32_t i = threadIdx.x; i < nb * n_vars; i += blockDim.x) {  // assemble/mod.rs:201-208: system.variables
+        const uint32_t b = i / n_vars, g = i - b * n_vars;
+        const size_t v = v0 + b;
+        vars_out[v * n_vars + g] = __ldg(solved + g) ? __ldg(scales + v) * vrow[i] : __ldg(raw_vars + v * raw_vars_stride + g);
+    }
+}
+
+int launch_system_sp_gather_scatter(uint32_t n, uint32_t n_vars, uint32_t n_expr, double* vt, const double* pt, uint32_t n_scatter,
+                                    const SpGroup* scatter, uint32_t n_reports, fk_report* reports_out, uint32_t n_perturb,
+                                    const uint32_t* perturb_var, const uint32_t* perturb_draw, const double* draws, uint32_t n_gather,
+                                    const SpGroup* gather, const uint8_t* solved, const double* raw_vars, uint32_t raw_vars_stride,
+                                    const double* scales, double* vars_out, void* stream) {
+    static_assert(sizeof(fk_report) % 8 == 0, "fk_report is moved as 64-bit words");
+    if (n == 0) return 0;
+    // up to 32 variants per CTA, fewer while that leaves under four CTAs per SM
+    const uint32_t vb = std::max<uint32_t>(1, std::min<uint32_t>(32, n / (148u * 4u)));
+    fk_system_sp_gather_scatter_kernel<<<(n + vb - 1) / vb, 256, 0, (cudaStream_t)stream>>>(
+        n, vb, n_vars, n_expr, vt, pt, n_scatter, scatter, n_reports, (uint64_t*)reports_out, n_perturb, perturb_var, perturb_draw, draws,
+        n_gather, gather, solved, raw_vars, raw_vars_stride, scales, vars_out);
+    return (int)cudaGetLastError();
 }
 
 int launch_system_batch_prepare(uint32_t n, uint32_t n_vars, uint32_t n_expr, uint32_t n_constraints, const uint8_t* kinds,

@@ -1,6 +1,7 @@
 // fk_system_batch_solve: System::solve over n variants of one drawing, every component solved in batches on the device.
 // system.cpp describes the drawing (SystemBatchLayout), capi.cu groups its components by structure and runs the chunks,
-// system_batch.cu holds the prepare / gather and scatter kernels.
+// system_batch.cu holds the prepare / gather and scatter kernels.  fk_system_batch_solve_single_pass (Decomposer::SinglePass)
+// shares the layout, the prepare kernel and the structure grouping, and adds the waves of strongly connected sets.
 #pragma once
 #include <cstdint>
 #include <memory>
@@ -26,6 +27,12 @@ struct SystemBatchLayout {
         std::vector<uint32_t> free_var;     // local free column -> system variable
     };
     std::vector<Component> comps;
+    // Decomposer::SinglePass (fk_system_batch_solve_single_pass): comps are the strongly connected sets in the order of the host
+    // loop (slot_draw unused), comp_wave their waves.  Per system variable: var_draw, the draw pair of its component's
+    // perturbation, and var_wave, the wave at whose start that perturbation runs (0: in the prepare kernel); kSbNone for a
+    // variable of no non-empty component's free set.
+    std::vector<uint32_t> comp_wave, var_draw, var_wave;
+    uint32_t n_waves = 0;
 };
 
 // Device descriptor of one structure (components of identical shape) for the two kernels: its batch buffers hold sketch
@@ -56,6 +63,26 @@ int launch_system_batch_scatter(uint32_t n, uint32_t n_vars, const double* raw_v
                                 const uint32_t* comp_member, const SbStructure* structures, double* vars_out, fk_report* reports_out,
                                 void* stream);
 
+// fk_system_batch_solve_single_pass: the sets of one structure inside one wave.  s.vars / s.params / s.out / s.reps are the
+// structure's batch buffers (sketch = variant * mult + member), s.slot_var [mult][nv] and s.expr [mult][ne] the members' rows
+// (s.slot_draw unused); free_var [mult][nf]: system variable of each solved column; step [mult]: the member's set index.
+struct SpGroup {
+    SbStructure s;
+    const uint32_t* free_var;
+    const uint32_t* step;
+};
+
+// One launch between two waves of fk_system_batch_solve_single_pass, per variant v < n on the resident rows vt[v][n_vars]
+// (scaled variables) and pt[v][n_expr] (scaled parameters), in this order: the solved values of the `scatter` groups into vt
+// and their reports into reports_out[v][step] (step < n_reports); the perturbations perturb_var[k] with draw pair
+// perturb_draw[k]; the input rows of the `gather` groups.  vars_out != null: then vars_out[v][i] = scales[v] * vt[v][i] for a
+// variable some set solves (solved[i] != 0), raw_vars[v][i] otherwise.
+int launch_system_sp_gather_scatter(uint32_t n, uint32_t n_vars, uint32_t n_expr, double* vt, const double* pt, uint32_t n_scatter,
+                                    const SpGroup* scatter, uint32_t n_reports, fk_report* reports_out, uint32_t n_perturb,
+                                    const uint32_t* perturb_var, const uint32_t* perturb_draw, const double* draws, uint32_t n_gather,
+                                    const SpGroup* gather, const uint8_t* solved, const double* raw_vars, uint32_t raw_vars_stride,
+                                    const double* scales, double* vars_out, void* stream);
+
 // Host plan of a drawing (capi.cu): components grouped by structure through the topology cache, device state per device.
 struct SystemBatch;
 int system_batch_create(SystemBatchLayout&& layout, const std::vector<const fk_problem*>& problems, std::shared_ptr<SystemBatch>* out);
@@ -74,6 +101,15 @@ struct SystemBatchCall {
 };
 // Refusals (checked before any device work) and the solve.  Errors leave a message for fk_last_error().
 int system_batch_solve(SystemBatch& b, const SystemBatchCall& call);
+
+// The same for Decomposer::SinglePass: layout.comps are the sets (problems: one per set), grouped by structure; per wave one
+// launch per structure present.  (call.optimizer is ignored: the reference runs LM under SinglePass.)
+struct SystemSpBatch;
+int system_sp_batch_create(SystemBatchLayout&& layout, const std::vector<const fk_problem*>& problems, std::shared_ptr<SystemSpBatch>* out);
+// (n_sets, n_waves, n_structures, wave and structure of each set)
+void system_sp_batch_layout(const SystemSpBatch& b, uint32_t* n_sets, uint32_t* n_waves, uint32_t* n_structures,
+                            std::vector<uint32_t>* set_wave, std::vector<uint32_t>* set_structure);
+int system_sp_batch_solve(SystemSpBatch& b, const SystemBatchCall& call);
 // fk_last_error()'s message for errors found outside capi.cu.
 int system_batch_fail(int code, const std::string& msg);
 

@@ -80,6 +80,23 @@ class System:
         (LevenbergMarquardt, the default) or 'lbfgs' (LBfgs)."""
         self._solve(0, perturb, optimizer, lib().fk_system_num_components(self._h))
 
+    def _variant_rows(self, vars, params, n):
+        """(n_variables, vars [count][n_variables] or None, params [count][n_constraints] or None, count) of a batch call."""
+        nv, ncon = lib().fk_system_num_variables(self._h), self.num_constraints()
+        def rows(a, width):
+            a = np.ascontiguousarray(a, dtype=np.float64)
+            return a.reshape(len(a) if a.ndim == 2 else -1, width)
+        if vars is not None:
+            vars = rows(vars, nv)
+        if params is not None:
+            params = rows(params, ncon)
+        sizes = {len(a) for a in (vars, params) if a is not None}
+        if n is not None:
+            sizes.add(int(n))
+        if len(sizes) != 1:
+            raise ValueError("give vars, params or n, with one number of variants")
+        return nv, vars, params, sizes.pop()
+
     def batch_layout(self):
         """(solved components, distinct component structures, [components per structure]) of batch_solve's plan (host
         only)."""
@@ -96,20 +113,7 @@ class System:
         (variables after each variant's solve [n][n_variables], reports [n][solved components] as REPORT_DTYPE)."""
         if optimizer not in _OPTIMIZERS:
             raise ValueError(f"optimizer must be 'lm' or 'lbfgs', not {optimizer!r}")
-        nv, ncon = lib().fk_system_num_variables(self._h), self.num_constraints()
-        def rows(a, width):
-            a = np.ascontiguousarray(a, dtype=np.float64)
-            return a.reshape(len(a) if a.ndim == 2 else -1, width)
-        if vars is not None:
-            vars = rows(vars, nv)
-        if params is not None:
-            params = rows(params, ncon)
-        sizes = {len(a) for a in (vars, params) if a is not None}
-        if n is not None:
-            sizes.add(int(n))
-        if len(sizes) != 1:
-            raise ValueError("give vars, params or n, with one number of variants")
-        count = sizes.pop()
+        nv, vars, params, count = self._variant_rows(vars, params, n)
         n_solved = self.batch_layout()[0]
         out = np.zeros((count, nv))
         reps = np.zeros((count, n_solved), dtype=REPORT_DTYPE)
@@ -125,6 +129,32 @@ class System:
         """System::solve with Decomposer::SinglePass (assemble/mod.rs:169-210) on the GPU.  The reference runs LM here
         whatever the optimizer (assemble/mod.rs:191)."""
         self._solve(1, perturb, optimizer, len(self.single_pass_plan()))
+
+    def single_pass_batch_layout(self):
+        """(sets, waves, distinct set structures, [wave of each set], [structure of each set]) of batch_solve_single_pass's
+        plan (host only)."""
+        n, nw, ns = C.c_uint32(0), C.c_uint32(0), C.c_uint32(0)
+        check(lib().fk_system_single_pass_batch_layout(self._h, C.byref(n), C.byref(nw), C.byref(ns), None, None))
+        wave = np.zeros(max(n.value, 1), np.uint32)
+        struct = np.zeros(max(n.value, 1), np.uint32)
+        check(lib().fk_system_single_pass_batch_layout(self._h, C.byref(n), C.byref(nw), C.byref(ns), ptr(wave, C.c_uint32),
+                                                       ptr(struct, C.c_uint32)))
+        return int(n.value), int(nw.value), int(ns.value), wave[:n.value].tolist(), struct[:n.value].tolist()
+
+    def batch_solve_single_pass(self, vars=None, params=None, perturb=True, n_gpus=1, n=None):
+        """System.solve_single_pass(perturb) of n variants of this drawing in one call (fk_system_batch_solve_single_pass);
+        arguments as batch_solve.  The system itself is not modified.  Returns (variables after each variant's solve
+        [n][n_variables], reports [n][solved sets] as REPORT_DTYPE, in the order solve_single_pass reports them)."""
+        nv, vars, params, count = self._variant_rows(vars, params, n)
+        n_sets = self.single_pass_batch_layout()[0]
+        out = np.zeros((count, nv))
+        reps = np.zeros((count, n_sets), dtype=REPORT_DTYPE)
+        got = C.c_uint32(0)
+        check(lib().fk_system_batch_solve_single_pass(
+            self._h, int(bool(perturb)), count, None if vars is None else ptr(vars, C.c_double),
+            None if params is None else ptr(params, C.c_double), ptr(out, C.c_double),
+            reps.ctypes.data_as(C.POINTER(FkReport)), n_sets, C.byref(got), int(n_gpus)))
+        return out, reps
 
     def solve_recursive_assembly(self, perturb=True, optimizer="lm"):
         """System::solve with Decomposer::RecursiveAssembly (assemble/mod.rs:212-277) on the GPU.  The reference runs LM

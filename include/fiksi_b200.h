@@ -457,6 +457,29 @@ FK_API int fk_system_batch_solve(const fk_system* s, const fk_solving_options* o
 /* Host-only probe of fk_system_batch_solve's plan (no device needed): solved components, distinct component structures,
  * and the components per structure in order of first appearance (multiplicity[n_structures], may be NULL). */
 FK_API int fk_system_batch_layout(const fk_system* s, uint32_t* n_components, uint32_t* n_structures, uint32_t* multiplicity);
+/* == System::solve(SolvingOptions { decomposer: SinglePass, perturb }) (assemble/mod.rs:169-210; the reference runs LM here
+ * whatever the optimizer, :191) applied to n variants of `s`; argument meaning as fk_system_batch_solve.  vars_out[v] and
+ * reports[v] are bit for bit what fk_system_solve_opts(decomposer = 1, perturb) gives on a copy of `s` with the variant's
+ * numbers (a set on the global sparse path runs the sparse batch kernel: the decisions of that call, coordinates within the
+ * documented difference).  reports[v][k]: the k-th solved set in the order fk_system_solve_opts(decomposer = 1) reports them,
+ * the first reports_per_variant of them; *n_solved = sets per variant.  `s` is not modified.
+ * The plan is kept on `s` until a structural edit, like fk_system_batch_solve's: the strongly connected sets, grouped by
+ * structure through the topology cache, and their waves.  A set's wave is one more than the latest wave of the sets it must
+ * follow in the host loop's order (one writes what the other reads or writes, or reads what it writes), directly or through
+ * a component's perturbation; a perturbation runs in the prepare kernel, or at the start of the wave after the last set that
+ * reads its component's variables before it.  On the device, per chunk of variants: one prepare kernel (scale, resident scaled
+ * rows), then per wave one gather / scatter kernel and one batched LM launch per structure present in the wave, and a last
+ * gather / scatter kernel that writes the unscaled rows.  perturb 0 or 1; refusals come before any device work and leave
+ * vars_out untouched: FK_ERR_INVALID for bad arguments, FK_ERR_TOO_LARGE when a set on the global sparse path has a largest
+ * supernodal front above the 236 rows of fk_batch_solve (the message names the set, its first expression and the front).
+ * Variants are chunked (about 1 GiB of device buffers, FK_SYSTEM_BATCH_CHUNK overrides) and sharded over n_gpus devices. */
+FK_API int fk_system_batch_solve_single_pass(const fk_system* s, int perturb, uint32_t n, const double* vars, const double* params,
+                                             double* vars_out, fk_report* reports, uint32_t reports_per_variant,
+                                             uint32_t* n_solved, int n_gpus);
+/* Host-only probe of its plan (no device needed): sets, waves, distinct set structures, and per set its wave and structure
+ * (structures in order of first appearance; step_wave[n_steps] and step_structure[n_steps] may be NULL). */
+FK_API int fk_system_single_pass_batch_layout(const fk_system* s, uint32_t* n_steps, uint32_t* n_waves, uint32_t* n_structures,
+                                              uint32_t* step_wave, uint32_t* step_structure);
 /* Host-only probe of the RecursiveAssembly plan (no device needed) as a stream of 32-bit words: per step
  * n_constraints, constraints..., n_elements, elements..., n_free, free elements..., then the maps on_frontiers,
  * owned_elements, frontier_elements (recursive_assembly.rs:75-114) as n_keys and per key (ascending) key, n,

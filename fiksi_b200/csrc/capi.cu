@@ -2129,6 +2129,7 @@ int system_batch_solve(SystemBatch& b, const SystemBatchCall& c) {
 }
 
 // ---- fk_system_batch_solve_single_pass: Decomposer::SinglePass over n variants of one drawing ---------------------------
+// (fk_system_batch_solve_recursive_assembly runs on the same plan: its steps in place of the sets, with their moves.)
 // The device state of fk_system_batch_solve plus the resident rows of the scaled variables (vt) and parameters (pt) that the
 // waves read and write, and the per-wave descriptors of the gather / scatter kernel.  d_desc holds the one identity structure
 // through which the prepare kernel writes vt and pt; plans are one per structure (capacity chunk * the structure's most sets
@@ -2164,11 +2165,11 @@ struct SystemSpBatch {
     std::vector<uint32_t> set_struct;
     struct Group {  // the sets of one structure in one wave, in plan order: the tables of its SpGroup
         uint32_t structure = 0;
-        std::vector<uint32_t> sets, slot_var, expr, free_var;
+        std::vector<uint32_t> sets, slot_var, expr, free_var, move_off{0}, moves;
     };
     std::vector<std::vector<Group>> waves;
     std::vector<std::vector<uint32_t>> wave_perturb;  // variables whose perturbation runs at the start of wave w >= 1
-    std::vector<uint8_t> solved;                      // per system variable: some set solves it
+    std::vector<uint8_t> solved;                      // per system variable: some set solves it (or a step moves it)
     std::mutex mu;
     std::map<int, std::unique_ptr<SystemSpDevice>> devices;
 };
@@ -2206,8 +2207,12 @@ int system_sp_batch_create(SystemBatchLayout&& layout, const std::vector<const f
         it->slot_var.insert(it->slot_var.end(), c.slot_var.begin(), c.slot_var.end());
         it->expr.insert(it->expr.end(), c.expr.begin(), c.expr.end());
         it->free_var.insert(it->free_var.end(), c.free_var.begin(), c.free_var.end());
+        it->moves.insert(it->moves.end(), c.moves.begin(), c.moves.end());
+        it->move_off.push_back((uint32_t)(it->moves.size() / 2));
         b->st[si].wave_mult = std::max(b->st[si].wave_mult, (uint32_t)it->sets.size());
-        for (uint32_t g : c.free_var) b->solved[g] = 1;
+        for (uint32_t g : c.free_var)
+            if (g != kSbNone) b->solved[g] = 1;
+        for (size_t m = 0; m < c.moves.size(); m += 2) b->solved[c.moves[m]] = b->solved[c.moves[m] + 1] = 1;
     }
     // (a perturbation scheduled behind the last wave precedes no set: nothing reads it, and vars_out keeps unsolved variables raw)
     b->wave_perturb.assign(L.n_waves, {});
@@ -2288,10 +2293,11 @@ static int system_sp_device(SystemSpBatch& b, SystemSpDevice* d, int device, uin
         };
         const size_t o_kind = add(L.kind), o_con = add(L.expr_constraint), o_draws = add(L.draws), o_iv = add(ident_var), o_id = add(ident_draw),
                      o_ie = add(ident_expr), o_solved = add(b.solved), o_pv = add(pvar), o_pd = add(pdraw);
-        struct GroupAt { size_t sv, ex, fv, st; };
+        struct GroupAt { size_t sv, ex, fv, st, mo, mv; };
         std::vector<GroupAt> at;
         for (const auto& wave : b.waves)
-            for (const SystemSpBatch::Group& g : wave) at.push_back({add(g.slot_var), add(g.expr), add(g.free_var), add(g.sets)});
+            for (const SystemSpBatch::Group& g : wave)
+                at.push_back({add(g.slot_var), add(g.expr), add(g.free_var), add(g.sets), add(g.move_off), add(g.moves)});
         std::vector<unsigned char> host(off + 16, 0);
         for (const Item& it : items)
             if (it.bytes) std::memcpy(host.data() + it.at, it.src, it.bytes);
@@ -2317,6 +2323,7 @@ static int system_sp_device(SystemSpBatch& b, SystemSpDevice* d, int device, uin
                 SpGroup G{};
                 G.s.slot_var = (const uint32_t*)(t + at[q].sv); G.s.expr = (const uint32_t*)(t + at[q].ex);
                 G.free_var = (const uint32_t*)(t + at[q].fv); G.step = (const uint32_t*)(t + at[q].st);
+                G.move_off = (const uint32_t*)(t + at[q].mo); G.moves = (const uint32_t*)(t + at[q].mv);
                 G.s.nv = tp.n_vars; G.s.ne = tp.n_expr; G.s.nf = tp.n_free; G.s.mult = (uint32_t)g.sets.size();
                 d->groups.push_back(G);
                 q++;
@@ -2415,7 +2422,7 @@ static int system_sp_range(SystemSpBatch& b, const SystemBatchCall& c, int devic
                                                     d->d_solved, raw, raw_stride, d->d_scales, w == nw ? d->d_vars_out : nullptr, st);
                 if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_sp_gather_scatter_kernel");
                 if (w == nw) break;
-                for (const SystemSpBatch::Group& g : b.waves[w]) {  // LM under SinglePass whatever the optimizer (assemble/mod.rs:191)
+                for (const SystemSpBatch::Group& g : b.waves[w]) {  // LM under SinglePass / RecursiveAssembly whatever the optimizer (assemble/mod.rs:191, :224)
                     fk_batch_plan* p = d->plans[g.structure];
                     p->n = cnt * (uint32_t)g.sets.size();
                     const int r = fk_batch_plan_run(p, st);
@@ -2433,16 +2440,18 @@ static int system_sp_range(SystemSpBatch& b, const SystemBatchCall& c, int devic
     rc = run();
     // (also after an error: no copy into the caller's buffers may still be running when the call returns)
     const cudaError_t e = cudaStreamSynchronize(st);
-    if (rc == FK_OK && e != cudaSuccess) rc = cuda_fail(e, "fk_system_batch_solve_single_pass kernels / copies");
+    if (rc == FK_OK && e != cudaSuccess) rc = cuda_fail(e, "fk_system_batch_solve_single_pass / _recursive_assembly kernels / copies");
     return rc;
 }
 
 int system_sp_batch_solve(SystemSpBatch& b, const SystemBatchCall& c) {
-    for (const SystemSpBatch::Structure& S : b.st)  // sets on the global sparse path: the front limit of fk_batch_solve
+    for (const SystemSpBatch::Structure& S : b.st)  // sets / steps on the global sparse path: the front limit of fk_batch_solve
         if (S.topo->t.path == 2 && S.topo->sb_check() != FK_OK) {
             const uint32_t k = S.members[0];
-            return fail(FK_ERR_TOO_LARGE, "set " + std::to_string(k) + " (first expression " + std::to_string(b.L.comps[k].expr[0]) +
-                                              "): " + S.topo->sb_err + "; fk_system_solve_opts solves it one variant at a time");
+            const std::string what = b.L.step_constraint.empty()
+                                         ? "set " + std::to_string(k) + " (first expression " + std::to_string(b.L.comps[k].expr[0])
+                                         : "step " + std::to_string(k) + " (first constraint " + std::to_string(b.L.step_constraint[k]);
+            return fail(FK_ERR_TOO_LARGE, what + "): " + S.topo->sb_err + "; fk_system_solve_opts solves it one variant at a time");
         }
     if (c.n == 0) return FK_OK;
     int n_gpus = c.n_gpus;

@@ -69,6 +69,7 @@ struct fk_system {
     mutable std::mutex batch_mu;
     mutable std::shared_ptr<fk::SystemBatch> batch;
     mutable std::shared_ptr<fk::SystemSpBatch> sp_batch;  // fk_system_batch_solve_single_pass's plan, kept and dropped alike
+    mutable std::shared_ptr<fk::SystemSpBatch> ra_batch;  // fk_system_batch_solve_recursive_assembly's plan, kept and dropped alike
 
     uint32_t new_element(uint8_t tag, uint32_t a, uint32_t b, const double* v, int nv) {
         uint32_t id = (uint32_t)elems.size();
@@ -131,6 +132,7 @@ struct fk_system {
         std::lock_guard<std::mutex> lock(batch_mu);
         batch.reset();
         sp_batch.reset();
+        ra_batch.reset();
     }
     void push_expr(uint8_t k, uint32_t i0, uint32_t i1, uint32_t i2, uint32_t i3, double p) {
         kind.push_back(k);
@@ -488,6 +490,7 @@ struct ClusteredProblem {
     std::vector<uint32_t> elements;                                        // step_plus_frontier_elements
     std::vector<std::pair<uint32_t, std::vector<uint32_t>>> clusters;      // cluster key -> frontier points, in first-seen order
     std::map<uint32_t, uint32_t> slot;                                     // system variable -> free variable of the step
+    std::vector<uint32_t> var_global, expr_global;  // local variable / expression -> system one, fk::kSbNone for a pose's
     std::vector<double> vars, param, x;
     std::vector<uint8_t> kind;
     std::vector<uint32_t> idx, free_vars, rows;
@@ -532,12 +535,14 @@ struct ClusteredProblem {
         }
         // free variables (:432-477)
         vars.assign(clusters.size() * 3, 0.0);
+        var_global.assign(clusters.size() * 3, fk::kSbNone);
         for (uint32_t el : elements) {
             const Elem& e = s->elems[el];
             const int n = e.tag == kLength ? 1 : (e.tag == kPoint ? 2 : 0);
             for (int k = 0; k < n; k++) {
                 slot[e.a + k] = (uint32_t)vars.size();
                 vars.push_back(vt[e.a + k]);
+                var_global.push_back(e.a + k);
             }
         }
         const uint32_t n_free = (uint32_t)vars.size();
@@ -550,7 +555,10 @@ struct ClusteredProblem {
                 const uint32_t at = (uint32_t)vars.size();
                 vars.push_back(vt[pv]);      // the point before the step: constant of the two rows
                 vars.push_back(vt[pv + 1]);
+                var_global.push_back(pv);
+                var_global.push_back(pv + 1);
                 for (int y = 0; y < 2; y++) {
+                    expr_global.push_back(fk::kSbNone);
                     rows.push_back((uint32_t)kind.size());
                     kind.push_back(y ? FK_POSE_POINT_Y : FK_POSE_POINT_X);
                     param.push_back(0.0);
@@ -561,6 +569,7 @@ struct ClusteredProblem {
         for (uint32_t c : step.constraints)
             for (uint8_t k = 0; k < s->constrs[c].n_expr; k++) {
                 const uint32_t e = s->constrs[c].first_expr + k;
+                expr_global.push_back(e);
                 rows.push_back((uint32_t)kind.size());
                 kind.push_back(s->kind[e]);
                 param.push_back(pt[e]);
@@ -581,6 +590,9 @@ struct ClusteredProblem {
         return true;
     }
 };
+
+// the reference panics here: unwrap on a missing cluster entry (recursive_assembly.rs:352-373)
+const char kRaPanic[] = "recursive assembly: the decomposition reaches a cluster without bookkeeping (the reference panics on this system)";
 
 // == System::solve(SolvingOptions { optimizer: LevenbergMarquardt, decomposer: RecursiveAssembly, perturb })
 // (assemble/mod.rs:212-277): every step of every component's plan is one LM solve on the GPU; afterwards the points a
@@ -615,8 +627,8 @@ int solve_recursive_assembly(fk_system* s, int perturb, fk_report* reports, uint
         std::vector<fk::RaStep> steps;
         try {
             steps = component_plan(s, c);
-        } catch (const std::out_of_range&) {  // the reference panics here: unwrap on a missing cluster entry (recursive_assembly.rs:352-373)
-            s->error = "recursive assembly: the decomposition reaches a cluster without bookkeeping (the reference panics on this system)";
+        } catch (const std::out_of_range&) {
+            s->error = kRaPanic;
             return FK_ERR_INVALID;
         }
         for (const fk::RaStep& step : steps) {
@@ -910,37 +922,75 @@ int batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemBatch>* out) {
     return FK_OK;
 }
 
+// The waves of the batched SinglePass and RecursiveAssembly plans.  The host loop is a sequence of nodes: per non-empty
+// component its perturbation (reads and writes the component's free variables) followed by its sets or steps.  Node b follows
+// an earlier node a when a writes what b reads or writes, or reads what b writes.  Times: a set or step of wave w at 2w + 1, a
+// perturbation at the start of wave w at 2w; every node goes to the earliest time after all nodes it follows (ASAP).  The
+// perturbation nodes count whether or not the call perturbs, so the waves do not depend on it.  Any schedule that respects
+// the edges computes the host loop's values.
+struct WaveScheduler {
+    std::vector<int64_t> last_write, last_read;  // per system variable: latest time of a writer / reader
+    explicit WaveScheduler(size_t n_vars) : last_write(n_vars, -1), last_read(n_vars, -1) {}
+    // earliest time after every node that the node reading `reads` and writing `writes` (a subset of reads) follows
+    int64_t earliest(const std::vector<uint32_t>& reads, const std::vector<uint32_t>& writes) const {
+        int64_t t = -1;
+        for (uint32_t g : reads) t = std::max(t, last_write[g]);
+        for (uint32_t g : writes) t = std::max(t, last_read[g]);
+        return t + 1;
+    }
+    void place(const std::vector<uint32_t>& reads, const std::vector<uint32_t>& writes, int64_t time) {
+        for (uint32_t g : reads) last_read[g] = std::max(last_read[g], time);
+        for (uint32_t g : writes) last_write[g] = std::max(last_write[g], time);
+    }
+    // a component's perturbation: the first wave start at or after its earliest time
+    uint32_t perturbation(const std::vector<uint32_t>& free_sorted) {
+        const uint32_t pw = (uint32_t)((earliest(free_sorted, free_sorted) + 1) / 2);
+        place(free_sorted, free_sorted, 2 * (int64_t)pw);
+        return pw;
+    }
+    // a set or step: the first solve time 2w + 1 at or after its earliest time
+    uint32_t solve(const std::vector<uint32_t>& reads, const std::vector<uint32_t>& writes) {
+        const uint32_t w = (uint32_t)(earliest(reads, writes) / 2);
+        place(reads, writes, 2 * (int64_t)w + 1);
+        return w;
+    }
+};
+
+// The parts of a wave plan that do not depend on the decomposer: the expressions and, per variable, no draw yet.
+fk::SystemBatchLayout wave_layout(const fk_system* s) {
+    fk::SystemBatchLayout lay;
+    lay.n_vars = (uint32_t)s->vars.size();
+    lay.n_constraints = (uint32_t)s->constrs.size();
+    lay.kind = s->kind;
+    lay.expr_constraint.assign(s->kind.size(), fk::kSbNone);
+    for (uint32_t c = 0; c < s->constrs.size(); c++) lay.expr_constraint[s->constrs[c].first_expr] = c;  // update_parameter
+    lay.var_draw.assign(s->vars.size(), fk::kSbNone);
+    lay.var_wave.assign(s->vars.size(), fk::kSbNone);
+    return lay;
+}
+
+// A component's perturbation node: its wave, and the draws of batch_plan_for for its free variables.
+int perturbation_node(fk::SystemBatchLayout& lay, WaveScheduler& sched, Lcg& rng, const std::vector<uint32_t>& free_sorted) {
+    const uint32_t pw = sched.perturbation(free_sorted);
+    for (uint32_t fv : free_sorted) {
+        if (lay.var_draw[fv] != fk::kSbNone) return fk::system_batch_fail(FK_ERR_INTERNAL, "a variable is free in two components");
+        lay.var_draw[fv] = (uint32_t)(lay.draws.size() / 2);
+        lay.var_wave[fv] = pw;
+        lay.draws.push_back(rng.next());
+        lay.draws.push_back(rng.next());
+    }
+    return FK_OK;
+}
+
 // fk_system_batch_solve_single_pass's plan: the sets of fk_system_solve_opts(decomposer = 1) in its order, each as its
-// LocalProblem numbering, the draws of batch_plan_for, and the waves.  The host loop is a sequence of nodes: per non-empty
-// component its perturbation (reads and writes the component's free variables) followed by its sets (read their variables,
-// write their free ones).  Node b follows an earlier node a when a writes what b reads or writes, or reads what b writes; sets
-// reach across components (SinglePass plans over the equation graph of every expression), so these edges are computed, not
-// assumed.  Times: a set of wave w at 2w + 1, a perturbation at the start of wave w at 2w; every node goes to the earliest
-// time after all nodes it follows (ASAP).  The perturbation nodes count whether or not the call perturbs, so the waves do not
-// depend on it.  Any schedule that respects the edges computes the host loop's values.
+// LocalProblem numbering (read: its variables, written: its free ones), the draws of batch_plan_for, and the waves.  Sets
+// reach across components (SinglePass plans over the equation graph of every expression), so the edges between nodes are
+// computed, not assumed.
 int single_pass_batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemSpBatch>* out) {
     std::lock_guard<std::mutex> lock(s->batch_mu);
     if (!s->sp_batch) {
-        fk::SystemBatchLayout lay;
-        lay.n_vars = (uint32_t)s->vars.size();
-        lay.n_constraints = (uint32_t)s->constrs.size();
-        lay.kind = s->kind;
-        lay.expr_constraint.assign(s->kind.size(), fk::kSbNone);
-        for (uint32_t c = 0; c < s->constrs.size(); c++) lay.expr_constraint[s->constrs[c].first_expr] = c;  // update_parameter
-        lay.var_draw.assign(s->vars.size(), fk::kSbNone);
-        lay.var_wave.assign(s->vars.size(), fk::kSbNone);
-        std::vector<int64_t> last_write(s->vars.size(), -1), last_read(s->vars.size(), -1);  // latest time of a writer / reader
-        // earliest time after every node that the node reading `reads` and writing `writes` (a subset of reads) follows
-        auto earliest = [&](const std::vector<uint32_t>& reads, const std::vector<uint32_t>& writes) {
-            int64_t t = -1;
-            for (uint32_t g : reads) t = std::max(t, last_write[g]);
-            for (uint32_t g : writes) t = std::max(t, last_read[g]);
-            return t + 1;
-        };
-        auto place = [&](const std::vector<uint32_t>& reads, const std::vector<uint32_t>& writes, int64_t time) {
-            for (uint32_t g : reads) last_read[g] = std::max(last_read[g], time);
-            for (uint32_t g : writes) last_write[g] = std::max(last_write[g], time);
-        };
+        fk::SystemBatchLayout lay = wave_layout(s);
+        WaveScheduler sched(s->vars.size());
         std::vector<std::vector<uint32_t>> var_exprs, expr_vars;
         equation_graph(s, var_exprs, expr_vars);
         fk::SinglePassPlanner planner(var_exprs, expr_vars);
@@ -949,21 +999,12 @@ int single_pass_batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemSpB
         for (const fk_system::Comp& c : s->comps) {
             if (c.elements.empty()) continue;  // assemble/mod.rs:87-89
             const std::vector<uint32_t> free_sorted = component_free_variables(s, c);
-            const int64_t tp = earliest(free_sorted, free_sorted);
-            const uint32_t pw = (uint32_t)((tp + 1) / 2);  // first wave start at or after tp
-            for (uint32_t fv : free_sorted) {
-                if (lay.var_draw[fv] != fk::kSbNone) return fk::system_batch_fail(FK_ERR_INTERNAL, "a variable is free in two components");
-                lay.var_draw[fv] = (uint32_t)(lay.draws.size() / 2);
-                lay.var_wave[fv] = pw;
-                lay.draws.push_back(rng.next());
-                lay.draws.push_back(rng.next());
-            }
-            place(free_sorted, free_sorted, 2 * (int64_t)pw);
+            const int rc = perturbation_node(lay, sched, rng, free_sorted);
+            if (rc != FK_OK) return rc;
             for (const fk::SinglePassStep& st : planner.plan(free_sorted)) {
                 std::unique_ptr<LocalProblem> L(new LocalProblem());
                 build_local(s, s->vars, s->param, st.free_variables, st.expressions, *L);
-                const uint32_t w = (uint32_t)(earliest(L->slot_global, st.free_variables) / 2);  // first set time 2w + 1 at or after it
-                place(L->slot_global, st.free_variables, 2 * (int64_t)w + 1);
+                const uint32_t w = sched.solve(L->slot_global, st.free_variables);
                 fk::SystemBatchLayout::Component comp;
                 comp.slot_var = L->slot_global;
                 comp.expr = st.expressions;
@@ -981,6 +1022,110 @@ int single_pass_batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemSpB
     }
     *out = s->sp_batch;
     return FK_OK;
+}
+
+// fk_system_batch_solve_recursive_assembly's plan: the steps of fk_system_solve_opts(decomposer = 2) in its order, each as
+// its ClusteredProblem (built once on the template values: its structure does not depend on them), the draws of
+// batch_plan_for, and the waves.  A step reads its variables (element variables and the point copies behind them) and the
+// points it moves, and writes its element variables and the points it moves; the moves are the host loop's, in its order.
+int recursive_assembly_batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemSpBatch>* out) {
+    std::lock_guard<std::mutex> lock(s->batch_mu);
+    if (!s->ra_batch) {
+        fk::SystemBatchLayout lay = wave_layout(s);
+        WaveScheduler sched(s->vars.size());
+        std::vector<std::unique_ptr<ClusteredProblem>> problems;
+        Lcg rng{42};
+        for (const fk_system::Comp& c : s->comps) {
+            if (c.elements.empty()) continue;  // assemble/mod.rs:87-89
+            const int rc = perturbation_node(lay, sched, rng, component_free_variables(s, c));
+            if (rc != FK_OK) return rc;
+            std::vector<fk::RaStep> steps;
+            try {
+                steps = component_plan(s, c);
+            } catch (const std::out_of_range&) {
+                return fk::system_batch_fail(FK_ERR_INVALID, kRaPanic);
+            }
+            for (const fk::RaStep& step : steps) {
+                std::unique_ptr<ClusteredProblem> P(new ClusteredProblem());
+                if (!P->build(s, step, s->vars, s->param)) return fk::system_batch_fail(FK_ERR_INVALID, P->error);
+                fk::SystemBatchLayout::Component comp;
+                comp.slot_var = P->var_global;
+                comp.expr = P->expr_global;
+                comp.free_var.assign(P->var_global.begin(), P->var_global.begin() + P->prob.n_free);
+                for (size_t ci = 0; ci < P->clusters.size(); ci++) {  // as solve_recursive_assembly walks them (:235-273)
+                    const std::vector<uint32_t>* owned = find_list(step.owned_elements, P->clusters[ci].first);
+                    if (!owned) continue;
+                    for (uint32_t el : *owned) {
+                        if (std::find(P->elements.begin(), P->elements.end(), el) != P->elements.end() || s->elems[el].tag != kPoint) continue;
+                        comp.moves.push_back(s->elems[el].a);
+                        comp.moves.push_back((uint32_t)(3 * ci));
+                    }
+                }
+                std::vector<uint32_t> reads, writes;
+                for (uint32_t g : comp.slot_var)
+                    if (g != fk::kSbNone) reads.push_back(g);
+                for (uint32_t g : comp.free_var)
+                    if (g != fk::kSbNone) writes.push_back(g);
+                for (size_t m = 0; m < comp.moves.size(); m += 2)
+                    for (uint32_t y = 0; y < 2; y++) {
+                        reads.push_back(comp.moves[m] + y);
+                        writes.push_back(comp.moves[m] + y);
+                    }
+                const uint32_t w = sched.solve(reads, writes);
+                lay.comps.push_back(std::move(comp));
+                lay.comp_wave.push_back(w);
+                lay.step_constraint.push_back(step.constraints[0]);
+                lay.n_waves = std::max(lay.n_waves, w + 1);
+                problems.push_back(std::move(P));
+            }
+        }
+        std::vector<const fk_problem*> probs;
+        for (const auto& P : problems) probs.push_back(&P->prob);
+        const int rc = fk::system_sp_batch_create(std::move(lay), probs, &s->ra_batch);
+        if (rc != FK_OK) return rc;
+    }
+    *out = s->ra_batch;
+    return FK_OK;
+}
+
+// The host probe and the call of the two wave plans (SinglePass, RecursiveAssembly), given how to build the plan.
+using WavePlanFor = int (*)(const fk_system*, std::shared_ptr<fk::SystemSpBatch>*);
+
+int wave_batch_layout(WavePlanFor plan_for, const fk_system* s, uint32_t* n_steps, uint32_t* n_waves, uint32_t* n_structures,
+                      uint32_t* step_wave, uint32_t* step_structure) {
+    if (!s) return fk::system_batch_fail(FK_ERR_INVALID, "null system");
+    std::shared_ptr<fk::SystemSpBatch> b;
+    const int rc = plan_for(s, &b);
+    if (rc != FK_OK) return rc;
+    std::vector<uint32_t> wave, structure;
+    fk::system_sp_batch_layout(*b, n_steps, n_waves, n_structures, &wave, &structure);
+    if (step_wave) std::copy(wave.begin(), wave.end(), step_wave);
+    if (step_structure) std::copy(structure.begin(), structure.end(), step_structure);
+    return FK_OK;
+}
+
+int wave_batch_solve(WavePlanFor plan_for, const fk_system* s, int perturb, uint32_t n, const double* vars, const double* params,
+                     double* vars_out, fk_report* reports, uint32_t reports_per_variant, uint32_t* n_solved, int n_gpus) {
+    if (!s || !vars_out) return fk::system_batch_fail(FK_ERR_INVALID, "null system or vars_out");
+    if (perturb != 0 && perturb != 1) return fk::system_batch_fail(FK_ERR_INVALID, "perturb must be 0 or 1");
+    std::shared_ptr<fk::SystemSpBatch> b;
+    int rc = plan_for(s, &b);
+    if (rc != FK_OK) return rc;
+    uint32_t n_steps = 0;
+    fk::system_sp_batch_layout(*b, &n_steps, nullptr, nullptr, nullptr, nullptr);
+    if (n_solved) *n_solved = n_steps;
+    fk::SystemBatchCall c;
+    c.perturb = perturb;
+    c.n_gpus = n_gpus;
+    c.n = n;
+    c.vars = vars;
+    c.params = params;
+    c.tmpl_vars = s->vars.data();
+    c.tmpl_param = s->param.data();
+    c.vars_out = vars_out;
+    c.reports = reports;
+    c.reports_per_variant = reports_per_variant;
+    return fk::system_sp_batch_solve(*b, c);
 }
 
 }  // namespace
@@ -1027,39 +1172,24 @@ int fk_system_batch_solve(const fk_system* s, const fk_solving_options* opts, ui
 
 int fk_system_single_pass_batch_layout(const fk_system* s, uint32_t* n_steps, uint32_t* n_waves, uint32_t* n_structures,
                                        uint32_t* step_wave, uint32_t* step_structure) {
-    if (!s) return fk::system_batch_fail(FK_ERR_INVALID, "null system");
-    std::shared_ptr<fk::SystemSpBatch> b;
-    const int rc = single_pass_batch_plan_for(s, &b);
-    if (rc != FK_OK) return rc;
-    std::vector<uint32_t> set_wave, set_structure;
-    fk::system_sp_batch_layout(*b, n_steps, n_waves, n_structures, &set_wave, &set_structure);
-    if (step_wave) std::copy(set_wave.begin(), set_wave.end(), step_wave);
-    if (step_structure) std::copy(set_structure.begin(), set_structure.end(), step_structure);
-    return FK_OK;
+    return wave_batch_layout(single_pass_batch_plan_for, s, n_steps, n_waves, n_structures, step_wave, step_structure);
 }
 
 int fk_system_batch_solve_single_pass(const fk_system* s, int perturb, uint32_t n, const double* vars, const double* params,
                                       double* vars_out, fk_report* reports, uint32_t reports_per_variant, uint32_t* n_solved, int n_gpus) {
-    if (!s || !vars_out) return fk::system_batch_fail(FK_ERR_INVALID, "null system or vars_out");
-    if (perturb != 0 && perturb != 1) return fk::system_batch_fail(FK_ERR_INVALID, "perturb must be 0 or 1");
-    std::shared_ptr<fk::SystemSpBatch> b;
-    int rc = single_pass_batch_plan_for(s, &b);
-    if (rc != FK_OK) return rc;
-    uint32_t n_sets = 0;
-    fk::system_sp_batch_layout(*b, &n_sets, nullptr, nullptr, nullptr, nullptr);
-    if (n_solved) *n_solved = n_sets;
-    fk::SystemBatchCall c;
-    c.perturb = perturb;
-    c.n_gpus = n_gpus;
-    c.n = n;
-    c.vars = vars;
-    c.params = params;
-    c.tmpl_vars = s->vars.data();
-    c.tmpl_param = s->param.data();
-    c.vars_out = vars_out;
-    c.reports = reports;
-    c.reports_per_variant = reports_per_variant;
-    return fk::system_sp_batch_solve(*b, c);
+    return wave_batch_solve(single_pass_batch_plan_for, s, perturb, n, vars, params, vars_out, reports, reports_per_variant, n_solved, n_gpus);
+}
+
+int fk_system_recursive_assembly_batch_layout(const fk_system* s, uint32_t* n_steps, uint32_t* n_waves, uint32_t* n_structures,
+                                              uint32_t* step_wave, uint32_t* step_structure) {
+    return wave_batch_layout(recursive_assembly_batch_plan_for, s, n_steps, n_waves, n_structures, step_wave, step_structure);
+}
+
+int fk_system_batch_solve_recursive_assembly(const fk_system* s, int perturb, uint32_t n, const double* vars, const double* params,
+                                             double* vars_out, fk_report* reports, uint32_t reports_per_variant, uint32_t* n_solved,
+                                             int n_gpus) {
+    return wave_batch_solve(recursive_assembly_batch_plan_for, s, perturb, n, vars, params, vars_out, reports, reports_per_variant,
+                            n_solved, n_gpus);
 }
 
 }  // extern "C"

@@ -1,8 +1,8 @@
 // Kernels of fk_system_batch_solve (System::solve over n variants of one drawing): the scale, perturbation and gather of
 // every component's input rows into its structure's batch buffers, and the write-back of the solved components into the
 // variants' variable rows.  The arithmetic of the pre-processing is prepare.cuh's, shared with fk_batch_prepare_kernel.
-// fk_system_batch_solve_single_pass reuses the prepare kernel (one identity structure: the resident scaled rows) and moves
-// values between the waves of strongly connected sets with fk_system_sp_gather_scatter_kernel.
+// fk_system_batch_solve_single_pass and _recursive_assembly reuse the prepare kernel (one identity structure: the resident
+// scaled rows) and move values between the waves of sets or steps with fk_system_sp_gather_scatter_kernel.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -96,10 +96,12 @@ fk_system_batch_scatter_kernel(uint32_t n, uint32_t n_vars, const double* __rest
     }
 }
 
-// Between two waves of fk_system_batch_solve_single_pass.  One CTA per `vb` consecutive variants, so that the phases (scatter,
-// perturbations, gather, write-back) of a variant are ordered by __syncthreads alone.  A group's rows of variants
-// [v0, v0 + nb) are contiguous in its batch buffers (sketch = variant * mult + member): consecutive threads read the solved
-// values and write the gathered rows at consecutive addresses; the resident rows vt / pt are read and written by index.
+// Between two waves of fk_system_batch_solve_single_pass / _recursive_assembly.  One CTA per `vb` consecutive variants, so
+// that the phases (scatter, moves and reports, perturbations, gather, write-back) of a variant are ordered by __syncthreads
+// alone.  A group's rows of variants [v0, v0 + nb) are contiguous in its batch buffers (sketch = variant * mult + member):
+// consecutive threads read the solved values and write the gathered rows at consecutive addresses; the resident rows vt / pt
+// are read and written by index.  Steps of one wave move disjoint points (the waves order every step after the steps that
+// read or write what it writes), so one thread per (variant, step) applies that step's moves in their recorded order.
 __global__ void __launch_bounds__(256)
 fk_system_sp_gather_scatter_kernel(uint32_t n, uint32_t vb, uint32_t n_vars, uint32_t n_expr, double* __restrict__ vt,
                                    const double* __restrict__ pt, uint32_t n_scatter, const SpGroup* __restrict__ scatter,
@@ -111,13 +113,34 @@ fk_system_sp_gather_scatter_kernel(uint32_t n, uint32_t vb, uint32_t n_vars, uin
     const uint32_t v0 = blockIdx.x * vb;
     const uint32_t nb = min(vb, n - v0);
     double* vrow = vt + (size_t)v0 * n_vars;
-    for (uint32_t g = 0; g < n_scatter; g++) {  // assemble/mod.rs:201-208: the set's solution replaces its free variables
+    for (uint32_t g = 0; g < n_scatter; g++) {  // assemble/mod.rs:201-208 (:226-233): the solution replaces its free variables
         const SpGroup G = scatter[g];
         const uint32_t row = G.s.mult * G.s.nf;
         const double* src = G.s.out + (size_t)v0 * row;
         for (uint32_t i = threadIdx.x; i < nb * row; i += blockDim.x) {
             const uint32_t b = i / row, r = i - b * row;
-            vrow[(size_t)b * n_vars + __ldg(G.free_var + r)] = src[i];
+            const uint32_t f = __ldg(G.free_var + r);
+            if (f != kSbNone) vrow[(size_t)b * n_vars + f] = src[i];
+        }
+    }
+    __syncthreads();
+    for (uint32_t g = 0; g < n_scatter; g++) {
+        const SpGroup G = scatter[g];
+        const uint32_t row = G.s.mult * G.s.nf;
+        for (uint32_t i = threadIdx.x; i < nb * G.s.mult; i += blockDim.x) {  // assemble/mod.rs:235-273: owned points follow the pose
+            const uint32_t b = i / G.s.mult, m = i - b * G.s.mult;
+            const double* x = G.s.out + (size_t)(v0 + b) * row + (size_t)m * G.s.nf;
+            double* p = vrow + (size_t)b * n_vars;
+            for (uint32_t k = __ldg(G.move_off + m), end = __ldg(G.move_off + m + 1); k < end; k++) {
+                const uint32_t pv = __ldg(G.moves + 2 * (size_t)k), col = __ldg(G.moves + 2 * (size_t)k + 1);
+                const double tx = x[col + 1], ty = x[col + 2];
+                double sn, cs;
+                sincos(x[col], &sn, &cs);
+                const double u = p[pv], w = p[pv + 1];  // Pose2D::transform_point, expressions.rs:1122-1136
+                const double uc = u * cs, us = u * sn, vc = w * cs, vs = w * sn;
+                p[pv] = tx + uc - vs;
+                p[pv + 1] = ty + us + vc;
+            }
         }
         constexpr uint32_t W = sizeof(fk_report) / 8;
         const uint32_t words = G.s.mult * W;
@@ -142,13 +165,15 @@ fk_system_sp_gather_scatter_kernel(uint32_t n, uint32_t vb, uint32_t n_vars, uin
         double* ov = G.s.vars + (size_t)v0 * row;
         for (uint32_t i = threadIdx.x; i < nb * row; i += blockDim.x) {
             const uint32_t b = i / row, r = i - b * row;
-            ov[i] = vrow[(size_t)b * n_vars + __ldg(G.s.slot_var + r)];
+            const uint32_t sv = __ldg(G.s.slot_var + r);
+            ov[i] = sv == kSbNone ? 0.0 : vrow[(size_t)b * n_vars + sv];  // (a pose column starts at the identity)
         }
         double* op = G.s.params + (size_t)v0 * prow;
         const double* prow_src = pt + (size_t)v0 * n_expr;
         for (uint32_t i = threadIdx.x; i < nb * prow; i += blockDim.x) {
             const uint32_t b = i / prow, r = i - b * prow;
-            op[i] = __ldg(prow_src + (size_t)b * n_expr + __ldg(G.s.expr + r));
+            const uint32_t e = __ldg(G.s.expr + r);
+            op[i] = e == kSbNone ? 0.0 : __ldg(prow_src + (size_t)b * n_expr + e);
         }
     }
     if (!vars_out) return;

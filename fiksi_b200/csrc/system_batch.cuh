@@ -1,7 +1,9 @@
 // fk_system_batch_solve: System::solve over n variants of one drawing, every component solved in batches on the device.
 // system.cpp describes the drawing (SystemBatchLayout), capi.cu groups its components by structure and runs the chunks,
 // system_batch.cu holds the prepare / gather and scatter kernels.  fk_system_batch_solve_single_pass (Decomposer::SinglePass)
-// shares the layout, the prepare kernel and the structure grouping, and adds the waves of strongly connected sets.
+// shares the layout, the prepare kernel and the structure grouping, and adds the waves of strongly connected sets;
+// fk_system_batch_solve_recursive_assembly (Decomposer::RecursiveAssembly) runs on the same waves with the recombination steps
+// in place of the sets, plus the owned-point moves that follow each step.
 #pragma once
 #include <cstdint>
 #include <memory>
@@ -25,6 +27,10 @@ struct SystemBatchLayout {
         std::vector<uint32_t> slot_draw;    // local variable -> draw pair already applied at the component's snapshot, or kSbNone
         std::vector<uint32_t> expr;         // local expression -> system expression
         std::vector<uint32_t> free_var;     // local free column -> system variable
+        // Decomposer::RecursiveAssembly: pairs (first variable of a point the step's cluster moves, the cluster's first pose
+        // column) in the host loop's order.  A pose column has slot_var and free_var kSbNone (gathered as 0.0, never
+        // scattered), a pose row expr kSbNone (parameter 0.0).
+        std::vector<uint32_t> moves;
     };
     std::vector<Component> comps;
     // Decomposer::SinglePass (fk_system_batch_solve_single_pass): comps are the strongly connected sets in the order of the host
@@ -33,6 +39,8 @@ struct SystemBatchLayout {
     // variable of no non-empty component's free set.
     std::vector<uint32_t> comp_wave, var_draw, var_wave;
     uint32_t n_waves = 0;
+    // Decomposer::RecursiveAssembly: comps are the steps, step_constraint[k] the first constraint of step k (refusals name it).
+    std::vector<uint32_t> step_constraint;
 };
 
 // Device descriptor of one structure (components of identical shape) for the two kernels: its batch buffers hold sketch
@@ -65,16 +73,22 @@ int launch_system_batch_scatter(uint32_t n, uint32_t n_vars, const double* raw_v
 
 // fk_system_batch_solve_single_pass: the sets of one structure inside one wave.  s.vars / s.params / s.out / s.reps are the
 // structure's batch buffers (sketch = variant * mult + member), s.slot_var [mult][nv] and s.expr [mult][ne] the members' rows
-// (s.slot_draw unused); free_var [mult][nf]: system variable of each solved column; step [mult]: the member's set index.
+// (s.slot_draw unused; kSbNone gathers 0.0); free_var [mult][nf]: system variable of each solved column (kSbNone: not
+// scattered); step [mult]: the member's set index.  fk_system_batch_solve_recursive_assembly: the members are steps and member
+// m moves the points of moves[2k] (variable of x, y follows) with the pose in its solved columns moves[2k + 1] .. + 2, for
+// move_off[m] <= k < move_off[m + 1] (all empty under SinglePass).
 struct SpGroup {
     SbStructure s;
     const uint32_t* free_var;
     const uint32_t* step;
+    const uint32_t* move_off;
+    const uint32_t* moves;
 };
 
-// One launch between two waves of fk_system_batch_solve_single_pass, per variant v < n on the resident rows vt[v][n_vars]
-// (scaled variables) and pt[v][n_expr] (scaled parameters), in this order: the solved values of the `scatter` groups into vt
-// and their reports into reports_out[v][step] (step < n_reports); the perturbations perturb_var[k] with draw pair
+// One launch between two waves of fk_system_batch_solve_single_pass / _recursive_assembly, per variant v < n on the resident
+// rows vt[v][n_vars] (scaled variables) and pt[v][n_expr] (scaled parameters), in this order: the solved values of the
+// `scatter` groups into vt; their owned-point moves (Pose2D::transform_point); their reports into reports_out[v][step]
+// (step < n_reports); the perturbations perturb_var[k] with draw pair
 // perturb_draw[k]; the input rows of the `gather` groups.  vars_out != null: then vars_out[v][i] = scales[v] * vt[v][i] for a
 // variable some set solves (solved[i] != 0), raw_vars[v][i] otherwise.
 int launch_system_sp_gather_scatter(uint32_t n, uint32_t n_vars, uint32_t n_expr, double* vt, const double* pt, uint32_t n_scatter,
@@ -103,7 +117,8 @@ struct SystemBatchCall {
 int system_batch_solve(SystemBatch& b, const SystemBatchCall& call);
 
 // The same for Decomposer::SinglePass: layout.comps are the sets (problems: one per set), grouped by structure; per wave one
-// launch per structure present.  (call.optimizer is ignored: the reference runs LM under SinglePass.)
+// launch per structure present.  (call.optimizer is ignored: the reference runs LM under SinglePass.)  Decomposer::
+// RecursiveAssembly uses the same plan and calls with layout.comps the steps (layout.step_constraint set, moves per step).
 struct SystemSpBatch;
 int system_sp_batch_create(SystemBatchLayout&& layout, const std::vector<const fk_problem*>& problems, std::shared_ptr<SystemSpBatch>* out);
 // (n_sets, n_waves, n_structures, wave and structure of each set)

@@ -130,31 +130,35 @@ class System:
         whatever the optimizer (assemble/mod.rs:191)."""
         self._solve(1, perturb, optimizer, len(self.single_pass_plan()))
 
+    def _wave_layout(self, fn):
+        n, nw, ns = C.c_uint32(0), C.c_uint32(0), C.c_uint32(0)
+        check(fn(self._h, C.byref(n), C.byref(nw), C.byref(ns), None, None))
+        wave = np.zeros(max(n.value, 1), np.uint32)
+        struct = np.zeros(max(n.value, 1), np.uint32)
+        check(fn(self._h, C.byref(n), C.byref(nw), C.byref(ns), ptr(wave, C.c_uint32), ptr(struct, C.c_uint32)))
+        return int(n.value), int(nw.value), int(ns.value), wave[:n.value].tolist(), struct[:n.value].tolist()
+
+    def _wave_solve(self, fn, n_steps, vars, params, perturb, n_gpus, n):
+        nv, vars, params, count = self._variant_rows(vars, params, n)
+        out = np.zeros((count, nv))
+        reps = np.zeros((count, n_steps), dtype=REPORT_DTYPE)
+        got = C.c_uint32(0)
+        check(fn(self._h, int(bool(perturb)), count, None if vars is None else ptr(vars, C.c_double),
+                 None if params is None else ptr(params, C.c_double), ptr(out, C.c_double),
+                 reps.ctypes.data_as(C.POINTER(FkReport)), n_steps, C.byref(got), int(n_gpus)))
+        return out, reps
+
     def single_pass_batch_layout(self):
         """(sets, waves, distinct set structures, [wave of each set], [structure of each set]) of batch_solve_single_pass's
         plan (host only)."""
-        n, nw, ns = C.c_uint32(0), C.c_uint32(0), C.c_uint32(0)
-        check(lib().fk_system_single_pass_batch_layout(self._h, C.byref(n), C.byref(nw), C.byref(ns), None, None))
-        wave = np.zeros(max(n.value, 1), np.uint32)
-        struct = np.zeros(max(n.value, 1), np.uint32)
-        check(lib().fk_system_single_pass_batch_layout(self._h, C.byref(n), C.byref(nw), C.byref(ns), ptr(wave, C.c_uint32),
-                                                       ptr(struct, C.c_uint32)))
-        return int(n.value), int(nw.value), int(ns.value), wave[:n.value].tolist(), struct[:n.value].tolist()
+        return self._wave_layout(lib().fk_system_single_pass_batch_layout)
 
     def batch_solve_single_pass(self, vars=None, params=None, perturb=True, n_gpus=1, n=None):
         """System.solve_single_pass(perturb) of n variants of this drawing in one call (fk_system_batch_solve_single_pass);
         arguments as batch_solve.  The system itself is not modified.  Returns (variables after each variant's solve
         [n][n_variables], reports [n][solved sets] as REPORT_DTYPE, in the order solve_single_pass reports them)."""
-        nv, vars, params, count = self._variant_rows(vars, params, n)
-        n_sets = self.single_pass_batch_layout()[0]
-        out = np.zeros((count, nv))
-        reps = np.zeros((count, n_sets), dtype=REPORT_DTYPE)
-        got = C.c_uint32(0)
-        check(lib().fk_system_batch_solve_single_pass(
-            self._h, int(bool(perturb)), count, None if vars is None else ptr(vars, C.c_double),
-            None if params is None else ptr(params, C.c_double), ptr(out, C.c_double),
-            reps.ctypes.data_as(C.POINTER(FkReport)), n_sets, C.byref(got), int(n_gpus)))
-        return out, reps
+        return self._wave_solve(lib().fk_system_batch_solve_single_pass, self.single_pass_batch_layout()[0], vars, params, perturb,
+                                n_gpus, n)
 
     def solve_recursive_assembly(self, perturb=True, optimizer="lm"):
         """System::solve with Decomposer::RecursiveAssembly (assemble/mod.rs:212-277) on the GPU.  The reference runs LM
@@ -168,6 +172,20 @@ class System:
         out = np.zeros(max(nw.value, 1), dtype=np.uint32)
         check(lib().fk_system_recursive_assembly_plan(self._h, ptr(out, C.c_uint32), nw.value, C.byref(nw), C.byref(ns)))
         return int(ns.value), out[:nw.value].tolist()
+
+    def recursive_assembly_batch_layout(self):
+        """(steps, waves, distinct step structures, [wave of each step], [structure of each step]) of
+        batch_solve_recursive_assembly's plan (host only)."""
+        return self._wave_layout(lib().fk_system_recursive_assembly_batch_layout)
+
+    def batch_solve_recursive_assembly(self, vars=None, params=None, perturb=True, n_gpus=1, n=None):
+        """System.solve_recursive_assembly(perturb) of n variants of this drawing in one call
+        (fk_system_batch_solve_recursive_assembly); arguments as batch_solve.  The system itself is not modified.  Returns
+        (variables after each variant's solve [n][n_variables], reports [n][steps] as REPORT_DTYPE, in the order
+        solve_recursive_assembly reports them).  Where a step moves points, coordinates may differ from the per-variant solve
+        in the last places (include/fiksi_b200.h states the contract)."""
+        return self._wave_solve(lib().fk_system_batch_solve_recursive_assembly, self.recursive_assembly_batch_layout()[0], vars,
+                                params, perturb, n_gpus, n)
 
     def single_pass_plan(self):
         """[(free variables, expressions), ...] of fk_system_single_pass_plan (host only)."""

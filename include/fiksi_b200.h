@@ -480,6 +480,36 @@ FK_API int fk_system_batch_solve_single_pass(const fk_system* s, int perturb, ui
  * (structures in order of first appearance; step_wave[n_steps] and step_structure[n_steps] may be NULL). */
 FK_API int fk_system_single_pass_batch_layout(const fk_system* s, uint32_t* n_steps, uint32_t* n_waves, uint32_t* n_structures,
                                               uint32_t* step_wave, uint32_t* step_structure);
+/* == System::solve(SolvingOptions { decomposer: RecursiveAssembly, perturb }) (assemble/mod.rs:212-277; the reference runs LM
+ * here whatever the optimizer, :224) applied to n variants of `s`; arguments as fk_system_batch_solve_single_pass.
+ * reports[v][k]: step k in the order fk_system_solve_opts(decomposer = 2) reports them (components in order, then the steps
+ * of each component's plan), the first reports_per_variant of them; *n_solved = steps per variant.  vars_out[v][i] is
+ * scale * the solved value for a variable some step writes (a variable of the step's elements, or a point a moved cluster
+ * owns), and the raw input for every other variable, even where the call perturbed it.  `s` is not modified.
+ * The plan is kept on `s` until a structural edit (add_*, fix / unfix): the recombination steps of every component, each
+ * as its clustered problem (pose columns, element variables, the fixed point copies behind them) grouped by structure
+ * through the topology cache, the points each step moves in the host loop's order, and the waves of
+ * fk_system_batch_solve_single_pass's rule (a step reads its variables and the points it moves, and writes its element
+ * variables and the points it moves).  On the device, per chunk of variants: one prepare kernel, then per wave one gather /
+ * scatter kernel (previous wave's solutions, its moves, its reports, perturbations, this wave's input rows with every pose at
+ * the identity) and one batched LM launch per structure present, and a last gather / scatter kernel with the write-back.
+ * Numerical contract: each step's LM runs the kernels of the host loop, so a drawing whose plan moves no point gives bit
+ * for bit what fk_system_solve_opts(decomposer = 2, perturb) gives on a copy of `s` with the variant's numbers.  A move is
+ * Pose2D::transform_point with CUDA's sincos on the device and glibc's sin / cos in the host loop, which may differ in
+ * the last place: with moves, every step's exit, iterations, factorisations and trace agree, and coordinates agree within
+ * 1e-11 relative to the variant's largest |value| unless a step's decisions flip on that last place.  perturb 0 or 1;
+ * refusals come before any device work and leave vars_out untouched: FK_ERR_INVALID for bad arguments, for a system the
+ * reference panics on and for an expression that reads a variable outside its step (the host loop's messages),
+ * FK_ERR_TOO_LARGE when a step on the global sparse path has a largest supernodal front above the 236 rows of
+ * fk_batch_solve (the message names the step, its first constraint and the front).  Chunks and devices as
+ * fk_system_batch_solve_single_pass. */
+FK_API int fk_system_batch_solve_recursive_assembly(const fk_system* s, int perturb, uint32_t n, const double* vars,
+                                                    const double* params, double* vars_out, fk_report* reports,
+                                                    uint32_t reports_per_variant, uint32_t* n_solved, int n_gpus);
+/* Host-only probe of its plan (no device needed): steps, waves, distinct step structures, and per step its wave and
+ * structure (structures in order of first appearance; step_wave[n_steps] and step_structure[n_steps] may be NULL). */
+FK_API int fk_system_recursive_assembly_batch_layout(const fk_system* s, uint32_t* n_steps, uint32_t* n_waves,
+                                                     uint32_t* n_structures, uint32_t* step_wave, uint32_t* step_structure);
 /* Host-only probe of the RecursiveAssembly plan (no device needed) as a stream of 32-bit words: per step
  * n_constraints, constraints..., n_elements, elements..., n_free, free elements..., then the maps on_frontiers,
  * owned_elements, frontier_elements (recursive_assembly.rs:75-114) as n_keys and per key (ascending) key, n,

@@ -70,7 +70,8 @@ EXPORTS = [
     "fk_topology_batch_kernel", "fk_topology_lbfgs_kernel", "fk_lbfgs_solve", "fk_lbfgs_solve_batch", "fk_batch_plan_run_lbfgs_global",
     "fk_system_solve_options", "fk_batch_system_solve", "fk_batch_system_solve_begin", "fk_batch_system_solve_wait", "fk_batch_solve_device_begin", "fk_batch_solve_device_wait", "fk_topology_cache_configure", "fk_topology_cache_clear", "fk_topology_cache_stats",
     "fk_system_batch_solve", "fk_system_batch_layout", "fk_system_batch_solve_single_pass", "fk_system_single_pass_batch_layout",
-    "fk_system_batch_solve_recursive_assembly", "fk_system_recursive_assembly_batch_layout",
+    "fk_system_batch_solve_recursive_assembly", "fk_system_recursive_assembly_batch_layout", "fk_system_batch_analyze",
+    "fk_system_batch_residuals",
 ]
 
 _lib = None
@@ -106,6 +107,8 @@ def lib() -> C.CDLL:
                                          C.c_int]
         for name in ("fk_system_single_pass_batch_layout", "fk_system_recursive_assembly_batch_layout"):
             getattr(L, name).argtypes = [C.c_void_p, u32p, u32p, u32p, u32p, u32p]
+        L.fk_system_batch_analyze.argtypes = [C.c_void_p, C.c_uint32, f64p, f64p, C.POINTER(C.c_uint8), C.c_int]
+        L.fk_system_batch_residuals.argtypes = [C.c_void_p, C.c_uint32, f64p, f64p, f64p, C.c_int]
         _lib = L
     return _lib
 

@@ -2464,4 +2464,195 @@ int system_sp_batch_solve(SystemSpBatch& b, const SystemBatchCall& c) {
     return r;
 }
 
+// ---- fk_system_batch_analyze / fk_system_batch_residuals: System::analyze and calculate_residual over n variants -----------
+// Per device: the layout's tables, the template rows, the chunk buffers (variables vt and expanded parameters pt are what the
+// analyze kernels and fk_system_residuals_kernel read) and the analyze workspace, grow-only within fk::kAnWorkspaceBytes.
+struct SystemAnDevice {
+    int device = -1;
+    std::mutex mu;
+    cudaStream_t stream = nullptr;
+    bool ready = false;  // tables and template buffers in place
+    void* d_tables = nullptr;
+    const uint8_t* d_kind = nullptr;
+    const uint32_t *d_slot = nullptr, *d_expr_con = nullptr, *d_con_off = nullptr;
+    double *d_tmpl_vars = nullptr, *d_tmpl_param = nullptr;
+    uint32_t chunk = 0, an_chunk = 0, res_chunk = 0;  // variants the inputs, the analyze outputs, the residual outputs hold
+    double *d_raw_param = nullptr, *d_vt = nullptr, *d_pt = nullptr, *d_res = nullptr;
+    uint8_t *d_indep = nullptr, *d_dep = nullptr;
+    double* d_ws = nullptr;
+    uint64_t ws_bytes = 0;
+    void release_buffers() {
+        cudaFree(d_raw_param); cudaFree(d_vt); cudaFree(d_pt); cudaFree(d_res); cudaFree(d_indep); cudaFree(d_dep);
+        d_raw_param = d_vt = d_pt = d_res = nullptr;
+        d_indep = d_dep = nullptr;
+        chunk = an_chunk = res_chunk = 0;
+    }
+    ~SystemAnDevice() {
+        if (device < 0) return;
+        cudaSetDevice(device);
+        release_buffers();
+        cudaFree(d_tables); cudaFree(d_tmpl_vars); cudaFree(d_tmpl_param); cudaFree(d_ws);
+        if (stream) cudaStreamDestroy(stream);
+    }
+};
+
+struct SystemAnBatch {
+    SystemAnLayout L;
+    uint32_t n_expr = 0, n_constraints = 0;
+    std::mutex mu;
+    std::map<int, std::unique_ptr<SystemAnDevice>> devices;
+};
+
+int system_an_batch_create(SystemAnLayout&& layout, std::shared_ptr<SystemAnBatch>* out) {
+    std::shared_ptr<SystemAnBatch> b = std::make_shared<SystemAnBatch>();
+    b->L = std::move(layout);
+    b->n_expr = (uint32_t)b->L.kind.size();
+    b->n_constraints = b->L.con_off.empty() ? 0 : (uint32_t)b->L.con_off.size() - 1;
+    *out = std::move(b);
+    return FK_OK;
+}
+
+// Tables once per device; the input buffers and the outputs of the call's operation (analyze: per-expression flags and
+// per-constraint counts; residuals: per-constraint values) grow with the chunk.  The caller holds d->mu.
+static int system_an_device(const SystemAnBatch& b, SystemAnDevice* d, int device, uint32_t chunk, bool analyze) {
+    CU(cudaSetDevice(device));
+    const SystemAnLayout& L = b.L;
+    if (!d->ready) {
+        d->device = device;
+        if (!d->stream) CU(cudaStreamCreateWithFlags(&d->stream, cudaStreamNonBlocking));
+        cudaFree(d->d_tables); cudaFree(d->d_tmpl_vars); cudaFree(d->d_tmpl_param);  // (an earlier attempt's)
+        d->d_tables = nullptr;
+        d->d_tmpl_vars = d->d_tmpl_param = nullptr;
+        size_t off = 0;
+        const size_t o_kind = reserve<uint8_t>(off, L.kind.size()), o_slot = reserve<uint32_t>(off, L.slot_var.size()),
+                     o_con = reserve<uint32_t>(off, L.expr_constraint.size()), o_off = reserve<uint32_t>(off, L.con_off.size());
+        std::vector<unsigned char> host(off + 16, 0);
+        std::memcpy(host.data() + o_kind, L.kind.data(), L.kind.size());
+        std::memcpy(host.data() + o_slot, L.slot_var.data(), L.slot_var.size() * sizeof(uint32_t));
+        std::memcpy(host.data() + o_con, L.expr_constraint.data(), L.expr_constraint.size() * sizeof(uint32_t));
+        std::memcpy(host.data() + o_off, L.con_off.data(), L.con_off.size() * sizeof(uint32_t));
+        CU(cudaMalloc(&d->d_tables, host.size()));
+        CU(cudaMalloc(&d->d_tmpl_vars, sizeof(double) * std::max<uint32_t>(L.n_vars, 1)));
+        CU(cudaMalloc(&d->d_tmpl_param, sizeof(double) * std::max<uint32_t>(b.n_expr, 1)));
+        CU(cudaMemcpyAsync(d->d_tables, host.data(), host.size(), cudaMemcpyHostToDevice, d->stream));
+        CU(cudaStreamSynchronize(d->stream));  // (host leaves scope)
+        unsigned char* p = (unsigned char*)d->d_tables;
+        d->d_kind = p + o_kind;
+        d->d_slot = (const uint32_t*)(p + o_slot);
+        d->d_expr_con = (const uint32_t*)(p + o_con);
+        d->d_con_off = (const uint32_t*)(p + o_off);
+        d->ready = true;
+    }
+    auto alloc = [&](auto** ptr, size_t count) -> int {
+        cudaFree(*ptr);
+        *ptr = nullptr;
+        CU(cudaMalloc((void**)ptr, sizeof(**ptr) * std::max<size_t>(count, 1)));
+        return FK_OK;
+    };
+    int rc = FK_OK;
+    if (d->chunk < chunk) {
+        d->chunk = 0;
+        if ((rc = alloc(&d->d_raw_param, (size_t)chunk * b.n_constraints)) != FK_OK || (rc = alloc(&d->d_vt, (size_t)chunk * L.n_vars)) != FK_OK ||
+            (rc = alloc(&d->d_pt, (size_t)chunk * b.n_expr)) != FK_OK)
+            return rc;
+        d->chunk = chunk;
+    }
+    if (analyze && d->an_chunk < chunk) {
+        d->an_chunk = 0;
+        if ((rc = alloc(&d->d_indep, (size_t)chunk * b.n_expr)) != FK_OK || (rc = alloc(&d->d_dep, (size_t)chunk * b.n_constraints)) != FK_OK)
+            return rc;
+        d->an_chunk = chunk;
+    }
+    if (!analyze && d->res_chunk < chunk) {
+        d->res_chunk = 0;
+        if ((rc = alloc(&d->d_res, (size_t)chunk * b.n_constraints)) != FK_OK) return rc;
+        d->res_chunk = chunk;
+    }
+    return FK_OK;
+}
+
+// Variants [lo, hi) on one device, chunk after chunk on its stream: upload (or broadcast the template), expand the parameters,
+// then analyze + reduce or the residuals, download.
+static int system_an_range(SystemAnBatch& b, const SystemAnCall& c, int device, uint32_t lo, uint32_t hi) {
+    const SystemAnLayout& L = b.L;
+    const uint32_t ne = b.n_expr, ncon = b.n_constraints;
+    const bool analyze = c.dependent != nullptr;
+    const uint64_t per_variant = sizeof(double) * ((uint64_t)L.n_vars + ncon + ne) + (analyze ? (uint64_t)ne + ncon : sizeof(double) * ncon);
+    const uint32_t env = system_batch_chunk_env();
+    const uint32_t chunk = (uint32_t)std::min<uint64_t>(env ? env : std::max<uint64_t>(1, (1ull << 30) / per_variant), hi - lo);
+    SystemAnDevice* d;
+    {
+        std::lock_guard<std::mutex> lock(b.mu);
+        auto& p = b.devices[device];
+        if (!p) p.reset(new SystemAnDevice());
+        d = p.get();
+    }
+    std::lock_guard<std::mutex> lock(d->mu);
+    int rc = system_an_device(b, d, device, chunk, analyze);
+    if (rc != FK_OK) return rc;
+    cudaStream_t st = d->stream;
+    auto run = [&]() -> int {
+        CU(cudaMemcpyAsync(d->d_tmpl_vars, c.tmpl_vars, sizeof(double) * L.n_vars, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(d->d_tmpl_param, c.tmpl_param, sizeof(double) * ne, cudaMemcpyHostToDevice, st));
+        for (uint32_t at = lo; at < hi; at += chunk) {
+            const uint32_t cnt = std::min(chunk, hi - at);
+            if (c.vars)
+                CU(cudaMemcpyAsync(d->d_vt, c.vars + (size_t)at * L.n_vars, sizeof(double) * (size_t)cnt * L.n_vars, cudaMemcpyHostToDevice, st));
+            if (c.params)
+                CU(cudaMemcpyAsync(d->d_raw_param, c.params + (size_t)at * ncon, sizeof(double) * (size_t)cnt * ncon, cudaMemcpyHostToDevice, st));
+            int e = launch_system_an_expand(cnt, L.n_vars, ne, ncon, c.vars ? nullptr : d->d_tmpl_vars, d->d_vt, d->d_expr_con,
+                                            c.params ? d->d_raw_param : nullptr, d->d_tmpl_param, d->d_pt, st);
+            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_an_expand_kernel");
+            if (!analyze) {
+                e = launch_system_residuals(cnt, L.n_vars, ne, ncon, d->d_kind, d->d_slot, d->d_con_off, d->d_vt, d->d_pt, d->d_res, st);
+                if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_residuals_kernel");
+                CU(cudaMemcpyAsync(c.residuals + (size_t)at * ncon, d->d_res, sizeof(double) * (size_t)cnt * ncon, cudaMemcpyDeviceToHost, st));
+                continue;
+            }
+            AnalyzePlan plan;  // the kernel for this chunk's size
+            std::string err;
+            const int prc = choose_analyze(L.n_vars, ne, cnt, device, &plan, &err);
+            if (prc != FK_OK) return fail(prc, err);
+            if (d->ws_bytes < plan.workspace_bytes()) {  // grow-only, within fk::kAnWorkspaceBytes
+                CU(cudaStreamSynchronize(st));  // (an earlier chunk's launch may still use the old workspace)
+                cudaFree(d->d_ws);
+                d->d_ws = nullptr;
+                d->ws_bytes = 0;
+                CU(cudaMalloc(&d->d_ws, plan.workspace_bytes()));
+                d->ws_bytes = plan.workspace_bytes();
+            }
+            e = plan.kernel == kAnWarp ? launch_batch_analyze(L.n_vars, ne, d->d_kind, d->d_slot, cnt, d->d_vt, d->d_pt, d->d_indep, st)
+                                       : launch_analyze(plan, L.n_vars, ne, d->d_kind, d->d_slot, cnt, d->d_vt, d->d_pt, d->d_indep, d->d_ws, st);
+            if (e != 0) return cuda_fail((cudaError_t)e, plan.kernel == kAnWarp ? "launch fk_batch_analyze_kernel" : "launch fk_analyze_cta_kernel");
+            e = launch_system_an_reduce(cnt, ne, ncon, d->d_indep, d->d_con_off, d->d_dep, st);
+            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_an_reduce_kernel");
+            CU(cudaMemcpyAsync(c.dependent + (size_t)at * ncon, d->d_dep, (size_t)cnt * ncon, cudaMemcpyDeviceToHost, st));
+        }
+        return FK_OK;
+    };
+    rc = run();
+    // (also after an error: no copy into the caller's buffers may still be running when the call returns)
+    const cudaError_t e = cudaStreamSynchronize(st);
+    if (rc == FK_OK && e != cudaSuccess) rc = cuda_fail(e, "fk_system_batch_analyze / _residuals kernels / copies");
+    return rc;
+}
+
+int system_an_batch_run(SystemAnBatch& b, const SystemAnCall& c) {
+    if (c.n == 0 || b.n_constraints == 0) return FK_OK;
+    int n_gpus = c.n_gpus;
+    int rc = clamp_gpus(n_gpus);
+    if (rc != FK_OK) return rc;
+    int cur = 0;
+    if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
+    if (c.dependent) {  // the size limit of the analyze kernels (it does not depend on the batch size)
+        AnalyzePlan plan;
+        std::string err;
+        rc = choose_analyze(b.L.n_vars, b.n_expr, c.n, cur, &plan, &err);
+        if (rc != FK_OK) return fail(rc, err);
+    }
+    const int r = shard_over_devices(n_gpus, c.n, [&](int device, uint32_t lo, uint32_t hi) { return system_an_range(b, c, device, lo, hi); });
+    if (cudaSetDevice(cur) != cudaSuccess) cudaGetLastError();
+    return r;
+}
+
 }  // namespace fk

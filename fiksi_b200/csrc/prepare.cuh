@@ -13,6 +13,16 @@ __device__ __forceinline__ bool prepare_is_distance(uint32_t kind) {
     return kind == FK_POINT_POINT_DISTANCE || kind == FK_POINT_LINE_DISTANCE;
 }
 
+// Raw parameter of expression e in variant v of a System batch: raw_param[v][c] where e holds constraint c's parameter
+// (expr_constraint[e] = c, 0xFFFFFFFF for none; update_parameter writes it at the constraint's first expression, constraints/mod.rs:992-1046) and
+// raw_param is given, tmpl_param[e] otherwise.
+__device__ __forceinline__ double variant_param(const double* __restrict__ raw_param, uint32_t n_constraints,
+                                                const uint32_t* __restrict__ expr_constraint, const double* __restrict__ tmpl_param,
+                                                size_t v, uint32_t e) {
+    const uint32_t c = raw_param ? __ldg(expr_constraint + e) : 0xFFFFFFFFu;
+    return c != 0xFFFFFFFFu ? __ldg(raw_param + v * n_constraints + c) : __ldg(tmpl_param + e);
+}
+
 // RMS scale of one sketch: every variable left to right, then the distance parameters in expression order, summed
 // sequentially (fiksi/src/utils.rs:12-19).  param(e) returns the raw parameter of expression e.
 template <class Param>

@@ -70,6 +70,7 @@ struct fk_system {
     mutable std::shared_ptr<fk::SystemBatch> batch;
     mutable std::shared_ptr<fk::SystemSpBatch> sp_batch;  // fk_system_batch_solve_single_pass's plan, kept and dropped alike
     mutable std::shared_ptr<fk::SystemSpBatch> ra_batch;  // fk_system_batch_solve_recursive_assembly's plan, kept and dropped alike
+    mutable std::shared_ptr<fk::SystemAnBatch> an_batch;  // fk_system_batch_analyze / _residuals' plan, kept and dropped alike
 
     uint32_t new_element(uint8_t tag, uint32_t a, uint32_t b, const double* v, int nv) {
         uint32_t id = (uint32_t)elems.size();
@@ -133,6 +134,7 @@ struct fk_system {
         batch.reset();
         sp_batch.reset();
         ra_batch.reset();
+        an_batch.reset();
     }
     void push_expr(uint8_t k, uint32_t i0, uint32_t i1, uint32_t i2, uint32_t i3, double p) {
         kind.push_back(k);
@@ -1128,9 +1130,58 @@ int wave_batch_solve(WavePlanFor plan_for, const fk_system* s, int perturb, uint
     return fk::system_sp_batch_solve(*b, c);
 }
 
+// fk_system_batch_analyze / _residuals' plan: the expressions with their slot tables and the constraints' expression ranges.
+int analyze_batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemAnBatch>* out) {
+    std::lock_guard<std::mutex> lock(s->batch_mu);
+    if (!s->an_batch) {
+        fk::SystemAnLayout lay;
+        lay.n_vars = (uint32_t)s->vars.size();
+        lay.kind = s->kind;
+        lay.slot_var.assign(s->kind.size() * 8, 0);
+        for (size_t e = 0; e < s->kind.size(); e++) fk::expand_slots(s->kind[e], &s->idx[4 * e], &lay.slot_var[8 * e]);
+        lay.expr_constraint.assign(s->kind.size(), fk::kSbNone);
+        lay.con_off.push_back(0);
+        for (uint32_t c = 0; c < s->constrs.size(); c++) {
+            // (fk_system_add_constraint appends a constraint's expressions: first_expr is the previous constraint's end)
+            lay.expr_constraint[s->constrs[c].first_expr] = c;  // update_parameter
+            lay.con_off.push_back(s->constrs[c].first_expr + s->constrs[c].n_expr);
+        }
+        const int rc = fk::system_an_batch_create(std::move(lay), &s->an_batch);
+        if (rc != FK_OK) return rc;
+    }
+    *out = s->an_batch;
+    return FK_OK;
+}
+
+int an_batch_run(const fk_system* s, uint32_t n, const double* vars, const double* params, uint8_t* dependent, double* residuals,
+                 int n_gpus) {
+    if (!s || (n && !dependent && !residuals)) return fk::system_batch_fail(FK_ERR_INVALID, "null system or output");
+    std::shared_ptr<fk::SystemAnBatch> b;
+    const int rc = analyze_batch_plan_for(s, &b);
+    if (rc != FK_OK) return rc;
+    fk::SystemAnCall c;
+    c.n_gpus = n_gpus;
+    c.n = n;
+    c.vars = vars;
+    c.params = params;
+    c.tmpl_vars = s->vars.data();
+    c.tmpl_param = s->param.data();
+    c.dependent = dependent;
+    c.residuals = residuals;
+    return fk::system_an_batch_run(*b, c);
+}
+
 }  // namespace
 
 extern "C" {
+
+int fk_system_batch_analyze(const fk_system* s, uint32_t n, const double* vars, const double* params, uint8_t* dependent, int n_gpus) {
+    return an_batch_run(s, n, vars, params, dependent, nullptr, n_gpus);
+}
+
+int fk_system_batch_residuals(const fk_system* s, uint32_t n, const double* vars, const double* params, double* out, int n_gpus) {
+    return an_batch_run(s, n, vars, params, nullptr, out, n_gpus);
+}
 
 int fk_system_batch_layout(const fk_system* s, uint32_t* n_components, uint32_t* n_structures, uint32_t* multiplicity) {
     if (!s) return fk::system_batch_fail(FK_ERR_INVALID, "null system");

@@ -3,10 +3,13 @@
 // variants' variable rows.  The arithmetic of the pre-processing is prepare.cuh's, shared with fk_batch_prepare_kernel.
 // fk_system_batch_solve_single_pass and _recursive_assembly reuse the prepare kernel (one identity structure: the resident
 // scaled rows) and move values between the waves of sets or steps with fk_system_sp_gather_scatter_kernel.
+// fk_system_batch_analyze and fk_system_batch_residuals expand the variants' parameter rows, then reduce the analyze flags
+// per constraint or evaluate every constraint's residual.
 #include <cuda_runtime.h>
 
 #include <algorithm>
 
+#include "expressions.cuh"
 #include "prepare.cuh"
 #include "system_batch.cuh"
 
@@ -29,11 +32,7 @@ fk_system_batch_prepare_kernel(uint32_t n, uint32_t n_vars, uint32_t n_expr, uin
     __shared__ double s_recip[kPrepVariants];
     const uint32_t v0 = blockIdx.x * kPrepVariants;
     const uint32_t nb = min(kPrepVariants, n - v0);
-    // raw parameter of expression e in variant v
-    auto param_of = [&](uint32_t v, uint32_t e) -> double {
-        const uint32_t c = raw_param ? __ldg(expr_constraint + e) : kSbNone;
-        return c != kSbNone ? __ldg(raw_param + (size_t)v * n_constraints + c) : __ldg(tmpl_param + e);
-    };
+    auto param_of = [&](uint32_t v, uint32_t e) { return variant_param(raw_param, n_constraints, expr_constraint, tmpl_param, v, e); };
     if (threadIdx.x < nb) {
         const uint32_t v = v0 + threadIdx.x;
         const double scale =
@@ -182,6 +181,94 @@ fk_system_sp_gather_scatter_kernel(uint32_t n, uint32_t vb, uint32_t n_vars, uin
         const size_t v = v0 + b;
         vars_out[v * n_vars + g] = __ldg(solved + g) ? __ldg(scales + v) * vrow[i] : __ldg(raw_vars + v * raw_vars_stride + g);
     }
+}
+
+// ---- fk_system_batch_analyze / fk_system_batch_residuals ---------------------------------------------------------------
+namespace {
+uint32_t grid_for(uint64_t total) { return (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((total + 255) / 256, 148u * 16u)); }
+}  // namespace
+
+// The variants' rows as the analyze kernels and fk_system_residuals_kernel read them: pt[v][e] = variant_param, and, given
+// tmpl_vars (the call passed no variables), vt[v] = tmpl_vars.
+__global__ void __launch_bounds__(256)
+fk_system_an_expand_kernel(uint32_t n, uint32_t n_vars, uint32_t n_expr, uint32_t n_constraints, const double* __restrict__ tmpl_vars,
+                           double* __restrict__ vt, const uint32_t* __restrict__ expr_constraint, const double* __restrict__ raw_param,
+                           const double* __restrict__ tmpl_param, double* __restrict__ pt) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    const uint64_t first = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (tmpl_vars)
+        for (uint64_t i = first; i < (uint64_t)n * n_vars; i += stride) vt[i] = __ldg(tmpl_vars + i % n_vars);
+    for (uint64_t i = first; i < (uint64_t)n * n_expr; i += stride) {
+        const uint64_t v = i / n_expr;
+        pt[i] = variant_param(raw_param, n_constraints, expr_constraint, tmpl_param, v, (uint32_t)(i - v * n_expr));
+    }
+}
+
+// dependent[v][c] = the expressions [con_off[c], con_off[c + 1]) of constraint c that analyze found dependent.
+__global__ void __launch_bounds__(256)
+fk_system_an_reduce_kernel(uint32_t n, uint32_t n_expr, uint32_t n_constraints, const uint8_t* __restrict__ independent,
+                           const uint32_t* __restrict__ con_off, uint8_t* __restrict__ dependent) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < (uint64_t)n * n_constraints; i += stride) {
+        const uint64_t v = i / n_constraints;
+        const uint32_t c = (uint32_t)(i - v * n_constraints);
+        uint32_t d = 0;
+        for (uint32_t e = __ldg(con_off + c), end = __ldg(con_off + c + 1); e < end; e++) d += independent[v * n_expr + e] ? 0u : 1u;
+        dependent[i] = (uint8_t)d;
+    }
+}
+
+// out[v][c] = calculate_residual (constraints/mod.rs:88-110) of constraint c in variant v, as fk_system_residuals combines the
+// expression residuals: a one-expression constraint its residual, otherwise q += r * r in expression order, then sqrt(q).
+// The slots are read as the analyze kernels read them (slot_var[e][8], arity_of), the residual is eval_expression's.
+__global__ void __launch_bounds__(256)
+fk_system_residuals_kernel(uint32_t n, uint32_t n_vars, uint32_t n_expr, uint32_t n_constraints, const uint8_t* __restrict__ kinds,
+                           const uint32_t* __restrict__ slot_var, const uint32_t* __restrict__ con_off, const double* __restrict__ vt,
+                           const double* __restrict__ pt, double* __restrict__ out) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < (uint64_t)n * n_constraints; i += stride) {
+        const uint64_t v = i / n_constraints;
+        const uint32_t c = (uint32_t)(i - v * n_constraints);
+        const double* vars = vt + v * n_vars;
+        const uint32_t e0 = __ldg(con_off + c), e1 = __ldg(con_off + c + 1);
+        double q = 0.0, r = 0.0;
+        for (uint32_t e = e0; e < e1; e++) {
+            const int kind = (int)__ldg(kinds + e);
+            const int ar = dev::arity_of(kind);
+            double x[8], g[8];
+#pragma unroll
+            for (int sl = 0; sl < 8; sl++) x[sl] = sl < ar ? __ldg(vars + __ldg(slot_var + (size_t)e * 8 + sl)) : 0.0;
+            r = dev::eval_expression(kind, x, __ldg(pt + v * n_expr + e), g);
+            q += r * r;
+        }
+        out[i] = e1 - e0 > 1 ? sqrt(q) : r;
+    }
+}
+
+int launch_system_an_expand(uint32_t n, uint32_t n_vars, uint32_t n_expr, uint32_t n_constraints, const double* tmpl_vars, double* vt,
+                            const uint32_t* expr_constraint, const double* raw_param, const double* tmpl_param, double* pt, void* stream) {
+    const uint64_t total = (uint64_t)n * std::max(tmpl_vars ? n_vars : 0u, n_expr);
+    if (total == 0) return 0;
+    fk_system_an_expand_kernel<<<grid_for(total), 256, 0, (cudaStream_t)stream>>>(n, n_vars, n_expr, n_constraints, tmpl_vars, vt,
+                                                                                  expr_constraint, raw_param, tmpl_param, pt);
+    return (int)cudaGetLastError();
+}
+
+int launch_system_an_reduce(uint32_t n, uint32_t n_expr, uint32_t n_constraints, const uint8_t* independent, const uint32_t* con_off,
+                            uint8_t* dependent, void* stream) {
+    const uint64_t total = (uint64_t)n * n_constraints;
+    if (total == 0) return 0;
+    fk_system_an_reduce_kernel<<<grid_for(total), 256, 0, (cudaStream_t)stream>>>(n, n_expr, n_constraints, independent, con_off, dependent);
+    return (int)cudaGetLastError();
+}
+
+int launch_system_residuals(uint32_t n, uint32_t n_vars, uint32_t n_expr, uint32_t n_constraints, const uint8_t* kinds, const uint32_t* slot_var,
+                            const uint32_t* con_off, const double* vt, const double* pt, double* out, void* stream) {
+    const uint64_t total = (uint64_t)n * n_constraints;
+    if (total == 0) return 0;
+    fk_system_residuals_kernel<<<grid_for(total), 256, 0, (cudaStream_t)stream>>>(n, n_vars, n_expr, n_constraints, kinds, slot_var, con_off,
+                                                                                  vt, pt, out);
+    return (int)cudaGetLastError();
 }
 
 int launch_system_sp_gather_scatter(uint32_t n, uint32_t n_vars, uint32_t n_expr, double* vt, const double* pt, uint32_t n_scatter,

@@ -125,6 +125,40 @@ int system_sp_batch_create(SystemBatchLayout&& layout, const std::vector<const f
 void system_sp_batch_layout(const SystemSpBatch& b, uint32_t* n_sets, uint32_t* n_waves, uint32_t* n_structures,
                             std::vector<uint32_t>* set_wave, std::vector<uint32_t>* set_structure);
 int system_sp_batch_solve(SystemSpBatch& b, const SystemBatchCall& call);
+
+// fk_system_batch_analyze / fk_system_batch_residuals: System::analyze and calculate_residual over n variants of one drawing.
+// The drawing's expressions as analyze and the residuals read them; no topology, ordering or symbolic analysis.
+struct SystemAnLayout {
+    uint32_t n_vars = 0;
+    std::vector<uint8_t> kind;              // [n_expr]
+    std::vector<uint32_t> slot_var;         // [n_expr][8] expand_slots of every expression, as fk_batch_analyze builds it
+    std::vector<uint32_t> expr_constraint;  // [n_expr] constraint whose parameter the expression holds, kSbNone for none
+    std::vector<uint32_t> con_off;          // [n_constraints + 1] constraint c owns expressions [con_off[c], con_off[c + 1])
+};
+// pt[v][e] = variant_param(raw_param, ..., v, e) (prepare.cuh) for v < n; tmpl_vars != null: vt[v] = tmpl_vars too.
+int launch_system_an_expand(uint32_t n, uint32_t n_vars, uint32_t n_expr, uint32_t n_constraints, const double* tmpl_vars, double* vt,
+                            const uint32_t* expr_constraint, const double* raw_param, const double* tmpl_param, double* pt, void* stream);
+// dependent[v][c] = number of expressions of constraint c with independent[v][e] == 0.
+int launch_system_an_reduce(uint32_t n, uint32_t n_expr, uint32_t n_constraints, const uint8_t* independent, const uint32_t* con_off,
+                            uint8_t* dependent, void* stream);
+// out[v][c] = fk_system_residuals of variant v (rows vt[v][n_vars], pt[v][n_expr]).
+int launch_system_residuals(uint32_t n, uint32_t n_vars, uint32_t n_expr, uint32_t n_constraints, const uint8_t* kinds, const uint32_t* slot_var,
+                            const uint32_t* con_off, const double* vt, const double* pt, double* out, void* stream);
+struct SystemAnBatch;
+int system_an_batch_create(SystemAnLayout&& layout, std::shared_ptr<SystemAnBatch>* out);
+struct SystemAnCall {
+    int n_gpus = 1;
+    uint32_t n = 0;
+    const double* vars = nullptr;        // [n][n_vars] or null
+    const double* params = nullptr;      // [n][n_constraints] or null
+    const double* tmpl_vars = nullptr;   // [n_vars]
+    const double* tmpl_param = nullptr;  // [n_expr]
+    uint8_t* dependent = nullptr;        // fk_system_batch_analyze: [n][n_constraints]
+    double* residuals = nullptr;         // fk_system_batch_residuals: [n][n_constraints] (exactly one of the two is set)
+};
+// Refusals (analyze: choose_analyze's size limit) before any device work, then the chunks on every device.
+int system_an_batch_run(SystemAnBatch& b, const SystemAnCall& call);
+
 // fk_last_error()'s message for errors found outside capi.cu.
 int system_batch_fail(int code, const std::string& msg);
 

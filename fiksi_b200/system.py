@@ -187,6 +187,25 @@ class System:
         return self._wave_solve(lib().fk_system_batch_solve_recursive_assembly, self.recursive_assembly_batch_layout()[0], vars,
                                 params, perturb, n_gpus, n)
 
+    def batch_analyze(self, vars=None, params=None, n_gpus=1, n=None):
+        """System.analyze() of n variants of this drawing in one call (fk_system_batch_analyze); arguments as batch_solve.
+        Returns uint8 [n][n_constraints]: how many of each constraint's expressions were found dependent, so that variant
+        v's analyze() is np.repeat(np.arange(n_constraints), dependent[v]).  The system itself is not modified."""
+        _, vars, params, count = self._variant_rows(vars, params, n)
+        out = np.zeros((count, self.num_constraints()), np.uint8)
+        check(lib().fk_system_batch_analyze(self._h, count, None if vars is None else ptr(vars, C.c_double),
+                                            None if params is None else ptr(params, C.c_double), ptr(out, C.c_uint8), int(n_gpus)))
+        return out
+
+    def batch_residuals(self, vars=None, params=None, n_gpus=1, n=None):
+        """System.residuals() of n variants of this drawing in one call (fk_system_batch_residuals); arguments as batch_solve.
+        Returns float64 [n][n_constraints].  The system itself is not modified."""
+        _, vars, params, count = self._variant_rows(vars, params, n)
+        out = np.zeros((count, self.num_constraints()))
+        check(lib().fk_system_batch_residuals(self._h, count, None if vars is None else ptr(vars, C.c_double),
+                                              None if params is None else ptr(params, C.c_double), ptr(out, C.c_double), int(n_gpus)))
+        return out
+
     def single_pass_plan(self):
         """[(free variables, expressions), ...] of fk_system_single_pass_plan (host only)."""
         sizes = np.zeros(3, dtype=np.uint32)

@@ -526,6 +526,35 @@ FK_API int fk_system_residuals(fk_system* s, double* out /* [num_constraints] */
  * through fk_batch_analyze as one sketch on device 0 (a group of CTAs once its matrix leaves shared memory), under
  * the same size limit. */
 FK_API int fk_system_analyze(fk_system* s, uint32_t* constraints, uint32_t cap, uint32_t* n_found);
+/* == System::analyze on n variants of `s` (variant v: every variable set to vars[v][i], every constraint parameter to
+ * params[v][c]; NULL = s's own values, as fk_system_batch_solve).  dependent[v][c] = number of constraint c's expressions
+ * the elimination found dependent (0 up to its expression count).  A constraint's expressions are consecutive and
+ * expression ids ascend with constraint ids, so the list fk_system_analyze returns for variant v is every c
+ * ascending, repeated dependent[v][c] times.
+ * Bit for bit per variant: dependent[v] gives exactly that list on a copy of `s` with the variant's numbers, quirks
+ * included (rows beyond min(n_expressions, n_variables) are never examined and count as dependent; every variable is a
+ * column, fixed or not).  All three analyze kernels repeat the reference's floating-point operations, so the flags do not
+ * depend on which one runs.  `s` is not modified; NaN and inf stay inside their own variant.
+ * The plan (expression kinds, slot tables, the constraints' expression ranges; per device those tables and a grow-only
+ * workspace within the 4 GiB of fk_batch_analyze) is built on first use and kept until a structural edit (add_*, fix /
+ * unfix); new variable or parameter values keep it, and the NULL rows are s's values at call time.  No topology is built.
+ * On the device, per chunk of variants on one stream per device: upload (or broadcast s's rows), one kernel expands the
+ * parameters per expression, the analyze kernel choose_analyze picks for the chunk's size (FK_ANALYZE_KERNEL honoured), one
+ * kernel counts each constraint's dependent expressions, download.  Chunks keep their buffers within about 1 GiB
+ * (FK_SYSTEM_BATCH_CHUNK overrides); variants are sharded over n_gpus devices (0 == all visible).
+ * Refusals come before any device work and leave `dependent` untouched: FK_ERR_INVALID for a null `s` or a null output with
+ * n > 0, FK_ERR_TOO_LARGE with choose_analyze's message for a drawing beyond the analyze limit (n_variables > 26,624, or one
+ * sketch's matrix beyond the 4 GiB workspace).  n = 0 and a drawing without constraints return FK_OK. */
+FK_API int fk_system_batch_analyze(const fk_system* s, uint32_t n, const double* vars, const double* params,
+                                   uint8_t* dependent /* [n][n_constraints] */, int n_gpus);
+/* == calculate_residual of every constraint for n variants: out[v][c] is what fk_system_residuals writes on a copy of s
+ * with the variant's numbers (unscaled; 2-norm of the two equalities of a coincidence), bit for bit on both of its paths
+ * (the batch plan's K2 evaluation and fk_topology_eval on the global sparse path: both evaluate with the same device
+ * formulas).  Arguments, plan, chunks, devices and FK_ERR_INVALID as fk_system_batch_analyze; one kernel evaluates every
+ * constraint of every variant from the plan's slot tables (q += r * r in expression order, then sqrt, as
+ * fk_system_residuals combines a coincidence).  Every drawing size is taken: no topology, batch plan or front limit. */
+FK_API int fk_system_batch_residuals(const fk_system* s, uint32_t n, const double* vars, const double* params,
+                                     double* out /* [n][n_constraints] */, int n_gpus);
 FK_API uint32_t fk_system_num_components(const fk_system* s);
 FK_API int fk_system_component(const fk_system* s, uint32_t index, uint32_t* n_elements, uint32_t* elements,
                                uint32_t* n_constraints, uint32_t* constraints);

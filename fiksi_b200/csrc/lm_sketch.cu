@@ -27,12 +27,23 @@ __device__ __forceinline__ double sk_rcp(double d) {
     return r;
 }
 
-// Entry e of a lane's region lives at byte (e << 8) behind the lane's region pointer (32 lanes x 8 bytes per entry).
-__device__ __forceinline__ double ldp(const char* p, uint32_t off) { return *reinterpret_cast<const double*>(p + off); }
-__device__ __forceinline__ void stp(char* p, uint32_t off, double v) { *reinterpret_cast<double*>(p + off) = v; }
+// Entry e of a lane's region lives at byte (e << 8) behind the lane's region address (32 lanes x 8 bytes per entry).
+// Regions are held as 32-bit shared-window addresses, so a target's address is one 32-bit add of the lane's region address
+// and the table word (generic pointers formed it as a 64-bit add folded into a three-input IADD3 with the window base).
+// The accesses are asm volatile with a memory clobber: the compiler keeps them in program order (a target's load, its
+// store; a later load of the same entry after that store), as it did for the plain loads and stores they replace.
+using SmAddr = uint32_t;
+__device__ __forceinline__ double lds(SmAddr a) {
+    double v;
+    asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a) : "memory");
+    return v;
+}
+__device__ __forceinline__ void sts(SmAddr a, double v) { asm volatile("st.shared.f64 [%0], %1;" ::"r"(a), "d"(v) : "memory"); }
+__device__ __forceinline__ double ldp(SmAddr p, uint32_t off) { return lds(p + off); }
+__device__ __forceinline__ void stp(SmAddr p, uint32_t off, double v) { sts(p + off, v); }
 
-__device__ __forceinline__ void cp_async8(void* smem_dst, const void* gmem_src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gmem_src) : "memory");
+__device__ __forceinline__ void cp_async8(SmAddr smem_dst, const void* gmem_src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_dst), "l"(gmem_src) : "memory");
 }
 
 __host__ __device__ constexpr int sk_arity(int kind) {
@@ -58,7 +69,7 @@ __device__ __forceinline__ void ld_words(const uint32_t* p, uint32_t (&wd)[(N + 
 // instead of forming a load-FMA-store chain.  SPECIAL: some slot of the row is a fixed variable.
 // rec: the row's record; h0: its first four words (already loaded).
 template <int KIND, bool SPECIAL>
-__device__ __forceinline__ void sk_eval_row(const uint32_t* rec, const uint4 h0, const char* x, const char* fx, const char* pr, char* w, char* f,
+__device__ __forceinline__ void sk_eval_row(const uint32_t* rec, const uint4 h0, SmAddr x, SmAddr fx, SmAddr pr, SmAddr w, SmAddr f,
                                             double& ssr) {
     constexpr int A = sk_arity(KIND);
     constexpr int NP = A * (A + 1) / 2;
@@ -80,41 +91,41 @@ __device__ __forceinline__ void sk_eval_row(const uint32_t* rec, const uint4 h0,
         else v[s] = ldp(x, src);
     }
     const double param = sk_has_param(KIND) ? ldp(pr, t[1]) : 0.0;
-    double* gp[A];
-    double* hp[NP];
+    SmAddr gp[A];
+    SmAddr hp[NP];
     double gv[A], hv[NP];
     // the targets do not depend on the row's arithmetic: fetch them before it
 #pragma unroll
     for (int s = 0; s < A; s++) {
         const uint32_t o = t[2 + A + s];
-        gp[s] = reinterpret_cast<double*>(w + o);
-        gv[s] = (!SPECIAL || o != kNone) ? *gp[s] : 0.0;
+        gp[s] = w + o;
+        gv[s] = (!SPECIAL || o != kNone) ? lds(gp[s]) : 0.0;
     }
 #pragma unroll
     for (int q = 0; q < NP; q++) {
         const uint32_t o = t[2 + 2 * A + q];
-        hp[q] = reinterpret_cast<double*>(f + o);
-        hv[q] = (!SPECIAL || o != kNone) ? *hp[q] : 0.0;
+        hp[q] = f + o;
+        hv[q] = (!SPECIAL || o != kNone) ? lds(hp[q]) : 0.0;
     }
     const double r = dev::eval_expression(KIND, v, param, g);
     ssr = ssr + r * r;  // lm.rs:195-197: sequential, not fused
     const double nr = -r;
 #pragma unroll
     for (int s = 0; s < A; s++)
-        if (!SPECIAL || t[2 + A + s] != kNone) *gp[s] = fma(g[s], nr, gv[s]);
+        if (!SPECIAL || t[2 + A + s] != kNone) sts(gp[s], fma(g[s], nr, gv[s]));
     int q = 0;
 #pragma unroll
     for (int a = 0; a < A; a++)
 #pragma unroll
         for (int b = 0; b <= a; b++, q++)
-            if (!SPECIAL || t[2 + 2 * A + q] != kNone) *hp[q] = fma(g[a], g[b], hv[q]);
+            if (!SPECIAL || t[2 + 2 * A + q] != kNone) sts(hp[q], fma(g[a], g[b], hv[q]));
 }
 
 // Two consecutive rows of one kind without fixed slots: loads and sqrt / divide chains of the two rows are independent
 // and issue together; the accumulations stay in row order (row r's stores precede row r+1's target loads).
 template <int KIND>
-__device__ __forceinline__ void sk_eval_rows2(const uint32_t* rec0, const uint4 h0, const uint32_t* rec1, const uint4 h1, const char* x,
-                                              const char* pr, char* w, char* f, double& ssr) {
+__device__ __forceinline__ void sk_eval_rows2(const uint32_t* rec0, const uint4 h0, const uint32_t* rec1, const uint4 h1, SmAddr x,
+                                              SmAddr pr, SmAddr w, SmAddr f, double& ssr) {
     constexpr int A = sk_arity(KIND);
     constexpr int NP = A * (A + 1) / 2;
     constexpr int NW = 2 + 2 * A + NP;
@@ -138,18 +149,18 @@ __device__ __forceinline__ void sk_eval_rows2(const uint32_t* rec0, const uint4 
     }
     const double p0 = sk_has_param(KIND) ? ldp(pr, t0[1]) : 0.0;
     const double p1 = sk_has_param(KIND) ? ldp(pr, t1[1]) : 0.0;
-    double* gp[A];
-    double* hp[NP];
+    SmAddr gp[A];
+    SmAddr hp[NP];
     double gv[A], hv[NP];
 #pragma unroll
     for (int s = 0; s < A; s++) {
-        gp[s] = reinterpret_cast<double*>(w + t0[2 + A + s]);
-        gv[s] = *gp[s];
+        gp[s] = w + t0[2 + A + s];
+        gv[s] = lds(gp[s]);
     }
 #pragma unroll
     for (int q = 0; q < NP; q++) {
-        hp[q] = reinterpret_cast<double*>(f + t0[2 + 2 * A + q]);
-        hv[q] = *hp[q];
+        hp[q] = f + t0[2 + 2 * A + q];
+        hv[q] = lds(hp[q]);
     }
     const double r0 = dev::eval_expression(KIND, v0, p0, g0);
     const double r1 = dev::eval_expression(KIND, v1, p1, g1);
@@ -158,32 +169,32 @@ __device__ __forceinline__ void sk_eval_rows2(const uint32_t* rec0, const uint4 
     {
         const double nr = -r0;
 #pragma unroll
-        for (int s = 0; s < A; s++) *gp[s] = fma(g0[s], nr, gv[s]);
+        for (int s = 0; s < A; s++) sts(gp[s], fma(g0[s], nr, gv[s]));
         int q = 0;
 #pragma unroll
         for (int a = 0; a < A; a++)
 #pragma unroll
-            for (int b = 0; b <= a; b++, q++) *hp[q] = fma(g0[a], g0[b], hv[q]);
+            for (int b = 0; b <= a; b++, q++) sts(hp[q], fma(g0[a], g0[b], hv[q]));
     }
     {
         const double nr = -r1;
 #pragma unroll
         for (int s = 0; s < A; s++) {
-            gp[s] = reinterpret_cast<double*>(w + t1[2 + A + s]);
-            gv[s] = *gp[s];
+            gp[s] = w + t1[2 + A + s];
+            gv[s] = lds(gp[s]);
         }
 #pragma unroll
         for (int q = 0; q < NP; q++) {
-            hp[q] = reinterpret_cast<double*>(f + t1[2 + 2 * A + q]);
-            hv[q] = *hp[q];
+            hp[q] = f + t1[2 + 2 * A + q];
+            hv[q] = lds(hp[q]);
         }
 #pragma unroll
-        for (int s = 0; s < A; s++) *gp[s] = fma(g1[s], nr, gv[s]);
+        for (int s = 0; s < A; s++) sts(gp[s], fma(g1[s], nr, gv[s]));
         int q = 0;
 #pragma unroll
         for (int a = 0; a < A; a++)
 #pragma unroll
-            for (int b = 0; b <= a; b++, q++) *hp[q] = fma(g1[a], g1[b], hv[q]);
+            for (int b = 0; b <= a; b++, q++) sts(hp[q], fma(g1[a], g1[b], hv[q]));
     }
 }
 
@@ -192,24 +203,24 @@ __device__ __forceinline__ void sk_eval_rows2(const uint32_t* rec0, const uint4 
 // rides along) is fetched, updated with one FMA and stored.  Same operations as the tile kernel's
 // L[dst] = fma(-(L[a] * inv), L[b], L[dst]).  body: C positions in f, C positions in w, C(C+1)/2 targets in f.
 template <int C>
-__device__ __forceinline__ void sk_column(const uint32_t* body, char* f, char* w, double wk, double inv) {
+__device__ __forceinline__ void sk_column(const uint32_t* body, SmAddr f, SmAddr w, double wk, double inv) {
     constexpr int NP = C * (C + 1) / 2;
     uint32_t t[(2 * C + NP + 3) / 4 * 4];
     ld_words<2 * C + NP>(body, t);
     double l[C], s[C], wv[C], d[NP];
-    double* wp[C];
-    double* dp[NP];
+    SmAddr wp[C];
+    SmAddr dp[NP];
 #pragma unroll
     for (int a = 0; a < C; a++) l[a] = ldp(f, t[a]);
 #pragma unroll
     for (int a = 0; a < C; a++) {
-        wp[a] = reinterpret_cast<double*>(w + t[C + a]);
-        wv[a] = *wp[a];
+        wp[a] = w + t[C + a];
+        wv[a] = lds(wp[a]);
     }
 #pragma unroll
     for (int q = 0; q < NP; q++) {
-        dp[q] = reinterpret_cast<double*>(f + t[2 * C + q]);
-        d[q] = *dp[q];
+        dp[q] = f + t[2 * C + q];
+        d[q] = lds(dp[q]);
     }
 #pragma unroll
     for (int a = 0; a < C; a++) s[a] = -(l[a] * inv);
@@ -217,30 +228,30 @@ __device__ __forceinline__ void sk_column(const uint32_t* body, char* f, char* w
 #pragma unroll
     for (int a = 0; a < C; a++)
 #pragma unroll
-        for (int b = 0; b <= a; b++, q++) *dp[q] = fma(s[a], l[b], d[q]);
+        for (int b = 0; b <= a; b++, q++) sts(dp[q], fma(s[a], l[b], d[q]));
 #pragma unroll
-    for (int a = 0; a < C; a++) *wp[a] = fma(s[a], wk, wv[a]);
+    for (int a = 0; a < C; a++) sts(wp[a], fma(s[a], wk, wv[a]));
 }
 
 // Columns with more than 8 entries below the diagonal: same operations, one at a time.
-__device__ __forceinline__ void sk_column_generic(const uint32_t* t, uint32_t C, char* f, char* w, double wk, double inv) {
+__device__ __forceinline__ void sk_column_generic(const uint32_t* t, uint32_t C, SmAddr f, SmAddr w, double wk, double inv) {
     uint32_t q = 0;
     for (uint32_t a = 0; a < C; a++) {
         const double la = ldp(f, t[a]);
         const double sa = -(la * inv);
         for (uint32_t b = 0; b <= a; b++, q++) {
-            double* dst = reinterpret_cast<double*>(f + t[2 * C + q]);
+            SmAddr dst = f + t[2 * C + q];
             const double lb = b == a ? la : ldp(f, t[b]);
-            *dst = fma(sa, lb, *dst);
+            sts(dst, fma(sa, lb, lds(dst)));
         }
-        double* wr = reinterpret_cast<double*>(w + t[C + a]);
-        *wr = fma(sa, wk, *wr);
+        SmAddr wr = w + t[C + a];
+        sts(wr, fma(sa, wk, lds(wr)));
     }
 }
 
 // acc - sum_{a} (L D)(row_a, k) z(row_a), rows descending as the tile kernel's scatter form applies them.
 template <int C>
-__device__ __forceinline__ double sk_back_column(const uint32_t* body, const char* f, const char* w, double acc) {
+__device__ __forceinline__ double sk_back_column(const uint32_t* body, SmAddr f, SmAddr w, double acc) {
     uint32_t t[(2 * C + 3) / 4 * 4];
     ld_words<2 * C>(body, t);
     double l[C], z[C];
@@ -261,7 +272,7 @@ __device__ __forceinline__ uint64_t sk_trace_push(uint64_t h, uint32_t code) { r
 // sketch's loads are in flight at once and the thread waits once (with one warp or two per SM nothing else would hide the
 // DRAM latency of a load-then-store loop).  Raw mode (SkRaw): the whole variable row (and the parameter row unless shared)
 // is staged in the g and H regions first, then scale, scaling and perturbation run exactly as fk_batch_prepare_kernel does.
-__device__ __forceinline__ double sk_stage_inputs(const SkProgram& P, const SkRaw& R, const uint32_t* tab, char* base, char* xp, uint32_t sk,
+__device__ __forceinline__ double sk_stage_inputs(const SkProgram& P, const SkRaw& R, const uint32_t* tab, SmAddr base, SmAddr xp, uint32_t sk,
                                                   const double* __restrict__ vars_all, const double* __restrict__ params_all) {
     const uint32_t n = P.n;
     if (R.raw_vars == nullptr) {
@@ -273,7 +284,7 @@ __device__ __forceinline__ double sk_stage_inputs(const SkProgram& P, const SkRa
         asm volatile("cp.async.commit_group;\n cp.async.wait_group 0;" ::: "memory");
         return 1.0;
     }
-    char* S = base + (P.w << 8);  // scratch: g and H regions, n + nnz(L) entries (sk_raw_fits)
+    SmAddr S = base + (P.w << 8);  // scratch: g and H regions, n + nnz(L) entries (sk_raw_fits)
     const double* rv = R.raw_vars + (size_t)sk * P.n_vars;
     const double* rp = R.raw_param + (R.shared_param ? 0 : (size_t)sk * P.n_expr);
     for (uint32_t i = 0; i < P.n_vars; i++) cp_async8(S + (i << 8), rv + i);
@@ -334,7 +345,7 @@ __device__ __forceinline__ double sk_stage_inputs(const SkProgram& P, const SkRa
         return j == kNone ? col : col + (col * (1.0 / 8196.0) * __ldg(R.draws + 2 * j) + (1.0 / 65568.0) * __ldg(R.draws + 2 * j + 1));
     };
     // count variables listed at tab[off_tab ..], their draw positions in draw_idx, into entries entry0.. of the region dst
-    auto stage_vars = [&](uint32_t count, uint32_t off_tab, const uint32_t* __restrict__ draw_idx, char* dst, uint32_t entry0) {
+    auto stage_vars = [&](uint32_t count, uint32_t off_tab, const uint32_t* __restrict__ draw_idx, SmAddr dst, uint32_t entry0) {
         uint32_t c = 0;
         for (; c + 4 <= count; c += 4) {
             uint32_t j[4];
@@ -396,21 +407,21 @@ fk_batch_lm_sketch_kernel(const SkProgram P, const SkRaw R, uint32_t n_sketches,
     for (uint32_t i = threadIdx.x; i < P.tab_words / 4; i += blockDim.x)
         reinterpret_cast<uint4*>(tab)[i] = __ldg(reinterpret_cast<const uint4*>(P.tab) + i);
     __syncthreads();
-    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+    const uint32_t lane = threadIdx.x & 31u, warp = __shfl_sync(0xFFFFFFFFu, threadIdx.x >> 5, 0);  // (lane 0's copy: nvcc then knows it is warp-uniform)
     const uint32_t sketch = (blockIdx.x * (blockDim.x >> 5) + warp) * 32u + lane;
     if (sketch - lane >= n_sketches) return;  // a whole warp without work
     const bool valid = sketch < n_sketches;
     const uint32_t sk = valid ? sketch : n_sketches - 1;  // idle lanes shadow the last sketch and store nothing
-    char* const base = sk_smem + (size_t)P.tab_words * 4 + (size_t)warp * P.entries * 256u + lane * 8u;
+    const SmAddr base = (SmAddr)__cvta_generic_to_shared(sk_smem) + P.tab_words * 4 + warp * P.entries * 256u + lane * 8u;
     const uint32_t n = P.n;
 
     // accepted / trial point: the two roles swap per lane on accept (a register exchange instead of a copy)
-    char* xp = base + (P.xa << 8);
-    char* xsp = base + (P.xb << 8);
-    char* const w = base + (P.w << 8);
-    char* const f = base + (P.f << 8);
-    const char* const fx = base + (P.fx << 8);
-    const char* const pr = base + (P.pr << 8);
+    SmAddr xp = base + (P.xa << 8);
+    SmAddr xsp = base + (P.xb << 8);
+    const SmAddr w = base + (P.w << 8);
+    const SmAddr f = base + (P.f << 8);
+    const SmAddr fx = base + (P.fx << 8);
+    const SmAddr pr = base + (P.pr << 8);
 
     const double scale = sk_stage_inputs(P, R, tab, base, xp, sk, vars_all, params_all);
 
@@ -424,7 +435,7 @@ fk_batch_lm_sketch_kernel(const SkProgram P, const SkRaw R, uint32_t n_sketches,
     // rejected / unsolved step of some sketch of the warp (its H and g were consumed by the factorisation;
     // sketches that accepted recompute the values they already hold).
     enum { kInit, kTrial, kRestore } mode = kInit;
-    const char* xe = xp;
+    SmAddr xe = xp;
 
     for (;;) {
         // ---- residuals, g = -J^T r (into w), H = J^T J (into f) at xe; s = sum of squared residuals ----------
@@ -498,7 +509,7 @@ fk_batch_lm_sketch_kernel(const SkProgram P, const SkRaw R, uint32_t n_sketches,
                     if (lambda < 1e-50) lambda = 1e-50;
                     accepted++;
                     trace = sk_trace_push(trace, 1);
-                    char* tmp = xp; xp = xsp; xsp = tmp;
+                    SmAddr tmp = xp; xp = xsp; xsp = tmp;
                     const bool stalled = (ssr - ssr_s) / ssr <= 1e-6;  // lm.rs:164-168
                     ssr = ssr_s;
                     if (stalled) {
@@ -540,15 +551,15 @@ fk_batch_lm_sketch_kernel(const SkProgram P, const SkRaw R, uint32_t n_sketches,
             uint4 hn = *reinterpret_cast<const uint4*>(rec);
             for (uint32_t c = 0; c < n; c++) {
                 const uint32_t C = hn.x;
-                double* dp = reinterpret_cast<double*>(f + hn.y);
+                SmAddr dp = f + hn.y;
                 const double wk = ldp(w, hn.z);
                 const uint32_t* body = rec + 4;
                 rec = body + ((2 * C + C * (C + 1) / 2 + 3u) & ~3u);
                 hn = *reinterpret_cast<const uint4*>(rec);  // next column's header
-                const double d = *dp + lam2;
+                const double d = lds(dp) + lam2;
                 if (fstat == 0 && !(d > 0.0 && d < INFINITY)) fstat = d != d ? 2 : 1;
                 const double inv = sk_rcp(d);
-                *dp = inv;
+                sts(dp, inv);
                 switch (C) {
                     case 0: break;
                     case 1: sk_column<1>(body, f, w, wk, inv); break;
@@ -569,12 +580,12 @@ fk_batch_lm_sketch_kernel(const SkProgram P, const SkRaw R, uint32_t n_sketches,
             for (uint32_t c = 0; c < n; c++) {
                 const uint32_t C = hn.x;
                 const double inv = ldp(f, hn.y);
-                double* zp = reinterpret_cast<double*>(w + hn.z);
-                double* xd = reinterpret_cast<double*>(xsp + hn.w);
+                SmAddr zp = w + hn.z;
+                SmAddr xd = xsp + hn.w;
                 const uint32_t* body = rec + 4;
                 rec = body + ((2 * C + 3u) & ~3u);
                 hn = *reinterpret_cast<const uint4*>(rec);
-                double acc = *zp;
+                double acc = lds(zp);
                 switch (C) {
                     case 0: break;
                     case 1: acc = sk_back_column<1>(body, f, w, acc); break;
@@ -590,8 +601,8 @@ fk_batch_lm_sketch_kernel(const SkProgram P, const SkRaw R, uint32_t n_sketches,
                         break;
                 }
                 const double z = acc * inv;
-                *zp = z;
-                *xd = z;
+                sts(zp, z);
+                sts(xd, z);
             }
         }
         {   // lm.rs:139 (sum of squared steps, in variable order) and lm.rs:144-146 (trial point)
@@ -656,7 +667,7 @@ fk_batch_lm_sketch_kernel(const SkProgram P, const SkRaw R, uint32_t n_sketches,
 constexpr uint32_t kPairExtra = 38;  // entries behind the solo state: 2 steps x 2 rows x (8 gradients + residual) staging, lambda, pad
 
 template <int KIND, bool SPECIAL>
-__device__ __forceinline__ void sk_row_produce(const uint32_t* rec, const uint4 h0, const char* x, const char* fx, const char* pr, char* stage,
+__device__ __forceinline__ void sk_row_produce(const uint32_t* rec, const uint4 h0, SmAddr x, SmAddr fx, SmAddr pr, SmAddr stage,
                                                double& ssr) {
     constexpr int A = sk_arity(KIND);
     uint32_t t[(2 + A + 3) / 4 * 4];
@@ -686,8 +697,8 @@ __device__ __forceinline__ void sk_row_produce(const uint32_t* rec, const uint4 
 // Two consecutive rows of the same kind without fixed slots: their loads and their sqrt / divide chains are independent,
 // so issuing them together hides most of one row's latency behind the other's.
 template <int KIND>
-__device__ __forceinline__ void sk_rows_produce2(const uint32_t* rec0, const uint4 h0, const uint32_t* rec1, const uint4 h1, const char* x,
-                                                 const char* pr, char* st0, char* st1, double& ssr) {
+__device__ __forceinline__ void sk_rows_produce2(const uint32_t* rec0, const uint4 h0, const uint32_t* rec1, const uint4 h1, SmAddr x,
+                                                 SmAddr pr, SmAddr st0, SmAddr st1, double& ssr) {
     constexpr int A = sk_arity(KIND);
     constexpr int NWD = (2 + A + 3) / 4 * 4;
     uint32_t t0[NWD], t1[NWD];
@@ -723,39 +734,39 @@ __device__ __forceinline__ void sk_rows_produce2(const uint32_t* rec0, const uin
 }
 
 template <int KIND, bool SPECIAL>
-__device__ __forceinline__ void sk_row_consume(const uint32_t* rec, const char* stage, char* w, char* f) {
+__device__ __forceinline__ void sk_row_consume(const uint32_t* rec, SmAddr stage, SmAddr w, SmAddr f) {
     constexpr int A = sk_arity(KIND);
     constexpr int NP = A * (A + 1) / 2;
     constexpr int NW = 2 + 2 * A + NP;
     uint32_t t[(NW + 3) / 4 * 4];
     ld_words<NW>(rec, t);
-    double* gp[A];
-    double* hp[NP];
+    SmAddr gp[A];
+    SmAddr hp[NP];
     double gv[A], hv[NP], g[A];
 #pragma unroll
     for (int s = 0; s < A; s++) {
         const uint32_t o = t[2 + A + s];
-        gp[s] = reinterpret_cast<double*>(w + o);
-        gv[s] = (!SPECIAL || o != kNone) ? *gp[s] : 0.0;
+        gp[s] = w + o;
+        gv[s] = (!SPECIAL || o != kNone) ? lds(gp[s]) : 0.0;
     }
 #pragma unroll
     for (int q = 0; q < NP; q++) {
         const uint32_t o = t[2 + 2 * A + q];
-        hp[q] = reinterpret_cast<double*>(f + o);
-        hv[q] = (!SPECIAL || o != kNone) ? *hp[q] : 0.0;
+        hp[q] = f + o;
+        hv[q] = (!SPECIAL || o != kNone) ? lds(hp[q]) : 0.0;
     }
 #pragma unroll
     for (int s = 0; s < A; s++) g[s] = ldp(stage, (uint32_t)s << 8);
     const double nr = ldp(stage, 8u << 8);
 #pragma unroll
     for (int s = 0; s < A; s++)
-        if (!SPECIAL || t[2 + A + s] != kNone) *gp[s] = fma(g[s], nr, gv[s]);
+        if (!SPECIAL || t[2 + A + s] != kNone) sts(gp[s], fma(g[s], nr, gv[s]));
     int q = 0;
 #pragma unroll
     for (int a = 0; a < A; a++)
 #pragma unroll
         for (int b = 0; b <= a; b++, q++)
-            if (!SPECIAL || t[2 + 2 * A + q] != kNone) *hp[q] = fma(g[a], g[b], hv[q]);
+            if (!SPECIAL || t[2 + 2 * A + q] != kNone) sts(hp[q], fma(g[a], g[b], hv[q]));
 }
 
 // The leader's share of a column's NT targets: less than half, because the leader also carries the pivot checks and,
@@ -766,27 +777,27 @@ __host__ __device__ constexpr int sk_leader_share(int nt) { return (nt * FK_SK_L
 // One part of a column's updates (HALF 0: the leader's first sk_leader_share(NT) targets in the order "pairs (a, b),
 // then the C right-hand-side entries", HALF 1: the rest).  Both parts read the whole column.
 template <int C, int HALF>
-__device__ __forceinline__ void sk_column_half(const uint32_t* body, char* f, char* w, double wk, double inv) {
+__device__ __forceinline__ void sk_column_half(const uint32_t* body, SmAddr f, SmAddr w, double wk, double inv) {
     constexpr int NP = C * (C + 1) / 2, NT = NP + C, H0 = sk_leader_share(NT);
     constexpr int LO = HALF ? H0 : 0, HI = HALF ? NT : H0;
     uint32_t t[(2 * C + NP + 3) / 4 * 4];
     ld_words<2 * C + NP>(body, t);
     double l[C], s[C], wv[C], d[NP];
-    double* wp[C];
-    double* dp[NP];
+    SmAddr wp[C];
+    SmAddr dp[NP];
 #pragma unroll
     for (int a = 0; a < C; a++) l[a] = ldp(f, t[a]);
 #pragma unroll
     for (int q = 0; q < NP; q++)
         if (q >= LO && q < HI) {
-            dp[q] = reinterpret_cast<double*>(f + t[2 * C + q]);
-            d[q] = *dp[q];
+            dp[q] = f + t[2 * C + q];
+            d[q] = lds(dp[q]);
         }
 #pragma unroll
     for (int a = 0; a < C; a++)
         if (NP + a >= LO && NP + a < HI) {
-            wp[a] = reinterpret_cast<double*>(w + t[C + a]);
-            wv[a] = *wp[a];
+            wp[a] = w + t[C + a];
+            wv[a] = lds(wp[a]);
         }
 #pragma unroll
     for (int a = 0; a < C; a++) s[a] = -(l[a] * inv);
@@ -795,13 +806,13 @@ __device__ __forceinline__ void sk_column_half(const uint32_t* body, char* f, ch
     for (int a = 0; a < C; a++)
 #pragma unroll
         for (int b = 0; b <= a; b++, q++)
-            if (q >= LO && q < HI) *dp[q] = fma(s[a], l[b], d[q]);
+            if (q >= LO && q < HI) sts(dp[q], fma(s[a], l[b], d[q]));
 #pragma unroll
     for (int a = 0; a < C; a++)
-        if (NP + a >= LO && NP + a < HI) *wp[a] = fma(s[a], wk, wv[a]);
+        if (NP + a >= LO && NP + a < HI) sts(wp[a], fma(s[a], wk, wv[a]));
 }
 
-__device__ __forceinline__ void sk_column_generic_half(const uint32_t* t, uint32_t C, int half, char* f, char* w, double wk, double inv) {
+__device__ __forceinline__ void sk_column_generic_half(const uint32_t* t, uint32_t C, int half, SmAddr f, SmAddr w, double wk, double inv) {
     const uint32_t NP = C * (C + 1) / 2, NT = NP + C, H0 = (uint32_t)sk_leader_share((int)NT);
     const uint32_t lo = half ? H0 : 0, hi = half ? NT : H0;
     uint32_t q = 0;
@@ -810,19 +821,19 @@ __device__ __forceinline__ void sk_column_generic_half(const uint32_t* t, uint32
         const double sa = -(la * inv);
         for (uint32_t b = 0; b <= a; b++, q++) {
             if (q < lo || q >= hi) continue;
-            double* dst = reinterpret_cast<double*>(f + t[2 * C + q]);
+            SmAddr dst = f + t[2 * C + q];
             const double lb = b == a ? la : ldp(f, t[b]);
-            *dst = fma(sa, lb, *dst);
+            sts(dst, fma(sa, lb, lds(dst)));
         }
         if (NP + a >= lo && NP + a < hi) {
-            double* wr = reinterpret_cast<double*>(w + t[C + a]);
-            *wr = fma(sa, wk, *wr);
+            SmAddr wr = w + t[C + a];
+            sts(wr, fma(sa, wk, lds(wr)));
         }
     }
 }
 
 template <int HALF>
-__device__ __forceinline__ void sk_column_dispatch_half(uint32_t C, const uint32_t* body, char* f, char* w, double wk, double inv) {
+__device__ __forceinline__ void sk_column_dispatch_half(uint32_t C, const uint32_t* body, SmAddr f, SmAddr w, double wk, double inv) {
     switch (C) {
         case 0: break;
         case 1: sk_column_half<1, HALF>(body, f, w, wk, inv); break;
@@ -846,15 +857,15 @@ fk_batch_lm_sketch_pair_kernel(const SkProgram P, const SkRaw R, uint32_t n_sket
     for (uint32_t i = threadIdx.x; i < P.tab_words / 4; i += blockDim.x)
         reinterpret_cast<uint4*>(tab)[i] = __ldg(reinterpret_cast<const uint4*>(P.tab) + i);
     __syncthreads();
-    const uint32_t lane = threadIdx.x & 31u, role = threadIdx.x >> 5;
+    const uint32_t lane = threadIdx.x & 31u, role = __shfl_sync(0xFFFFFFFFu, threadIdx.x >> 5, 0);  // (lane 0's copy: nvcc then knows it is warp-uniform)
     const uint32_t sketch = blockIdx.x * 32u + lane;
     const bool valid = sketch < n_sketches;
     const uint32_t sk = valid ? sketch : n_sketches - 1;
-    char* const base = sk_smem + (size_t)P.tab_words * 4 + lane * 8u;
+    const SmAddr base = (SmAddr)__cvta_generic_to_shared(sk_smem) + P.tab_words * 4 + lane * 8u;
     const uint32_t n = P.n;
-    char* const w = base + (P.w << 8);
-    char* const f = base + (P.f << 8);
-    char* const stage = base + (P.entries << 8);  // [2 steps][2 rows][9] staging, then lambda
+    const SmAddr w = base + (P.w << 8);
+    const SmAddr f = base + (P.f << 8);
+    const SmAddr stage = base + (P.entries << 8);  // [2 steps][2 rows][9] staging, then lambda
 
     if (role == 1) {
         // ---- helper ---------------------------------------------------------------------------------------
@@ -879,8 +890,8 @@ fk_batch_lm_sketch_pair_kernel(const SkProgram P, const SkRaw R, uint32_t n_sket
                 const uint32_t* rec1 = cur + (h >> 16);
                 const uint32_t h1 = rec1[0];
                 const bool two = r + 1 < P.m && (h & 0x1FFu) < 0x100u && (h1 & 0x1FFu) == (h & 0x1FFu);
-                const char* st0 = stage + ((step & 1u) * 18u << 8);
-                const char* st1 = st0 + (9u << 8);
+                SmAddr st0 = stage + ((step & 1u) * 18u << 8);
+                SmAddr st1 = st0 + (9u << 8);
                 if (two) {
                     rec = rec1 + (h1 >> 16);
                     r += 2;
@@ -912,12 +923,12 @@ fk_batch_lm_sketch_pair_kernel(const SkProgram P, const SkRaw R, uint32_t n_sket
             uint4 hn = *reinterpret_cast<const uint4*>(frec);
             for (uint32_t col = 0; col < n; col++) {
                 const uint32_t C = hn.x;
-                const double* dp = reinterpret_cast<const double*>(f + hn.y);
+                const SmAddr dp = f + hn.y;
                 const double wk = ldp(w, hn.z);
                 const uint32_t* body = frec + 4;
                 frec = body + ((2 * C + C * (C + 1) / 2 + 3u) & ~3u);
                 hn = *reinterpret_cast<const uint4*>(frec);
-                const double inv = sk_rcp(*dp + lam2);  // (the leader stores 1 / d one column later)
+                const double inv = sk_rcp(lds(dp) + lam2);  // (the leader stores 1 / d one column later)
                 sk_column_dispatch_half<1>(C, body, f, w, wk, inv);
                 __syncthreads();
             }
@@ -927,10 +938,10 @@ fk_batch_lm_sketch_pair_kernel(const SkProgram P, const SkRaw R, uint32_t n_sket
     }
 
     // ---- leader ---------------------------------------------------------------------------------------------
-    char* xp = base + (P.xa << 8);
-    char* xsp = base + (P.xb << 8);
-    const char* const fx = base + (P.fx << 8);
-    const char* const pr = base + (P.pr << 8);
+    SmAddr xp = base + (P.xa << 8);
+    SmAddr xsp = base + (P.xb << 8);
+    const SmAddr fx = base + (P.fx << 8);
+    const SmAddr pr = base + (P.pr << 8);
     const double scale = sk_stage_inputs(P, R, tab, base, xp, sk, vars_all, params_all);
     if (R.raw_vars != nullptr) __syncthreads();  // the helper may clear g and H now
 
@@ -940,7 +951,7 @@ fk_batch_lm_sketch_pair_kernel(const SkProgram P, const SkRaw R, uint32_t n_sket
     bool active = valid;
     int fstat = 0;
     enum { kInit, kTrial, kRestore } mode = kInit;
-    const char* xe = xp;
+    SmAddr xe = xp;
     for (;;) {
         double s = 0.0;
         {
@@ -951,8 +962,8 @@ fk_batch_lm_sketch_pair_kernel(const SkProgram P, const SkRaw R, uint32_t n_sket
                 const uint32_t* rec1 = cur + (h.x >> 16);
                 const uint4 h1 = *reinterpret_cast<const uint4*>(rec1);
                 const bool two = r + 1 < P.m && (h.x & 0x1FFu) < 0x100u && (h1.x & 0x1FFu) == (h.x & 0x1FFu);
-                char* st0 = stage + ((step & 1u) * 18u << 8);
-                char* st1 = st0 + (9u << 8);
+                SmAddr st0 = stage + ((step & 1u) * 18u << 8);
+                SmAddr st1 = st0 + (9u << 8);
 #define FK_SK_ROW(K)                                                                           \
     case K:                                                                                    \
         if (two) sk_rows_produce2<K>(cur, h, rec1, h1, xe, pr, st0, st1, s);                   \
@@ -1002,7 +1013,7 @@ fk_batch_lm_sketch_pair_kernel(const SkProgram P, const SkRaw R, uint32_t n_sket
                     if (lambda < 1e-50) lambda = 1e-50;
                     accepted++;
                     trace = sk_trace_push(trace, 1);
-                    char* tmp = xp; xp = xsp; xsp = tmp;
+                    SmAddr tmp = xp; xp = xsp; xsp = tmp;
                     const bool stalled = (ssr - ssr_s) / ssr <= 1e-6;
                     ssr = ssr_s;
                     if (stalled) {
@@ -1046,27 +1057,27 @@ fk_batch_lm_sketch_pair_kernel(const SkProgram P, const SkRaw R, uint32_t n_sket
         if (c == 2) break;
         {
             fstat = 0;
-            double* dp_prev = nullptr;
+            SmAddr dp_prev = kNone;
             double inv_prev = 0.0;
             const uint32_t* rec = tab + P.off_factor;
             uint4 hn = *reinterpret_cast<const uint4*>(rec);
             for (uint32_t col = 0; col < n; col++) {
                 const uint32_t C = hn.x;
-                double* dp = reinterpret_cast<double*>(f + hn.y);
+                SmAddr dp = f + hn.y;
                 const double wk = ldp(w, hn.z);
                 const uint32_t* body = rec + 4;
                 rec = body + ((2 * C + C * (C + 1) / 2 + 3u) & ~3u);
                 hn = *reinterpret_cast<const uint4*>(rec);
-                const double d = *dp + lam2;
+                const double d = lds(dp) + lam2;
                 if (fstat == 0 && !(d > 0.0 && d < INFINITY)) fstat = d != d ? 2 : 1;
                 const double inv = sk_rcp(d);
-                if (dp_prev) *dp_prev = inv_prev;  // the helper read that pivot before the last barrier
+                if (dp_prev != kNone) sts(dp_prev, inv_prev);  // the helper read that pivot before the last barrier
                 sk_column_dispatch_half<0>(C, body, f, w, wk, inv);
                 dp_prev = dp;
                 inv_prev = inv;
                 __syncthreads();
             }
-            if (dp_prev) *dp_prev = inv_prev;
+            if (dp_prev != kNone) sts(dp_prev, inv_prev);
         }
         {
             const uint32_t* rec = tab + P.off_back;
@@ -1074,12 +1085,12 @@ fk_batch_lm_sketch_pair_kernel(const SkProgram P, const SkRaw R, uint32_t n_sket
             for (uint32_t col = 0; col < n; col++) {
                 const uint32_t C = hn.x;
                 const double inv = ldp(f, hn.y);
-                double* zp = reinterpret_cast<double*>(w + hn.z);
-                double* xd = reinterpret_cast<double*>(xsp + hn.w);
+                SmAddr zp = w + hn.z;
+                SmAddr xd = xsp + hn.w;
                 const uint32_t* body = rec + 4;
                 rec = body + ((2 * C + 3u) & ~3u);
                 hn = *reinterpret_cast<const uint4*>(rec);
-                double acc = *zp;
+                double acc = lds(zp);
                 switch (C) {
                     case 0: break;
                     case 1: acc = sk_back_column<1>(body, f, w, acc); break;
@@ -1095,8 +1106,8 @@ fk_batch_lm_sketch_pair_kernel(const SkProgram P, const SkRaw R, uint32_t n_sket
                         break;
                 }
                 const double z = acc * inv;
-                *zp = z;
-                *xd = z;
+                sts(zp, z);
+                sts(xd, z);
             }
         }
         __syncthreads();  // H and g are consumed: the helper clears them for the trial evaluation

@@ -9,6 +9,7 @@
 
 #include "expressions.cuh"
 #include "lm_kernels.cuh"
+#include "symbolic.hpp"
 
 namespace fk {
 
@@ -233,6 +234,61 @@ __device__ __forceinline__ void sk_column(const uint32_t* body, SmAddr f, SmAddr
     for (int a = 0; a < C; a++) sts(wp[a], fma(s[a], wk, wv[a]));
 }
 
+// Target q of a column record is the pair (a, b), b <= a, of the column's rows: q = a(a+1)/2 + b.
+__host__ __device__ constexpr int sk_tri(int a, int b) { return a * (a + 1) / 2 + b; }
+
+// Columns k and k+1 of a pair record (symbolic.hpp): L(:,k) = {k+1} u L(:,k+1), so column k+1's pivot, entries and
+// right-hand side entry are column k's targets (0, 0), (a, 0) and w row 0, and its targets are column k's targets
+// (a, b), a >= b >= 1.  Every target is loaded once, receives column k's FMA and then column k+1's, and is stored once;
+// per entry the operations and their order are those of sk_column for k and then for k+1.  Column k+1's pivot is checked
+// after column k's (the caller's), so fstat still records the first bad pivot in column order.
+template <int C>
+__device__ __forceinline__ void sk_column2(const uint32_t* body, SmAddr f, SmAddr w, double wk, double inv, double lam2, int& fstat) {
+    constexpr int NP = C * (C + 1) / 2;
+    uint32_t t[(2 * C + NP + 3) / 4 * 4];
+    ld_words<2 * C + NP>(body, t);
+    double l[C], s[C], wv[C], d[NP];
+    SmAddr wp[C];
+    SmAddr dp[NP];
+#pragma unroll
+    for (int a = 0; a < C; a++) l[a] = ldp(f, t[a]);
+#pragma unroll
+    for (int a = 0; a < C; a++) {
+        wp[a] = w + t[C + a];
+        wv[a] = lds(wp[a]);
+    }
+#pragma unroll
+    for (int q = 0; q < NP; q++) {
+        dp[q] = f + t[2 * C + q];
+        d[q] = lds(dp[q]);
+    }
+#pragma unroll
+    for (int a = 0; a < C; a++) s[a] = -(l[a] * inv);
+    int q = 0;
+#pragma unroll
+    for (int a = 0; a < C; a++)
+#pragma unroll
+        for (int b = 0; b <= a; b++, q++) d[q] = fma(s[a], l[b], d[q]);
+#pragma unroll
+    for (int a = 0; a < C; a++) wv[a] = fma(s[a], wk, wv[a]);
+    // column k+1's entries and right-hand side entry are final now
+#pragma unroll
+    for (int a = 1; a < C; a++) sts(dp[sk_tri(a, 0)], d[sk_tri(a, 0)]);
+    sts(wp[0], wv[0]);
+    const double d1 = d[0] + lam2;
+    if (fstat == 0 && !(d1 > 0.0 && d1 < INFINITY)) fstat = d1 != d1 ? 2 : 1;
+    const double inv1 = sk_rcp(d1);
+    sts(dp[0], inv1);
+#pragma unroll
+    for (int a = 1; a < C; a++) s[a] = -(d[sk_tri(a, 0)] * inv1);
+#pragma unroll
+    for (int a = 1; a < C; a++)
+#pragma unroll
+        for (int b = 1; b <= a; b++) sts(dp[sk_tri(a, b)], fma(s[a], d[sk_tri(b, 0)], d[sk_tri(a, b)]));
+#pragma unroll
+    for (int a = 1; a < C; a++) sts(wp[a], fma(s[a], wv[0], wv[a]));
+}
+
 // Columns with more than 8 entries below the diagonal: same operations, one at a time.
 __device__ __forceinline__ void sk_column_generic(const uint32_t* t, uint32_t C, SmAddr f, SmAddr w, double wk, double inv) {
     uint32_t q = 0;
@@ -263,6 +319,76 @@ __device__ __forceinline__ double sk_back_column(const uint32_t* body, SmAddr f,
 #pragma unroll
     for (int a = C - 1; a >= 0; a--) acc = fma(-l[a], z[a], acc);
     return acc;
+}
+
+// Back substitution of a pair record: column k+1, then column k (acc: column k's right-hand side).  Rows descend and row
+// k+1 is column k's last, so both sums run side by side over the rows below k+1 and share their z loads; z(k+1) goes to w
+// and to the trial point's slot xs here.  Returns column k's sum, to be multiplied by 1 / d(k).
+template <int C>
+__device__ __forceinline__ double sk_back_column2(const uint32_t* body, SmAddr f, SmAddr w, SmAddr xs, double acc) {
+    uint32_t t[(3 * C + 1 + 3) / 4 * 4];
+    ld_words<3 * C + 1>(body, t);  // column k's entries, rows, column k+1's entries, its diagonal, perm[k+1]
+    double l[C], l1[C], z[C];
+#pragma unroll
+    for (int a = 0; a < C; a++) l[a] = ldp(f, t[a]);
+#pragma unroll
+    for (int a = 1; a < C; a++) {
+        z[a] = ldp(w, t[C + a]);
+        l1[a] = ldp(f, t[2 * C + a - 1]);
+    }
+    const SmAddr zp1 = w + t[C];
+    double acc1 = lds(zp1);
+    const double inv1 = ldp(f, t[3 * C - 1]);
+#pragma unroll
+    for (int a = C - 1; a >= 1; a--) {
+        acc1 = fma(-l1[a], z[a], acc1);
+        acc = fma(-l[a], z[a], acc);
+    }
+    const double z1 = acc1 * inv1;
+    sts(zp1, z1);
+    stp(xs, t[3 * C], z1);
+    return fma(-l[0], z1, acc);
+}
+
+// D L^T z = y in place in w (rec: the back section), delta in variable order (qr.rs:354) into the trial point's slots xs.
+__device__ __forceinline__ void sk_back_solve(const uint32_t* rec, uint32_t n, SmAddr f, SmAddr w, SmAddr xs) {
+    uint4 hn = *reinterpret_cast<const uint4*>(rec);
+    for (uint32_t c = 0; c < n;) {
+        const uint32_t hx = hn.x, C = hx & (kSkPairFlag - 1), two = hx & kSkPairFlag;
+        const double inv = ldp(f, hn.y);
+        SmAddr zp = w + hn.z;
+        SmAddr xd = xs + hn.w;
+        const uint32_t* body = rec + 4;
+        rec = body + ((two ? 3 * C + 1 + 3u : 2 * C + 3u) & ~3u);
+        hn = *reinterpret_cast<const uint4*>(rec);
+        double acc = lds(zp);
+        c += two ? 2 : 1;
+        switch (hx) {
+            case 0: break;
+            case 1: acc = sk_back_column<1>(body, f, w, acc); break;
+            case 2: acc = sk_back_column<2>(body, f, w, acc); break;
+            case 3: acc = sk_back_column<3>(body, f, w, acc); break;
+            case 4: acc = sk_back_column<4>(body, f, w, acc); break;
+            case 5: acc = sk_back_column<5>(body, f, w, acc); break;
+            case 6: acc = sk_back_column<6>(body, f, w, acc); break;
+            case 7: acc = sk_back_column<7>(body, f, w, acc); break;
+            case 8: acc = sk_back_column<8>(body, f, w, acc); break;
+            case kSkPairFlag | 1: acc = sk_back_column2<1>(body, f, w, xs, acc); break;
+            case kSkPairFlag | 2: acc = sk_back_column2<2>(body, f, w, xs, acc); break;
+            case kSkPairFlag | 3: acc = sk_back_column2<3>(body, f, w, xs, acc); break;
+            case kSkPairFlag | 4: acc = sk_back_column2<4>(body, f, w, xs, acc); break;
+            case kSkPairFlag | 5: acc = sk_back_column2<5>(body, f, w, xs, acc); break;
+            case kSkPairFlag | 6: acc = sk_back_column2<6>(body, f, w, xs, acc); break;
+            case kSkPairFlag | 7: acc = sk_back_column2<7>(body, f, w, xs, acc); break;
+            case kSkPairFlag | 8: acc = sk_back_column2<8>(body, f, w, xs, acc); break;
+            default:  // single columns with more than 8 entries below the diagonal
+                for (uint32_t a = C; a-- > 0;) acc = fma(-ldp(f, body[a]), ldp(w, body[C + a]), acc);
+                break;
+        }
+        const double z = acc * inv;
+        sts(zp, z);
+        sts(xd, z);
+    }
 }
 
 __device__ __forceinline__ uint64_t sk_trace_push(uint64_t h, uint32_t code) { return h * 3ull + code + 1ull; }
@@ -549,17 +675,31 @@ fk_batch_lm_sketch_kernel(const SkProgram P, const SkRaw R, uint32_t n_sketches,
             fstat = 0;
             const uint32_t* rec = tab + P.off_factor;
             uint4 hn = *reinterpret_cast<const uint4*>(rec);
-            for (uint32_t c = 0; c < n; c++) {
-                const uint32_t C = hn.x;
+            for (uint32_t c = 0; c < n;) {
+                const uint32_t C = hn.x & (kSkPairFlag - 1), two = hn.x & kSkPairFlag;
                 SmAddr dp = f + hn.y;
                 const double wk = ldp(w, hn.z);
                 const uint32_t* body = rec + 4;
                 rec = body + ((2 * C + C * (C + 1) / 2 + 3u) & ~3u);
-                hn = *reinterpret_cast<const uint4*>(rec);  // next column's header
+                hn = *reinterpret_cast<const uint4*>(rec);  // next record's header
                 const double d = lds(dp) + lam2;
                 if (fstat == 0 && !(d > 0.0 && d < INFINITY)) fstat = d != d ? 2 : 1;
                 const double inv = sk_rcp(d);
                 sts(dp, inv);
+                c += two ? 2 : 1;
+                if (two) {
+                    switch (C) {
+                        case 1: sk_column2<1>(body, f, w, wk, inv, lam2, fstat); break;
+                        case 2: sk_column2<2>(body, f, w, wk, inv, lam2, fstat); break;
+                        case 3: sk_column2<3>(body, f, w, wk, inv, lam2, fstat); break;
+                        case 4: sk_column2<4>(body, f, w, wk, inv, lam2, fstat); break;
+                        case 5: sk_column2<5>(body, f, w, wk, inv, lam2, fstat); break;
+                        case 6: sk_column2<6>(body, f, w, wk, inv, lam2, fstat); break;
+                        case 7: sk_column2<7>(body, f, w, wk, inv, lam2, fstat); break;
+                        default: sk_column2<8>(body, f, w, wk, inv, lam2, fstat); break;
+                    }
+                    continue;
+                }
                 switch (C) {
                     case 0: break;
                     case 1: sk_column<1>(body, f, w, wk, inv); break;
@@ -574,37 +714,7 @@ fk_batch_lm_sketch_kernel(const SkProgram P, const SkRaw R, uint32_t n_sketches,
                 }
             }
         }
-        {   // D L^T z = y in place in w; delta in variable order (qr.rs:354) into the trial point's slots
-            const uint32_t* rec = tab + P.off_back;
-            uint4 hn = *reinterpret_cast<const uint4*>(rec);
-            for (uint32_t c = 0; c < n; c++) {
-                const uint32_t C = hn.x;
-                const double inv = ldp(f, hn.y);
-                SmAddr zp = w + hn.z;
-                SmAddr xd = xsp + hn.w;
-                const uint32_t* body = rec + 4;
-                rec = body + ((2 * C + 3u) & ~3u);
-                hn = *reinterpret_cast<const uint4*>(rec);
-                double acc = lds(zp);
-                switch (C) {
-                    case 0: break;
-                    case 1: acc = sk_back_column<1>(body, f, w, acc); break;
-                    case 2: acc = sk_back_column<2>(body, f, w, acc); break;
-                    case 3: acc = sk_back_column<3>(body, f, w, acc); break;
-                    case 4: acc = sk_back_column<4>(body, f, w, acc); break;
-                    case 5: acc = sk_back_column<5>(body, f, w, acc); break;
-                    case 6: acc = sk_back_column<6>(body, f, w, acc); break;
-                    case 7: acc = sk_back_column<7>(body, f, w, acc); break;
-                    case 8: acc = sk_back_column<8>(body, f, w, acc); break;
-                    default:
-                        for (uint32_t a = C; a-- > 0;) acc = fma(-ldp(f, body[a]), ldp(w, body[C + a]), acc);
-                        break;
-                }
-                const double z = acc * inv;
-                sts(zp, z);
-                sts(xd, z);
-            }
-        }
+        sk_back_solve(tab + P.off_back, n, f, w, xsp);
         {   // lm.rs:139 (sum of squared steps, in variable order) and lm.rs:144-146 (trial point)
             dn = 0.0;
             uint32_t i = 0;
@@ -656,11 +766,12 @@ fk_batch_lm_sketch_kernel(const SkProgram P, const SkRaw R, uint32_t n_sketches,
 // CTA is TWO warps working on the SAME 32 sketches (thread l of both warps serves sketch l):
 //   * evaluation: the leader computes a row (loads, sqrt / divide / atan2) and leaves gradient and residual in a
 //     double-buffered staging area; the helper adds them into g and H while the leader is already on the next row;
-//   * factorisation: both warps read the pivot column into registers, each applies one half of the column's updates;
+//   * factorisation: both warps read the pivot column (or column pair) into registers, each applies its share of the
+//     updates;
 //   * back substitution and the LM bookkeeping stay with the leader (dependent chains), the helper clears g and H
 //     for the next evaluation meanwhile.
-// One CTA barrier per row and per column hands the data over.  Operations and their order per entry are those of the
-// solo kernel, so the results are bit-identical.
+// One CTA barrier per row and per factorisation step (one column or a column pair) hands the data over.  Operations and
+// their order per entry are those of the solo kernel, so the results are bit-identical.
 #ifndef FK_SK_LEADER_PCT
 #define FK_SK_LEADER_PCT 20  // (30: 71.7, 20: 72.7, 10: 72.5 M sketches/s on the 65,536-truss batch)
 #endif
@@ -832,6 +943,81 @@ __device__ __forceinline__ void sk_column_generic_half(const uint32_t* t, uint32
     }
 }
 
+// One part of a pair record's updates (columns k and k+1, see sk_column2).  Both warps read column k's entries and apply
+// its update to column k+1's pivot, entries and right-hand side entry, then take 1 / d(k+1); the remaining targets
+// ((a, b) with a >= b >= 1, then the w rows a >= 1) receive both updates and are split as sk_column_half splits a column's.
+// The step's barrier is part of the body: the helper reads column k+1's values and the pivot of column k during the step,
+// so HALF 0 (the leader), which also checks column k+1's pivot, stores them (and 1 / d of both pivots; dpk: column k's
+// diagonal) only after the barrier.  Only the back substitution reads them afterwards.
+template <int C, int HALF>
+__device__ __forceinline__ void sk_column2_half(const uint32_t* body, SmAddr f, SmAddr w, double wk, double inv, double lam2, int& fstat,
+                                                SmAddr dpk) {
+    constexpr int NP = C * (C + 1) / 2, NP1 = C * (C - 1) / 2, NT = NP1 + C - 1, H0 = sk_leader_share(NT);
+    constexpr int LO = HALF ? H0 : 0, HI = HALF ? NT : H0;
+    uint32_t t[(2 * C + NP + 3) / 4 * 4];
+    ld_words<2 * C + NP>(body, t);
+    double l[C], s[C], s1[C], wv[C], d[NP];
+    SmAddr wp[C];
+    SmAddr dp[NP];
+#pragma unroll
+    for (int a = 0; a < C; a++) l[a] = ldp(f, t[a]);
+#pragma unroll
+    for (int a = 0; a < C; a++) {
+        dp[sk_tri(a, 0)] = f + t[2 * C + sk_tri(a, 0)];
+        d[sk_tri(a, 0)] = lds(dp[sk_tri(a, 0)]);
+    }
+    wp[0] = w + t[C];
+    wv[0] = lds(wp[0]);
+#pragma unroll
+    for (int a = 1; a < C; a++)
+#pragma unroll
+        for (int b = 1; b <= a; b++)
+            if (sk_tri(a - 1, b - 1) >= LO && sk_tri(a - 1, b - 1) < HI) {
+                dp[sk_tri(a, b)] = f + t[2 * C + sk_tri(a, b)];
+                d[sk_tri(a, b)] = lds(dp[sk_tri(a, b)]);
+            }
+#pragma unroll
+    for (int a = 1; a < C; a++)
+        if (NP1 + a - 1 >= LO && NP1 + a - 1 < HI) {
+            wp[a] = w + t[C + a];
+            wv[a] = lds(wp[a]);
+        }
+#pragma unroll
+    for (int a = 0; a < C; a++) s[a] = -(l[a] * inv);
+#pragma unroll
+    for (int a = 0; a < C; a++) {
+        d[sk_tri(a, 0)] = fma(s[a], l[0], d[sk_tri(a, 0)]);
+#pragma unroll
+        for (int b = 1; b <= a; b++)
+            if (sk_tri(a - 1, b - 1) >= LO && sk_tri(a - 1, b - 1) < HI) d[sk_tri(a, b)] = fma(s[a], l[b], d[sk_tri(a, b)]);
+    }
+    wv[0] = fma(s[0], wk, wv[0]);
+#pragma unroll
+    for (int a = 1; a < C; a++)
+        if (NP1 + a - 1 >= LO && NP1 + a - 1 < HI) wv[a] = fma(s[a], wk, wv[a]);
+    const double d1 = d[0] + lam2;
+    if (HALF == 0 && fstat == 0 && !(d1 > 0.0 && d1 < INFINITY)) fstat = d1 != d1 ? 2 : 1;
+    const double inv1 = sk_rcp(d1);
+#pragma unroll
+    for (int a = 1; a < C; a++) s1[a] = -(d[sk_tri(a, 0)] * inv1);
+#pragma unroll
+    for (int a = 1; a < C; a++)
+#pragma unroll
+        for (int b = 1; b <= a; b++)
+            if (sk_tri(a - 1, b - 1) >= LO && sk_tri(a - 1, b - 1) < HI) sts(dp[sk_tri(a, b)], fma(s1[a], d[sk_tri(b, 0)], d[sk_tri(a, b)]));
+#pragma unroll
+    for (int a = 1; a < C; a++)
+        if (NP1 + a - 1 >= LO && NP1 + a - 1 < HI) sts(wp[a], fma(s1[a], wv[0], wv[a]));
+    __syncthreads();
+    if (HALF == 0) {
+        sts(dpk, inv);
+        sts(dp[0], inv1);
+        sts(wp[0], wv[0]);
+#pragma unroll
+        for (int a = 1; a < C; a++) sts(dp[sk_tri(a, 0)], d[sk_tri(a, 0)]);
+    }
+}
+
 template <int HALF>
 __device__ __forceinline__ void sk_column_dispatch_half(uint32_t C, const uint32_t* body, SmAddr f, SmAddr w, double wk, double inv) {
     switch (C) {
@@ -845,6 +1031,22 @@ __device__ __forceinline__ void sk_column_dispatch_half(uint32_t C, const uint32
         case 7: sk_column_half<7, HALF>(body, f, w, wk, inv); break;
         case 8: sk_column_half<8, HALF>(body, f, w, wk, inv); break;
         default: sk_column_generic_half(body, C, HALF, f, w, wk, inv); break;
+    }
+}
+
+// A pair record (1 <= C <= kSkPairMaxC); ends with the step's barrier.
+template <int HALF>
+__device__ __forceinline__ void sk_column2_dispatch_half(uint32_t C, const uint32_t* body, SmAddr f, SmAddr w, double wk, double inv,
+                                                         double lam2, int& fstat, SmAddr dpk) {
+    switch (C) {
+        case 1: sk_column2_half<1, HALF>(body, f, w, wk, inv, lam2, fstat, dpk); break;
+        case 2: sk_column2_half<2, HALF>(body, f, w, wk, inv, lam2, fstat, dpk); break;
+        case 3: sk_column2_half<3, HALF>(body, f, w, wk, inv, lam2, fstat, dpk); break;
+        case 4: sk_column2_half<4, HALF>(body, f, w, wk, inv, lam2, fstat, dpk); break;
+        case 5: sk_column2_half<5, HALF>(body, f, w, wk, inv, lam2, fstat, dpk); break;
+        case 6: sk_column2_half<6, HALF>(body, f, w, wk, inv, lam2, fstat, dpk); break;
+        case 7: sk_column2_half<7, HALF>(body, f, w, wk, inv, lam2, fstat, dpk); break;
+        default: sk_column2_half<8, HALF>(body, f, w, wk, inv, lam2, fstat, dpk); break;
     }
 }
 
@@ -921,16 +1123,23 @@ fk_batch_lm_sketch_pair_kernel(const SkProgram P, const SkRaw R, uint32_t n_sket
             const double lam2 = ldp(stage, 36u << 8);
             const uint32_t* frec = tab + P.off_factor;
             uint4 hn = *reinterpret_cast<const uint4*>(frec);
-            for (uint32_t col = 0; col < n; col++) {
-                const uint32_t C = hn.x;
+            int fstat_unused = 0;
+            for (uint32_t col = 0; col < n;) {
+                const uint32_t hx = hn.x, C = hx & (kSkPairFlag - 1);
                 const SmAddr dp = f + hn.y;
                 const double wk = ldp(w, hn.z);
                 const uint32_t* body = frec + 4;
                 frec = body + ((2 * C + C * (C + 1) / 2 + 3u) & ~3u);
                 hn = *reinterpret_cast<const uint4*>(frec);
-                const double inv = sk_rcp(lds(dp) + lam2);  // (the leader stores 1 / d one column later)
-                sk_column_dispatch_half<1>(C, body, f, w, wk, inv);
-                __syncthreads();
+                const double inv = sk_rcp(lds(dp) + lam2);  // (the leader stores 1 / d after the step's barrier)
+                if (hx & kSkPairFlag) {
+                    sk_column2_dispatch_half<1>(C, body, f, w, wk, inv, lam2, fstat_unused, dp);
+                    col += 2;
+                } else {
+                    sk_column_dispatch_half<1>(C, body, f, w, wk, inv);
+                    __syncthreads();
+                    col += 1;
+                }
             }
             __syncthreads();  // the leader is through with the back substitution
         }
@@ -1061,8 +1270,8 @@ fk_batch_lm_sketch_pair_kernel(const SkProgram P, const SkRaw R, uint32_t n_sket
             double inv_prev = 0.0;
             const uint32_t* rec = tab + P.off_factor;
             uint4 hn = *reinterpret_cast<const uint4*>(rec);
-            for (uint32_t col = 0; col < n; col++) {
-                const uint32_t C = hn.x;
+            for (uint32_t col = 0; col < n;) {
+                const uint32_t hx = hn.x, C = hx & (kSkPairFlag - 1);
                 SmAddr dp = f + hn.y;
                 const double wk = ldp(w, hn.z);
                 const uint32_t* body = rec + 4;
@@ -1072,44 +1281,21 @@ fk_batch_lm_sketch_pair_kernel(const SkProgram P, const SkRaw R, uint32_t n_sket
                 if (fstat == 0 && !(d > 0.0 && d < INFINITY)) fstat = d != d ? 2 : 1;
                 const double inv = sk_rcp(d);
                 if (dp_prev != kNone) sts(dp_prev, inv_prev);  // the helper read that pivot before the last barrier
-                sk_column_dispatch_half<0>(C, body, f, w, wk, inv);
-                dp_prev = dp;
-                inv_prev = inv;
-                __syncthreads();
+                if (hx & kSkPairFlag) {
+                    sk_column2_dispatch_half<0>(C, body, f, w, wk, inv, lam2, fstat, dp);  // stores 1 / d itself
+                    dp_prev = kNone;
+                    col += 2;
+                } else {
+                    sk_column_dispatch_half<0>(C, body, f, w, wk, inv);
+                    dp_prev = dp;
+                    inv_prev = inv;
+                    __syncthreads();
+                    col += 1;
+                }
             }
             if (dp_prev != kNone) sts(dp_prev, inv_prev);
         }
-        {
-            const uint32_t* rec = tab + P.off_back;
-            uint4 hn = *reinterpret_cast<const uint4*>(rec);
-            for (uint32_t col = 0; col < n; col++) {
-                const uint32_t C = hn.x;
-                const double inv = ldp(f, hn.y);
-                SmAddr zp = w + hn.z;
-                SmAddr xd = xsp + hn.w;
-                const uint32_t* body = rec + 4;
-                rec = body + ((2 * C + 3u) & ~3u);
-                hn = *reinterpret_cast<const uint4*>(rec);
-                double acc = lds(zp);
-                switch (C) {
-                    case 0: break;
-                    case 1: acc = sk_back_column<1>(body, f, w, acc); break;
-                    case 2: acc = sk_back_column<2>(body, f, w, acc); break;
-                    case 3: acc = sk_back_column<3>(body, f, w, acc); break;
-                    case 4: acc = sk_back_column<4>(body, f, w, acc); break;
-                    case 5: acc = sk_back_column<5>(body, f, w, acc); break;
-                    case 6: acc = sk_back_column<6>(body, f, w, acc); break;
-                    case 7: acc = sk_back_column<7>(body, f, w, acc); break;
-                    case 8: acc = sk_back_column<8>(body, f, w, acc); break;
-                    default:
-                        for (uint32_t a = C; a-- > 0;) acc = fma(-ldp(f, body[a]), ldp(w, body[C + a]), acc);
-                        break;
-                }
-                const double z = acc * inv;
-                sts(zp, z);
-                sts(xd, z);
-            }
-        }
+        sk_back_solve(tab + P.off_back, n, f, w, xsp);
         __syncthreads();  // H and g are consumed: the helper clears them for the trial evaluation
         {
             dn = 0.0;

@@ -631,10 +631,27 @@ void Topology::build_sketch_tables() {
         pad4();
     }
     T.insert(T.end(), 4, 0u);  // the kernel prefetches the header of the record after the last one
-    k.off_factor = (uint32_t)T.size();
-    for (uint32_t c = 0; c < n; c++) {
+    // Column pairs: column c pairs with c + 1 when L(:,c) = {c+1} u L(:,c+1) and C(c) <= kSkPairMaxC, taken greedily in
+    // column order (a wider supernode splits into consecutive pairs).  Then every target of column c+1 is a target of
+    // column c, and c+1's diagonal, entries and right-hand side entry are column c's targets (0, 0), (a >= 1, 0) and its
+    // first w row, so one kernel step eliminates both columns with one load and one store per target.
+    // FK_SK_COLPAIR=0 emits single-column records only (A/B knob; read here, when a topology's tables are built).
+    const char* env_pairs = std::getenv("FK_SK_COLPAIR");
+    const bool use_pairs = !(env_pairs && std::atoi(env_pairs) == 0);
+    std::vector<uint8_t> pair_first(n, 0);  // 1: column c is the first of a pair
+    for (uint32_t c = 0; use_pairs && c + 1 < n; c++) {
         const uint32_t b0 = l_colptr[c] + 1, e0 = l_colptr[c + 1], C = e0 - b0;
-        T.push_back(C); T.push_back(pos(l_colptr[c])); T.push_back(pos(c)); T.push_back(0);
+        const uint32_t b1 = l_colptr[c + 1] + 1, e1 = l_colptr[c + 2];
+        if (C < 1 || C > kSkPairMaxC || l_rowidx[b0] != c + 1 || e1 - b1 != C - 1) continue;
+        if (!std::equal(l_rowidx.begin() + b0 + 1, l_rowidx.begin() + e0, l_rowidx.begin() + b1)) continue;
+        pair_first[c] = 1;
+        c++;
+    }
+    k.off_factor = (uint32_t)T.size();
+    for (uint32_t c = 0; c < n; c += pair_first[c] ? 2 : 1) {
+        const uint32_t b0 = l_colptr[c] + 1, e0 = l_colptr[c + 1], C = e0 - b0;
+        if (C >= kSkPairFlag) return refuse("a column's count collides with the pair flag");  // (the kernel reads C as the bits below it)
+        T.push_back(C | (pair_first[c] ? kSkPairFlag : 0u)); T.push_back(pos(l_colptr[c])); T.push_back(pos(c)); T.push_back(0);
         for (uint32_t q = b0; q < e0; q++) T.push_back(pos(q));
         for (uint32_t q = b0; q < e0; q++) T.push_back(pos(l_rowidx[q]));
         for (uint32_t qa = b0; qa < e0; qa++)
@@ -648,10 +665,17 @@ void Topology::build_sketch_tables() {
     T.insert(T.end(), 4, 0u);
     k.off_back = (uint32_t)T.size();
     for (uint32_t cc = n; cc-- > 0;) {
-        const uint32_t b0 = l_colptr[cc] + 1, e0 = l_colptr[cc + 1];
-        T.push_back(e0 - b0); T.push_back(pos(l_colptr[cc])); T.push_back(pos(cc)); T.push_back(pos((uint32_t)perm[cc]));
+        const bool pair = cc > 0 && pair_first[cc - 1];
+        const uint32_t c = pair ? cc - 1 : cc;  // a pair record is column c's record plus what column c+1 needs
+        const uint32_t b0 = l_colptr[c] + 1, e0 = l_colptr[c + 1];
+        T.push_back((e0 - b0) | (pair ? kSkPairFlag : 0u)); T.push_back(pos(l_colptr[c])); T.push_back(pos(c)); T.push_back(pos((uint32_t)perm[c]));
         for (uint32_t q = b0; q < e0; q++) T.push_back(pos(q));
         for (uint32_t q = b0; q < e0; q++) T.push_back(pos(l_rowidx[q]));
+        if (pair) {
+            for (uint32_t q = l_colptr[cc] + 1; q < l_colptr[cc + 1]; q++) T.push_back(pos(q));
+            T.push_back(pos(l_colptr[cc])); T.push_back(pos((uint32_t)perm[cc]));
+            cc--;
+        }
         pad4();
     }
     T.insert(T.end(), 4, 0u);

@@ -28,6 +28,11 @@ inline int kind_arity(uint8_t kind) {
 // Expands the stored base indices into variable slots.  Returns arity or -1.
 int expand_slots(uint8_t kind, const uint32_t idx[4], uint32_t out[8]);
 
+// Sketch-kernel table records that eliminate two columns (Topology::SketchTables): the flag in the record's first word,
+// and the largest C (entries below column k's diagonal) such a record takes.
+constexpr uint32_t kSkPairFlag = 0x10000u;
+constexpr uint32_t kSkPairMaxC = 8;
+
 struct Topology {
     // ---- copy of the structural inputs -----------------------------------------------------
     uint32_t n_vars = 0, n_expr = 0, n_free = 0, n_rows = 0;
@@ -121,6 +126,11 @@ struct Topology {
         //          C positions in f, C positions in w (rows), C(C+1)/2 update targets in f ((a, b), b <= a)
         //   back   per column k descending: C, diagonal position, position of k in w, position of perm[k] in x,
         //          C positions in f, C positions in w (rows)
+        //   Column pairs (build_sketch_tables): when L(:,k) = {k+1} u L(:,k+1) and C <= kSkPairMaxC, ONE record
+        //   eliminates columns k and k+1 and carries kSkPairFlag in its first word.  The factor pair record is column
+        //   k's record: column k+1's diagonal, entries and w position are column k's target (0, 0), targets (a, 0) for
+        //   a >= 1 and first w row.  The back pair record (for k+1, then k) is column k's back record followed by the
+        //   C - 1 positions in f of column k+1's entries, column k+1's diagonal position and the position of perm[k+1].
         uint32_t off_free = 0, off_fix = 0, off_par = 0, off_eval = 0, off_factor = 0, off_back = 0;
         std::vector<uint32_t> tab;
     } sk;

@@ -93,6 +93,15 @@ int shard_over_devices(int n_gpus, uint32_t n, const Fn& fn) {
     return FK_OK;
 }
 
+// The per-device state in `slots` for `device`, created empty on first use, under `mu`.
+template <class T>
+T* device_slot(std::mutex& mu, std::map<int, std::unique_ptr<T>>& slots, int device) {
+    std::lock_guard<std::mutex> lock(mu);
+    std::unique_ptr<T>& p = slots[device];
+    if (!p) p.reset(new T());
+    return p.get();
+}
+
 // Packs the topology tables into one device allocation and fills the DevProgram view.
 struct DeviceProgram {
     int device = -1;
@@ -110,57 +119,64 @@ struct DeviceProgram {
     }
 };
 
-template <class T>
-size_t reserve(size_t& off, size_t count) {
-    off = (off + 15) & ~size_t(15);
-    size_t at = off;
-    off += std::max<size_t>(count, 1) * sizeof(T);
-    return at;
-}
+// Host tables packed into one device allocation: add() copies a vector in at the next 16-byte boundary (room for at least one
+// element) and returns its offset, upload() makes the allocation, at() points into it.
+struct TablePack {
+    std::vector<unsigned char> host;
+    const unsigned char* base = nullptr;
+    template <class V>
+    size_t add(const V& vec) {
+        using T = typename V::value_type;
+        const size_t at = (host.size() + 15) & ~size_t(15);
+        host.resize(at + std::max<size_t>(vec.size(), 1) * sizeof(T), 0);
+        if (!vec.empty()) std::memcpy(host.data() + at, vec.data(), vec.size() * sizeof(T));
+        return at;
+    }
+    // One cudaMalloc (16 zero bytes behind the last table) into *buf, which the caller frees also after an error, and one copy on
+    // `stream` (0: the legacy default stream), complete on return.  The caller has selected the device.
+    int upload(cudaStream_t stream, void** buf) {
+        host.resize(host.size() + 16, 0);
+        CU(cudaMalloc(buf, host.size()));
+        base = (const unsigned char*)*buf;
+        CU(cudaMemcpyAsync(*buf, host.data(), host.size(), cudaMemcpyHostToDevice, stream));
+        CU(cudaStreamSynchronize(stream));
+        return FK_OK;
+    }
+    template <class T>
+    const T* at(size_t off) const { return (const T*)(base + off); }
+};
 
 int upload_program(const fk::Topology& t, int device, DeviceProgram& out) {
     CU(cudaSetDevice(device));
-    struct Item { const void* src; size_t bytes; size_t at; };
-    std::vector<Item> items;
-    size_t off = 0;
-    auto add = [&](const auto& vec) {
-        using T = typename std::decay<decltype(vec)>::type::value_type;
-        size_t at = reserve<T>(off, vec.size());
-        items.push_back({vec.data(), vec.size() * sizeof(T), at});
-        return at;
-    };
+    TablePack pk;
     const fk::Topology::Tables& tb = t.tab;
     std::vector<uint32_t> jcolptr(t.n_free + 1), jrow(t.jac_nnz);  // CSC of the Jacobian without damping rows (L-BFGS gradient)
     for (uint32_t c = 0; c <= t.n_free; c++) jcolptr[c] = t.aug_colptr[c] - c;
     for (uint32_t c = 0; c < t.n_free; c++)
         for (uint32_t q = t.aug_colptr[c]; q + 1 < t.aug_colptr[c + 1]; q++) jrow[q - c] = t.aug_rowidx[q];
-    const size_t o_jcp = add(jcolptr), o_jrow = add(jrow);
-    size_t o_free = add(t.free_vars), o_rh = add(tb.row_hdr), o_rs = add(tb.row_slots),
-           o_af = add(tb.a_flags), o_ao = add(tb.a_ops), o_ad = add(tb.a_dst),
-           o_gf = add(tb.g_flags), o_go = add(tb.g_ops), o_gd = add(tb.g_dst),
-           o_fs = add(tb.f_steps), o_fo = add(tb.f_ops), o_ss = add(tb.s_steps), o_so = add(tb.s_ops),
-           o_bs = add(tb.b_steps), o_bo = add(tb.b_ops);
-    const size_t o_sk = (t.sk.ok && fk::sk_fits(t.sk.entries, t.sk.tab.size())) ? add(t.sk.tab) : SIZE_MAX;
-    std::vector<unsigned char> host(off + 16, 0);
-    for (const Item& it : items)
-        if (it.bytes) std::memcpy(host.data() + it.at, it.src, it.bytes);
-    CU(cudaMalloc(&out.buf, host.size()));
+    const size_t o_jcp = pk.add(jcolptr), o_jrow = pk.add(jrow);
+    size_t o_free = pk.add(t.free_vars), o_rh = pk.add(tb.row_hdr), o_rs = pk.add(tb.row_slots),
+           o_af = pk.add(tb.a_flags), o_ao = pk.add(tb.a_ops), o_ad = pk.add(tb.a_dst),
+           o_gf = pk.add(tb.g_flags), o_go = pk.add(tb.g_ops), o_gd = pk.add(tb.g_dst),
+           o_fs = pk.add(tb.f_steps), o_fo = pk.add(tb.f_ops), o_ss = pk.add(tb.s_steps), o_so = pk.add(tb.s_ops),
+           o_bs = pk.add(tb.b_steps), o_bo = pk.add(tb.b_ops);
+    const size_t o_sk = (t.sk.ok && fk::sk_fits(t.sk.entries, t.sk.tab.size())) ? pk.add(t.sk.tab) : SIZE_MAX;
     out.device = device;
-    CU(cudaMemcpy(out.buf, host.data(), host.size(), cudaMemcpyHostToDevice));
-    unsigned char* b = (unsigned char*)out.buf;
+    const int rc = pk.upload(0, &out.buf);
+    if (rc != FK_OK) return rc;
     fk::DevProgram& v = out.view;
     v.n_vars = t.n_vars; v.n_expr = t.n_expr; v.n = t.n_free; v.m = t.n_rows;
     v.jnnz = t.jac_nnz; v.lnnz = (uint32_t)t.l_rowidx.size(); v.tile = t.tile; v.uniform_kind = tb.uniform_kind;
     v.eval_rounds = tb.eval_rounds; v.a_nsteps = tb.a_nsteps; v.g_nsteps = tb.g_nsteps;
     v.f_nsteps = tb.f_nsteps; v.s_nsteps = tb.s_nsteps; v.b_nsteps = tb.b_nsteps;
-    v.free_vars = (const uint32_t*)(b + o_free);
-    v.row_hdr = (const uint32_t*)(b + o_rh); v.row_slots = (const uint2*)(b + o_rs);
-    v.a_flags = (const uint32_t*)(b + o_af); v.a_ops = (const uint32_t*)(b + o_ao); v.a_dst = (const uint32_t*)(b + o_ad);
-    v.g_flags = (const uint32_t*)(b + o_gf); v.g_ops = (const uint32_t*)(b + o_go); v.g_dst = (const uint32_t*)(b + o_gd);
-    v.f_steps = (const uint32_t*)(b + o_fs); v.f_ops = (const uint2*)(b + o_fo);
-    v.s_steps = (const uint2*)(b + o_ss); v.s_ops = (const uint32_t*)(b + o_so);
-    v.b_steps = (const uint2*)(b + o_bs); v.b_ops = (const uint32_t*)(b + o_bo);
-    out.jcolptr = (const uint32_t*)(b + o_jcp); out.jrow = (const uint32_t*)(b + o_jrow);
+    v.free_vars = pk.at<uint32_t>(o_free);
+    v.row_hdr = pk.at<uint32_t>(o_rh); v.row_slots = pk.at<uint2>(o_rs);
+    v.a_flags = pk.at<uint32_t>(o_af); v.a_ops = pk.at<uint32_t>(o_ao); v.a_dst = pk.at<uint32_t>(o_ad);
+    v.g_flags = pk.at<uint32_t>(o_gf); v.g_ops = pk.at<uint32_t>(o_go); v.g_dst = pk.at<uint32_t>(o_gd);
+    v.f_steps = pk.at<uint32_t>(o_fs); v.f_ops = pk.at<uint2>(o_fo);
+    v.s_steps = pk.at<uint2>(o_ss); v.s_ops = pk.at<uint32_t>(o_so);
+    v.b_steps = pk.at<uint2>(o_bs); v.b_ops = pk.at<uint32_t>(o_bo);
+    out.jcolptr = pk.at<uint32_t>(o_jcp); out.jrow = pk.at<uint32_t>(o_jrow);
     v.sketch_prog = nullptr;
     if (o_sk != SIZE_MAX) {
         const fk::Topology::SketchTables& k = t.sk;
@@ -172,7 +188,7 @@ int upload_program(const fk::Topology& t, int device, DeviceProgram& out) {
         p.off_free = k.off_free; p.off_fix = k.off_fix; p.off_par = k.off_par;
         p.off_eval = k.off_eval; p.off_factor = k.off_factor; p.off_back = k.off_back;
         p.tab_words = (uint32_t)k.tab.size();
-        p.tab = (const uint32_t*)(b + o_sk);
+        p.tab = pk.at<uint32_t>(o_sk);
         v.sketch_prog = out.sketch.get();
     }
     return FK_OK;
@@ -241,8 +257,9 @@ struct DevicePipeline {
 struct AnalyzePool {
     int device = -1;
     std::mutex mu;
-    uint8_t* d_kind = nullptr;
-    uint32_t* d_slot = nullptr;
+    void* d_tables = nullptr;
+    const uint8_t* d_kind = nullptr;
+    const uint32_t* d_slot = nullptr;
     double *d_vars = nullptr, *d_param = nullptr;
     uint8_t* d_out = nullptr;
     uint32_t capacity = 0;
@@ -251,7 +268,7 @@ struct AnalyzePool {
     cudaStream_t stream = nullptr;
     ~AnalyzePool() {
         if (device >= 0) cudaSetDevice(device);
-        cudaFree(d_kind); cudaFree(d_slot); cudaFree(d_vars); cudaFree(d_param); cudaFree(d_out); cudaFree(d_ws);
+        cudaFree(d_tables); cudaFree(d_vars); cudaFree(d_param); cudaFree(d_out); cudaFree(d_ws);
         if (stream) cudaStreamDestroy(stream);
     }
 };
@@ -262,14 +279,15 @@ struct PrepareTables {
     int device = -1;
     std::vector<uint32_t> perturb_vars;
     uint32_t seed = 0;
-    uint8_t* d_kind = nullptr;
-    uint32_t* d_perturb = nullptr;
-    double* d_draws = nullptr;
-    uint32_t* d_free_draw = nullptr;  // sketch kernel's raw mode: draw index per free column / per fixed variable the rows read
-    uint32_t* d_fix_draw = nullptr;
+    void* d_tables = nullptr;
+    const uint8_t* d_kind = nullptr;
+    const uint32_t* d_perturb = nullptr;
+    const double* d_draws = nullptr;
+    const uint32_t* d_free_draw = nullptr;  // sketch kernel's raw mode: draw index per free column / per fixed variable the rows read
+    const uint32_t* d_fix_draw = nullptr;
     ~PrepareTables() {
         if (device >= 0) cudaSetDevice(device);
-        cudaFree(d_kind); cudaFree(d_perturb); cudaFree(d_draws); cudaFree(d_free_draw); cudaFree(d_fix_draw);
+        cudaFree(d_tables);
     }
 };
 
@@ -664,13 +682,7 @@ int fk_batch_analyze(const fk_topology* topo_c, int device, uint32_t n, const do
     std::string err;
     const int prc = fk::choose_analyze(t.n_vars, t.n_expr, n, device, &plan, &err);  // the limit rule, before any allocation
     if (prc != FK_OK) return fail(prc, err);
-    AnalyzePool* pool;
-    {
-        std::lock_guard<std::mutex> lock(topo->mu);
-        auto& p = topo->analyze_pools[device];
-        if (!p) p.reset(new AnalyzePool());
-        pool = p.get();
-    }
+    AnalyzePool* pool = device_slot(topo->mu, topo->analyze_pools, device);
     std::lock_guard<std::mutex> lock(pool->mu);
     if (pool->device < 0) {  // tables: once per (topology, device)
         std::vector<uint32_t> slot_var((size_t)t.n_expr * 8, 0);
@@ -680,12 +692,13 @@ int fk_batch_analyze(const fk_topology* topo_c, int device, uint32_t n, const do
             for (int k = 0; k < a; k++) slot_var[(size_t)e * 8 + k] = sv[k];
         }
         pool->device = device;
-        CU(cudaMalloc(&pool->d_kind, t.n_expr));
-        CU(cudaMalloc(&pool->d_slot, slot_var.size() * sizeof(uint32_t)));
         CU(cudaStreamCreateWithFlags(&pool->stream, cudaStreamNonBlocking));
-        CU(cudaMemcpyAsync(pool->d_kind, t.kind.data(), t.n_expr, cudaMemcpyHostToDevice, pool->stream));
-        CU(cudaMemcpyAsync(pool->d_slot, slot_var.data(), slot_var.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, pool->stream));
-        CU(cudaStreamSynchronize(pool->stream));  // slot_var leaves scope
+        TablePack pk;
+        const size_t o_kind = pk.add(t.kind), o_slot = pk.add(slot_var);
+        const int rc = pk.upload(pool->stream, &pool->d_tables);
+        if (rc != FK_OK) return rc;
+        pool->d_kind = pk.at<uint8_t>(o_kind);
+        pool->d_slot = pk.at<uint32_t>(o_slot);
     }
     if (pool->capacity < n) {  // grow-only
         cudaFree(pool->d_vars); cudaFree(pool->d_param); cudaFree(pool->d_out);
@@ -1181,23 +1194,17 @@ static int prepare_tables_for(fk_topology* topo, int device, const fk_prepare_op
         st = st * 1664525u + 1013904223u;
         draws[k] = (1.0 / 4294967295.0) * (double)st;
     }
-    CU(cudaMalloc(&q->d_kind, std::max<uint32_t>(t.n_expr, 1)));
-    CU(cudaMalloc(&q->d_perturb, sizeof(uint32_t) * std::max<size_t>(list.size(), 1)));
-    CU(cudaMalloc(&q->d_draws, sizeof(double) * draws.size()));
-    if (t.n_expr) CU(cudaMemcpy(q->d_kind, t.kind.data(), t.n_expr, cudaMemcpyHostToDevice));
-    if (!list.empty()) CU(cudaMemcpy(q->d_perturb, list.data(), sizeof(uint32_t) * list.size(), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(q->d_draws, draws.data(), sizeof(double) * draws.size(), cudaMemcpyHostToDevice));
-    {
-        std::vector<uint32_t> where(t.n_vars, 0xFFFFFFFFu), free_draw(std::max<uint32_t>(t.n_free, 1), 0xFFFFFFFFu), fix_draw(std::max<uint32_t>(t.sk.nfix, 1), 0xFFFFFFFFu);
-        for (size_t j = 0; j < list.size(); j++) where[list[j]] = (uint32_t)j;
-        for (uint32_t c = 0; c < t.n_free; c++) free_draw[c] = where[t.free_vars[c]];
-        if (t.sk.ok)
-            for (uint32_t i = 0; i < t.sk.nfix; i++) fix_draw[i] = where[t.sk.tab[t.sk.off_fix + i]];
-        CU(cudaMalloc(&q->d_free_draw, sizeof(uint32_t) * free_draw.size()));
-        CU(cudaMalloc(&q->d_fix_draw, sizeof(uint32_t) * fix_draw.size()));
-        CU(cudaMemcpy(q->d_free_draw, free_draw.data(), sizeof(uint32_t) * free_draw.size(), cudaMemcpyHostToDevice));
-        CU(cudaMemcpy(q->d_fix_draw, fix_draw.data(), sizeof(uint32_t) * fix_draw.size(), cudaMemcpyHostToDevice));
-    }
+    std::vector<uint32_t> where(t.n_vars, 0xFFFFFFFFu), free_draw(std::max<uint32_t>(t.n_free, 1), 0xFFFFFFFFu), fix_draw(std::max<uint32_t>(t.sk.nfix, 1), 0xFFFFFFFFu);
+    for (size_t j = 0; j < list.size(); j++) where[list[j]] = (uint32_t)j;
+    for (uint32_t c = 0; c < t.n_free; c++) free_draw[c] = where[t.free_vars[c]];
+    if (t.sk.ok)
+        for (uint32_t i = 0; i < t.sk.nfix; i++) fix_draw[i] = where[t.sk.tab[t.sk.off_fix + i]];
+    TablePack pk;
+    const size_t o_kind = pk.add(t.kind), o_perturb = pk.add(list), o_draws = pk.add(draws), o_free = pk.add(free_draw), o_fix = pk.add(fix_draw);
+    const int rc = pk.upload(0, &q->d_tables);
+    if (rc != FK_OK) return rc;
+    q->d_kind = pk.at<uint8_t>(o_kind); q->d_perturb = pk.at<uint32_t>(o_perturb); q->d_draws = pk.at<double>(o_draws);
+    q->d_free_draw = pk.at<uint32_t>(o_free); q->d_fix_draw = pk.at<uint32_t>(o_fix);
     p = std::move(q);
     *out = p.get();
     return FK_OK;
@@ -1841,46 +1848,209 @@ namespace fk {
 
 int system_batch_fail(int code, const std::string& msg) { return fail(code, msg); }
 
-// The buffers of one device: the structures' batch plans (capacity chunk * multiplicity), the chunk's raw input and output
-// rows, and the index tables of the two kernels, all on one stream.
-struct SystemBatchDevice {
+// The problems grouped by structure, one topology per group (group_by_topology without free values).
+static int group_by_structure(const std::vector<const fk_problem*>& problems, std::vector<BatchGroup>& groups) {
+    if (problems.empty()) return FK_OK;
+    static double dummy = 0.0;  // (group_by_topology checks the free-value pointers; nothing is written through them)
+    std::vector<double*> fv(problems.size(), &dummy);
+    return group_by_topology((uint32_t)problems.size(), problems.data(), fv.data(), groups);
+}
+
+// Variants per chunk of n: FK_SYSTEM_BATCH_CHUNK=n (test knob), else the chunk's buffers (`bytes` per variant) within about 1 GiB
+// of device memory, at least one; then at most INT32_MAX sketches per launch (`sketches` per variant) and rows of `row` values
+// per variant within 32-bit offsets.
+static uint32_t system_batch_chunk(uint32_t n, uint64_t bytes, uint64_t sketches, uint64_t row) {
+    static const uint32_t env = [] {
+        const char* e = std::getenv("FK_SYSTEM_BATCH_CHUNK");
+        const long v = e ? std::atol(e) : 0;
+        return (uint32_t)(v >= 1 && v <= (long)UINT32_MAX ? v : 0);
+    }();
+    uint64_t chunk = env ? env : std::max<uint64_t>(1, (1ull << 30) / bytes);
+    chunk = std::min<uint64_t>(chunk, std::max<uint64_t>(1, (uint64_t)INT32_MAX / std::max<uint64_t>(1, sketches)));
+    chunk = std::min<uint64_t>(chunk, std::max<uint64_t>(1, (uint64_t)UINT32_MAX / std::max<uint64_t>(1, row)));
+    return (uint32_t)std::min<uint64_t>(chunk, n);
+}
+
+// The state of a system batch call on one device, all on one stream: the layout's tables, the template rows and the chunk buffers
+// (grow / release_buffers).  d_vt / d_pt: the variants' scaled variables and parameters where the call keeps them resident (not
+// fk_system_batch_solve).  The caller holds mu.
+struct SystemDevice {
     std::mutex mu;
     int device = -1;
-    bool ready = false;          // tables uploaded
     cudaStream_t stream = nullptr;
-    uint32_t chunk = 0;          // variants the buffers hold
-    bool lm = false;             // the plans were made for LM (which on the global sparse path needs the sparse batch tables)
-    std::vector<fk_batch_plan*> plans;
-    void* d_tables = nullptr;    // kinds, expression -> constraint, draws, slot / expression tables, scatter tables, descriptors
-    const uint8_t* d_kind = nullptr;
-    const uint32_t *d_expr_con = nullptr, *d_var_struct = nullptr, *d_var_off = nullptr, *d_comp_struct = nullptr, *d_comp_member = nullptr;
-    const double* d_draws = nullptr;
-    SbStructure* d_desc = nullptr;
-    std::vector<SbStructure> desc;  // (host copy; the buffer pointers change with the plans)
-    double *d_raw_vars = nullptr, *d_raw_param = nullptr, *d_tmpl_vars = nullptr, *d_tmpl_param = nullptr, *d_scales = nullptr, *d_vars_out = nullptr;
-    fk_report* d_rep_out = nullptr;
+    bool ready = false;  // tables uploaded
+    uint32_t chunk = 0;  // variants the chunk buffers hold
+    void* d_tables = nullptr;
+    double *d_tmpl_vars = nullptr, *d_tmpl_param = nullptr;
+    double *d_raw_param = nullptr, *d_vt = nullptr, *d_pt = nullptr;
+    // What grow has allocated: the member it set and the buffer (the destructor frees the buffers of members that derived
+    // classes own after those members are gone).
+    struct Grown { void** member; void* buf; };
+    std::vector<Grown> grown;
+
+    // *ptr = a new buffer of `count` elements (at least one), freed by release_buffers; frees the one grow put there before.
+    template <class T>
+    int grow(T** ptr, size_t count) {
+        void** member = (void**)ptr;
+        auto it = std::find_if(grown.begin(), grown.end(), [&](const Grown& g) { return g.member == member; });
+        if (it != grown.end()) {
+            cudaFree(it->buf);
+            grown.erase(it);
+        }
+        *member = nullptr;
+        void* buf = nullptr;
+        CU(cudaMalloc(&buf, sizeof(T) * std::max<size_t>(count, 1)));
+        grown.push_back({member, buf});
+        *member = buf;
+        return FK_OK;
+    }
     void release_buffers() {
-        for (fk_batch_plan* p : plans) delete p;
-        plans.clear();
-        cudaFree(d_raw_vars); cudaFree(d_raw_param); cudaFree(d_scales); cudaFree(d_vars_out); cudaFree(d_rep_out);
-        d_raw_vars = d_raw_param = d_scales = d_vars_out = nullptr;
-        d_rep_out = nullptr;
+        for (const Grown& g : grown) {
+            cudaFree(g.buf);
+            *g.member = nullptr;
+        }
+        grown.clear();
         chunk = 0;
     }
-    ~SystemBatchDevice() {
+    // Once per device: the stream, the tables of `pk` and the template rows (an earlier failed attempt's are freed first).
+    int upload_tables(int dev, TablePack& pk, uint32_t n_vars, uint32_t n_expr) {
+        device = dev;
+        if (!stream) CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+        cudaFree(d_tables); cudaFree(d_tmpl_vars); cudaFree(d_tmpl_param);
+        d_tables = nullptr;
+        d_tmpl_vars = d_tmpl_param = nullptr;
+        const int rc = pk.upload(stream, &d_tables);
+        if (rc != FK_OK) return rc;
+        CU(cudaMalloc(&d_tmpl_vars, sizeof(double) * std::max<uint32_t>(n_vars, 1)));
+        CU(cudaMalloc(&d_tmpl_param, sizeof(double) * std::max<uint32_t>(n_expr, 1)));
+        return FK_OK;
+    }
+    ~SystemDevice() {
         if (device < 0) return;
         cudaSetDevice(device);
-        release_buffers();
-        cudaFree(d_tables); cudaFree(d_desc); cudaFree(d_tmpl_vars); cudaFree(d_tmpl_param);
+        for (const Grown& g : grown) cudaFree(g.buf);
+        cudaFree(d_tables); cudaFree(d_tmpl_vars); cudaFree(d_tmpl_param);
         if (stream) cudaStreamDestroy(stream);
     }
 };
+
+// The template rows up, then body(at, cnt) for the chunks [at, at + cnt) of variants [lo, hi) on d's stream, then a synchronise
+// whether or not one failed: no copy into the caller's buffers may still be running when the call returns.  `what` names a
+// failure the synchronise reports.
+template <class Chunk>
+static int run_chunks(SystemDevice* d, uint32_t n_vars, uint32_t n_expr, const double* tmpl_vars, const double* tmpl_param, uint32_t lo,
+                      uint32_t hi, uint32_t chunk, const char* what, const Chunk& body) {
+    auto run = [&]() -> int {
+        if (n_vars) CU(cudaMemcpyAsync(d->d_tmpl_vars, tmpl_vars, sizeof(double) * n_vars, cudaMemcpyHostToDevice, d->stream));
+        if (n_expr) CU(cudaMemcpyAsync(d->d_tmpl_param, tmpl_param, sizeof(double) * n_expr, cudaMemcpyHostToDevice, d->stream));
+        for (uint32_t at = lo; at < hi; at += chunk) {
+            const int rc = body(at, std::min(chunk, hi - at));
+            if (rc != FK_OK) return rc;
+        }
+        return FK_OK;
+    };
+    int rc = run();
+    const cudaError_t e = cudaStreamSynchronize(d->stream);
+    if (rc == FK_OK && e != cudaSuccess) rc = cuda_fail(e, what);
+    return rc;
+}
+
+// The solve batches' device state: the prepare kernel's tables and descriptors (d_desc), the structures' batch plans, and the
+// chunk's raw, scale and output rows.  Plus, for fk_system_batch_solve, the scatter kernel's tables.
+struct SystemBatchDevice : SystemDevice {
+    bool lm = false;  // the plans were made for LM (which on the global sparse path needs the sparse batch tables)
+    std::vector<std::unique_ptr<fk_batch_plan>> plans;
+    const uint8_t* d_kind = nullptr;
+    const uint32_t *d_expr_con = nullptr, *d_var_struct = nullptr, *d_var_off = nullptr, *d_comp_struct = nullptr, *d_comp_member = nullptr;
+    const double* d_draws = nullptr;
+    std::vector<SbStructure> desc;  // (host copy; the buffer pointers change with the plans)
+    SbStructure* d_desc = nullptr;
+    double *d_raw_vars = nullptr, *d_scales = nullptr, *d_vars_out = nullptr;
+    fk_report* d_rep_out = nullptr;
+
+    // The chunk buffers of `cap` variants, everything released first and again after a failure: per structure s a plan of
+    // cap * st[s].mult sketches, the raw, scale and output rows with n_rep reports per variant, and with `resident` vt and pt.
+    template <class Structure>
+    int grow_chunk(const SystemBatchLayout& L, const std::vector<Structure>& st, uint32_t cap, bool lm_plans, uint32_t n_rep, bool resident) {
+        plans.clear();
+        release_buffers();
+        int rc = FK_OK;
+        for (size_t s = 0; s < st.size() && rc == FK_OK; s++) {
+            fk_batch_plan* p = nullptr;
+            if ((rc = plan_create(st[s].topo.get(), cap * st[s].mult, device, lm_plans, &p)) == FK_OK) plans.emplace_back(p);
+        }
+        if (rc == FK_OK) rc = grow(&d_raw_vars, (size_t)cap * L.n_vars);
+        if (rc == FK_OK) rc = grow(&d_raw_param, (size_t)cap * L.n_constraints);
+        if (rc == FK_OK) rc = grow(&d_scales, cap);
+        if (rc == FK_OK) rc = grow(&d_vars_out, (size_t)cap * L.n_vars);
+        if (rc == FK_OK) rc = grow(&d_rep_out, (size_t)cap * n_rep);
+        if (rc == FK_OK && resident) rc = grow(&d_vt, (size_t)cap * L.n_vars);
+        if (rc == FK_OK && resident) rc = grow(&d_pt, (size_t)cap * L.kind.size());
+        if (rc == FK_OK) rc = grow(&d_desc, desc.size());
+        if (rc != FK_OK) {
+            plans.clear();
+            release_buffers();
+            return rc;
+        }
+        chunk = cap;
+        lm = lm_plans;
+        return FK_OK;
+    }
+};
+
+// Bytes per variant of the structures' plan rows (st[s].mult sketches each); *max_mult: the most sketches per variant of one plan.
+template <class Structure>
+static uint64_t plan_bytes(const std::vector<Structure>& st, uint64_t* max_mult) {
+    uint64_t bytes = 0;
+    *max_mult = 1;
+    for (const Structure& S : st) {
+        const fk::Topology& t = S.topo->t;
+        bytes += S.mult * (sizeof(double) * ((uint64_t)t.n_vars + t.n_expr + t.n_free) + sizeof(fk_report));
+        *max_mult = std::max<uint64_t>(*max_mult, S.mult);
+    }
+    return bytes;
+}
+
+// Variants [lo, hi) of a solve batch on one device, chunk after chunk on its stream: the raw rows up, the prepare kernel over the
+// n_desc descriptors of d_desc, step(cnt, raw, raw_stride) (the solves and the write-back into d_vars_out / d_rep_out), then
+// vars_out and n_rep reports per variant down.
+template <class Step>
+static int solve_chunks(SystemBatchDevice* d, const SystemBatchLayout& L, const SystemBatchCall& c, uint32_t lo, uint32_t hi, uint32_t chunk,
+                        uint32_t n_rep, uint32_t n_desc, const char* what, const Step& step) {
+    const uint32_t n_expr = (uint32_t)L.kind.size();
+    const cudaStream_t st = d->stream;
+    return run_chunks(d, L.n_vars, n_expr, c.tmpl_vars, c.tmpl_param, lo, hi, chunk, what, [&](uint32_t at, uint32_t cnt) -> int {
+        const double* raw = d->d_tmpl_vars;
+        uint32_t raw_stride = 0;
+        if (c.vars) {
+            if (L.n_vars)
+                CU(cudaMemcpyAsync(d->d_raw_vars, c.vars + (size_t)at * L.n_vars, sizeof(double) * (size_t)cnt * L.n_vars, cudaMemcpyHostToDevice, st));
+            raw = d->d_raw_vars;
+            raw_stride = L.n_vars;
+        }
+        if (c.params && L.n_constraints)
+            CU(cudaMemcpyAsync(d->d_raw_param, c.params + (size_t)at * L.n_constraints, sizeof(double) * (size_t)cnt * L.n_constraints,
+                               cudaMemcpyHostToDevice, st));
+        const int e = launch_system_batch_prepare(cnt, L.n_vars, n_expr, L.n_constraints, d->d_kind, d->d_expr_con, d->d_draws, c.perturb, raw,
+                                                  raw_stride, c.params ? d->d_raw_param : nullptr, d->d_tmpl_param, n_desc, d->d_desc, d->d_scales, st);
+        if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_batch_prepare_kernel");
+        const int rc = step(cnt, raw, raw_stride);
+        if (rc != FK_OK) return rc;
+        if (L.n_vars)
+            CU(cudaMemcpyAsync(c.vars_out + (size_t)at * L.n_vars, d->d_vars_out, sizeof(double) * (size_t)cnt * L.n_vars, cudaMemcpyDeviceToHost, st));
+        if (n_rep)
+            CU(cudaMemcpy2DAsync(c.reports + (size_t)at * c.reports_per_variant, sizeof(fk_report) * c.reports_per_variant, d->d_rep_out,
+                                 sizeof(fk_report) * n_rep, sizeof(fk_report) * n_rep, cnt, cudaMemcpyDeviceToHost, st));
+        return FK_OK;
+    });
+}
 
 struct SystemBatch {
     SystemBatchLayout L;
     struct Structure {
         std::shared_ptr<fk_topology> topo;
-        std::vector<uint32_t> members;                 // component indices
+        std::vector<uint32_t> members;                    // component indices
+        uint32_t mult = 0;                                // members.size(): the plan's sketches per variant
         std::vector<uint32_t> slot_var, slot_draw, expr;  // [mult][nv], [mult][nv], [mult][ne]
     };
     std::vector<Structure> st;
@@ -1896,12 +2066,8 @@ int system_batch_create(SystemBatchLayout&& layout, const std::vector<const fk_p
     const SystemBatchLayout& L = b->L;
     const uint32_t nc = (uint32_t)problems.size();
     std::vector<BatchGroup> groups;
-    if (nc) {
-        static double dummy = 0.0;  // (group_by_topology checks the free-value pointers; nothing is written through them)
-        std::vector<double*> fv(nc, &dummy);
-        const int rc = group_by_topology(nc, problems.data(), fv.data(), groups);
-        if (rc != FK_OK) return rc;
-    }
+    const int rc = group_by_structure(problems, groups);
+    if (rc != FK_OK) return rc;
     b->comp_struct.assign(nc, kSbNone);
     b->comp_member.assign(nc, 0);
     b->var_struct.assign(L.n_vars, kSbNone);
@@ -1910,6 +2076,7 @@ int system_batch_create(SystemBatchLayout&& layout, const std::vector<const fk_p
         SystemBatch::Structure S;
         S.topo = g.topo;
         S.members = g.members;
+        S.mult = (uint32_t)g.members.size();
         const uint32_t si = (uint32_t)b->st.size(), nf = g.topo->t.n_free;
         for (uint32_t m = 0; m < S.members.size(); m++) {
             const SystemBatchLayout::Component& c = L.comps[S.members[m]];
@@ -1934,181 +2101,84 @@ void system_batch_layout(const SystemBatch& b, uint32_t* n_components, uint32_t*
     if (n_structures) *n_structures = (uint32_t)b.st.size();
     if (multiplicity) {
         multiplicity->clear();
-        for (const SystemBatch::Structure& S : b.st) multiplicity->push_back((uint32_t)S.members.size());
+        for (const SystemBatch::Structure& S : b.st) multiplicity->push_back(S.mult);
     }
 }
 
-// FK_SYSTEM_BATCH_CHUNK=n: variants per chunk of both system batch calls (test knob), 0 when unset.
-static uint32_t system_batch_chunk_env() {
-    static const uint32_t env = [] {
-        const char* e = std::getenv("FK_SYSTEM_BATCH_CHUNK");
-        const long v = e ? std::atol(e) : 0;
-        return (uint32_t)(v >= 1 && v <= (long)UINT32_MAX ? v : 0);
-    }();
-    return env;
-}
-
-// Variants per chunk: the chunk's buffers within about 1 GiB of device memory (FK_SYSTEM_BATCH_CHUNK=n overrides), at least one.
-static uint32_t system_batch_chunk(const SystemBatch& b, uint32_t n, uint32_t n_reports) {
-    const uint32_t env = system_batch_chunk_env();
-    uint64_t bytes = sizeof(double) * (2ull * b.L.n_vars + b.L.n_constraints + 1) + sizeof(fk_report) * (uint64_t)n_reports;
-    uint64_t max_mult = 1;
-    for (const SystemBatch::Structure& S : b.st) {
-        const fk::Topology& t = S.topo->t;
-        bytes += S.members.size() * (sizeof(double) * ((uint64_t)t.n_vars + t.n_expr + t.n_free) + sizeof(fk_report));
-        max_mult = std::max<uint64_t>(max_mult, S.members.size());
-    }
-    uint64_t chunk = env ? env : std::max<uint64_t>(1, (1ull << 30) / bytes);
-    chunk = std::min<uint64_t>(chunk, std::max<uint64_t>(1, (uint64_t)INT32_MAX / max_mult));  // sketches per launch stay in range
-    return (uint32_t)std::min<uint64_t>(chunk, n);
-}
-
-static SystemBatchDevice* system_batch_device_slot(SystemBatch& b, int device) {
-    std::lock_guard<std::mutex> lock(b.mu);
-    auto& p = b.devices[device];
-    if (!p) p.reset(new SystemBatchDevice());
-    return p.get();
-}
-
-// Tables once per device; plans and chunk buffers grow with the chunk (and are made again when LM follows L-BFGS).  The caller
-// holds d->mu.
-static int system_batch_device(SystemBatch& b, SystemBatchDevice* d, int device, uint32_t chunk, uint32_t n_reports, bool lm) {
+// Tables once per device; plans and chunk buffers grow with the chunk (and are made again when LM follows L-BFGS).  *chunk: the
+// variants per chunk for n variants.  The caller holds d->mu.
+static int system_batch_device(SystemBatch& b, SystemBatchDevice* d, int device, uint32_t n, bool lm, uint32_t* chunk) {
     CU(cudaSetDevice(device));
     const SystemBatchLayout& L = b.L;
-    const uint32_t n_expr = (uint32_t)L.kind.size(), ns = (uint32_t)b.st.size(), nc = (uint32_t)L.comps.size();
+    const uint32_t ns = (uint32_t)b.st.size(), nc = (uint32_t)L.comps.size();
     if (!d->ready) {
-        d->device = device;
-        if (!d->stream) CU(cudaStreamCreateWithFlags(&d->stream, cudaStreamNonBlocking));
-        cudaFree(d->d_tables); cudaFree(d->d_desc); cudaFree(d->d_tmpl_vars); cudaFree(d->d_tmpl_param);  // (an earlier attempt's)
-        d->d_tables = nullptr; d->d_desc = nullptr; d->d_tmpl_vars = d->d_tmpl_param = nullptr;
-        struct Item { const void* src; size_t bytes; size_t at; };
-        std::vector<Item> items;
-        size_t off = 0;
-        auto add = [&](const auto& vec) {
-            using T = typename std::decay<decltype(vec)>::type::value_type;
-            const size_t at = reserve<T>(off, vec.size());
-            items.push_back({vec.data(), vec.size() * sizeof(T), at});
-            return at;
-        };
-        const size_t o_kind = add(L.kind), o_con = add(L.expr_constraint), o_draws = add(L.draws), o_vs = add(b.var_struct), o_vo = add(b.var_off),
-                     o_cs = add(b.comp_struct), o_cm = add(b.comp_member);
+        TablePack pk;
+        const size_t o_kind = pk.add(L.kind), o_con = pk.add(L.expr_constraint), o_draws = pk.add(L.draws), o_vs = pk.add(b.var_struct),
+                     o_vo = pk.add(b.var_off), o_cs = pk.add(b.comp_struct), o_cm = pk.add(b.comp_member);
         std::vector<size_t> o_sv(ns), o_sd(ns), o_ex(ns);
         for (uint32_t s = 0; s < ns; s++) {
-            o_sv[s] = add(b.st[s].slot_var);
-            o_sd[s] = add(b.st[s].slot_draw);
-            o_ex[s] = add(b.st[s].expr);
+            o_sv[s] = pk.add(b.st[s].slot_var);
+            o_sd[s] = pk.add(b.st[s].slot_draw);
+            o_ex[s] = pk.add(b.st[s].expr);
         }
-        std::vector<unsigned char> host(off + 16, 0);
-        for (const Item& it : items)
-            if (it.bytes) std::memcpy(host.data() + it.at, it.src, it.bytes);
-        CU(cudaMalloc(&d->d_tables, host.size()));
-        CU(cudaMemcpyAsync(d->d_tables, host.data(), host.size(), cudaMemcpyHostToDevice, d->stream));
-        CU(cudaStreamSynchronize(d->stream));  // (host leaves scope)
-        unsigned char* t = (unsigned char*)d->d_tables;
-        d->d_kind = t + o_kind;
-        d->d_expr_con = (const uint32_t*)(t + o_con);
-        d->d_draws = (const double*)(t + o_draws);
-        d->d_var_struct = (const uint32_t*)(t + o_vs); d->d_var_off = (const uint32_t*)(t + o_vo);
-        d->d_comp_struct = (const uint32_t*)(t + o_cs); d->d_comp_member = (const uint32_t*)(t + o_cm);
+        const int rc = d->upload_tables(device, pk, L.n_vars, (uint32_t)L.kind.size());
+        if (rc != FK_OK) return rc;
+        d->d_kind = pk.at<uint8_t>(o_kind);
+        d->d_expr_con = pk.at<uint32_t>(o_con);
+        d->d_draws = pk.at<double>(o_draws);
+        d->d_var_struct = pk.at<uint32_t>(o_vs); d->d_var_off = pk.at<uint32_t>(o_vo);
+        d->d_comp_struct = pk.at<uint32_t>(o_cs); d->d_comp_member = pk.at<uint32_t>(o_cm);
         d->desc.assign(ns, SbStructure{});
         for (uint32_t s = 0; s < ns; s++) {
             const fk::Topology& tp = b.st[s].topo->t;
             SbStructure& S = d->desc[s];
-            S.slot_var = (const uint32_t*)(t + o_sv[s]); S.slot_draw = (const uint32_t*)(t + o_sd[s]); S.expr = (const uint32_t*)(t + o_ex[s]);
-            S.nv = tp.n_vars; S.ne = tp.n_expr; S.nf = tp.n_free; S.mult = (uint32_t)b.st[s].members.size();
+            S.slot_var = pk.at<uint32_t>(o_sv[s]); S.slot_draw = pk.at<uint32_t>(o_sd[s]); S.expr = pk.at<uint32_t>(o_ex[s]);
+            S.nv = tp.n_vars; S.ne = tp.n_expr; S.nf = tp.n_free; S.mult = b.st[s].mult;
         }
-        CU(cudaMalloc(&d->d_desc, sizeof(SbStructure) * std::max<uint32_t>(ns, 1)));
-        CU(cudaMalloc(&d->d_tmpl_vars, sizeof(double) * std::max<uint32_t>(L.n_vars, 1)));
-        CU(cudaMalloc(&d->d_tmpl_param, sizeof(double) * std::max<uint32_t>(n_expr, 1)));
         d->ready = true;
     }
-    if (d->chunk >= chunk && (d->lm || !lm) && d->plans.size() == ns) return FK_OK;
-    const uint32_t cap = std::max(chunk, d->chunk);
-    d->release_buffers();
+    // per variant: the raw rows, its scale, vars_out and a report per component, and the plans' rows
+    uint64_t mult = 1;
+    const uint64_t bytes = sizeof(double) * (2ull * L.n_vars + L.n_constraints + 1) + sizeof(fk_report) * (uint64_t)nc + plan_bytes(b.st, &mult);
+    *chunk = system_batch_chunk(n, bytes, mult, std::max({L.n_vars, L.n_constraints, nc}));
+    if (d->chunk >= *chunk && (d->lm || !lm) && d->plans.size() == ns) return FK_OK;
+    const int rc = d->grow_chunk(L, b.st, std::max(*chunk, d->chunk), lm, nc, false);
+    if (rc != FK_OK) return rc;
     for (uint32_t s = 0; s < ns; s++) {
-        fk_batch_plan* p = nullptr;
-        const int rc = plan_create(b.st[s].topo.get(), cap * (uint32_t)b.st[s].members.size(), device, lm, &p);
-        if (rc != FK_OK) {
-            d->release_buffers();
-            return rc;
-        }
-        d->plans.push_back(p);
+        const fk_batch_plan* p = d->plans[s].get();
         SbStructure& S = d->desc[s];
         S.vars = p->d_vars; S.params = p->d_params; S.out = p->d_out; S.reps = p->d_rep;
     }
-    auto alloc = [&](auto** ptr, size_t count) -> int {
-        CU(cudaMalloc((void**)ptr, sizeof(**ptr) * std::max<size_t>(count, 1)));
-        return FK_OK;
-    };
-    int rc = FK_OK;
-    if ((rc = alloc(&d->d_raw_vars, (size_t)cap * L.n_vars)) != FK_OK || (rc = alloc(&d->d_raw_param, (size_t)cap * L.n_constraints)) != FK_OK ||
-        (rc = alloc(&d->d_scales, cap)) != FK_OK || (rc = alloc(&d->d_vars_out, (size_t)cap * L.n_vars)) != FK_OK ||
-        (rc = alloc(&d->d_rep_out, (size_t)cap * std::max<uint32_t>(std::min(n_reports, nc), 1))) != FK_OK) {
-        d->release_buffers();
-        return rc;
-    }
     if (ns) CU(cudaMemcpyAsync(d->d_desc, d->desc.data(), sizeof(SbStructure) * ns, cudaMemcpyHostToDevice, d->stream));
     CU(cudaStreamSynchronize(d->stream));  // (desc may change before a later call's copy)
-    d->chunk = cap;
-    d->lm = lm;
     return FK_OK;
 }
 
-// Variants [lo, hi) on one device, chunk after chunk on its stream: upload, prepare + gather, one launch per structure, scatter,
-// download.
+// Variants [lo, hi) on one device: per chunk the prepare kernel (gather into every structure's rows), one launch per structure
+// and the scatter kernel.
 static int system_batch_range(SystemBatch& b, const SystemBatchCall& c, int device, uint32_t lo, uint32_t hi) {
     const SystemBatchLayout& L = b.L;
-    const uint32_t n_expr = (uint32_t)L.kind.size(), ns = (uint32_t)b.st.size(), nc = (uint32_t)L.comps.size();
+    const uint32_t ns = (uint32_t)b.st.size(), nc = (uint32_t)L.comps.size();
     const uint32_t n_rep = c.reports ? std::min(c.reports_per_variant, nc) : 0;
-    const uint32_t chunk = system_batch_chunk(b, hi - lo, n_rep);
-    SystemBatchDevice* d = system_batch_device_slot(b, device);
+    SystemBatchDevice* d = device_slot(b.mu, b.devices, device);
     std::lock_guard<std::mutex> lock(d->mu);
-    int rc = system_batch_device(b, d, device, chunk, nc, c.optimizer == 0);
+    uint32_t chunk = 0;
+    const int rc = system_batch_device(b, d, device, hi - lo, c.optimizer == 0, &chunk);
     if (rc != FK_OK) return rc;
-    cudaStream_t st = d->stream;
-    auto run = [&]() -> int {
-        if (L.n_vars) CU(cudaMemcpyAsync(d->d_tmpl_vars, c.tmpl_vars, sizeof(double) * L.n_vars, cudaMemcpyHostToDevice, st));
-        if (n_expr) CU(cudaMemcpyAsync(d->d_tmpl_param, c.tmpl_param, sizeof(double) * n_expr, cudaMemcpyHostToDevice, st));
-        for (uint32_t at = lo; at < hi; at += chunk) {
-            const uint32_t cnt = std::min(chunk, hi - at);
-            const double* raw = d->d_tmpl_vars;
-            uint32_t raw_stride = 0;
-            if (c.vars) {
-                if (L.n_vars)
-                    CU(cudaMemcpyAsync(d->d_raw_vars, c.vars + (size_t)at * L.n_vars, sizeof(double) * (size_t)cnt * L.n_vars, cudaMemcpyHostToDevice, st));
-                raw = d->d_raw_vars;
-                raw_stride = L.n_vars;
-            }
-            if (c.params && L.n_constraints)
-                CU(cudaMemcpyAsync(d->d_raw_param, c.params + (size_t)at * L.n_constraints, sizeof(double) * (size_t)cnt * L.n_constraints,
-                                   cudaMemcpyHostToDevice, st));
-            int e = launch_system_batch_prepare(cnt, L.n_vars, n_expr, L.n_constraints, d->d_kind, d->d_expr_con, d->d_draws, c.perturb, raw,
-                                                raw_stride, c.params ? d->d_raw_param : nullptr, d->d_tmpl_param, ns, d->d_desc, d->d_scales, st);
-            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_batch_prepare_kernel");
-            for (uint32_t s = 0; s < ns; s++) {
-                fk_batch_plan* p = d->plans[s];
-                p->n = cnt * (uint32_t)b.st[s].members.size();
-                const int r = c.optimizer == 0                    ? fk_batch_plan_run(p, st)
-                              : choose_lbfgs(p->topo, p->n) == 1 ? fk_batch_plan_run_lbfgs_global(p, st)
-                                                                 : fk_batch_plan_run_lbfgs(p, st);
-                if (r != FK_OK) return r;
-            }
-            e = launch_system_batch_scatter(cnt, L.n_vars, raw, raw_stride, d->d_scales, d->d_var_struct, d->d_var_off, n_rep, d->d_comp_struct,
-                                            d->d_comp_member, d->d_desc, d->d_vars_out, d->d_rep_out, st);
-            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_batch_scatter_kernel");
-            if (L.n_vars)
-                CU(cudaMemcpyAsync(c.vars_out + (size_t)at * L.n_vars, d->d_vars_out, sizeof(double) * (size_t)cnt * L.n_vars, cudaMemcpyDeviceToHost, st));
-            if (n_rep)
-                CU(cudaMemcpy2DAsync(c.reports + (size_t)at * c.reports_per_variant, sizeof(fk_report) * c.reports_per_variant, d->d_rep_out,
-                                     sizeof(fk_report) * n_rep, sizeof(fk_report) * n_rep, cnt, cudaMemcpyDeviceToHost, st));
-        }
-        return FK_OK;
-    };
-    rc = run();
-    // (also after an error: no copy into the caller's buffers may still be running when the call returns)
-    const cudaError_t e = cudaStreamSynchronize(st);
-    if (rc == FK_OK && e != cudaSuccess) rc = cuda_fail(e, "fk_system_batch_solve kernels / copies");
-    return rc;
+    return solve_chunks(d, L, c, lo, hi, chunk, n_rep, ns, "fk_system_batch_solve kernels / copies",
+                        [&](uint32_t cnt, const double* raw, uint32_t raw_stride) -> int {
+                            for (uint32_t s = 0; s < ns; s++) {
+                                fk_batch_plan* p = d->plans[s].get();
+                                p->n = cnt * b.st[s].mult;
+                                const int r = c.optimizer == 0                    ? fk_batch_plan_run(p, d->stream)
+                                              : choose_lbfgs(p->topo, p->n) == 1 ? fk_batch_plan_run_lbfgs_global(p, d->stream)
+                                                                                 : fk_batch_plan_run_lbfgs(p, d->stream);
+                                if (r != FK_OK) return r;
+                            }
+                            const int e = launch_system_batch_scatter(cnt, L.n_vars, raw, raw_stride, d->d_scales, d->d_var_struct, d->d_var_off, n_rep,
+                                                                      d->d_comp_struct, d->d_comp_member, d->d_desc, d->d_vars_out, d->d_rep_out, d->stream);
+                            return e != 0 ? cuda_fail((cudaError_t)e, "launch fk_system_batch_scatter_kernel") : FK_OK;
+                        });
 }
 
 int system_batch_solve(SystemBatch& b, const SystemBatchCall& c) {
@@ -2121,37 +2191,21 @@ int system_batch_solve(SystemBatch& b, const SystemBatchCall& c) {
     int n_gpus = c.n_gpus;
     const int rc = clamp_gpus(n_gpus);
     if (rc != FK_OK) return rc;
-    int cur = 0;
-    if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
-    const int r = shard_over_devices(n_gpus, c.n, [&](int device, uint32_t lo, uint32_t hi) { return system_batch_range(b, c, device, lo, hi); });
-    if (cudaSetDevice(cur) != cudaSuccess) cudaGetLastError();
-    return r;
+    return shard_over_devices(n_gpus, c.n, [&](int device, uint32_t lo, uint32_t hi) { return system_batch_range(b, c, device, lo, hi); });
 }
 
 // ---- fk_system_batch_solve_single_pass: Decomposer::SinglePass over n variants of one drawing ---------------------------
 // (fk_system_batch_solve_recursive_assembly runs on the same plan: its steps in place of the sets, with their moves.)
-// The device state of fk_system_batch_solve plus the resident rows of the scaled variables (vt) and parameters (pt) that the
-// waves read and write, and the per-wave descriptors of the gather / scatter kernel.  d_desc holds the one identity structure
-// through which the prepare kernel writes vt and pt; plans are one per structure (capacity chunk * the structure's most sets
-// in one wave).
+// The solve batches' device state plus the per-wave descriptors of the gather / scatter kernel.  The resident rows vt and pt are
+// what the waves read and write; d_desc holds the one identity structure through which the prepare kernel writes them.  Plans are
+// one per structure (capacity chunk * the structure's most sets in one wave).
 struct SystemSpDevice : SystemBatchDevice {
-    double *d_vt = nullptr, *d_pt = nullptr;
     const uint8_t* d_solved = nullptr;
     const uint32_t *d_pvar = nullptr, *d_pdraw = nullptr;  // the perturbations of waves >= 1, wave after wave
     std::vector<uint32_t> pert_off;                        // [n_waves + 1]
     std::vector<SpGroup> groups;                           // (host copy) every wave's groups, wave after wave
     std::vector<uint32_t> group_off;                       // [n_waves + 1]
     SpGroup* d_groups = nullptr;
-    void release_sp_buffers() {
-        cudaFree(d_vt); cudaFree(d_pt);
-        d_vt = d_pt = nullptr;
-        release_buffers();
-    }
-    ~SystemSpDevice() {
-        if (device < 0) return;
-        cudaSetDevice(device);
-        cudaFree(d_vt); cudaFree(d_pt); cudaFree(d_groups);
-    }
 };
 
 struct SystemSpBatch {
@@ -2159,7 +2213,7 @@ struct SystemSpBatch {
     struct Structure {
         std::shared_ptr<fk_topology> topo;
         std::vector<uint32_t> members;  // set indices
-        uint32_t wave_mult = 0;         // most sets of the structure in one wave: the plan's sketches per variant
+        uint32_t mult = 0;              // most sets of the structure in one wave: the plan's sketches per variant
     };
     std::vector<Structure> st;
     std::vector<uint32_t> set_struct;
@@ -2180,12 +2234,8 @@ int system_sp_batch_create(SystemBatchLayout&& layout, const std::vector<const f
     const SystemBatchLayout& L = b->L;
     const uint32_t n_sets = (uint32_t)problems.size();
     std::vector<BatchGroup> groups;
-    if (n_sets) {
-        static double dummy = 0.0;  // (group_by_topology checks the free-value pointers; nothing is written through them)
-        std::vector<double*> fv(n_sets, &dummy);
-        const int rc = group_by_topology(n_sets, problems.data(), fv.data(), groups);
-        if (rc != FK_OK) return rc;
-    }
+    const int rc = group_by_structure(problems, groups);
+    if (rc != FK_OK) return rc;
     b->set_struct.assign(n_sets, kSbNone);
     for (BatchGroup& g : groups) {
         for (uint32_t k : g.members) b->set_struct[k] = (uint32_t)b->st.size();
@@ -2209,7 +2259,7 @@ int system_sp_batch_create(SystemBatchLayout&& layout, const std::vector<const f
         it->free_var.insert(it->free_var.end(), c.free_var.begin(), c.free_var.end());
         it->moves.insert(it->moves.end(), c.moves.begin(), c.moves.end());
         it->move_off.push_back((uint32_t)(it->moves.size() / 2));
-        b->st[si].wave_mult = std::max(b->st[si].wave_mult, (uint32_t)it->sets.size());
+        b->st[si].mult = std::max(b->st[si].mult, (uint32_t)it->sets.size());
         for (uint32_t g : c.free_var)
             if (g != kSbNone) b->solved[g] = 1;
         for (size_t m = 0; m < c.moves.size(); m += 2) b->solved[c.moves[m]] = b->solved[c.moves[m] + 1] = 1;
@@ -2231,40 +2281,13 @@ void system_sp_batch_layout(const SystemSpBatch& b, uint32_t* n_sets, uint32_t* 
     if (set_structure) *set_structure = b.set_struct;
 }
 
-// Variants per chunk, as system_batch_chunk: raw, resident and output rows plus every structure's plan buffers.
-static uint32_t system_sp_chunk(const SystemSpBatch& b, uint32_t n, uint32_t n_reports) {
-    const uint32_t env = system_batch_chunk_env();
-    const uint64_t n_expr = b.L.kind.size();
-    uint64_t bytes = sizeof(double) * (3ull * b.L.n_vars + b.L.n_constraints + n_expr + 1) + sizeof(fk_report) * (uint64_t)n_reports;
-    uint64_t max_mult = 1;
-    for (const SystemSpBatch::Structure& S : b.st) {
-        const fk::Topology& t = S.topo->t;
-        bytes += S.wave_mult * (sizeof(double) * ((uint64_t)t.n_vars + t.n_expr + t.n_free) + sizeof(fk_report));
-        max_mult = std::max<uint64_t>(max_mult, S.wave_mult);
-    }
-    uint64_t chunk = env ? env : std::max<uint64_t>(1, (1ull << 30) / bytes);
-    chunk = std::min<uint64_t>(chunk, std::max<uint64_t>(1, (uint64_t)INT32_MAX / max_mult));  // sketches per launch stay in range
-    chunk = std::min<uint64_t>(chunk, std::max<uint64_t>(1, (uint64_t)UINT32_MAX / std::max<uint64_t>({1, b.L.n_vars, n_expr})));
-    return (uint32_t)std::min<uint64_t>(chunk, n);
-}
-
-static SystemSpDevice* system_sp_device_slot(SystemSpBatch& b, int device) {
-    std::lock_guard<std::mutex> lock(b.mu);
-    auto& p = b.devices[device];
-    if (!p) p.reset(new SystemSpDevice());
-    return p.get();
-}
-
-// Tables once per device; plans, buffers and descriptors grow with the chunk.  The caller holds d->mu.
-static int system_sp_device(SystemSpBatch& b, SystemSpDevice* d, int device, uint32_t chunk, uint32_t n_reports) {
+// Tables once per device; plans, buffers and descriptors grow with the chunk.  *chunk: the variants per chunk for n variants.
+// The caller holds d->mu.
+static int system_sp_device(SystemSpBatch& b, SystemSpDevice* d, int device, uint32_t n, uint32_t* chunk) {
     CU(cudaSetDevice(device));
     const SystemBatchLayout& L = b.L;
-    const uint32_t n_expr = (uint32_t)L.kind.size(), ns = (uint32_t)b.st.size(), nw = L.n_waves;
+    const uint32_t n_expr = (uint32_t)L.kind.size(), ns = (uint32_t)b.st.size(), nw = L.n_waves, n_sets = (uint32_t)L.comps.size();
     if (!d->ready) {
-        d->device = device;
-        if (!d->stream) CU(cudaStreamCreateWithFlags(&d->stream, cudaStreamNonBlocking));
-        cudaFree(d->d_tables); cudaFree(d->d_desc); cudaFree(d->d_tmpl_vars); cudaFree(d->d_tmpl_param); cudaFree(d->d_groups);  // (an earlier attempt's)
-        d->d_tables = nullptr; d->d_desc = nullptr; d->d_tmpl_vars = d->d_tmpl_param = nullptr; d->d_groups = nullptr;
         // the identity structure of the prepare kernel: every variable (with its draw where the perturbation runs before any
         // set) and every expression
         std::vector<uint32_t> ident_var(L.n_vars), ident_draw(L.n_vars, kSbNone), ident_expr(n_expr);
@@ -2282,37 +2305,24 @@ static int system_sp_device(SystemSpBatch& b, SystemSpDevice* d, int device, uin
             }
             d->pert_off.push_back((uint32_t)pvar.size());
         }
-        struct Item { const void* src; size_t bytes; size_t at; };
-        std::vector<Item> items;
-        size_t off = 0;
-        auto add = [&](const auto& vec) {
-            using T = typename std::decay<decltype(vec)>::type::value_type;
-            const size_t at = reserve<T>(off, vec.size());
-            items.push_back({vec.data(), vec.size() * sizeof(T), at});
-            return at;
-        };
-        const size_t o_kind = add(L.kind), o_con = add(L.expr_constraint), o_draws = add(L.draws), o_iv = add(ident_var), o_id = add(ident_draw),
-                     o_ie = add(ident_expr), o_solved = add(b.solved), o_pv = add(pvar), o_pd = add(pdraw);
+        TablePack pk;
+        const size_t o_kind = pk.add(L.kind), o_con = pk.add(L.expr_constraint), o_draws = pk.add(L.draws), o_iv = pk.add(ident_var),
+                     o_id = pk.add(ident_draw), o_ie = pk.add(ident_expr), o_solved = pk.add(b.solved), o_pv = pk.add(pvar), o_pd = pk.add(pdraw);
         struct GroupAt { size_t sv, ex, fv, st, mo, mv; };
         std::vector<GroupAt> at;
         for (const auto& wave : b.waves)
             for (const SystemSpBatch::Group& g : wave)
-                at.push_back({add(g.slot_var), add(g.expr), add(g.free_var), add(g.sets), add(g.move_off), add(g.moves)});
-        std::vector<unsigned char> host(off + 16, 0);
-        for (const Item& it : items)
-            if (it.bytes) std::memcpy(host.data() + it.at, it.src, it.bytes);
-        CU(cudaMalloc(&d->d_tables, host.size()));
-        CU(cudaMemcpyAsync(d->d_tables, host.data(), host.size(), cudaMemcpyHostToDevice, d->stream));
-        CU(cudaStreamSynchronize(d->stream));  // (host leaves scope)
-        unsigned char* t = (unsigned char*)d->d_tables;
-        d->d_kind = t + o_kind;
-        d->d_expr_con = (const uint32_t*)(t + o_con);
-        d->d_draws = (const double*)(t + o_draws);
-        d->d_solved = t + o_solved;
-        d->d_pvar = (const uint32_t*)(t + o_pv); d->d_pdraw = (const uint32_t*)(t + o_pd);
+                at.push_back({pk.add(g.slot_var), pk.add(g.expr), pk.add(g.free_var), pk.add(g.sets), pk.add(g.move_off), pk.add(g.moves)});
+        const int rc = d->upload_tables(device, pk, L.n_vars, n_expr);
+        if (rc != FK_OK) return rc;
+        d->d_kind = pk.at<uint8_t>(o_kind);
+        d->d_expr_con = pk.at<uint32_t>(o_con);
+        d->d_draws = pk.at<double>(o_draws);
+        d->d_solved = pk.at<uint8_t>(o_solved);
+        d->d_pvar = pk.at<uint32_t>(o_pv); d->d_pdraw = pk.at<uint32_t>(o_pd);
         d->desc.assign(1, SbStructure{});
         SbStructure& I = d->desc[0];
-        I.slot_var = (const uint32_t*)(t + o_iv); I.slot_draw = (const uint32_t*)(t + o_id); I.expr = (const uint32_t*)(t + o_ie);
+        I.slot_var = pk.at<uint32_t>(o_iv); I.slot_draw = pk.at<uint32_t>(o_id); I.expr = pk.at<uint32_t>(o_ie);
         I.nv = L.n_vars; I.ne = n_expr; I.nf = 0; I.mult = 1;
         d->groups.clear();
         d->group_off.assign(1, 0);
@@ -2321,127 +2331,78 @@ static int system_sp_device(SystemSpBatch& b, SystemSpDevice* d, int device, uin
             for (const SystemSpBatch::Group& g : wave) {
                 const fk::Topology& tp = b.st[g.structure].topo->t;
                 SpGroup G{};
-                G.s.slot_var = (const uint32_t*)(t + at[q].sv); G.s.expr = (const uint32_t*)(t + at[q].ex);
-                G.free_var = (const uint32_t*)(t + at[q].fv); G.step = (const uint32_t*)(t + at[q].st);
-                G.move_off = (const uint32_t*)(t + at[q].mo); G.moves = (const uint32_t*)(t + at[q].mv);
+                G.s.slot_var = pk.at<uint32_t>(at[q].sv); G.s.expr = pk.at<uint32_t>(at[q].ex);
+                G.free_var = pk.at<uint32_t>(at[q].fv); G.step = pk.at<uint32_t>(at[q].st);
+                G.move_off = pk.at<uint32_t>(at[q].mo); G.moves = pk.at<uint32_t>(at[q].mv);
                 G.s.nv = tp.n_vars; G.s.ne = tp.n_expr; G.s.nf = tp.n_free; G.s.mult = (uint32_t)g.sets.size();
                 d->groups.push_back(G);
                 q++;
             }
             d->group_off.push_back((uint32_t)d->groups.size());
         }
-        CU(cudaMalloc(&d->d_desc, sizeof(SbStructure)));
-        CU(cudaMalloc(&d->d_groups, sizeof(SpGroup) * std::max<size_t>(d->groups.size(), 1)));
-        CU(cudaMalloc(&d->d_tmpl_vars, sizeof(double) * std::max<uint32_t>(L.n_vars, 1)));
-        CU(cudaMalloc(&d->d_tmpl_param, sizeof(double) * std::max<uint32_t>(n_expr, 1)));
         d->ready = true;
     }
-    if (d->chunk >= chunk && d->plans.size() == ns) return FK_OK;
-    const uint32_t cap = std::max(chunk, d->chunk);
-    d->release_sp_buffers();
-    for (uint32_t s = 0; s < ns; s++) {
-        fk_batch_plan* p = nullptr;
-        const int rc = plan_create(b.st[s].topo.get(), cap * b.st[s].wave_mult, device, true, &p);
-        if (rc != FK_OK) {
-            d->release_sp_buffers();
-            return rc;
-        }
-        d->plans.push_back(p);
-    }
-    auto alloc = [&](auto** ptr, size_t count) -> int {
-        CU(cudaMalloc((void**)ptr, sizeof(**ptr) * std::max<size_t>(count, 1)));
-        return FK_OK;
-    };
-    const uint32_t n_sets = (uint32_t)L.comps.size();
-    int rc = FK_OK;
-    if ((rc = alloc(&d->d_raw_vars, (size_t)cap * L.n_vars)) != FK_OK || (rc = alloc(&d->d_raw_param, (size_t)cap * L.n_constraints)) != FK_OK ||
-        (rc = alloc(&d->d_scales, cap)) != FK_OK || (rc = alloc(&d->d_vars_out, (size_t)cap * L.n_vars)) != FK_OK ||
-        (rc = alloc(&d->d_vt, (size_t)cap * L.n_vars)) != FK_OK || (rc = alloc(&d->d_pt, (size_t)cap * n_expr)) != FK_OK ||
-        (rc = alloc(&d->d_rep_out, (size_t)cap * std::max<uint32_t>(std::min(n_reports, n_sets), 1))) != FK_OK) {
-        d->release_sp_buffers();
+    // per variant: the raw rows, its scale, vars_out, the resident rows, a report per set, and the plans' rows
+    uint64_t mult = 1;
+    const uint64_t bytes = sizeof(double) * (3ull * L.n_vars + L.n_constraints + n_expr + 1) + sizeof(fk_report) * (uint64_t)n_sets +
+                           plan_bytes(b.st, &mult);
+    *chunk = system_batch_chunk(n, bytes, mult, std::max({L.n_vars, L.n_constraints, n_expr, n_sets}));
+    if (d->chunk >= *chunk && d->plans.size() == ns) return FK_OK;
+    int rc = d->grow_chunk(L, b.st, std::max(*chunk, d->chunk), true, n_sets, true);
+    if (rc == FK_OK) rc = d->grow(&d->d_groups, d->groups.size());
+    if (rc != FK_OK) {
+        d->plans.clear();
+        d->release_buffers();
         return rc;
     }
     d->desc[0].vars = d->d_vt;
     d->desc[0].params = d->d_pt;
-    {
-        size_t q = 0;
-        for (const auto& wave : b.waves)
-            for (const SystemSpBatch::Group& g : wave) {
-                const fk_batch_plan* p = d->plans[g.structure];
-                SpGroup& G = d->groups[q++];
-                G.s.vars = p->d_vars; G.s.params = p->d_params; G.s.out = p->d_out; G.s.reps = p->d_rep;
-            }
-    }
+    for (size_t q = 0, w = 0; w < b.waves.size(); w++)
+        for (const SystemSpBatch::Group& g : b.waves[w]) {
+            const fk_batch_plan* p = d->plans[g.structure].get();
+            SpGroup& G = d->groups[q++];
+            G.s.vars = p->d_vars; G.s.params = p->d_params; G.s.out = p->d_out; G.s.reps = p->d_rep;
+        }
     CU(cudaMemcpyAsync(d->d_desc, d->desc.data(), sizeof(SbStructure), cudaMemcpyHostToDevice, d->stream));
     if (!d->groups.empty())
         CU(cudaMemcpyAsync(d->d_groups, d->groups.data(), sizeof(SpGroup) * d->groups.size(), cudaMemcpyHostToDevice, d->stream));
     CU(cudaStreamSynchronize(d->stream));  // (the descriptors may change before a later call's copy)
-    d->chunk = cap;
-    d->lm = true;
     return FK_OK;
 }
 
-// Variants [lo, hi) on one device, chunk after chunk on its stream: upload; prepare (scale, the perturbations that precede every
-// set, the resident rows vt / pt); per wave one gather / scatter launch and one LM launch per structure present; a last gather /
-// scatter launch with the write-back; download.
+// Variants [lo, hi) on one device: per chunk the prepare kernel (scale, the perturbations that precede every set, the resident rows
+// vt / pt); per wave one gather / scatter launch and one LM launch per structure present; a last gather / scatter launch with the
+// write-back.
 static int system_sp_range(SystemSpBatch& b, const SystemBatchCall& c, int device, uint32_t lo, uint32_t hi) {
     const SystemBatchLayout& L = b.L;
     const uint32_t n_expr = (uint32_t)L.kind.size(), nw = L.n_waves, n_sets = (uint32_t)L.comps.size();
     const uint32_t n_rep = c.reports ? std::min(c.reports_per_variant, n_sets) : 0;
-    const uint32_t chunk = system_sp_chunk(b, hi - lo, n_rep);
-    SystemSpDevice* d = system_sp_device_slot(b, device);
+    SystemSpDevice* d = device_slot(b.mu, b.devices, device);
     std::lock_guard<std::mutex> lock(d->mu);
-    int rc = system_sp_device(b, d, device, chunk, n_sets);
+    uint32_t chunk = 0;
+    const int rc = system_sp_device(b, d, device, hi - lo, &chunk);
     if (rc != FK_OK) return rc;
-    cudaStream_t st = d->stream;
-    auto run = [&]() -> int {
-        if (L.n_vars) CU(cudaMemcpyAsync(d->d_tmpl_vars, c.tmpl_vars, sizeof(double) * L.n_vars, cudaMemcpyHostToDevice, st));
-        if (n_expr) CU(cudaMemcpyAsync(d->d_tmpl_param, c.tmpl_param, sizeof(double) * n_expr, cudaMemcpyHostToDevice, st));
-        for (uint32_t at = lo; at < hi; at += chunk) {
-            const uint32_t cnt = std::min(chunk, hi - at);
-            const double* raw = d->d_tmpl_vars;
-            uint32_t raw_stride = 0;
-            if (c.vars) {
-                if (L.n_vars)
-                    CU(cudaMemcpyAsync(d->d_raw_vars, c.vars + (size_t)at * L.n_vars, sizeof(double) * (size_t)cnt * L.n_vars, cudaMemcpyHostToDevice, st));
-                raw = d->d_raw_vars;
-                raw_stride = L.n_vars;
-            }
-            if (c.params && L.n_constraints)
-                CU(cudaMemcpyAsync(d->d_raw_param, c.params + (size_t)at * L.n_constraints, sizeof(double) * (size_t)cnt * L.n_constraints,
-                                   cudaMemcpyHostToDevice, st));
-            int e = launch_system_batch_prepare(cnt, L.n_vars, n_expr, L.n_constraints, d->d_kind, d->d_expr_con, d->d_draws, c.perturb, raw,
-                                                raw_stride, c.params ? d->d_raw_param : nullptr, d->d_tmpl_param, 1, d->d_desc, d->d_scales, st);
-            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_batch_prepare_kernel");
-            for (uint32_t w = 0; w <= nw; w++) {
-                const uint32_t s_lo = w ? d->group_off[w - 1] : 0, s_hi = w ? d->group_off[w] : 0;
-                const uint32_t g_lo = w < nw ? d->group_off[w] : 0, g_hi = w < nw ? d->group_off[w + 1] : 0;
-                const uint32_t p_lo = c.perturb && w < nw ? d->pert_off[w] : 0, p_hi = c.perturb && w < nw ? d->pert_off[w + 1] : 0;
-                e = launch_system_sp_gather_scatter(cnt, L.n_vars, n_expr, d->d_vt, d->d_pt, s_hi - s_lo, d->d_groups + s_lo, n_rep, d->d_rep_out,
-                                                    p_hi - p_lo, d->d_pvar + p_lo, d->d_pdraw + p_lo, d->d_draws, g_hi - g_lo, d->d_groups + g_lo,
-                                                    d->d_solved, raw, raw_stride, d->d_scales, w == nw ? d->d_vars_out : nullptr, st);
-                if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_sp_gather_scatter_kernel");
-                if (w == nw) break;
-                for (const SystemSpBatch::Group& g : b.waves[w]) {  // LM under SinglePass / RecursiveAssembly whatever the optimizer (assemble/mod.rs:191, :224)
-                    fk_batch_plan* p = d->plans[g.structure];
-                    p->n = cnt * (uint32_t)g.sets.size();
-                    const int r = fk_batch_plan_run(p, st);
-                    if (r != FK_OK) return r;
-                }
-            }
-            if (L.n_vars)
-                CU(cudaMemcpyAsync(c.vars_out + (size_t)at * L.n_vars, d->d_vars_out, sizeof(double) * (size_t)cnt * L.n_vars, cudaMemcpyDeviceToHost, st));
-            if (n_rep)
-                CU(cudaMemcpy2DAsync(c.reports + (size_t)at * c.reports_per_variant, sizeof(fk_report) * c.reports_per_variant, d->d_rep_out,
-                                     sizeof(fk_report) * n_rep, sizeof(fk_report) * n_rep, cnt, cudaMemcpyDeviceToHost, st));
-        }
-        return FK_OK;
-    };
-    rc = run();
-    // (also after an error: no copy into the caller's buffers may still be running when the call returns)
-    const cudaError_t e = cudaStreamSynchronize(st);
-    if (rc == FK_OK && e != cudaSuccess) rc = cuda_fail(e, "fk_system_batch_solve_single_pass / _recursive_assembly kernels / copies");
-    return rc;
+    return solve_chunks(d, L, c, lo, hi, chunk, n_rep, 1, "fk_system_batch_solve_single_pass / _recursive_assembly kernels / copies",
+                        [&](uint32_t cnt, const double* raw, uint32_t raw_stride) -> int {
+                            for (uint32_t w = 0; w <= nw; w++) {
+                                const uint32_t s_lo = w ? d->group_off[w - 1] : 0, s_hi = w ? d->group_off[w] : 0;
+                                const uint32_t g_lo = w < nw ? d->group_off[w] : 0, g_hi = w < nw ? d->group_off[w + 1] : 0;
+                                const uint32_t p_lo = c.perturb && w < nw ? d->pert_off[w] : 0, p_hi = c.perturb && w < nw ? d->pert_off[w + 1] : 0;
+                                const int e = launch_system_sp_gather_scatter(
+                                    cnt, L.n_vars, n_expr, d->d_vt, d->d_pt, s_hi - s_lo, d->d_groups + s_lo, n_rep, d->d_rep_out, p_hi - p_lo,
+                                    d->d_pvar + p_lo, d->d_pdraw + p_lo, d->d_draws, g_hi - g_lo, d->d_groups + g_lo, d->d_solved, raw, raw_stride,
+                                    d->d_scales, w == nw ? d->d_vars_out : nullptr, d->stream);
+                                if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_sp_gather_scatter_kernel");
+                                if (w == nw) break;
+                                for (const SystemSpBatch::Group& g : b.waves[w]) {  // LM under SinglePass / RecursiveAssembly whatever the optimizer (assemble/mod.rs:191, :224)
+                                    fk_batch_plan* p = d->plans[g.structure].get();
+                                    p->n = cnt * (uint32_t)g.sets.size();
+                                    const int r = fk_batch_plan_run(p, d->stream);
+                                    if (r != FK_OK) return r;
+                                }
+                            }
+                            return FK_OK;
+                        });
 }
 
 int system_sp_batch_solve(SystemSpBatch& b, const SystemBatchCall& c) {
@@ -2457,43 +2418,21 @@ int system_sp_batch_solve(SystemSpBatch& b, const SystemBatchCall& c) {
     int n_gpus = c.n_gpus;
     const int rc = clamp_gpus(n_gpus);
     if (rc != FK_OK) return rc;
-    int cur = 0;
-    if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
-    const int r = shard_over_devices(n_gpus, c.n, [&](int device, uint32_t lo, uint32_t hi) { return system_sp_range(b, c, device, lo, hi); });
-    if (cudaSetDevice(cur) != cudaSuccess) cudaGetLastError();
-    return r;
+    return shard_over_devices(n_gpus, c.n, [&](int device, uint32_t lo, uint32_t hi) { return system_sp_range(b, c, device, lo, hi); });
 }
 
 // ---- fk_system_batch_analyze / fk_system_batch_residuals: System::analyze and calculate_residual over n variants -----------
 // Per device: the layout's tables, the template rows, the chunk buffers (variables vt and expanded parameters pt are what the
-// analyze kernels and fk_system_residuals_kernel read) and the analyze workspace, grow-only within fk::kAnWorkspaceBytes.
-struct SystemAnDevice {
-    int device = -1;
-    std::mutex mu;
-    cudaStream_t stream = nullptr;
-    bool ready = false;  // tables and template buffers in place
-    void* d_tables = nullptr;
+// analyze kernels and fk_system_residuals_kernel read), the outputs of each operation (grown on its first call) and the analyze
+// workspace, grow-only within fk::kAnWorkspaceBytes.
+struct SystemAnDevice : SystemDevice {
     const uint8_t* d_kind = nullptr;
     const uint32_t *d_slot = nullptr, *d_expr_con = nullptr, *d_con_off = nullptr;
-    double *d_tmpl_vars = nullptr, *d_tmpl_param = nullptr;
-    uint32_t chunk = 0, an_chunk = 0, res_chunk = 0;  // variants the inputs, the analyze outputs, the residual outputs hold
-    double *d_raw_param = nullptr, *d_vt = nullptr, *d_pt = nullptr, *d_res = nullptr;
+    uint32_t an_chunk = 0, res_chunk = 0;  // variants the analyze outputs, the residual outputs hold
+    double* d_res = nullptr;
     uint8_t *d_indep = nullptr, *d_dep = nullptr;
     double* d_ws = nullptr;
     uint64_t ws_bytes = 0;
-    void release_buffers() {
-        cudaFree(d_raw_param); cudaFree(d_vt); cudaFree(d_pt); cudaFree(d_res); cudaFree(d_indep); cudaFree(d_dep);
-        d_raw_param = d_vt = d_pt = d_res = nullptr;
-        d_indep = d_dep = nullptr;
-        chunk = an_chunk = res_chunk = 0;
-    }
-    ~SystemAnDevice() {
-        if (device < 0) return;
-        cudaSetDevice(device);
-        release_buffers();
-        cudaFree(d_tables); cudaFree(d_tmpl_vars); cudaFree(d_tmpl_param); cudaFree(d_ws);
-        if (stream) cudaStreamDestroy(stream);
-    }
 };
 
 struct SystemAnBatch {
@@ -2513,128 +2452,94 @@ int system_an_batch_create(SystemAnLayout&& layout, std::shared_ptr<SystemAnBatc
 }
 
 // Tables once per device; the input buffers and the outputs of the call's operation (analyze: per-expression flags and
-// per-constraint counts; residuals: per-constraint values) grow with the chunk.  The caller holds d->mu.
-static int system_an_device(const SystemAnBatch& b, SystemAnDevice* d, int device, uint32_t chunk, bool analyze) {
+// per-constraint counts; residuals: per-constraint values) grow with the chunk.  *chunk: the variants per chunk for n variants.
+// The caller holds d->mu.
+static int system_an_device(const SystemAnBatch& b, SystemAnDevice* d, int device, uint32_t n, bool analyze, uint32_t* chunk) {
     CU(cudaSetDevice(device));
     const SystemAnLayout& L = b.L;
+    const uint32_t ne = b.n_expr, ncon = b.n_constraints;
     if (!d->ready) {
-        d->device = device;
-        if (!d->stream) CU(cudaStreamCreateWithFlags(&d->stream, cudaStreamNonBlocking));
-        cudaFree(d->d_tables); cudaFree(d->d_tmpl_vars); cudaFree(d->d_tmpl_param);  // (an earlier attempt's)
-        d->d_tables = nullptr;
-        d->d_tmpl_vars = d->d_tmpl_param = nullptr;
-        size_t off = 0;
-        const size_t o_kind = reserve<uint8_t>(off, L.kind.size()), o_slot = reserve<uint32_t>(off, L.slot_var.size()),
-                     o_con = reserve<uint32_t>(off, L.expr_constraint.size()), o_off = reserve<uint32_t>(off, L.con_off.size());
-        std::vector<unsigned char> host(off + 16, 0);
-        std::memcpy(host.data() + o_kind, L.kind.data(), L.kind.size());
-        std::memcpy(host.data() + o_slot, L.slot_var.data(), L.slot_var.size() * sizeof(uint32_t));
-        std::memcpy(host.data() + o_con, L.expr_constraint.data(), L.expr_constraint.size() * sizeof(uint32_t));
-        std::memcpy(host.data() + o_off, L.con_off.data(), L.con_off.size() * sizeof(uint32_t));
-        CU(cudaMalloc(&d->d_tables, host.size()));
-        CU(cudaMalloc(&d->d_tmpl_vars, sizeof(double) * std::max<uint32_t>(L.n_vars, 1)));
-        CU(cudaMalloc(&d->d_tmpl_param, sizeof(double) * std::max<uint32_t>(b.n_expr, 1)));
-        CU(cudaMemcpyAsync(d->d_tables, host.data(), host.size(), cudaMemcpyHostToDevice, d->stream));
-        CU(cudaStreamSynchronize(d->stream));  // (host leaves scope)
-        unsigned char* p = (unsigned char*)d->d_tables;
-        d->d_kind = p + o_kind;
-        d->d_slot = (const uint32_t*)(p + o_slot);
-        d->d_expr_con = (const uint32_t*)(p + o_con);
-        d->d_con_off = (const uint32_t*)(p + o_off);
+        TablePack pk;
+        const size_t o_kind = pk.add(L.kind), o_slot = pk.add(L.slot_var), o_con = pk.add(L.expr_constraint), o_off = pk.add(L.con_off);
+        const int rc = d->upload_tables(device, pk, L.n_vars, ne);
+        if (rc != FK_OK) return rc;
+        d->d_kind = pk.at<uint8_t>(o_kind);
+        d->d_slot = pk.at<uint32_t>(o_slot);
+        d->d_expr_con = pk.at<uint32_t>(o_con);
+        d->d_con_off = pk.at<uint32_t>(o_off);
         d->ready = true;
     }
-    auto alloc = [&](auto** ptr, size_t count) -> int {
-        cudaFree(*ptr);
-        *ptr = nullptr;
-        CU(cudaMalloc((void**)ptr, sizeof(**ptr) * std::max<size_t>(count, 1)));
-        return FK_OK;
-    };
+    // per variant: the raw parameters, vt and pt, and the operation's outputs
+    const uint64_t bytes = sizeof(double) * ((uint64_t)L.n_vars + ncon + ne) + (analyze ? (uint64_t)ne + ncon : sizeof(double) * ncon);
+    *chunk = system_batch_chunk(n, bytes, 1, std::max({L.n_vars, ncon, ne}));
+    const uint32_t cap = *chunk;
     int rc = FK_OK;
-    if (d->chunk < chunk) {
+    if (d->chunk < cap) {
         d->chunk = 0;
-        if ((rc = alloc(&d->d_raw_param, (size_t)chunk * b.n_constraints)) != FK_OK || (rc = alloc(&d->d_vt, (size_t)chunk * L.n_vars)) != FK_OK ||
-            (rc = alloc(&d->d_pt, (size_t)chunk * b.n_expr)) != FK_OK)
+        if ((rc = d->grow(&d->d_raw_param, (size_t)cap * ncon)) != FK_OK || (rc = d->grow(&d->d_vt, (size_t)cap * L.n_vars)) != FK_OK ||
+            (rc = d->grow(&d->d_pt, (size_t)cap * ne)) != FK_OK)
             return rc;
-        d->chunk = chunk;
+        d->chunk = cap;
     }
-    if (analyze && d->an_chunk < chunk) {
+    if (analyze && d->an_chunk < cap) {
         d->an_chunk = 0;
-        if ((rc = alloc(&d->d_indep, (size_t)chunk * b.n_expr)) != FK_OK || (rc = alloc(&d->d_dep, (size_t)chunk * b.n_constraints)) != FK_OK)
-            return rc;
-        d->an_chunk = chunk;
+        if ((rc = d->grow(&d->d_indep, (size_t)cap * ne)) != FK_OK || (rc = d->grow(&d->d_dep, (size_t)cap * ncon)) != FK_OK) return rc;
+        d->an_chunk = cap;
     }
-    if (!analyze && d->res_chunk < chunk) {
+    if (!analyze && d->res_chunk < cap) {
         d->res_chunk = 0;
-        if ((rc = alloc(&d->d_res, (size_t)chunk * b.n_constraints)) != FK_OK) return rc;
-        d->res_chunk = chunk;
+        if ((rc = d->grow(&d->d_res, (size_t)cap * ncon)) != FK_OK) return rc;
+        d->res_chunk = cap;
     }
     return FK_OK;
 }
 
-// Variants [lo, hi) on one device, chunk after chunk on its stream: upload (or broadcast the template), expand the parameters,
-// then analyze + reduce or the residuals, download.
+// Variants [lo, hi) on one device, per chunk: upload (or broadcast the template), expand the parameters, then analyze + reduce or
+// the residuals, download.
 static int system_an_range(SystemAnBatch& b, const SystemAnCall& c, int device, uint32_t lo, uint32_t hi) {
     const SystemAnLayout& L = b.L;
     const uint32_t ne = b.n_expr, ncon = b.n_constraints;
     const bool analyze = c.dependent != nullptr;
-    const uint64_t per_variant = sizeof(double) * ((uint64_t)L.n_vars + ncon + ne) + (analyze ? (uint64_t)ne + ncon : sizeof(double) * ncon);
-    const uint32_t env = system_batch_chunk_env();
-    const uint32_t chunk = (uint32_t)std::min<uint64_t>(env ? env : std::max<uint64_t>(1, (1ull << 30) / per_variant), hi - lo);
-    SystemAnDevice* d;
-    {
-        std::lock_guard<std::mutex> lock(b.mu);
-        auto& p = b.devices[device];
-        if (!p) p.reset(new SystemAnDevice());
-        d = p.get();
-    }
+    SystemAnDevice* d = device_slot(b.mu, b.devices, device);
     std::lock_guard<std::mutex> lock(d->mu);
-    int rc = system_an_device(b, d, device, chunk, analyze);
+    uint32_t chunk = 0;
+    const int rc = system_an_device(b, d, device, hi - lo, analyze, &chunk);
     if (rc != FK_OK) return rc;
-    cudaStream_t st = d->stream;
-    auto run = [&]() -> int {
-        CU(cudaMemcpyAsync(d->d_tmpl_vars, c.tmpl_vars, sizeof(double) * L.n_vars, cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(d->d_tmpl_param, c.tmpl_param, sizeof(double) * ne, cudaMemcpyHostToDevice, st));
-        for (uint32_t at = lo; at < hi; at += chunk) {
-            const uint32_t cnt = std::min(chunk, hi - at);
-            if (c.vars)
-                CU(cudaMemcpyAsync(d->d_vt, c.vars + (size_t)at * L.n_vars, sizeof(double) * (size_t)cnt * L.n_vars, cudaMemcpyHostToDevice, st));
-            if (c.params)
-                CU(cudaMemcpyAsync(d->d_raw_param, c.params + (size_t)at * ncon, sizeof(double) * (size_t)cnt * ncon, cudaMemcpyHostToDevice, st));
-            int e = launch_system_an_expand(cnt, L.n_vars, ne, ncon, c.vars ? nullptr : d->d_tmpl_vars, d->d_vt, d->d_expr_con,
-                                            c.params ? d->d_raw_param : nullptr, d->d_tmpl_param, d->d_pt, st);
-            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_an_expand_kernel");
-            if (!analyze) {
-                e = launch_system_residuals(cnt, L.n_vars, ne, ncon, d->d_kind, d->d_slot, d->d_con_off, d->d_vt, d->d_pt, d->d_res, st);
-                if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_residuals_kernel");
-                CU(cudaMemcpyAsync(c.residuals + (size_t)at * ncon, d->d_res, sizeof(double) * (size_t)cnt * ncon, cudaMemcpyDeviceToHost, st));
-                continue;
-            }
-            AnalyzePlan plan;  // the kernel for this chunk's size
-            std::string err;
-            const int prc = choose_analyze(L.n_vars, ne, cnt, device, &plan, &err);
-            if (prc != FK_OK) return fail(prc, err);
-            if (d->ws_bytes < plan.workspace_bytes()) {  // grow-only, within fk::kAnWorkspaceBytes
-                CU(cudaStreamSynchronize(st));  // (an earlier chunk's launch may still use the old workspace)
-                cudaFree(d->d_ws);
-                d->d_ws = nullptr;
-                d->ws_bytes = 0;
-                CU(cudaMalloc(&d->d_ws, plan.workspace_bytes()));
-                d->ws_bytes = plan.workspace_bytes();
-            }
-            e = plan.kernel == kAnWarp ? launch_batch_analyze(L.n_vars, ne, d->d_kind, d->d_slot, cnt, d->d_vt, d->d_pt, d->d_indep, st)
-                                       : launch_analyze(plan, L.n_vars, ne, d->d_kind, d->d_slot, cnt, d->d_vt, d->d_pt, d->d_indep, d->d_ws, st);
-            if (e != 0) return cuda_fail((cudaError_t)e, plan.kernel == kAnWarp ? "launch fk_batch_analyze_kernel" : "launch fk_analyze_cta_kernel");
-            e = launch_system_an_reduce(cnt, ne, ncon, d->d_indep, d->d_con_off, d->d_dep, st);
-            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_an_reduce_kernel");
-            CU(cudaMemcpyAsync(c.dependent + (size_t)at * ncon, d->d_dep, (size_t)cnt * ncon, cudaMemcpyDeviceToHost, st));
+    const cudaStream_t st = d->stream;
+    return run_chunks(d, L.n_vars, ne, c.tmpl_vars, c.tmpl_param, lo, hi, chunk, "fk_system_batch_analyze / _residuals kernels / copies",
+                      [&](uint32_t at, uint32_t cnt) -> int {
+        if (c.vars)
+            CU(cudaMemcpyAsync(d->d_vt, c.vars + (size_t)at * L.n_vars, sizeof(double) * (size_t)cnt * L.n_vars, cudaMemcpyHostToDevice, st));
+        if (c.params)
+            CU(cudaMemcpyAsync(d->d_raw_param, c.params + (size_t)at * ncon, sizeof(double) * (size_t)cnt * ncon, cudaMemcpyHostToDevice, st));
+        int e = launch_system_an_expand(cnt, L.n_vars, ne, ncon, c.vars ? nullptr : d->d_tmpl_vars, d->d_vt, d->d_expr_con,
+                                        c.params ? d->d_raw_param : nullptr, d->d_tmpl_param, d->d_pt, st);
+        if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_an_expand_kernel");
+        if (!analyze) {
+            e = launch_system_residuals(cnt, L.n_vars, ne, ncon, d->d_kind, d->d_slot, d->d_con_off, d->d_vt, d->d_pt, d->d_res, st);
+            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_residuals_kernel");
+            CU(cudaMemcpyAsync(c.residuals + (size_t)at * ncon, d->d_res, sizeof(double) * (size_t)cnt * ncon, cudaMemcpyDeviceToHost, st));
+            return FK_OK;
         }
+        AnalyzePlan plan;  // the kernel for this chunk's size
+        std::string err;
+        const int prc = choose_analyze(L.n_vars, ne, cnt, device, &plan, &err);
+        if (prc != FK_OK) return fail(prc, err);
+        if (d->ws_bytes < plan.workspace_bytes()) {  // grow-only, within fk::kAnWorkspaceBytes
+            CU(cudaStreamSynchronize(st));  // (an earlier chunk's launch may still use the old workspace)
+            d->ws_bytes = 0;
+            const int grc = d->grow(&d->d_ws, plan.workspace_bytes() / sizeof(double));
+            if (grc != FK_OK) return grc;
+            d->ws_bytes = plan.workspace_bytes();
+        }
+        e = plan.kernel == kAnWarp ? launch_batch_analyze(L.n_vars, ne, d->d_kind, d->d_slot, cnt, d->d_vt, d->d_pt, d->d_indep, st)
+                                   : launch_analyze(plan, L.n_vars, ne, d->d_kind, d->d_slot, cnt, d->d_vt, d->d_pt, d->d_indep, d->d_ws, st);
+        if (e != 0) return cuda_fail((cudaError_t)e, plan.kernel == kAnWarp ? "launch fk_batch_analyze_kernel" : "launch fk_analyze_cta_kernel");
+        e = launch_system_an_reduce(cnt, ne, ncon, d->d_indep, d->d_con_off, d->d_dep, st);
+        if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_an_reduce_kernel");
+        CU(cudaMemcpyAsync(c.dependent + (size_t)at * ncon, d->d_dep, (size_t)cnt * ncon, cudaMemcpyDeviceToHost, st));
         return FK_OK;
-    };
-    rc = run();
-    // (also after an error: no copy into the caller's buffers may still be running when the call returns)
-    const cudaError_t e = cudaStreamSynchronize(st);
-    if (rc == FK_OK && e != cudaSuccess) rc = cuda_fail(e, "fk_system_batch_analyze / _residuals kernels / copies");
-    return rc;
+    });
 }
 
 int system_an_batch_run(SystemAnBatch& b, const SystemAnCall& c) {
@@ -2642,17 +2547,15 @@ int system_an_batch_run(SystemAnBatch& b, const SystemAnCall& c) {
     int n_gpus = c.n_gpus;
     int rc = clamp_gpus(n_gpus);
     if (rc != FK_OK) return rc;
-    int cur = 0;
-    if (cudaGetDevice(&cur) != cudaSuccess) cur = 0;
-    if (c.dependent) {  // the size limit of the analyze kernels (it does not depend on the batch size)
+    if (c.dependent) {  // the size limit of the analyze kernels (it depends on neither the batch size nor the device: the current one)
+        int device = 0;
+        if (cudaGetDevice(&device) != cudaSuccess) device = 0;
         AnalyzePlan plan;
         std::string err;
-        rc = choose_analyze(b.L.n_vars, b.n_expr, c.n, cur, &plan, &err);
+        rc = choose_analyze(b.L.n_vars, b.n_expr, c.n, device, &plan, &err);
         if (rc != FK_OK) return fail(rc, err);
     }
-    const int r = shard_over_devices(n_gpus, c.n, [&](int device, uint32_t lo, uint32_t hi) { return system_an_range(b, c, device, lo, hi); });
-    if (cudaSetDevice(cur) != cudaSuccess) cudaGetLastError();
-    return r;
+    return shard_over_devices(n_gpus, c.n, [&](int device, uint32_t lo, uint32_t hi) { return system_an_range(b, c, device, lo, hi); });
 }
 
 }  // namespace fk

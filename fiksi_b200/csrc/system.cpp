@@ -878,30 +878,44 @@ int fk_system_component(const fk_system* s, uint32_t ci, uint32_t* n_elements, u
 // ---- System::solve over n variants of one drawing ------------------------------------------------------------------
 namespace {
 
+// The parts of a batch plan that do not depend on the decomposer: the expressions and, per variable, no draw or wave yet.
+fk::SystemBatchLayout batch_layout(const fk_system* s) {
+    fk::SystemBatchLayout lay;
+    lay.n_vars = (uint32_t)s->vars.size();
+    lay.n_constraints = (uint32_t)s->constrs.size();
+    lay.kind = s->kind;
+    lay.expr_constraint.assign(s->kind.size(), fk::kSbNone);
+    for (uint32_t c = 0; c < s->constrs.size(); c++) lay.expr_constraint[s->constrs[c].first_expr] = c;  // update_parameter
+    lay.var_draw.assign(s->vars.size(), fk::kSbNone);
+    lay.var_wave.assign(s->vars.size(), fk::kSbNone);
+    return lay;
+}
+
+// A component's draws from the solve's generator: two per free variable, in the ascending free set; var_draw their pair.
+int component_draws(fk::SystemBatchLayout& lay, Lcg& rng, const std::vector<uint32_t>& free_sorted) {
+    for (uint32_t fv : free_sorted) {
+        if (lay.var_draw[fv] != fk::kSbNone) return fk::system_batch_fail(FK_ERR_INTERNAL, "a variable is free in two components");
+        lay.var_draw[fv] = (uint32_t)(lay.draws.size() / 2);
+        lay.draws.push_back(rng.next());
+        lay.draws.push_back(rng.next());
+    }
+    return FK_OK;
+}
+
 // The drawing's batch plan: per non-empty component (component order) its LocalProblem numbering, the draws of the solve's
 // generator and, per local variable, the draw already applied at the component's snapshot -- prepare_components perturbs
 // component by component, so a variable of a later component is read unperturbed and one of an earlier component perturbed.
 int batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemBatch>* out) {
     std::lock_guard<std::mutex> lock(s->batch_mu);
     if (!s->batch) {
-        fk::SystemBatchLayout lay;
-        lay.n_vars = (uint32_t)s->vars.size();
-        lay.n_constraints = (uint32_t)s->constrs.size();
-        lay.kind = s->kind;
-        lay.expr_constraint.assign(s->kind.size(), fk::kSbNone);
-        for (uint32_t c = 0; c < s->constrs.size(); c++) lay.expr_constraint[s->constrs[c].first_expr] = c;  // update_parameter
-        std::vector<uint32_t> var_draw(s->vars.size(), fk::kSbNone);
+        fk::SystemBatchLayout lay = batch_layout(s);
         std::vector<std::unique_ptr<LocalProblem>> locals;
         Lcg rng{42};
         for (const fk_system::Comp& c : s->comps) {
             if (c.elements.empty()) continue;  // assemble/mod.rs:87-89
             const std::vector<uint32_t> free_sorted = component_free_variables(s, c);
-            for (uint32_t fv : free_sorted) {
-                if (var_draw[fv] != fk::kSbNone) return fk::system_batch_fail(FK_ERR_INTERNAL, "a variable is free in two components");
-                var_draw[fv] = (uint32_t)(lay.draws.size() / 2);
-                lay.draws.push_back(rng.next());
-                lay.draws.push_back(rng.next());
-            }
+            const int rc = component_draws(lay, rng, free_sorted);
+            if (rc != FK_OK) return rc;
             std::vector<uint32_t> exprs;
             for (uint32_t ci : c.constraints)
                 for (uint8_t k = 0; k < s->constrs[ci].n_expr; k++) exprs.push_back(s->constrs[ci].first_expr + k);
@@ -909,7 +923,7 @@ int batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemBatch>* out) {
             build_local(s, s->vars, s->param, free_sorted, exprs, *L);
             fk::SystemBatchLayout::Component comp;
             comp.slot_var = L->slot_global;
-            for (uint32_t g : L->slot_global) comp.slot_draw.push_back(var_draw[g]);
+            for (uint32_t g : L->slot_global) comp.slot_draw.push_back(lay.var_draw[g]);
             comp.expr = exprs;
             comp.free_var = free_sorted;
             lay.comps.push_back(std::move(comp));
@@ -958,30 +972,11 @@ struct WaveScheduler {
     }
 };
 
-// The parts of a wave plan that do not depend on the decomposer: the expressions and, per variable, no draw yet.
-fk::SystemBatchLayout wave_layout(const fk_system* s) {
-    fk::SystemBatchLayout lay;
-    lay.n_vars = (uint32_t)s->vars.size();
-    lay.n_constraints = (uint32_t)s->constrs.size();
-    lay.kind = s->kind;
-    lay.expr_constraint.assign(s->kind.size(), fk::kSbNone);
-    for (uint32_t c = 0; c < s->constrs.size(); c++) lay.expr_constraint[s->constrs[c].first_expr] = c;  // update_parameter
-    lay.var_draw.assign(s->vars.size(), fk::kSbNone);
-    lay.var_wave.assign(s->vars.size(), fk::kSbNone);
-    return lay;
-}
-
-// A component's perturbation node: its wave, and the draws of batch_plan_for for its free variables.
+// A component's perturbation node: its wave, and the component's draws.
 int perturbation_node(fk::SystemBatchLayout& lay, WaveScheduler& sched, Lcg& rng, const std::vector<uint32_t>& free_sorted) {
     const uint32_t pw = sched.perturbation(free_sorted);
-    for (uint32_t fv : free_sorted) {
-        if (lay.var_draw[fv] != fk::kSbNone) return fk::system_batch_fail(FK_ERR_INTERNAL, "a variable is free in two components");
-        lay.var_draw[fv] = (uint32_t)(lay.draws.size() / 2);
-        lay.var_wave[fv] = pw;
-        lay.draws.push_back(rng.next());
-        lay.draws.push_back(rng.next());
-    }
-    return FK_OK;
+    for (uint32_t fv : free_sorted) lay.var_wave[fv] = pw;
+    return component_draws(lay, rng, free_sorted);
 }
 
 // fk_system_batch_solve_single_pass's plan: the sets of fk_system_solve_opts(decomposer = 1) in its order, each as its
@@ -991,7 +986,7 @@ int perturbation_node(fk::SystemBatchLayout& lay, WaveScheduler& sched, Lcg& rng
 int single_pass_batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemSpBatch>* out) {
     std::lock_guard<std::mutex> lock(s->batch_mu);
     if (!s->sp_batch) {
-        fk::SystemBatchLayout lay = wave_layout(s);
+        fk::SystemBatchLayout lay = batch_layout(s);
         WaveScheduler sched(s->vars.size());
         std::vector<std::vector<uint32_t>> var_exprs, expr_vars;
         equation_graph(s, var_exprs, expr_vars);
@@ -1033,7 +1028,7 @@ int single_pass_batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemSpB
 int recursive_assembly_batch_plan_for(const fk_system* s, std::shared_ptr<fk::SystemSpBatch>* out) {
     std::lock_guard<std::mutex> lock(s->batch_mu);
     if (!s->ra_batch) {
-        fk::SystemBatchLayout lay = wave_layout(s);
+        fk::SystemBatchLayout lay = batch_layout(s);
         WaveScheduler sched(s->vars.size());
         std::vector<std::unique_ptr<ClusteredProblem>> problems;
         Lcg rng{42};
@@ -1090,6 +1085,12 @@ int recursive_assembly_batch_plan_for(const fk_system* s, std::shared_ptr<fk::Sy
     return FK_OK;
 }
 
+// A solve batch call on s's template rows.
+fk::SystemBatchCall batch_call(const fk_system* s, int optimizer, int perturb, uint32_t n, const double* vars, const double* params,
+                               double* vars_out, fk_report* reports, uint32_t reports_per_variant, int n_gpus) {
+    return {optimizer, perturb, n_gpus, n, vars, params, s->vars.data(), s->param.data(), vars_out, reports, reports_per_variant};
+}
+
 // The host probe and the call of the two wave plans (SinglePass, RecursiveAssembly), given how to build the plan.
 using WavePlanFor = int (*)(const fk_system*, std::shared_ptr<fk::SystemSpBatch>*);
 
@@ -1116,18 +1117,7 @@ int wave_batch_solve(WavePlanFor plan_for, const fk_system* s, int perturb, uint
     uint32_t n_steps = 0;
     fk::system_sp_batch_layout(*b, &n_steps, nullptr, nullptr, nullptr, nullptr);
     if (n_solved) *n_solved = n_steps;
-    fk::SystemBatchCall c;
-    c.perturb = perturb;
-    c.n_gpus = n_gpus;
-    c.n = n;
-    c.vars = vars;
-    c.params = params;
-    c.tmpl_vars = s->vars.data();
-    c.tmpl_param = s->param.data();
-    c.vars_out = vars_out;
-    c.reports = reports;
-    c.reports_per_variant = reports_per_variant;
-    return fk::system_sp_batch_solve(*b, c);
+    return fk::system_sp_batch_solve(*b, batch_call(s, 0, perturb, n, vars, params, vars_out, reports, reports_per_variant, n_gpus));
 }
 
 // fk_system_batch_analyze / _residuals' plan: the expressions with their slot tables and the constraints' expression ranges.
@@ -1206,19 +1196,8 @@ int fk_system_batch_solve(const fk_system* s, const fk_solving_options* opts, ui
     uint32_t nc = 0;
     fk::system_batch_layout(*b, &nc, nullptr, nullptr);
     if (n_solved) *n_solved = nc;
-    fk::SystemBatchCall c;
-    c.optimizer = (int)opts->optimizer;
-    c.perturb = (int)opts->perturb;
-    c.n_gpus = n_gpus;
-    c.n = n;
-    c.vars = vars;
-    c.params = params;
-    c.tmpl_vars = s->vars.data();
-    c.tmpl_param = s->param.data();
-    c.vars_out = vars_out;
-    c.reports = reports;
-    c.reports_per_variant = reports_per_variant;
-    return fk::system_batch_solve(*b, c);
+    return fk::system_batch_solve(*b, batch_call(s, (int)opts->optimizer, (int)opts->perturb, n, vars, params, vars_out, reports,
+                                                 reports_per_variant, n_gpus));
 }
 
 int fk_system_single_pass_batch_layout(const fk_system* s, uint32_t* n_steps, uint32_t* n_waves, uint32_t* n_structures,

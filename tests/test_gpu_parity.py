@@ -9,6 +9,7 @@ kernels are bit-exact for every kind that has no atan2 and within 4 ulp of pi ot
 import numpy as np
 import pytest
 
+import cad_drawings as cd
 import scenarios as sc
 import fiksi_b200 as fk
 from fiksi_b200 import workloads as wl
@@ -75,7 +76,12 @@ def test_uniform_batch_matches_oracle(oracle, maker, n):
 
 
 def test_eval_kernels_bit_exact_where_possible(oracle):
-    for maker in (wl.truss, wl.cad_mix):
+    """K1 / K2 of paths 0 and 1 against oracle.evaluate.  The CAD drawings bring every kind, fixed variables and, with
+    shared vertices, rows that name a free variable twice (K1's scatter sums those slots); the last one is on path 1."""
+    cad = [lambda n: cd.workload(*cd.PATH0, n, seed=1, shared_vertices=True),
+           lambda n: cd.workload(*cd.PATH0, n, seed=1, shared_vertices=False),
+           lambda n: cd.workload(*cd.PATH1_MID, n, seed=1, shared_vertices=True)]
+    for maker in [wl.truss, wl.cad_mix] + cad:
         w = maker(500)  # ragged last tile of the tile-staged kernel (S = 32 / 128)
         v, p, scale = w.prepare()
         topo = fk.Topology.from_arrays(w.n_vars, w.kind, w.idx, w.free_vars, w.rows)

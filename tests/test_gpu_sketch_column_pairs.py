@@ -6,6 +6,7 @@ in the solo kernel and in the warp-pair kernel alike, including rejected steps, 
 import numpy as np
 import pytest
 
+import cad_drawings as cd
 import fiksi_b200 as fk
 from fiksi_b200 import api, workloads as wl
 
@@ -15,6 +16,7 @@ TOPOLOGIES = {
     "truss10": lambda n: wl.truss(n, n_points=10),
     "cad_mix": lambda n: wl.cad_mix(n),
     "hinged4": lambda n: wl.hinged_triangles(4, n),
+    "cad4x4": lambda n: cd.workload(*cd.PATH0, n, seed=1, shared_vertices=False),  # every kind, fixed points
 }
 FIELDS = ("exit_reason", "outer_iters", "factorizations", "accepted", "trace_hash", "lambda", "ssr")
 

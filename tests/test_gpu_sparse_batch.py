@@ -7,6 +7,7 @@ import os
 import numpy as np
 import pytest
 
+import cad_drawings as cd
 import scenarios as sc
 import fiksi_b200 as fk
 from fiksi_b200 import workloads as wl
@@ -86,9 +87,12 @@ def test_small_lattices_forced_batched(oracle, force_sparse, nx, ny):
 
 
 # ---- 2. parity with the single-system path at natural size ---------------------------------------------------
-@pytest.mark.parametrize("shape,n", [((30, 20), 64), ((32, 32), 16), ((64, 50), 8), ("truss", 32)])
+@pytest.mark.parametrize("shape,n", [((30, 20), 64), ((32, 32), 16), ((64, 50), 8), ("truss", 32), ("cad", 6)])
 def test_natural_size_matches_single_system_path(oracle, shape, n):
-    w = wl.truss(n, 1000) if shape == "truss" else wl.lattice(*shape, n_sketches=n)
+    if shape == "cad":  # every kind, fixed points, rows that name a variable twice, far-apart length equalities
+        w = cd.workload(*cd.PATH2_NATURAL, n, seed=1)
+    else:
+        w = wl.truss(n, 1000) if shape == "truss" else wl.lattice(*shape, n_sketches=n)
     v, p, _ = w.prepare()
     topo = _topo(w)
     xb, rb = topo.batch_solve(v, p)

@@ -10,6 +10,7 @@ import zlib
 import numpy as np
 import pytest
 
+import cad_drawings as cd
 import scenarios as sc
 import fiksi_b200 as fk
 from fiksi_b200 import workloads as wl
@@ -99,6 +100,16 @@ def _grouping_drawing():
         sc.single_triangle(lambda: s)
     sc.circle_triangle_line(lambda: s)
     _add_ppd(s, wl.truss(1, 20))
+    return s
+
+
+def _cad_drawing(S):
+    """Three components: a mixed-kind CAD grid on the one-CTA-per-sketch path (path 1), a smaller one with shared vertices
+    on the tile path and a single triangle."""
+    s = S()
+    cd.cad_grid(lambda: s, *cd.PATH1_LOW, seed=3)
+    cd.cad_grid(lambda: s, *cd.PATH0, seed=4)
+    sc.single_triangle(lambda: s)
     return s
 
 
@@ -225,6 +236,40 @@ def test_lattice_component_on_the_sparse_batch_kernel():
     ref_out, ref_reps = _loop(s, vars_, params, "lbfgs")
     assert np.array_equal(out, ref_out)
     _same_reports(reps, ref_reps)
+
+
+def test_cad_drawing_components_take_paths_1_and_0(oracle):
+    paths = [fk.Topology.from_arrays(len(k[0]), k[1], k[2], k[4], k[5]).info["path"]
+             for _, _, k in _cad_drawing(oracle.System).prepare(perturb=False)]
+    assert sorted(paths) == [0, 0, 1]
+    assert _cad_drawing(RecSystem).batch_layout() == (3, 3, [1, 1, 1])
+
+
+@pytest.mark.gpu
+def test_cad_drawing_with_a_path1_component(oracle):
+    """Mixed kinds, fixed points and duplicated slots in every batched component kernel the system batch has for small
+    systems: 64 variants equal the per-variant solve bit for bit, three of them the oracle's System.solve."""
+    s = _cad_drawing(RecSystem)
+    vars_, params = _variants(s, 64, seed=17)
+    out, reps = s.batch_solve(vars_, params)
+    ref_out, ref_reps = _loop(s, vars_, params)
+    assert np.array_equal(out, ref_out, equal_nan=True)
+    _same_reports(reps, ref_reps)
+    for k in (0, 10, 40):
+        so = _cad_drawing(oracle.System)
+        for i, x in enumerate(vars_[k]):
+            so.set_variable(i, float(x))
+        for c, x in enumerate(params[k]):
+            so.set_parameter(c, float(x))
+        so.solve()
+        ro = so.reports()
+        assert len(ro) == reps.shape[1] == 3
+        for a, b in zip(ro, reps[k]):
+            for f in ("exit_reason", "trace_hash", "outer_iters", "factorizations", "accepted", "lambda"):
+                assert a[f] == b[f], (k, f, a, b)
+            assert abs(a["ssr"] - b["ssr"]) <= 1e-9 * max(a["ssr"], 1.0)
+        vo = so.variables
+        assert np.max(np.abs(vo - out[k])) <= 1e-9 * np.max(np.abs(vo))
 
 
 _CHUNK_SCRIPT = """

@@ -6,4 +6,4 @@ ctypes face used by the tests and the benchmark.
 from ._lib import FiksiError, FkProblem, FkReport, REPORT_DTYPE, LIB_PATH, lib, make_problem  # noqa: F401
 from .api import (BatchPlan, Topology, device_count, fp64_peak_tflops, lbfgs_solve, lbfgs_solve_batch, lm_solve,  # noqa: F401
                   lm_solve_batch)
-from .system import System  # noqa: F401
+from .system import System, solve_systems, systems_layout  # noqa: F401

@@ -1559,7 +1559,37 @@ static HeteroPool* hetero_pool_for(int device) {
     return p;
 }
 
-// Solves jobs (group index, member) of small path-0 groups with ONE launch of fk_hetero_lm_kernel on `device`.
+// Whether a structure of `instances` systems goes to fk_hetero_lm_kernel (one warp per system) rather than a uniform batch
+// launch: path 0, fewer than 64 systems (from there the sketch-per-thread kernel is the faster one) and an LM state within
+// 48 KiB.  The caller also needs the topology's 32-lane tables (fk_topology::lanes32).
+static bool hetero_fits(const fk::Topology& t, size_t instances) {
+    return t.path == 0 && instances < 64 && fk::lm_smem_doubles(t.n_free, t.n_rows, t.jac_nnz, (uint32_t)t.l_rowidx.size()) * 8 <= 48 * 1024;
+}
+
+// The programs of fk_hetero_lm_kernel on `device` (32-lane tables, no sketch-kernel block) and the largest LM state among them.
+static int hetero_programs(int device, const std::vector<fk_topology*>& topos32, std::vector<fk::DevProgram>& progs, uint32_t* max_state) {
+    progs.assign(topos32.size(), fk::DevProgram{});
+    *max_state = 1;
+    for (size_t g = 0; g < topos32.size(); g++) {
+        const fk::DevProgram* v = nullptr;
+        const int rc = topos32[g]->program_for(device, &v);
+        if (rc != FK_OK) return rc;
+        progs[g] = *v;
+        progs[g].sketch_prog = nullptr;
+        *max_state = std::max(*max_state, fk::lm_smem_doubles(v->n, v->m, v->jnnz, v->lnnz));
+    }
+    return FK_OK;
+}
+
+// One launch of fk_hetero_lm_kernel over device-resident programs, jobs and input rows.
+static int hetero_launch(const fk::DevProgram* d_progs, const fk::HeteroJob* d_jobs, size_t nj, uint32_t max_state, const double* d_in,
+                         double* d_out, fk_report* d_rep, cudaStream_t st) {
+    const int e = fk::launch_hetero_lm(d_progs, d_jobs, (uint32_t)nj, max_state, d_in, d_out, d_rep, st);
+    return e != 0 ? cuda_fail((cudaError_t)e, "launch fk_hetero_lm_kernel") : FK_OK;
+}
+
+// Solves jobs (group index, member) of small path-0 groups with ONE launch of fk_hetero_lm_kernel on `device`: the programs,
+// jobs and input rows staged in a pinned block, one copy up, the launch, one copy down.
 struct HeteroItem { uint32_t group, problem; };
 static int hetero_solve(int device, const std::vector<fk_topology*>& topos32, const std::vector<HeteroItem>& items,
                         const fk_problem* const* problems, double* const* free_values, fk_report* reports) {
@@ -1567,16 +1597,9 @@ static int hetero_solve(int device, const std::vector<fk_topology*>& topos32, co
     std::lock_guard<std::mutex> lock(pool->mu);
     CU(cudaSetDevice(device));
     const size_t ng = topos32.size(), nj = items.size();
-    std::vector<fk::DevProgram> progs(ng);
+    std::vector<fk::DevProgram> progs;
     uint32_t max_state = 1;
-    for (size_t g = 0; g < ng; g++) {
-        const fk::DevProgram* v = nullptr;
-        int rc = topos32[g]->program_for(device, &v);
-        if (rc != FK_OK) return rc;
-        progs[g] = *v;
-        progs[g].sketch_prog = nullptr;
-        max_state = std::max(max_state, fk::lm_smem_doubles(v->n, v->m, v->jnnz, v->lnnz));
-    }
+    if (const int rc = hetero_programs(device, topos32, progs, &max_state); rc != FK_OK) return rc;
     // layout of the staging block: [programs][jobs][inputs: vars row + param row per job] | [outputs][reports]
     auto align = [](size_t x) { return (x + 255) & ~size_t(255); };
     std::vector<fk::HeteroJob> jobs(nj);
@@ -1618,10 +1641,10 @@ static int hetero_solve(int device, const std::vector<fk_topology*>& topos32, co
         }
     }
     CU(cudaMemcpyAsync(pool->d, pool->h, o_out, cudaMemcpyHostToDevice, pool->stream));
-    const int e = fk::launch_hetero_lm(reinterpret_cast<const fk::DevProgram*>(pool->d + o_progs), reinterpret_cast<const fk::HeteroJob*>(pool->d + o_jobs),
-                                       (uint32_t)nj, max_state, reinterpret_cast<const double*>(pool->d + o_in), reinterpret_cast<double*>(pool->d + o_out),
-                                       reinterpret_cast<fk_report*>(pool->d + o_rep), pool->stream);
-    if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_hetero_lm_kernel");
+    const int rc = hetero_launch(reinterpret_cast<const fk::DevProgram*>(pool->d + o_progs), reinterpret_cast<const fk::HeteroJob*>(pool->d + o_jobs),
+                                 nj, max_state, reinterpret_cast<const double*>(pool->d + o_in), reinterpret_cast<double*>(pool->d + o_out),
+                                 reinterpret_cast<fk_report*>(pool->d + o_rep), pool->stream);
+    if (rc != FK_OK) return rc;
     CU(cudaMemcpyAsync(pool->h + o_out, pool->d + o_out, total - o_out, cudaMemcpyDeviceToHost, pool->stream));
     CU(cudaStreamSynchronize(pool->stream));
     const double* out = reinterpret_cast<const double*>(pool->h + o_out);
@@ -1748,9 +1771,7 @@ int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems, double* con
         static const bool no_hetero = std::getenv("FK_NO_HETERO") != nullptr;
         std::vector<size_t> small;
         for (size_t g = 0; g < groups.size(); g++) {
-            const fk::Topology& t = groups[g].topo->t;
-            if (t.path == 0 && groups[g].members.size() < 64 && fk::lm_smem_doubles(t.n_free, t.n_rows, t.jac_nnz, (uint32_t)t.l_rowidx.size()) * 8 <= 48 * 1024)
-                small.push_back(g);
+            if (hetero_fits(groups[g].topo->t, groups[g].members.size())) small.push_back(g);
         }
         if (!no_hetero && small.size() >= 2) {
             std::vector<fk_topology*> topos32;
@@ -1859,12 +1880,16 @@ static int group_by_structure(const std::vector<const fk_problem*>& problems, st
 // Variants per chunk of n: FK_SYSTEM_BATCH_CHUNK=n (test knob), else the chunk's buffers (`bytes` per variant) within about 1 GiB
 // of device memory, at least one; then at most INT32_MAX sketches per launch (`sketches` per variant) and rows of `row` values
 // per variant within 32-bit offsets.
-static uint32_t system_batch_chunk(uint32_t n, uint64_t bytes, uint64_t sketches, uint64_t row) {
+static uint32_t system_batch_chunk_env() {  // FK_SYSTEM_BATCH_CHUNK, read once (0: not set)
     static const uint32_t env = [] {
         const char* e = std::getenv("FK_SYSTEM_BATCH_CHUNK");
         const long v = e ? std::atol(e) : 0;
         return (uint32_t)(v >= 1 && v <= (long)UINT32_MAX ? v : 0);
     }();
+    return env;
+}
+static uint32_t system_batch_chunk(uint32_t n, uint64_t bytes, uint64_t sketches, uint64_t row) {
+    const uint32_t env = system_batch_chunk_env();
     uint64_t chunk = env ? env : std::max<uint64_t>(1, (1ull << 30) / bytes);
     chunk = std::min<uint64_t>(chunk, std::max<uint64_t>(1, (uint64_t)INT32_MAX / std::max<uint64_t>(1, sketches)));
     chunk = std::min<uint64_t>(chunk, std::max<uint64_t>(1, (uint64_t)UINT32_MAX / std::max<uint64_t>(1, row)));
@@ -2556,6 +2581,433 @@ int system_an_batch_run(SystemAnBatch& b, const SystemAnCall& c) {
         if (rc != FK_OK) return fail(rc, err);
     }
     return shard_over_devices(n_gpus, c.n, [&](int device, uint32_t lo, uint32_t hi) { return system_an_range(b, c, device, lo, hi); });
+}
+
+// ---- fk_systems_solve: System::solve over n different drawings ------------------------------------------------------------
+// The call's plan: the structures of every drawing's SystemBatch merged across drawings (same structural signature and an
+// exact comparison -- not the topology pointer, which differs with the topology cache off or after an eviction), each with
+// its launch kind, and the instances (solved components) in drawing order, component order inside a drawing.  Built per call.
+struct SystemsPlan {
+    struct Structure {
+        std::shared_ptr<fk_topology> topo;
+        uint32_t kind = 1;                           // 0 heterogeneous launch, 1 uniform batch, 2 sparse batch kernel (LM, path 2)
+        uint32_t instances = 0;
+        uint32_t hetero = kSbNone;                   // kind 0: its program in the heterogeneous launch
+        uint32_t first_drawing = 0, first_comp = 0;  // where it first appears (named by refusals)
+    };
+    std::vector<Structure> st;
+    std::vector<uint32_t> inst_struct;           // per instance
+    std::vector<size_t> inst_off;                // [n + 1] first instance of each drawing
+    std::vector<size_t> var_off;                 // [n + 1] first variable of each drawing in the call's flat rows
+    std::vector<fk_topology*> topos32;           // the 32-lane topologies of the kind-0 structures
+    const std::vector<double>* draws = nullptr;  // the longest of the drawings' draws: each drawing's are a prefix (LCG seeded 42)
+};
+
+static void systems_plan_create(const std::vector<SystemsDrawing>& d, int optimizer, SystemsPlan& P) {
+    static const std::vector<double> no_draws;
+    P.draws = &no_draws;
+    P.inst_off.assign(1, 0);
+    P.var_off.assign(1, 0);
+    std::multimap<uint64_t, uint32_t> by_sig;
+    std::unordered_map<const fk_topology*, uint32_t> by_topo;  // (one topology is one structure: skips the signature)
+    for (uint32_t i = 0; i < d.size(); i++) {
+        const SystemBatch& b = *d[i].plan;
+        std::vector<uint32_t> merged(b.st.size());
+        for (uint32_t s = 0; s < b.st.size(); s++) {
+            const auto known = by_topo.find(b.st[s].topo.get());
+            if (known != by_topo.end()) {
+                merged[s] = known->second;
+                P.st[known->second].instances += b.st[s].mult;
+                continue;
+            }
+            const fk_problem p = structure_of(b.st[s].topo->t);
+            const uint64_t sig = structural_signature(p);
+            uint32_t m = kSbNone;
+            for (auto r = by_sig.equal_range(sig); r.first != r.second && m == kSbNone; ++r.first)
+                if (same_structure(structure_of(P.st[r.first->second].topo->t), p)) m = r.first->second;
+            by_topo.emplace(b.st[s].topo.get(), m == kSbNone ? (uint32_t)P.st.size() : m);
+            if (m == kSbNone) {
+                m = (uint32_t)P.st.size();
+                by_sig.emplace(sig, m);
+                SystemsPlan::Structure S;
+                S.topo = b.st[s].topo;
+                S.first_drawing = i;
+                S.first_comp = b.st[s].members[0];
+                P.st.push_back(std::move(S));
+            }
+            merged[s] = m;
+            P.st[m].instances += b.st[s].mult;
+        }
+        for (uint32_t k = 0; k < b.L.comps.size(); k++) P.inst_struct.push_back(merged[b.comp_struct[k]]);
+        P.inst_off.push_back(P.inst_struct.size());
+        P.var_off.push_back(P.var_off.back() + b.L.n_vars);
+        if (b.L.draws.size() > P.draws->size()) P.draws = &b.L.draws;
+    }
+    // fk_lm_solve_batch's rule; L-BFGS has no heterogeneous kernel, so every structure gets its own launch
+    for (SystemsPlan::Structure& S : P.st) {
+        const fk::Topology& t = S.topo->t;
+        S.kind = optimizer == 0 && t.path == 2 ? 2 : 1;
+        if (optimizer == 0 && hetero_fits(t, S.instances)) {
+            fk_topology* t32 = S.topo->lanes32();
+            if (t32->t.tile != 32) continue;  // no 32-lane tables (FK_NO_LATENCY_TWIN): a uniform batch
+            S.kind = 0;
+            S.hetero = (uint32_t)P.topos32.size();
+            P.topos32.push_back(t32);
+        }
+    }
+}
+
+void systems_layout(const std::vector<SystemsDrawing>& d, int optimizer, uint32_t* n_components, std::vector<uint32_t>* instances,
+                    std::vector<uint32_t>* launch_kind) {
+    SystemsPlan P;
+    systems_plan_create(d, optimizer, P);
+    *n_components = (uint32_t)P.inst_struct.size();
+    instances->clear();
+    launch_kind->clear();
+    for (const SystemsPlan::Structure& S : P.st) {
+        instances->push_back(S.instances);
+        launch_kind->push_back(S.kind);
+    }
+}
+
+// Per device, reused across calls (never destroyed: CUDA may be gone at static-destruction time): one stream, a grow-only
+// pinned staging block and device arena, and the grow-only workspaces of the sparse batch LM kernel and the L-BFGS CTA kernel
+// (launches on the one stream run one after the other, so one workspace serves them all).
+struct SystemsDevice {
+    std::mutex mu;
+    cudaStream_t stream = nullptr;
+    unsigned char *h = nullptr, *d = nullptr;
+    size_t h_cap = 0, d_cap = 0;
+    double *lm_ws = nullptr, *lb_ws = nullptr;
+    uint64_t lm_ws_doubles = 0, lb_ws_doubles = 0;
+};
+static SystemsDevice* systems_device_for(int device) {
+    static std::mutex m;
+    static std::map<int, SystemsDevice*> devs;
+    std::lock_guard<std::mutex> lock(m);
+    SystemsDevice*& p = devs[device];
+    if (!p) p = new SystemsDevice();
+    return p;
+}
+
+// One chunk of drawings [a, b) on one device and where its rows live in the arena: [0, o_output) the input the host stages in
+// pinned memory (same offsets) and sends with one copy, [o_output, o_work) the rows that come back with one copy, [o_work, end)
+// device only.
+struct SystemsChunk {
+    uint32_t a = 0, b = 0;
+    size_t i0 = 0, i1 = 0;       // its instances
+    std::vector<uint32_t> count;  // per structure: instances in the chunk
+    struct Rows { size_t vars = 0, params = 0, out = 0, reps = 0; };
+    std::vector<Rows> rows;       // per uniform / sparse structure present: its batch rows
+    size_t nj = 0, tab_words = 0, nvars = 0, nexpr = 0, hin = 0, hout = 0;
+    size_t o_draws = 0, o_progs = 0, o_jobs = 0, o_inst = 0, o_ioff = 0, o_voff = 0, o_eoff = 0, o_tabs = 0, o_rawv = 0, o_rawp = 0,
+           o_kinds = 0, o_output = 0, o_outv = 0, o_outr = 0, o_work = 0, o_scales = 0, o_hin = 0, o_hout = 0, o_hrep = 0, end = 0;
+};
+
+static void systems_chunk_layout(const std::vector<SystemsDrawing>& d, const SystemsPlan& P, SystemsChunk& c) {
+    const size_t ns = P.st.size(), n = c.b - c.a;
+    c.i0 = P.inst_off[c.a];
+    c.i1 = P.inst_off[c.b];
+    c.count.assign(ns, 0);
+    for (uint32_t i = c.a; i < c.b; i++) {
+        const SystemBatchLayout& L = d[i].plan->L;
+        c.nvars += L.n_vars;
+        c.nexpr += L.kind.size();
+        for (size_t g = P.inst_off[i]; g < P.inst_off[i + 1]; g++) {
+            const SystemsPlan::Structure& S = P.st[P.inst_struct[g]];
+            const fk::Topology& t = S.topo->t;
+            c.count[P.inst_struct[g]]++;
+            c.tab_words += 2 * (size_t)t.n_vars + t.n_expr + t.n_free;
+            if (S.kind == 0) {
+                c.nj++;
+                c.hin += (size_t)t.n_vars + t.n_expr;
+                c.hout += t.n_free;
+            }
+        }
+    }
+    size_t at = 0;
+    auto put = [&](size_t bytes) {
+        const size_t o = at;
+        at = (at + std::max<size_t>(bytes, 1) + 255) & ~size_t(255);
+        return o;
+    };
+    const size_t ni = c.i1 - c.i0;
+    c.o_draws = put(sizeof(double) * P.draws->size());
+    c.o_progs = put(sizeof(fk::DevProgram) * P.topos32.size());
+    c.o_jobs = put(sizeof(fk::HeteroJob) * c.nj);
+    c.o_inst = put(sizeof(SysInst) * ni);
+    c.o_ioff = put(sizeof(uint32_t) * (n + 1));
+    c.o_voff = put(sizeof(uint64_t) * (n + 1));
+    c.o_eoff = put(sizeof(uint64_t) * (n + 1));
+    c.o_tabs = put(sizeof(uint32_t) * c.tab_words);
+    c.o_rawv = put(sizeof(double) * c.nvars);
+    c.o_rawp = put(sizeof(double) * c.nexpr);
+    c.o_kinds = put(c.nexpr);
+    c.o_output = at;
+    c.o_outv = put(sizeof(double) * c.nvars);
+    c.o_outr = put(sizeof(fk_report) * ni);
+    c.o_work = at;
+    c.o_scales = put(sizeof(double) * n);
+    c.o_hin = put(sizeof(double) * c.hin);
+    c.o_hout = put(sizeof(double) * c.hout);
+    c.o_hrep = put(sizeof(fk_report) * c.nj);
+    c.rows.assign(ns, SystemsChunk::Rows{});
+    for (size_t s = 0; s < ns; s++) {
+        if (P.st[s].kind == 0 || c.count[s] == 0) continue;
+        const fk::Topology& t = P.st[s].topo->t;
+        SystemsChunk::Rows& r = c.rows[s];
+        r.vars = put(sizeof(double) * c.count[s] * t.n_vars);
+        r.params = put(sizeof(double) * c.count[s] * t.n_expr);
+        r.out = put(sizeof(double) * c.count[s] * t.n_free);
+        r.reps = put(sizeof(fk_report) * c.count[s]);
+    }
+    c.end = at;
+}
+
+// Device bytes one drawing adds to a chunk (the budget of system_batch_chunk: about 1 GiB per chunk).
+static uint64_t systems_drawing_bytes(const std::vector<SystemsDrawing>& d, const SystemsPlan& P, uint32_t i) {
+    const SystemBatchLayout& L = d[i].plan->L;
+    uint64_t bytes = sizeof(double) * (2ull * L.n_vars + L.kind.size() + 1) + L.kind.size() + 20;
+    for (size_t g = P.inst_off[i]; g < P.inst_off[i + 1]; g++) {
+        const fk::Topology& t = P.st[P.inst_struct[g]].topo->t;
+        bytes += sizeof(SysInst) + sizeof(fk::HeteroJob) + 2 * sizeof(fk_report) + sizeof(uint32_t) * (2ull * t.n_vars + t.n_expr + t.n_free) +
+                 sizeof(double) * ((uint64_t)t.n_vars + t.n_expr + t.n_free);
+    }
+    return bytes;
+}
+
+// Grow-only device buffer of at least `bytes` (the stream is idle: every call ends with a synchronise).
+template <class T>
+static int systems_grow(T** buf, uint64_t* have, uint64_t need) {
+    if (*have >= need) return FK_OK;
+    cudaFree(*buf);
+    *buf = nullptr;
+    *have = 0;
+    CU(cudaMalloc((void**)buf, std::max<uint64_t>(need, 1)));
+    *have = need;
+    return FK_OK;
+}
+
+// Drawings [lo, hi) on one device, chunk after chunk on its stream: stage and upload, fk_systems_prepare_kernel, one
+// heterogeneous launch, one launch per uniform or sparse structure, fk_systems_scatter_kernel, download; then the chunk's
+// variables and reports into the call's rows (vars_out, reports).
+static int systems_range(const std::vector<SystemsDrawing>& d, const SystemsPlan& P, int optimizer, int perturb, int device, uint32_t lo,
+                         uint32_t hi, double* vars_out, fk_report* reports) {
+    CU(cudaSetDevice(device));
+    SystemsDevice* D = systems_device_for(device);
+    std::lock_guard<std::mutex> lock(D->mu);
+    if (!D->stream) CU(cudaStreamCreateWithFlags(&D->stream, cudaStreamNonBlocking));
+    const cudaStream_t st = D->stream;
+    const bool lm = optimizer == 0;
+    const size_t ns = P.st.size();
+    // ---- chunks: drawings in order, closed at about 1 GiB (FK_SYSTEM_BATCH_CHUNK caps the drawings), at least one drawing,
+    // at most INT32_MAX instances (so every launch stays within INT32_MAX sketches)
+    std::vector<SystemsChunk> chunks;
+    std::vector<uint32_t> max_count(ns, 0);
+    size_t h_need = 0, d_need = 0;
+    const uint32_t cap = system_batch_chunk_env();
+    for (uint32_t a = lo; a < hi;) {
+        uint32_t b = a;
+        uint64_t bytes = 0, inst = 0;
+        while (b < hi) {
+            const uint64_t db = systems_drawing_bytes(d, P, b), di = P.inst_off[b + 1] - P.inst_off[b];
+            if (b > a && (bytes + db > (1ull << 30) || (cap && b - a >= cap) || inst + di > (uint64_t)INT32_MAX)) break;
+            bytes += db;
+            inst += di;
+            b++;
+        }
+        chunks.emplace_back();
+        SystemsChunk& c = chunks.back();
+        c.a = a;
+        c.b = b;
+        systems_chunk_layout(d, P, c);
+        for (size_t s = 0; s < ns; s++) max_count[s] = std::max(max_count[s], c.count[s]);
+        h_need = std::max(h_need, c.o_work);
+        d_need = std::max(d_need, c.end);
+        a = b;
+    }
+    // ---- programs of the structures present and the workspaces of their largest launch
+    std::vector<const DeviceProgram*> full(ns, nullptr);
+    uint64_t lm_ws = 0, lb_ws = 0;
+    for (size_t s = 0; s < ns; s++) {
+        if (P.st[s].kind == 0 || max_count[s] == 0) continue;
+        const fk::DevProgram* v = nullptr;
+        const int rc = P.st[s].topo->program_for(device, &v, &full[s], lm);
+        if (rc != FK_OK) return rc;
+        if (lm && full[s]->sparse_batch) {
+            const fk::SparseBatchProgram& sb = *full[s]->sparse_batch;
+            lm_ws = std::max(lm_ws, sb.workspace_doubles(sb.workspace_ctas(max_count[s])));
+        } else if (!lm && choose_lbfgs(P.st[s].topo.get(), max_count[s]) == 1) {
+            const uint32_t ctas = fk::lbfgs_workspace_ctas(*v, max_count[s]);
+            if (ctas == 0) return fail(FK_ERR_CUDA, "occupancy query of fk_lbfgs_cta_kernel failed");
+            lb_ws = std::max(lb_ws, fk::lbfgs_workspace_doubles(*v, ctas));
+        }
+    }
+    std::vector<fk::DevProgram> progs;
+    uint32_t max_state = 1;
+    if (!P.topos32.empty())
+        if (const int rc = hetero_programs(device, P.topos32, progs, &max_state); rc != FK_OK) return rc;
+    if (D->h_cap < h_need) {
+        if (D->h) cudaFreeHost(D->h);
+        D->h = nullptr;
+        D->h_cap = 0;
+        const size_t want = h_need + h_need / 4;
+        CU(cudaMallocHost((void**)&D->h, want));
+        D->h_cap = want;
+    }
+    uint64_t d_cap = D->d_cap, lm_have = D->lm_ws_doubles * sizeof(double), lb_have = D->lb_ws_doubles * sizeof(double);
+    int grc = systems_grow(&D->d, &d_cap, d_need + d_need / 4);
+    D->d_cap = d_cap;
+    if (grc == FK_OK) grc = systems_grow(&D->lm_ws, &lm_have, lm_ws * sizeof(double));
+    D->lm_ws_doubles = lm_have / sizeof(double);
+    if (grc == FK_OK) grc = systems_grow(&D->lb_ws, &lb_have, lb_ws * sizeof(double));
+    D->lb_ws_doubles = lb_have / sizeof(double);
+    if (grc != FK_OK) return grc;
+
+    auto run = [&](const SystemsChunk& c) -> int {
+        unsigned char* H = D->h;
+        unsigned char* G = D->d;
+        const uint32_t n = c.b - c.a;
+        if (!P.draws->empty()) std::memcpy(H + c.o_draws, P.draws->data(), sizeof(double) * P.draws->size());
+        if (!progs.empty()) std::memcpy(H + c.o_progs, progs.data(), sizeof(fk::DevProgram) * progs.size());
+        fk::HeteroJob* jobs = (fk::HeteroJob*)(H + c.o_jobs);
+        SysInst* inst = (SysInst*)(H + c.o_inst);
+        uint32_t* ioff = (uint32_t*)(H + c.o_ioff);
+        uint64_t* voff = (uint64_t*)(H + c.o_voff);
+        uint64_t* eoff = (uint64_t*)(H + c.o_eoff);
+        uint32_t* tabs = (uint32_t*)(H + c.o_tabs);
+        double* rawv = (double*)(H + c.o_rawv);
+        double* rawp = (double*)(H + c.o_rawp);
+        uint8_t* kinds = (uint8_t*)(H + c.o_kinds);
+        double* hin = (double*)(G + c.o_hin);
+        double* hout = (double*)(G + c.o_hout);
+        fk_report* hrep = (fk_report*)(G + c.o_hrep);
+        std::vector<uint32_t> rank(ns, 0);
+        size_t j = 0, tw = 0, jin = 0, jout = 0, vo = 0, eo = 0;
+        for (uint32_t i = c.a; i < c.b; i++) {
+            const SystemBatchLayout& L = d[i].plan->L;
+            const uint32_t di = i - c.a, ne = (uint32_t)L.kind.size();
+            ioff[di] = (uint32_t)(P.inst_off[i] - c.i0);
+            voff[di] = vo;
+            eoff[di] = eo;
+            if (L.n_vars) std::memcpy(rawv + vo, d[i].vars, sizeof(double) * L.n_vars);
+            if (ne) {
+                std::memcpy(rawp + eo, d[i].param, sizeof(double) * ne);
+                std::memcpy(kinds + eo, L.kind.data(), ne);
+            }
+            for (size_t k = 0; k < L.comps.size(); k++) {
+                const size_t g = P.inst_off[i] + k;
+                const uint32_t s = P.inst_struct[g];
+                const SystemsPlan::Structure& S = P.st[s];
+                const SystemBatchLayout::Component& comp = L.comps[k];
+                const uint32_t nv = (uint32_t)comp.slot_var.size(), nx = (uint32_t)comp.expr.size(), nf = (uint32_t)comp.free_var.size();
+                SysInst& I = inst[g - c.i0];
+                I.tab = tw;
+                I.drawing = di;
+                I.nv = nv;
+                I.ne = nx;
+                I.nf = nf;
+                for (const std::vector<uint32_t>* v : {&comp.slot_var, &comp.slot_draw, &comp.expr, &comp.free_var}) {
+                    if (!v->empty()) std::memcpy(tabs + tw, v->data(), sizeof(uint32_t) * v->size());
+                    tw += v->size();
+                }
+                if (S.kind == 0) {
+                    fk::HeteroJob& J = jobs[j];
+                    J.prog = S.hetero;
+                    J.pad = 0;
+                    J.vars_off = jin;
+                    J.param_off = jin + nv;
+                    J.out_off = jout;
+                    I.vars = hin + jin;
+                    I.params = hin + jin + nv;
+                    I.out = hout + jout;
+                    I.rep = hrep + j;
+                    jin += (size_t)nv + nx;
+                    jout += nf;
+                    j++;
+                } else {
+                    const SystemsChunk::Rows& r = c.rows[s];
+                    const size_t q = rank[s]++;
+                    I.vars = (double*)(G + r.vars) + q * nv;
+                    I.params = (double*)(G + r.params) + q * nx;
+                    I.out = (const double*)(G + r.out) + q * nf;
+                    I.rep = (const fk_report*)(G + r.reps) + q;
+                }
+            }
+            vo += L.n_vars;
+            eo += ne;
+        }
+        ioff[n] = (uint32_t)(c.i1 - c.i0);
+        voff[n] = vo;
+        eoff[n] = eo;
+        CU(cudaMemcpyAsync(G, H, c.o_output, cudaMemcpyHostToDevice, st));
+        const uint64_t* d_voff = (const uint64_t*)(G + c.o_voff);
+        const uint32_t* d_ioff = (const uint32_t*)(G + c.o_ioff);
+        const SysInst* d_inst = (const SysInst*)(G + c.o_inst);
+        const uint32_t* d_tabs = (const uint32_t*)(G + c.o_tabs);
+        const double* d_rawv = (const double*)(G + c.o_rawv);
+        double* d_scales = (double*)(G + c.o_scales);
+        int e = launch_systems_prepare(n, d_voff, (const uint64_t*)(G + c.o_eoff), d_ioff, (const uint8_t*)(G + c.o_kinds), d_rawv,
+                                       (const double*)(G + c.o_rawp), (const double*)(G + c.o_draws), perturb, d_inst, d_tabs, d_scales, st);
+        if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_systems_prepare_kernel");
+        if (c.nj) {
+            const int rc = hetero_launch((const fk::DevProgram*)(G + c.o_progs), (const fk::HeteroJob*)(G + c.o_jobs), c.nj, max_state, hin, hout,
+                                         hrep, st);
+            if (rc != FK_OK) return rc;
+        }
+        for (size_t s = 0; s < ns; s++) {
+            const uint32_t cnt = c.count[s];
+            if (P.st[s].kind == 0 || cnt == 0) continue;
+            const DeviceProgram& F = *full[s];
+            const SystemsChunk::Rows& r = c.rows[s];
+            const double* v = (const double*)(G + r.vars);
+            const double* q = (const double*)(G + r.params);
+            double* o = (double*)(G + r.out);
+            fk_report* rp = (fk_report*)(G + r.reps);
+            if (lm) {
+                const uint32_t ws_ctas = F.sparse_batch ? F.sparse_batch->workspace_ctas(cnt) : 0;
+                e = launch_lm(F, cnt, v, q, o, rp, D->lm_ws, ws_ctas, st);
+                if (e != 0) return cuda_fail((cudaError_t)e, "launch batched LM kernel");
+            } else if (choose_lbfgs(P.st[s].topo.get(), cnt) == 1) {
+                e = fk::launch_lbfgs_cta(F.view, F.jcolptr, F.jrow, cnt, v, q, o, rp, D->lb_ws, fk::lbfgs_workspace_ctas(F.view, cnt), st);
+                if (e == (int)cudaErrorInvalidConfiguration) return fail(FK_ERR_TOO_LARGE, "more than 2^24 Jacobian entries");
+                if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_lbfgs_cta_kernel");
+            } else {
+                e = fk::launch_batch_lbfgs(F.view, F.jcolptr, F.jrow, cnt, v, q, o, rp, st);
+                if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_batch_lbfgs_kernel");
+            }
+        }
+        e = launch_systems_scatter(n, d_voff, d_ioff, d_rawv, d_scales, d_inst, d_tabs, (double*)(G + c.o_outv), (fk_report*)(G + c.o_outr), st);
+        if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_systems_scatter_kernel");
+        CU(cudaMemcpyAsync(H + c.o_output, G + c.o_output, c.o_work - c.o_output, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        if (c.nvars) std::memcpy(vars_out + P.var_off[c.a], H + c.o_outv, sizeof(double) * c.nvars);
+        if (c.i1 > c.i0) std::memcpy(reports + c.i0, H + c.o_outr, sizeof(fk_report) * (c.i1 - c.i0));
+        return FK_OK;
+    };
+    for (const SystemsChunk& c : chunks) {
+        const int rc = run(c);
+        if (rc != FK_OK) {
+            cudaStreamSynchronize(st);  // (nothing of a failed chunk may still run when the staging is reused)
+            return rc;
+        }
+    }
+    return FK_OK;
+}
+
+int systems_solve(const std::vector<SystemsDrawing>& d, int optimizer, int perturb, int n_gpus, double* vars_out, fk_report* reports) {
+    SystemsPlan P;
+    systems_plan_create(d, optimizer, P);
+    for (const SystemsPlan::Structure& S : P.st)  // LM on the global sparse path: the front limit of fk_batch_solve
+        if (S.kind == 2 && S.topo->sb_check() != FK_OK)
+            return fail(FK_ERR_TOO_LARGE, "drawing " + std::to_string(S.first_drawing) + ", component " + std::to_string(S.first_comp) + ": " +
+                                              S.topo->sb_err + "; Optimizer::LBfgs takes systems of every size");
+    if (d.empty()) return FK_OK;
+    const int rc = clamp_gpus(n_gpus);
+    if (rc != FK_OK) return rc;
+    return shard_over_devices(n_gpus, (uint32_t)d.size(), [&](int device, uint32_t lo, uint32_t hi) {
+        return systems_range(d, P, optimizer, perturb, device, lo, hi, vars_out, reports);
+    });
 }
 
 }  // namespace fk

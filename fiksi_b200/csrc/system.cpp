@@ -1161,9 +1161,76 @@ int an_batch_run(const fk_system* s, uint32_t n, const double* vars, const doubl
     return fk::system_an_batch_run(*b, c);
 }
 
+// fk_systems_solve / fk_systems_layout: the refusals of the call (before any device work) and every drawing's batch plan.
+int systems_drawings(uint32_t n, fk_system* const* systems, const fk_solving_options* opts, std::vector<fk::SystemsDrawing>& d,
+                     std::vector<std::shared_ptr<fk::SystemBatch>>& plans) {
+    if (!opts) return fk::system_batch_fail(FK_ERR_INVALID, "null options");
+    if (opts->optimizer > 1 || opts->perturb > 1 || opts->pad != 0 || opts->decomposer > 2)
+        return fk::system_batch_fail(FK_ERR_INVALID, "invalid solving options");
+    if (opts->decomposer != 0) return fk::system_batch_fail(FK_ERR_INVALID, "fk_systems_solve takes Decomposer::None only (decomposer 0)");
+    if (n && !systems) return fk::system_batch_fail(FK_ERR_INVALID, "null systems");
+    std::set<const fk_system*> seen;
+    for (uint32_t i = 0; i < n; i++) {
+        if (!systems[i]) return fk::system_batch_fail(FK_ERR_INVALID, "null system at index " + std::to_string(i));
+        if (!seen.insert(systems[i]).second)
+            return fk::system_batch_fail(FK_ERR_INVALID, "system at index " + std::to_string(i) + " is given twice");
+    }
+    plans.resize(n);
+    d.resize(n);
+    for (uint32_t i = 0; i < n; i++) {
+        const int rc = batch_plan_for(systems[i], &plans[i]);
+        if (rc != FK_OK) return rc;
+        d[i] = {plans[i].get(), systems[i]->vars.data(), systems[i]->param.data()};
+    }
+    return FK_OK;
+}
+
 }  // namespace
 
 extern "C" {
+
+int fk_systems_layout(uint32_t n, fk_system* const* systems, const fk_solving_options* opts, uint32_t* n_components, uint32_t* n_structures,
+                      uint32_t* instances, uint32_t* launch_kind) {
+    std::vector<fk::SystemsDrawing> d;
+    std::vector<std::shared_ptr<fk::SystemBatch>> plans;
+    const int rc = systems_drawings(n, systems, opts, d, plans);
+    if (rc != FK_OK) return rc;
+    uint32_t nc = 0;
+    std::vector<uint32_t> inst, kind;
+    fk::systems_layout(d, (int)opts->optimizer, &nc, &inst, &kind);
+    if (n_components) *n_components = nc;
+    if (n_structures) *n_structures = (uint32_t)inst.size();
+    if (instances) std::copy(inst.begin(), inst.end(), instances);
+    if (launch_kind) std::copy(kind.begin(), kind.end(), launch_kind);
+    return FK_OK;
+}
+
+int fk_systems_solve(uint32_t n, fk_system* const* systems, const fk_solving_options* opts, fk_report* reports, uint32_t reports_cap,
+                     uint32_t* n_solved, int n_gpus) {
+    std::vector<fk::SystemsDrawing> d;
+    std::vector<std::shared_ptr<fk::SystemBatch>> plans;
+    int rc = systems_drawings(n, systems, opts, d, plans);
+    if (rc != FK_OK || n == 0) return rc;
+    std::vector<size_t> var_off(n + 1, 0), rep_off(n + 1, 0);
+    for (uint32_t i = 0; i < n; i++) {
+        uint32_t nc = 0;
+        fk::system_batch_layout(*plans[i], &nc, nullptr, nullptr);
+        var_off[i + 1] = var_off[i] + systems[i]->vars.size();
+        rep_off[i + 1] = rep_off[i] + nc;
+    }
+    // all or nothing: the results land in the call's rows, and only a complete call writes them into the systems
+    std::vector<double> vars_out(std::max<size_t>(var_off[n], 1));
+    std::vector<fk_report> reps(std::max<size_t>(rep_off[n], 1));
+    rc = fk::systems_solve(d, (int)opts->optimizer, (int)opts->perturb, n_gpus, vars_out.data(), reps.data());
+    if (rc != FK_OK) return rc;
+    for (uint32_t i = 0; i < n; i++) {  // assemble/mod.rs:161-166
+        std::vector<double>& v = systems[i]->vars;
+        if (!v.empty()) std::memcpy(v.data(), vars_out.data() + var_off[i], sizeof(double) * v.size());
+        if (n_solved) n_solved[i] = (uint32_t)(rep_off[i + 1] - rep_off[i]);
+    }
+    if (reports) std::copy(reps.begin(), reps.begin() + std::min<size_t>(reports_cap, rep_off[n]), reports);
+    return FK_OK;
+}
 
 int fk_system_batch_analyze(const fk_system* s, uint32_t n, const double* vars, const double* params, uint8_t* dependent, int n_gpus) {
     return an_batch_run(s, n, vars, params, dependent, nullptr, n_gpus);

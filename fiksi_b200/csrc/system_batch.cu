@@ -4,7 +4,8 @@
 // fk_system_batch_solve_single_pass and _recursive_assembly reuse the prepare kernel (one identity structure: the resident
 // scaled rows) and move values between the waves of sets or steps with fk_system_sp_gather_scatter_kernel.
 // fk_system_batch_analyze and fk_system_batch_residuals expand the variants' parameter rows, then reduce the analyze flags
-// per constraint or evaluate every constraint's residual.
+// per constraint or evaluate every constraint's residual.  fk_systems_solve (n different drawings) has its own prepare and
+// scatter kernels over ragged rows: every drawing its own size, every component its own destination.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -181,6 +182,97 @@ fk_system_sp_gather_scatter_kernel(uint32_t n, uint32_t vb, uint32_t n_vars, uin
         const size_t v = v0 + b;
         vars_out[v * n_vars + g] = __ldg(solved + g) ? __ldg(scales + v) * vrow[i] : __ldg(raw_vars + v * raw_vars_stride + g);
     }
+}
+
+// ---- fk_systems_solve: n different drawings ----------------------------------------------------------------------------
+namespace {
+// Drawings per CTA of the two kernels of fk_systems_solve.  One thread owns a drawing's scale (the reference's sequential
+// sum); 32 keeps a call of a thousand mid-size drawings on 32 CTAs rather than 8.
+constexpr uint32_t kSysDrawings = 32, kSysThreads = 128;
+}  // namespace
+
+// One CTA per kSysDrawings consecutive drawings.  The first warp computes their scales, then the CTA's warps take the drawings'
+// instances (consecutive: [inst_off[d0], inst_off[d0 + nb])) one each, the lanes over its local variables and expressions.
+__global__ void __launch_bounds__(kSysThreads)
+fk_systems_prepare_kernel(uint32_t n, const uint64_t* __restrict__ var_off, const uint64_t* __restrict__ expr_off,
+                          const uint32_t* __restrict__ inst_off, const uint8_t* __restrict__ kinds, const double* __restrict__ raw_vars,
+                          const double* __restrict__ raw_param, const double* __restrict__ draws, uint32_t perturb,
+                          const SysInst* __restrict__ inst, const uint32_t* __restrict__ tabs, double* __restrict__ scales) {
+    __shared__ double s_recip[kSysDrawings];
+    const uint32_t d0 = blockIdx.x * kSysDrawings;
+    const uint32_t nb = min(kSysDrawings, n - d0);
+    if (threadIdx.x < nb) {
+        const uint32_t d = d0 + threadIdx.x;
+        const uint64_t v0 = __ldg(var_off + d), e0 = __ldg(expr_off + d);
+        const double* q = raw_param + e0;
+        const double scale = prepare_scale(raw_vars + v0, (uint32_t)(__ldg(var_off + d + 1) - v0), (uint32_t)(__ldg(expr_off + d + 1) - e0),
+                                           kinds + e0, [&](uint32_t e) { return __ldg(q + e); });
+        s_recip[threadIdx.x] = 1.0 / scale;
+        scales[d] = scale;
+    }
+    __syncthreads();
+    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+    for (uint32_t k = __ldg(inst_off + d0) + warp, end = __ldg(inst_off + d0 + nb); k < end; k += kSysThreads / 32) {
+        const SysInst I = inst[k];
+        const double recip = s_recip[I.drawing - d0];
+        const double* rv = raw_vars + __ldg(var_off + I.drawing);
+        const uint64_t e0 = __ldg(expr_off + I.drawing);
+        const uint32_t* slot_var = tabs + I.tab;
+        const uint32_t* slot_draw = slot_var + I.nv;
+        const uint32_t* expr = slot_draw + I.nv;
+        for (uint32_t j = lane; j < I.nv; j += 32) {
+            const uint32_t dr = __ldg(slot_draw + j);
+            double col = __ldg(rv + __ldg(slot_var + j)) * recip;
+            if (perturb && dr != kSbNone) col = prepare_perturb(col, __ldg(draws + 2 * (size_t)dr), __ldg(draws + 2 * (size_t)dr + 1));
+            I.vars[j] = col;
+        }
+        for (uint32_t j = lane; j < I.ne; j += 32) {
+            const uint64_t e = e0 + __ldg(expr + j);
+            const double q = __ldg(raw_param + e);
+            I.params[j] = prepare_is_distance(__ldg(kinds + e)) ? recip * q : q;
+        }
+    }
+}
+
+// system.variables after the solve (assemble/mod.rs:161-166), per drawing: every variable as it came in, then (after the
+// CTA's barrier, so the raw copy never lands on a solved value) scale * x for the solved free variables.  The reports go to
+// the instance's slot.
+__global__ void __launch_bounds__(kSysThreads)
+fk_systems_scatter_kernel(uint32_t n, const uint64_t* __restrict__ var_off, const uint32_t* __restrict__ inst_off,
+                          const double* __restrict__ raw_vars, const double* __restrict__ scales, const SysInst* __restrict__ inst,
+                          const uint32_t* __restrict__ tabs, double* __restrict__ vars_out, uint64_t* __restrict__ reports_out) {
+    const uint32_t d0 = blockIdx.x * kSysDrawings;
+    const uint32_t nb = min(kSysDrawings, n - d0);
+    for (uint64_t i = __ldg(var_off + d0) + threadIdx.x, end = __ldg(var_off + d0 + nb); i < end; i += kSysThreads) vars_out[i] = __ldg(raw_vars + i);
+    __syncthreads();
+    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+    constexpr uint32_t W = sizeof(fk_report) / 8;
+    for (uint32_t k = __ldg(inst_off + d0) + warp, end = __ldg(inst_off + d0 + nb); k < end; k += kSysThreads / 32) {
+        const SysInst I = inst[k];
+        const double scale = __ldg(scales + I.drawing);
+        double* row = vars_out + __ldg(var_off + I.drawing);
+        const uint32_t* free_var = tabs + I.tab + 2 * (uint64_t)I.nv + I.ne;
+        for (uint32_t j = lane; j < I.nf; j += 32) row[__ldg(free_var + j)] = scale * __ldg(I.out + j);
+        if (lane < W) reports_out[(uint64_t)k * W + lane] = __ldg((const unsigned long long*)I.rep + lane);
+    }
+}
+
+int launch_systems_prepare(uint32_t n, const uint64_t* var_off, const uint64_t* expr_off, const uint32_t* inst_off, const uint8_t* kinds,
+                           const double* raw_vars, const double* raw_param, const double* draws, int perturb, const SysInst* inst,
+                           const uint32_t* tabs, double* scales, void* stream) {
+    if (n == 0) return 0;
+    fk_systems_prepare_kernel<<<(n + kSysDrawings - 1) / kSysDrawings, kSysThreads, 0, (cudaStream_t)stream>>>(
+        n, var_off, expr_off, inst_off, kinds, raw_vars, raw_param, draws, perturb ? 1u : 0u, inst, tabs, scales);
+    return (int)cudaGetLastError();
+}
+
+int launch_systems_scatter(uint32_t n, const uint64_t* var_off, const uint32_t* inst_off, const double* raw_vars, const double* scales,
+                           const SysInst* inst, const uint32_t* tabs, double* vars_out, fk_report* reports_out, void* stream) {
+    static_assert(sizeof(fk_report) % 8 == 0 && sizeof(fk_report) / 8 <= 32, "fk_report is moved as 64-bit words by one warp");
+    if (n == 0) return 0;
+    fk_systems_scatter_kernel<<<(n + kSysDrawings - 1) / kSysDrawings, kSysThreads, 0, (cudaStream_t)stream>>>(
+        n, var_off, inst_off, raw_vars, scales, inst, tabs, vars_out, (uint64_t*)reports_out);
+    return (int)cudaGetLastError();
 }
 
 // ---- fk_system_batch_analyze / fk_system_batch_residuals ---------------------------------------------------------------

@@ -159,6 +159,49 @@ struct SystemAnCall {
 // Refusals (analyze: choose_analyze's size limit) before any device work, then the chunks on every device.
 int system_an_batch_run(SystemAnBatch& b, const SystemAnCall& call);
 
+// fk_systems_solve: System::solve over n different drawings, each with its own SystemBatch plan (its components, grouped by
+// structure inside the drawing).  capi.cu merges the structures of all drawings, runs chunks of drawings and returns every
+// drawing's variables and reports; system.cpp validates the call and writes the results into the systems.
+//
+// One instance per solved component of a chunk's drawings, in drawing order and component order inside a drawing, so that the
+// k-th instance's report is the k-th report of the chunk.  vars / params: where the prepare kernel writes its input rows (its
+// structure's batch rows, or its heterogeneous job's rows); out / rep: its solution.  tab: offset in the chunk's u32 table of
+// the component's slot_var[nv], slot_draw[nv], expr[ne] and free_var[nf] (SystemBatchLayout::Component).
+struct SysInst {
+    double* vars;
+    double* params;
+    const double* out;
+    const fk_report* rep;
+    uint64_t tab;
+    uint32_t drawing;  // in the chunk
+    uint32_t nv, ne, nf;
+};
+// Ragged rows of the chunk's n drawings: drawing d owns raw_vars[var_off[d] .. var_off[d + 1]) and raw_param / kinds
+// [expr_off[d] .. expr_off[d + 1]) (s->vars, s->param, s->kind), and the instances [inst_off[d], inst_off[d + 1]).
+// Per drawing: scales[d] = prepare_scale of its rows, then every instance's input rows (perturb 0: no draws applied; draws: the
+// one table of the call, pair k is the same in every drawing).
+int launch_systems_prepare(uint32_t n, const uint64_t* var_off, const uint64_t* expr_off, const uint32_t* inst_off, const uint8_t* kinds,
+                           const double* raw_vars, const double* raw_param, const double* draws, int perturb, const SysInst* inst,
+                           const uint32_t* tabs, double* scales, void* stream);
+// vars_out[var_off[d] + i] = raw_vars[var_off[d] + i], then scales[d] * x for every solved free variable; reports_out[k] = the
+// k-th instance's report.
+int launch_systems_scatter(uint32_t n, const uint64_t* var_off, const uint32_t* inst_off, const double* raw_vars, const double* scales,
+                           const SysInst* inst, const uint32_t* tabs, double* vars_out, fk_report* reports_out, void* stream);
+
+struct SystemsDrawing {
+    const SystemBatch* plan;
+    const double* vars;   // [plan n_vars]
+    const double* param;  // [plan n_expr]
+};
+// Host-only: solved components, distinct structures across the drawings (order of first appearance), per structure its
+// instances and launch kind (0 heterogeneous, 1 uniform batch, 2 sparse batch) under `optimizer`.
+void systems_layout(const std::vector<SystemsDrawing>& d, int optimizer, uint32_t* n_components, std::vector<uint32_t>* instances,
+                    std::vector<uint32_t>* launch_kind);
+// The solve: vars_out receives every drawing's variables after the solve (drawing after drawing), reports every solved
+// component's report (drawing after drawing, component order).  Refusals before any device work; vars_out and reports are only
+// complete when FK_OK is returned.
+int systems_solve(const std::vector<SystemsDrawing>& d, int optimizer, int perturb, int n_gpus, double* vars_out, fk_report* reports);
+
 // fk_last_error()'s message for errors found outside capi.cu.
 int system_batch_fail(int code, const std::string& msg);
 

@@ -258,3 +258,38 @@ class System:
             self.close()
         except Exception:
             pass
+
+
+def _systems_call(systems, optimizer, perturb):
+    if optimizer not in _OPTIMIZERS:
+        raise ValueError(f"optimizer must be 'lm' or 'lbfgs', not {optimizer!r}")
+    handles = (C.c_void_p * max(len(systems), 1))(*[s._h for s in systems])
+    return handles, FkSolvingOptions(_OPTIMIZERS[optimizer], 0, int(bool(perturb)), 0)
+
+
+def systems_layout(systems, optimizer="lm"):
+    """(solved components, distinct structures across the drawings, [instances per structure], [launch kind per structure:
+    0 heterogeneous, 1 uniform batch, 2 sparse batch]) of solve_systems' plan (host only, fk_systems_layout)."""
+    handles, opts = _systems_call(systems, optimizer, True)
+    nc, ns = C.c_uint32(0), C.c_uint32(0)
+    check(lib().fk_systems_layout(len(systems), handles, C.byref(opts), C.byref(nc), C.byref(ns), None, None))
+    inst = np.zeros(max(ns.value, 1), np.uint32)
+    kind = np.zeros(max(ns.value, 1), np.uint32)
+    check(lib().fk_systems_layout(len(systems), handles, C.byref(opts), C.byref(nc), C.byref(ns), ptr(inst, C.c_uint32),
+                                  ptr(kind, C.c_uint32)))
+    return int(nc.value), int(ns.value), inst[:ns.value].tolist(), kind[:ns.value].tolist()
+
+
+def solve_systems(systems, optimizer="lm", perturb=True, n_gpus=1):
+    """System.solve(perturb, optimizer) of every system in `systems` (different drawings) in one call (fk_systems_solve).
+    The systems are modified in place, exactly as each one's own solve() would modify it; nothing is modified when the call
+    fails.  Returns one REPORT_DTYPE array per system: the reports of its solved components, in component order."""
+    handles, opts = _systems_call(systems, optimizer, perturb)
+    n = len(systems)
+    cap = sum(lib().fk_system_num_constraints(s._h) for s in systems)  # every solved component holds a constraint
+    reps = np.zeros(max(cap, 1), dtype=REPORT_DTYPE)
+    solved = np.zeros(max(n, 1), np.uint32)
+    check(lib().fk_systems_solve(n, handles, C.byref(opts), reps.ctypes.data_as(C.POINTER(FkReport)), len(reps), ptr(solved, C.c_uint32),
+                                 int(n_gpus)))
+    ends = np.cumsum(solved[:n])
+    return [reps[e - k:e].copy() for e, k in zip(ends.tolist(), solved[:n].tolist())]

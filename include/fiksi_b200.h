@@ -457,6 +457,36 @@ FK_API int fk_system_batch_solve(const fk_system* s, const fk_solving_options* o
 /* Host-only probe of fk_system_batch_solve's plan (no device needed): solved components, distinct component structures,
  * and the components per structure in order of first appearance (multiplicity[n_structures], may be NULL). */
 FK_API int fk_system_batch_layout(const fk_system* s, uint32_t* n_components, uint32_t* n_structures, uint32_t* multiplicity);
+/* == System::solve(*opts) (lib.rs:464, assemble/mod.rs:46-167) on each of n different drawings, in one call.  systems[i] is
+ * solved in place exactly as fk_system_solve_options(systems[i], opts, ...) would solve it: after the call it holds bit for bit
+ * what that call gives on an identically built copy, and so do its reports -- for both optimizers, with and without
+ * perturbation, fixed variables, stale-index components (SURVEY F7), empty drawings and NaN / inf inputs (which stay inside
+ * their own drawing).  One exception: an LM component on the global sparse path runs the sparse batch kernel, with the
+ * decisions, traces and counters of that call and coordinates within the 1e-11 relative difference of fk_system_batch_solve.
+ * reports: the solved components of systems[0] in component order, then those of systems[1], ...; at most reports_cap are
+ * written.  n_solved[i] (may be NULL) = components solved in systems[i].
+ * Only Decomposer::None.  Refusals come before any device work and modify no system: FK_ERR_INVALID for null `systems` or
+ * `opts`, a null entry, the same fk_system twice (the results would depend on the order), opts->decomposer != 0 or other bad
+ * options; FK_ERR_TOO_LARGE with LM when a component's largest supernodal front exceeds the 236 rows of fk_batch_solve (the
+ * message names the drawing's index, the component and the front's order).  n == 0 returns FK_OK.  All or nothing: the systems
+ * are written only after every chunk on every device has succeeded, so a device error leaves every system as it was.
+ * Each drawing's plan is fk_system_batch_solve's, kept on the system until a structural edit.  Per call, the structures of
+ * all drawings are merged (same structure, whatever the drawing) and each goes to one launch kind: under LM, fk_lm_solve_batch's
+ * rule (path 0 with fewer than 64 instances, 32-lane tables and at most 48 KiB of state: the one heterogeneous launch of the
+ * chunk), the uniform batch kernels for the other path-0 / 1 structures, the sparse batch kernel on path 2; under L-BFGS one
+ * uniform launch per structure.  On the device, per chunk of drawings on one stream per device: one copy up of the drawings'
+ * raw rows and the call's tables, one kernel computes every drawing's scale and gathers every component's input rows, the
+ * solve launches, one kernel writes the unscaled rows and the reports, one copy down.  Drawings go in order in chunks of about
+ * 1 GiB of device buffers (FK_SYSTEM_BATCH_CHUNK caps the drawings per chunk), sharded by count over n_gpus devices (0 == all
+ * visible). */
+FK_API int fk_systems_solve(uint32_t n, fk_system* const* systems, const fk_solving_options* opts, fk_report* reports,
+                            uint32_t reports_cap, uint32_t* n_solved, int n_gpus);
+/* Host-only probe of fk_systems_solve's plan (no device needed): total solved components, distinct structures across the
+ * drawings, and per structure (order of first appearance) its instance count and launch kind (0 heterogeneous, 1 uniform
+ * batch, 2 sparse batch).  instances[n_structures] and launch_kind[n_structures] may be NULL; refusals as fk_systems_solve's
+ * FK_ERR_INVALID. */
+FK_API int fk_systems_layout(uint32_t n, fk_system* const* systems, const fk_solving_options* opts, uint32_t* n_components,
+                             uint32_t* n_structures, uint32_t* instances, uint32_t* launch_kind);
 /* == System::solve(SolvingOptions { decomposer: SinglePass, perturb }) (assemble/mod.rs:169-210; the reference runs LM here
  * whatever the optimizer, :191) applied to n variants of `s`; argument meaning as fk_system_batch_solve.  vars_out[v] and
  * reports[v] are bit for bit what fk_system_solve_opts(decomposer = 1, perturb) gives on a copy of `s` with the variant's

@@ -71,7 +71,8 @@ EXPORTS = [
     "fk_system_solve_options", "fk_batch_system_solve", "fk_batch_system_solve_begin", "fk_batch_system_solve_wait", "fk_batch_solve_device_begin", "fk_batch_solve_device_wait", "fk_topology_cache_configure", "fk_topology_cache_clear", "fk_topology_cache_stats",
     "fk_system_batch_solve", "fk_system_batch_layout", "fk_system_batch_solve_single_pass", "fk_system_single_pass_batch_layout",
     "fk_system_batch_solve_recursive_assembly", "fk_system_recursive_assembly_batch_layout", "fk_system_batch_analyze",
-    "fk_system_batch_residuals", "fk_systems_solve", "fk_systems_layout",
+    "fk_system_batch_residuals", "fk_systems_solve", "fk_systems_layout", "fk_systems_analyze", "fk_systems_residuals",
+    "fk_systems_analyze_layout",
 ]
 
 _lib = None
@@ -112,6 +113,9 @@ def lib() -> C.CDLL:
         sysp, optp = C.POINTER(C.c_void_p), C.POINTER(FkSolvingOptions)
         L.fk_systems_solve.argtypes = [C.c_uint32, sysp, optp, C.POINTER(FkReport), C.c_uint32, u32p, C.c_int]
         L.fk_systems_layout.argtypes = [C.c_uint32, sysp, optp, u32p, u32p, u32p, u32p]
+        L.fk_systems_analyze.argtypes = [C.c_uint32, sysp, C.POINTER(C.c_uint8), C.c_uint64, C.c_int]
+        L.fk_systems_residuals.argtypes = [C.c_uint32, sysp, f64p, C.c_uint64, C.c_int]
+        L.fk_systems_analyze_layout.argtypes = [C.c_uint32, sysp, u32p, u32p, u32p]
         _lib = L
     return _lib
 

@@ -218,8 +218,6 @@ fk_analyze_cta_kernel(AnArgs a) {
     }
 }
 
-namespace {
-
 int forced_analyze_kernel() {
     const char* e = std::getenv("FK_ANALYZE_KERNEL");
     if (!e) return -1;
@@ -228,8 +226,6 @@ int forced_analyze_kernel() {
     if (!std::strcmp(e, "group")) return kAnGroup;
     return -1;
 }
-
-}  // namespace
 
 int choose_analyze(uint32_t n_vars, uint32_t n_expr, uint32_t n_sketches, int device, AnalyzePlan* plan, std::string* err) {
     AnalyzePlan p;

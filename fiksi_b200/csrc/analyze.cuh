@@ -41,6 +41,8 @@ struct AnalyzePlan {
 // A/B); a forced warp kernel on a matrix it cannot hold is refused.  Returns FK_OK, FK_ERR_TOO_LARGE (with the sizes in
 // *err) or a CUDA failure as FK_ERR_CUDA.
 int choose_analyze(uint32_t n_vars, uint32_t n_expr, uint32_t n_sketches, int device, AnalyzePlan* plan, std::string* err);
+// The kernel FK_ANALYZE_KERNEL forces (kAnWarp, kAnCta, kAnGroup), or -1 when it is unset or names none of them.
+int forced_analyze_kernel();
 
 // Launches plan.kernel (cta / group) on `ws` (plan.workspace_bytes(), used by this launch alone until it completes).
 int launch_analyze(const AnalyzePlan& plan, uint32_t n_vars, uint32_t n_expr, const uint8_t* kinds, const uint32_t* slot_var,

@@ -2463,6 +2463,7 @@ struct SystemAnDevice : SystemDevice {
 struct SystemAnBatch {
     SystemAnLayout L;
     uint32_t n_expr = 0, n_constraints = 0;
+    uint64_t sig = 0;  // hash of the structure (n_vars, kinds, slot table, constraint ranges): fk_systems_analyze merges by it
     std::mutex mu;
     std::map<int, std::unique_ptr<SystemAnDevice>> devices;
 };
@@ -2472,6 +2473,15 @@ int system_an_batch_create(SystemAnLayout&& layout, std::shared_ptr<SystemAnBatc
     b->L = std::move(layout);
     b->n_expr = (uint32_t)b->L.kind.size();
     b->n_constraints = b->L.con_off.empty() ? 0 : (uint32_t)b->L.con_off.size() - 1;
+    uint64_t h = 1469598103934665603ull;  // FNV-1a
+    auto mix = [&h](const void* p, size_t bytes) {
+        for (size_t i = 0; i < bytes; i++) h = (h ^ ((const unsigned char*)p)[i]) * 1099511628211ull;
+    };
+    mix(&b->L.n_vars, sizeof(uint32_t));
+    mix(b->L.kind.data(), b->L.kind.size());
+    mix(b->L.slot_var.data(), sizeof(uint32_t) * b->L.slot_var.size());
+    mix(b->L.con_off.data(), sizeof(uint32_t) * b->L.con_off.size());
+    b->sig = h;
     *out = std::move(b);
     return FK_OK;
 }
@@ -2671,15 +2681,16 @@ void systems_layout(const std::vector<SystemsDrawing>& d, int optimizer, uint32_
 }
 
 // Per device, reused across calls (never destroyed: CUDA may be gone at static-destruction time): one stream, a grow-only
-// pinned staging block and device arena, and the grow-only workspaces of the sparse batch LM kernel and the L-BFGS CTA kernel
-// (launches on the one stream run one after the other, so one workspace serves them all).
+// pinned staging block and device arena, and the grow-only workspaces of the sparse batch LM kernel, the L-BFGS CTA kernel and
+// the global-memory analyze kernels (launches on the one stream run one after the other, so one workspace serves them all).
+// fk_systems_solve, fk_systems_analyze and fk_systems_residuals share it.
 struct SystemsDevice {
     std::mutex mu;
     cudaStream_t stream = nullptr;
     unsigned char *h = nullptr, *d = nullptr;
     size_t h_cap = 0, d_cap = 0;
-    double *lm_ws = nullptr, *lb_ws = nullptr;
-    uint64_t lm_ws_doubles = 0, lb_ws_doubles = 0;
+    double *lm_ws = nullptr, *lb_ws = nullptr, *an_ws = nullptr;
+    uint64_t lm_ws_doubles = 0, lb_ws_doubles = 0, an_ws_bytes = 0;
 };
 static SystemsDevice* systems_device_for(int device) {
     static std::mutex m;
@@ -3007,6 +3018,331 @@ int systems_solve(const std::vector<SystemsDrawing>& d, int optimizer, int pertu
     if (rc != FK_OK) return rc;
     return shard_over_devices(n_gpus, (uint32_t)d.size(), [&](int device, uint32_t lo, uint32_t hi) {
         return systems_range(d, P, optimizer, perturb, device, lo, hi, vars_out, reports);
+    });
+}
+
+// ---- fk_systems_analyze / fk_systems_residuals: System::analyze and calculate_residual over n different drawings -------------
+// The call's plan: the drawings' SystemAnBatch plans merged into structures (one plan object is one structure; other plans join
+// one when the signature and an exact comparison of n_vars, kinds, slot table and constraint ranges agree), each with its analyze
+// launch kind, and every drawing's first constraint in the call's output.  Built per call.
+struct SystemsAnPlan {
+    struct Structure {
+        const SystemAnBatch* b = nullptr;  // its first drawing's plan: the tables
+        uint32_t kind = 0;                 // 0 heterogeneous warp launch, 1 one launch of the kernel choose_analyze picks
+        uint32_t instances = 0, first_drawing = 0;
+        size_t tab_words = 0;              // slot_var[8 n_expr], the kinds in whole words, con_off[n_constraints + 1]
+    };
+    std::vector<Structure> st;
+    std::vector<uint32_t> drawing_struct;  // per drawing
+    std::vector<size_t> con_off;           // [n + 1]
+};
+
+constexpr uint32_t kSystemsAnUniform = 64;  // instances from which a warp-sized structure gets a launch of its own
+
+// analyze == false (the residuals): every structure kind 0, the rows in drawing order.
+static void systems_an_plan_create(const std::vector<SystemsAnDrawing>& d, bool analyze, SystemsAnPlan& P) {
+    const int forced = analyze ? forced_analyze_kernel() : -1;
+    std::multimap<uint64_t, uint32_t> by_sig;
+    std::unordered_map<const SystemAnBatch*, uint32_t> by_plan;
+    P.con_off.assign(1, 0);
+    for (uint32_t i = 0; i < d.size(); i++) {
+        const SystemAnBatch* b = d[i].plan;
+        uint32_t m = kSbNone;
+        const auto known = by_plan.find(b);
+        if (known != by_plan.end()) {
+            m = known->second;
+        } else {
+            for (auto r = by_sig.equal_range(b->sig); r.first != r.second && m == kSbNone; ++r.first) {
+                const SystemAnLayout& L = P.st[r.first->second].b->L;
+                if (L.n_vars == b->L.n_vars && L.kind == b->L.kind && L.slot_var == b->L.slot_var && L.con_off == b->L.con_off) m = r.first->second;
+            }
+            if (m == kSbNone) {
+                m = (uint32_t)P.st.size();
+                by_sig.emplace(b->sig, m);
+                SystemsAnPlan::Structure S;
+                S.b = b;
+                S.first_drawing = i;
+                const bool warp = (forced < 0 || forced == kAnWarp) && batch_analyze_warp_fits(b->L.n_vars, b->n_expr);
+                S.kind = analyze && !warp ? 1 : 0;  // (kind 0 may still become 1 below, by its instance count)
+                S.tab_words = 8 * (size_t)b->n_expr + (b->n_expr + 3) / 4 + b->n_constraints + 1;
+                P.st.push_back(S);
+            }
+            by_plan.emplace(b, m);
+        }
+        P.st[m].instances++;
+        P.drawing_struct.push_back(m);
+        P.con_off.push_back(P.con_off.back() + d[i].plan->n_constraints);
+    }
+    // A structure with many instances runs faster in its own fk_batch_analyze_kernel launch (choose_analyze's warp kernel): its
+    // exact footprint rather than the class's power of two sets the warps per SM.  The cut is fk_lm_solve_batch's for its
+    // heterogeneous launch.
+    for (SystemsAnPlan::Structure& S : P.st)
+        if (analyze && S.instances >= kSystemsAnUniform) S.kind = 1;
+}
+
+void systems_an_layout(const std::vector<SystemsAnDrawing>& d, std::vector<uint32_t>* instances, std::vector<uint32_t>* launch_kind) {
+    SystemsAnPlan P;
+    systems_an_plan_create(d, true, P);
+    instances->clear();
+    launch_kind->clear();
+    for (const SystemsAnPlan::Structure& S : P.st) {
+        instances->push_back(S.instances);
+        launch_kind->push_back(S.kind);
+    }
+}
+
+// One chunk of drawings [a, b) on one device.  Arena: [0, o_output) the input staged in pinned memory (same offsets) and sent with
+// one copy -- per drawing its SysAnJob, the constraint offsets, the kind-0 jobs, the tables of the structures present, the
+// variable and parameter rows --, [o_output, o_work) the counts or residuals that come back with one copy, [o_work, end) the
+// flags.  Rows (and flags, at the parameter offsets): the kind-0 drawings in drawing order, then one block per kind-1 structure
+// present, its drawings in drawing order, so that its uniform launch reads them in place.
+struct SystemsAnChunk {
+    uint32_t a = 0, b = 0;
+    std::vector<uint32_t> count;                 // per structure: drawings in the chunk
+    std::vector<size_t> tab, vblk, eblk;         // per structure present: table offset (words); kind 1: its block's row offsets
+    size_t nj = 0, tab_words = 0, nvars = 0, nexpr = 0, ncon = 0;
+    size_t o_desc = 0, o_base = 0, o_jobs = 0, o_tabs = 0, o_vars = 0, o_params = 0, o_output = 0, o_work = 0, end = 0;
+};
+
+static void systems_an_chunk_layout(const std::vector<SystemsAnDrawing>& d, const SystemsAnPlan& P, bool analyze, SystemsAnChunk& c) {
+    const size_t ns = P.st.size(), n = c.b - c.a;
+    c.count.assign(ns, 0);
+    c.tab.assign(ns, 0);
+    c.vblk.assign(ns, 0);
+    c.eblk.assign(ns, 0);
+    for (uint32_t i = c.a; i < c.b; i++) {
+        const uint32_t s = P.drawing_struct[i];
+        const SystemAnBatch& B = *d[i].plan;
+        if (c.count[s]++ == 0) {
+            c.tab[s] = c.tab_words;
+            c.tab_words += P.st[s].tab_words;
+        }
+        if (P.st[s].kind == 0) {
+            c.nvars += B.L.n_vars;
+            c.nexpr += B.n_expr;
+            if (B.n_expr) c.nj++;
+        }
+    }
+    for (size_t s = 0; s < ns; s++) {
+        if (P.st[s].kind == 0 || c.count[s] == 0) continue;
+        c.vblk[s] = c.nvars;
+        c.eblk[s] = c.nexpr;
+        c.nvars += (size_t)c.count[s] * P.st[s].b->L.n_vars;
+        c.nexpr += (size_t)c.count[s] * P.st[s].b->n_expr;
+    }
+    c.ncon = P.con_off[c.b] - P.con_off[c.a];
+    size_t at = 0;
+    auto put = [&](size_t bytes) {
+        const size_t o = at;
+        at = (at + std::max<size_t>(bytes, 1) + 255) & ~size_t(255);
+        return o;
+    };
+    c.o_desc = put(sizeof(SysAnJob) * n);
+    c.o_base = put(sizeof(uint64_t) * (n + 1));
+    c.o_jobs = put(sizeof(SysAnJob) * c.nj);
+    c.o_tabs = put(sizeof(uint32_t) * c.tab_words);
+    c.o_vars = put(sizeof(double) * c.nvars);
+    c.o_params = put(sizeof(double) * c.nexpr);
+    c.o_output = at;
+    put(analyze ? c.ncon : sizeof(double) * c.ncon);
+    c.o_work = at;
+    if (analyze) put(c.nexpr);
+    c.end = at;
+}
+
+// The warp footprint class of a drawing: its batch_analyze_warp_bytes rounded up to a power of two, at most 200 KiB.  One
+// heterogeneous launch per class, so that one large drawing does not set the shared memory (and the warps per CTA) of every
+// small one.
+static size_t an_footprint_class(uint32_t n_vars, uint32_t n_expr) {
+    const size_t bytes = batch_analyze_warp_bytes(n_vars, n_expr);
+    size_t c = 16;
+    while (c < bytes) c <<= 1;
+    return std::min<size_t>(c, 200 * 1024);
+}
+
+// Drawings [lo, hi) on one device, chunk after chunk on its stream: stage and upload; analyze: one heterogeneous launch per
+// footprint class, one launch per kind-1 structure, fk_systems_an_reduce_kernel; residuals: fk_systems_residuals_kernel;
+// download, then the chunk's counts or residuals into the call's output.
+static int systems_an_range(const std::vector<SystemsAnDrawing>& d, const SystemsAnPlan& P, int device, uint32_t lo, uint32_t hi,
+                            uint8_t* dependent, double* residuals) {
+    CU(cudaSetDevice(device));
+    SystemsDevice* D = systems_device_for(device);
+    std::lock_guard<std::mutex> lock(D->mu);
+    if (!D->stream) CU(cudaStreamCreateWithFlags(&D->stream, cudaStreamNonBlocking));
+    const cudaStream_t st = D->stream;
+    const bool analyze = dependent != nullptr;
+    const size_t ns = P.st.size();
+    // ---- chunks: drawings in order, closed at about 1 GiB (FK_SYSTEM_BATCH_CHUNK caps the drawings), at least one drawing
+    std::vector<SystemsAnChunk> chunks;
+    std::vector<uint32_t> seen(ns, kSbNone);  // the chunk that last counted a structure's tables
+    size_t h_need = 0, d_need = 0;
+    const uint32_t cap = system_batch_chunk_env();
+    for (uint32_t a = lo; a < hi;) {
+        uint32_t b = a;
+        uint64_t bytes = 0;
+        while (b < hi) {
+            const uint32_t s = P.drawing_struct[b];
+            const SystemAnBatch& B = *d[b].plan;
+            uint64_t db = sizeof(double) * ((uint64_t)B.L.n_vars + B.n_expr) + B.n_expr + 2 * sizeof(SysAnJob) + sizeof(uint64_t) +
+                          (analyze ? 1 : sizeof(double)) * (uint64_t)B.n_constraints;
+            if (seen[s] != a) db += sizeof(uint32_t) * P.st[s].tab_words;
+            if (b > a && (bytes + db > (1ull << 30) || (cap && b - a >= cap))) break;
+            seen[s] = a;
+            bytes += db;
+            b++;
+        }
+        chunks.emplace_back();
+        SystemsAnChunk& c = chunks.back();
+        c.a = a;
+        c.b = b;
+        systems_an_chunk_layout(d, P, analyze, c);
+        h_need = std::max(h_need, c.o_work);
+        d_need = std::max(d_need, c.end);
+        a = b;
+    }
+    if (D->h_cap < h_need) {
+        if (D->h) cudaFreeHost(D->h);
+        D->h = nullptr;
+        D->h_cap = 0;
+        const size_t want = h_need + h_need / 4;
+        CU(cudaMallocHost((void**)&D->h, want));
+        D->h_cap = want;
+    }
+    uint64_t d_cap = D->d_cap;
+    const int grc = systems_grow(&D->d, &d_cap, d_need + d_need / 4);
+    D->d_cap = d_cap;
+    if (grc != FK_OK) return grc;
+
+    auto run = [&](const SystemsAnChunk& c) -> int {
+        unsigned char* H = D->h;
+        unsigned char* G = D->d;
+        const uint32_t n = c.b - c.a;
+        SysAnJob* desc = (SysAnJob*)(H + c.o_desc);
+        uint64_t* base = (uint64_t*)(H + c.o_base);
+        SysAnJob* jobs = (SysAnJob*)(H + c.o_jobs);
+        uint32_t* tabs = (uint32_t*)(H + c.o_tabs);
+        double* rv = (double*)(H + c.o_vars);
+        double* rp = (double*)(H + c.o_params);
+        for (size_t s = 0; s < ns; s++) {
+            if (c.count[s] == 0) continue;
+            const SystemAnBatch& B = *P.st[s].b;
+            uint32_t* t = tabs + c.tab[s];
+            std::memcpy(t, B.L.slot_var.data(), sizeof(uint32_t) * B.L.slot_var.size());
+            std::memset(t + 8 * (size_t)B.n_expr, 0, sizeof(uint32_t) * ((B.n_expr + 3) / 4));
+            if (B.n_expr) std::memcpy(t + 8 * (size_t)B.n_expr, B.L.kind.data(), B.n_expr);
+            std::memcpy(t + 8 * (size_t)B.n_expr + (B.n_expr + 3) / 4, B.L.con_off.data(), sizeof(uint32_t) * B.L.con_off.size());
+        }
+        std::vector<uint32_t> rank(ns, 0);
+        std::vector<std::pair<size_t, uint32_t>> cls;  // (footprint class, drawing in the chunk) of every job
+        cls.reserve(c.nj);
+        uint64_t v0 = 0, e0 = 0;
+        for (uint32_t i = c.a; i < c.b; i++) {
+            const uint32_t s = P.drawing_struct[i], di = i - c.a;
+            const SystemAnBatch& B = *d[i].plan;
+            SysAnJob& J = desc[di];
+            J.tab = (uint32_t)c.tab[s];
+            J.n_vars = B.L.n_vars;
+            J.n_expr = B.n_expr;
+            J.pad = 0;
+            if (P.st[s].kind == 0) {
+                J.vars = v0;
+                J.exprs = e0;
+                v0 += B.L.n_vars;
+                e0 += B.n_expr;
+                if (B.n_expr) cls.emplace_back(an_footprint_class(B.L.n_vars, B.n_expr), di);
+            } else {
+                const uint64_t q = rank[s]++;
+                J.vars = c.vblk[s] + q * B.L.n_vars;
+                J.exprs = c.eblk[s] + q * B.n_expr;
+            }
+            if (B.L.n_vars) std::memcpy(rv + J.vars, d[i].vars, sizeof(double) * B.L.n_vars);
+            if (B.n_expr) std::memcpy(rp + J.exprs, d[i].param, sizeof(double) * B.n_expr);
+            base[di] = P.con_off[i] - P.con_off[c.a];
+        }
+        base[n] = c.ncon;
+        std::stable_sort(cls.begin(), cls.end(), [](const auto& x, const auto& y) { return x.first < y.first; });
+        for (size_t k = 0; k < cls.size(); k++) jobs[k] = desc[cls[k].second];
+        CU(cudaMemcpyAsync(G, H, c.o_output, cudaMemcpyHostToDevice, st));
+        const SysAnJob* d_desc = (const SysAnJob*)(G + c.o_desc);
+        const uint64_t* d_base = (const uint64_t*)(G + c.o_base);
+        const uint32_t* d_tabs = (const uint32_t*)(G + c.o_tabs);
+        const double* d_vars = (const double*)(G + c.o_vars);
+        const double* d_params = (const double*)(G + c.o_params);
+        int e;
+        if (!analyze) {
+            e = launch_systems_residuals(n, c.ncon, d_base, d_desc, d_tabs, d_vars, d_params, (double*)(G + c.o_output), st);
+            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_systems_residuals_kernel");
+        } else {
+            uint8_t* d_flags = G + c.o_work;
+            for (size_t k = 0; k < cls.size();) {  // one launch per footprint class
+                size_t k1 = k;
+                while (k1 < cls.size() && cls[k1].first == cls[k].first) k1++;
+                e = launch_systems_analyze((const SysAnJob*)(G + c.o_jobs) + k, (uint32_t)(k1 - k), cls[k].first, d_tabs, d_vars, d_params, d_flags, st);
+                if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_systems_analyze_kernel");
+                k = k1;
+            }
+            for (size_t s = 0; s < ns; s++) {
+                if (P.st[s].kind == 0 || c.count[s] == 0) continue;
+                const SystemAnBatch& B = *P.st[s].b;
+                AnalyzePlan plan;
+                std::string err;
+                const int prc = choose_analyze(B.L.n_vars, B.n_expr, c.count[s], device, &plan, &err);
+                if (prc != FK_OK) return fail(prc, err);
+                if (D->an_ws_bytes < plan.workspace_bytes()) {  // grow-only, within fk::kAnWorkspaceBytes
+                    CU(cudaStreamSynchronize(st));  // (an earlier launch may still use the old workspace)
+                    uint64_t have = D->an_ws_bytes;
+                    const int rc = systems_grow(&D->an_ws, &have, plan.workspace_bytes());
+                    D->an_ws_bytes = have;
+                    if (rc != FK_OK) return rc;
+                }
+                const uint32_t* slot = d_tabs + c.tab[s];
+                const uint8_t* kinds = sys_an_kinds(slot, B.n_expr);
+                const double* v = d_vars + c.vblk[s];
+                const double* q = d_params + c.eblk[s];
+                e = plan.kernel == kAnWarp ? launch_batch_analyze(B.L.n_vars, B.n_expr, kinds, slot, c.count[s], v, q, d_flags + c.eblk[s], st)
+                                           : launch_analyze(plan, B.L.n_vars, B.n_expr, kinds, slot, c.count[s], v, q, d_flags + c.eblk[s],
+                                                            D->an_ws, st);
+                if (e != 0) return cuda_fail((cudaError_t)e, plan.kernel == kAnWarp ? "launch fk_batch_analyze_kernel" : "launch fk_analyze_cta_kernel");
+            }
+            e = launch_systems_an_reduce(n, c.ncon, d_base, d_desc, d_tabs, d_flags, G + c.o_output, st);
+            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_systems_an_reduce_kernel");
+        }
+        const size_t out_bytes = (analyze ? 1 : sizeof(double)) * c.ncon;
+        if (out_bytes) CU(cudaMemcpyAsync(H + c.o_output, G + c.o_output, out_bytes, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        if (out_bytes) {
+            if (analyze) std::memcpy(dependent + P.con_off[c.a], H + c.o_output, out_bytes);
+            else std::memcpy(residuals + P.con_off[c.a], H + c.o_output, out_bytes);
+        }
+        return FK_OK;
+    };
+    for (const SystemsAnChunk& c : chunks) {
+        const int rc = run(c);
+        if (rc != FK_OK) {
+            cudaStreamSynchronize(st);  // (nothing of a failed chunk may still run when the staging is reused)
+            return rc;
+        }
+    }
+    return FK_OK;
+}
+
+int systems_an_run(const std::vector<SystemsAnDrawing>& d, uint8_t* dependent, double* residuals, int n_gpus) {
+    SystemsAnPlan P;
+    systems_an_plan_create(d, dependent != nullptr, P);
+    for (const SystemsAnPlan::Structure& S : P.st) {  // the size limit of the analyze kernels (the kernel itself is chosen per chunk)
+        if (S.kind == 0) continue;
+        int device = 0;
+        if (cudaGetDevice(&device) != cudaSuccess) device = 0;
+        AnalyzePlan plan;
+        std::string err;
+        const int rc = choose_analyze(S.b->L.n_vars, S.b->n_expr, S.instances, device, &plan, &err);
+        if (rc != FK_OK) return fail(rc, "drawing " + std::to_string(S.first_drawing) + ": " + err);
+    }
+    if (P.con_off.back() == 0) return FK_OK;
+    const int rc = clamp_gpus(n_gpus);
+    if (rc != FK_OK) return rc;
+    return shard_over_devices(n_gpus, (uint32_t)d.size(), [&](int device, uint32_t lo, uint32_t hi) {
+        return systems_an_range(d, P, device, lo, hi, dependent, residuals);
     });
 }
 

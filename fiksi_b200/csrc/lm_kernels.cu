@@ -612,15 +612,13 @@ fk_batch_eval_tiled_kernel(const DevProgram P, uint32_t n_sketches, const double
 // matrix in shared memory, lanes across the columns; every floating-point operation is the
 // reference's (multiply, then subtract; one IEEE reciprocal per pivot row), so the flags are
 // bit-for-bit those of the CPU restatement.  out[sketch][row] = 1 iff the row increased the rank.
-constexpr int kAnalyzeWarps = 4;
-__global__ void __launch_bounds__(kAnalyzeWarps * 32)
-fk_batch_analyze_kernel(uint32_t n_vars, uint32_t n_expr, const uint8_t* __restrict__ kinds, const uint32_t* __restrict__ slot_var,
-                        uint32_t n_sketches, const double* __restrict__ vars_all, const double* __restrict__ params_all,
-                        uint8_t* __restrict__ out, uint32_t warp_doubles, uint32_t warps_per_cta) {
-    extern __shared__ __align__(16) double smem_an[];
-    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t sketch = blockIdx.x * warps_per_cta + warp;
-    if (warp >= warps_per_cta || sketch >= n_sketches) return;
+// The body of both analyze warp kernels, so that their flags agree by construction: sketch `sketch` of the rows vars_all / params_all
+// (n_vars / n_expr per sketch) in the warp's slice of smem_an, its flags to out[sketch][n_expr].  The parameters keep the uniform
+// kernel's own names and arithmetic: taking pre-offset row pointers instead changes fk_batch_analyze_kernel's SASS.
+__device__ __forceinline__ void analyze_warp(uint32_t n_vars, uint32_t n_expr, const uint8_t* __restrict__ kinds,
+                                             const uint32_t* __restrict__ slot_var, uint32_t sketch, const double* __restrict__ vars_all,
+                                             const double* __restrict__ params_all, uint8_t* __restrict__ out, double* smem_an,
+                                             uint32_t warp_doubles, uint32_t warp, uint32_t lane) {
     const uint32_t m = n_expr, n = n_vars;
     double* M = smem_an + (size_t)warp * warp_doubles;
     uint32_t* ci = reinterpret_cast<uint32_t*>(M + (size_t)m * n);
@@ -696,6 +694,33 @@ fk_batch_analyze_kernel(uint32_t n_vars, uint32_t n_expr, const uint8_t* __restr
     for (uint32_t r = lane; r < m; r += 32) out[(size_t)sketch * m + r] = (uint8_t)inc[r];
 }
 
+constexpr int kAnalyzeWarps = 4;
+__global__ void __launch_bounds__(kAnalyzeWarps * 32)
+fk_batch_analyze_kernel(uint32_t n_vars, uint32_t n_expr, const uint8_t* __restrict__ kinds, const uint32_t* __restrict__ slot_var,
+                        uint32_t n_sketches, const double* __restrict__ vars_all, const double* __restrict__ params_all,
+                        uint8_t* __restrict__ out, uint32_t warp_doubles, uint32_t warps_per_cta) {
+    extern __shared__ __align__(16) double smem_an[];
+    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t sketch = blockIdx.x * warps_per_cta + warp;
+    if (warp >= warps_per_cta || sketch >= n_sketches) return;
+    analyze_warp(n_vars, n_expr, kinds, slot_var, sketch, vars_all, params_all, out, smem_an, warp_doubles, warp, lane);
+}
+
+// fk_systems_analyze: one warp per job, every job its own drawing (sizes, tables, rows); one footprint class per launch.
+__global__ void __launch_bounds__(kAnalyzeWarps * 32)
+fk_systems_analyze_kernel(const SysAnJob* __restrict__ jobs, uint32_t n_jobs, const uint32_t* __restrict__ tabs,
+                          const double* __restrict__ vars, const double* __restrict__ params, uint8_t* __restrict__ flags,
+                          uint32_t warp_doubles, uint32_t warps_per_cta) {
+    extern __shared__ __align__(16) double smem_an[];
+    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t j = blockIdx.x * warps_per_cta + warp;
+    if (warp >= warps_per_cta || j >= n_jobs) return;
+    const SysAnJob J = jobs[j];
+    const uint32_t* slot_var = tabs + J.tab;
+    analyze_warp(J.n_vars, J.n_expr, sys_an_kinds(slot_var, J.n_expr), slot_var, 0, vars + J.vars, params + J.exprs, flags + J.exprs,
+                 smem_an, warp_doubles, warp, lane);
+}
+
 size_t batch_analyze_warp_bytes(uint32_t n_vars, uint32_t n_expr) {
     return (((size_t)n_expr * n_vars * sizeof(double) + ((size_t)n_vars + n_expr) * sizeof(uint32_t)) + 15) & ~(size_t)15;
 }
@@ -713,6 +738,19 @@ int launch_batch_analyze(uint32_t n_vars, uint32_t n_expr, const uint8_t* kinds,
     const uint32_t grid = (n_sketches + wpc - 1) / wpc;
     fk_batch_analyze_kernel<<<grid, kAnalyzeWarps * 32, smem, (cudaStream_t)stream>>>(n_vars, n_expr, kinds, slot_var, n_sketches, vars, params, out,
                                                                                        (uint32_t)(per_warp / sizeof(double)), wpc);
+    return (int)cudaGetLastError();
+}
+
+int launch_systems_analyze(const SysAnJob* jobs, uint32_t n_jobs, size_t warp_bytes, const uint32_t* tabs, const double* vars,
+                           const double* params, uint8_t* flags, void* stream) {
+    if (n_jobs == 0) return 0;
+    if (warp_bytes > 200 * 1024 || warp_bytes % 16) return (int)cudaErrorInvalidConfiguration;
+    const uint32_t wpc = (uint32_t)std::max<size_t>(1, std::min<size_t>(kAnalyzeWarps, (200 * 1024) / warp_bytes));
+    const size_t smem = warp_bytes * wpc;
+    cudaError_t e = cudaFuncSetAttribute(fk_systems_analyze_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    fk_systems_analyze_kernel<<<(n_jobs + wpc - 1) / wpc, kAnalyzeWarps * 32, smem, (cudaStream_t)stream>>>(
+        jobs, n_jobs, tabs, vars, params, flags, (uint32_t)(warp_bytes / sizeof(double)), wpc);
     return (int)cudaGetLastError();
 }
 

@@ -72,6 +72,24 @@ size_t batch_analyze_warp_bytes(uint32_t n_vars, uint32_t n_expr);
 bool batch_analyze_warp_fits(uint32_t n_vars, uint32_t n_expr);
 int launch_batch_analyze(uint32_t n_vars, uint32_t n_expr, const uint8_t* kinds, const uint32_t* slot_var, uint32_t n_sketches,
                          const double* vars, const double* params, uint8_t* out, void* stream);
+// fk_systems_analyze: one drawing of a call over many different drawings.  Its tables start at tabs + tab: slot_var[n_expr][8],
+// the kinds (n_expr bytes, padded to whole words), con_off[n_constraints + 1] (the constraints' expression ranges).  vars: offset of
+// its variable row; exprs: offset of its parameter row and of its flags (one per expression in both).
+struct SysAnJob {
+    uint64_t vars, exprs;
+    uint32_t tab, n_vars, n_expr, pad;
+};
+__host__ __device__ inline const uint8_t* sys_an_kinds(const uint32_t* slot_var, uint32_t n_expr) {
+    return reinterpret_cast<const uint8_t*>(slot_var + 8 * (size_t)n_expr);
+}
+__host__ __device__ inline const uint32_t* sys_an_con_off(const uint32_t* slot_var, uint32_t n_expr) {
+    return slot_var + 8 * (size_t)n_expr + (n_expr + 3) / 4;
+}
+// The analyze warp kernel over n_jobs different drawings, jobs[j] one warp each: flags[J.exprs + r] = 1 iff row r increased the
+// rank, as launch_batch_analyze's flags.  warp_bytes: every job's shared memory (at least its batch_analyze_warp_bytes, a
+// multiple of 16, at most 200 KiB); warps per CTA as launch_batch_analyze takes them for that footprint.
+int launch_systems_analyze(const SysAnJob* jobs, uint32_t n_jobs, size_t warp_bytes, const uint32_t* tabs, const double* vars,
+                           const double* params, uint8_t* flags, void* stream);
 // L-BFGS on a uniform batch (tile paths with 4 / 8 / 16 / 32 lanes only); d_jcolptr[n+1], d_jrow[jnnz]: CSC
 // of the Jacobian.  Returns cudaErrorInvalidConfiguration when the topology does not take a tile path.
 // batch_lbfgs_tile_fits: whether it takes a topology with these sizes and lanes (host only).

@@ -1185,9 +1185,65 @@ int systems_drawings(uint32_t n, fk_system* const* systems, const fk_solving_opt
     return FK_OK;
 }
 
+// fk_systems_analyze / _residuals / _analyze_layout: the FK_ERR_INVALID refusals (before any device work) and every drawing's
+// analyze plan.  The same system may appear more than once: nothing is written into a system.  *total: the constraints of all.
+int systems_an_drawings(uint32_t n, const fk_system* const* systems, std::vector<fk::SystemsAnDrawing>& d,
+                        std::vector<std::shared_ptr<fk::SystemAnBatch>>& plans, uint64_t* total) {
+    if (n && !systems) return fk::system_batch_fail(FK_ERR_INVALID, "null systems");
+    *total = 0;
+    for (uint32_t i = 0; i < n; i++) {
+        if (!systems[i]) return fk::system_batch_fail(FK_ERR_INVALID, "null system at index " + std::to_string(i));
+        *total += systems[i]->constrs.size();
+    }
+    plans.resize(n);
+    d.resize(n);
+    for (uint32_t i = 0; i < n; i++) {
+        const int rc = analyze_batch_plan_for(systems[i], &plans[i]);
+        if (rc != FK_OK) return rc;
+        d[i] = {plans[i].get(), systems[i]->vars.data(), systems[i]->param.data()};
+    }
+    return FK_OK;
+}
+
+int systems_an_call(uint32_t n, const fk_system* const* systems, uint8_t* dependent, double* residuals, uint64_t cap, int n_gpus) {
+    std::vector<fk::SystemsAnDrawing> d;
+    std::vector<std::shared_ptr<fk::SystemAnBatch>> plans;
+    uint64_t total = 0;
+    const int rc = systems_an_drawings(n, systems, d, plans, &total);
+    if (rc != FK_OK) return rc;
+    if (total && !dependent && !residuals) return fk::system_batch_fail(FK_ERR_INVALID, "null output");
+    if (cap < total)
+        return fk::system_batch_fail(FK_ERR_INVALID, "output capacity " + std::to_string(cap) + " is below the " + std::to_string(total) +
+                                                         " constraints of the drawings");
+    return fk::systems_an_run(d, dependent, residuals, n_gpus);
+}
+
 }  // namespace
 
 extern "C" {
+
+int fk_systems_analyze(uint32_t n, const fk_system* const* systems, uint8_t* dependent, uint64_t cap, int n_gpus) {
+    return systems_an_call(n, systems, dependent, nullptr, cap, n_gpus);
+}
+
+int fk_systems_residuals(uint32_t n, const fk_system* const* systems, double* out, uint64_t cap, int n_gpus) {
+    return systems_an_call(n, systems, nullptr, out, cap, n_gpus);
+}
+
+int fk_systems_analyze_layout(uint32_t n, const fk_system* const* systems, uint32_t* n_structures, uint32_t* instances,
+                              uint32_t* launch_kind) {
+    std::vector<fk::SystemsAnDrawing> d;
+    std::vector<std::shared_ptr<fk::SystemAnBatch>> plans;
+    uint64_t total = 0;
+    const int rc = systems_an_drawings(n, systems, d, plans, &total);
+    if (rc != FK_OK) return rc;
+    std::vector<uint32_t> inst, kind;
+    fk::systems_an_layout(d, &inst, &kind);
+    if (n_structures) *n_structures = (uint32_t)inst.size();
+    if (instances) std::copy(inst.begin(), inst.end(), instances);
+    if (launch_kind) std::copy(kind.begin(), kind.end(), launch_kind);
+    return FK_OK;
+}
 
 int fk_systems_layout(uint32_t n, fk_system* const* systems, const fk_solving_options* opts, uint32_t* n_components, uint32_t* n_structures,
                       uint32_t* instances, uint32_t* launch_kind) {

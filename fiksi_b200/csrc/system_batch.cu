@@ -5,12 +5,14 @@
 // scaled rows) and move values between the waves of sets or steps with fk_system_sp_gather_scatter_kernel.
 // fk_system_batch_analyze and fk_system_batch_residuals expand the variants' parameter rows, then reduce the analyze flags
 // per constraint or evaluate every constraint's residual.  fk_systems_solve (n different drawings) has its own prepare and
-// scatter kernels over ragged rows: every drawing its own size, every component its own destination.
+// scatter kernels over ragged rows: every drawing its own size, every component its own destination.  fk_systems_analyze and
+// fk_systems_residuals reduce the flags or evaluate the residuals over ragged drawings, one thread per constraint.
 #include <cuda_runtime.h>
 
 #include <algorithm>
 
 #include "expressions.cuh"
+#include "lm_kernels.cuh"
 #include "prepare.cuh"
 #include "system_batch.cuh"
 
@@ -310,9 +312,25 @@ fk_system_an_reduce_kernel(uint32_t n, uint32_t n_expr, uint32_t n_constraints, 
     }
 }
 
-// out[v][c] = calculate_residual (constraints/mod.rs:88-110) of constraint c in variant v, as fk_system_residuals combines the
-// expression residuals: a one-expression constraint its residual, otherwise q += r * r in expression order, then sqrt(q).
+// calculate_residual (constraints/mod.rs:88-110) of the constraint owning expressions [e0, e1), as fk_system_residuals combines
+// the expression residuals: a one-expression constraint its residual, otherwise q += r * r in expression order, then sqrt(q).
 // The slots are read as the analyze kernels read them (slot_var[e][8], arity_of), the residual is eval_expression's.
+__device__ __forceinline__ double constraint_residual(const uint8_t* __restrict__ kinds, const uint32_t* __restrict__ slot_var, uint32_t e0,
+                                                      uint32_t e1, const double* __restrict__ vars, const double* __restrict__ params) {
+    double q = 0.0, r = 0.0;
+    for (uint32_t e = e0; e < e1; e++) {
+        const int kind = (int)__ldg(kinds + e);
+        const int ar = dev::arity_of(kind);
+        double x[8], g[8];
+#pragma unroll
+        for (int sl = 0; sl < 8; sl++) x[sl] = sl < ar ? __ldg(vars + __ldg(slot_var + (size_t)e * 8 + sl)) : 0.0;
+        r = dev::eval_expression(kind, x, __ldg(params + e), g);
+        q += r * r;
+    }
+    return e1 - e0 > 1 ? sqrt(q) : r;
+}
+
+// out[v][c] = constraint_residual of constraint c in variant v.
 __global__ void __launch_bounds__(256)
 fk_system_residuals_kernel(uint32_t n, uint32_t n_vars, uint32_t n_expr, uint32_t n_constraints, const uint8_t* __restrict__ kinds,
                            const uint32_t* __restrict__ slot_var, const uint32_t* __restrict__ con_off, const double* __restrict__ vt,
@@ -321,19 +339,54 @@ fk_system_residuals_kernel(uint32_t n, uint32_t n_vars, uint32_t n_expr, uint32_
     for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < (uint64_t)n * n_constraints; i += stride) {
         const uint64_t v = i / n_constraints;
         const uint32_t c = (uint32_t)(i - v * n_constraints);
-        const double* vars = vt + v * n_vars;
-        const uint32_t e0 = __ldg(con_off + c), e1 = __ldg(con_off + c + 1);
-        double q = 0.0, r = 0.0;
-        for (uint32_t e = e0; e < e1; e++) {
-            const int kind = (int)__ldg(kinds + e);
-            const int ar = dev::arity_of(kind);
-            double x[8], g[8];
-#pragma unroll
-            for (int sl = 0; sl < 8; sl++) x[sl] = sl < ar ? __ldg(vars + __ldg(slot_var + (size_t)e * 8 + sl)) : 0.0;
-            r = dev::eval_expression(kind, x, __ldg(pt + v * n_expr + e), g);
-            q += r * r;
-        }
-        out[i] = e1 - e0 > 1 ? sqrt(q) : r;
+        out[i] = constraint_residual(kinds, slot_var, __ldg(con_off + c), __ldg(con_off + c + 1), vt + v * n_vars, pt + v * n_expr);
+    }
+}
+
+// ---- fk_systems_analyze / fk_systems_residuals: n different drawings, one thread per constraint of the chunk --------------
+// The drawing of the chunk's constraint i: the last d < n with con_base[d] <= i (con_base[0] = 0 <= i < con_base[n]; a drawing
+// without constraints shares its con_base with the next one and is skipped).
+__device__ __forceinline__ uint32_t systems_drawing_of(const uint64_t* __restrict__ con_base, uint32_t n, uint64_t i) {
+    uint32_t lo = 0, hi = n;
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) / 2;
+        if (__ldg(con_base + mid) <= i) lo = mid;
+        else hi = mid;
+    }
+    return lo;
+}
+
+// dependent[i] = the expressions of the chunk's constraint i that analyze found dependent (zero flags of its drawing).
+__global__ void __launch_bounds__(256)
+fk_systems_an_reduce_kernel(uint32_t n, uint64_t total, const uint64_t* __restrict__ con_base, const SysAnJob* __restrict__ drawings,
+                            const uint32_t* __restrict__ tabs, const uint8_t* __restrict__ flags, uint8_t* __restrict__ dependent) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < total; i += stride) {
+        const uint32_t d = systems_drawing_of(con_base, n, i);
+        const SysAnJob D = drawings[d];
+        const uint32_t c = (uint32_t)(i - __ldg(con_base + d));
+        const uint32_t* con_off = sys_an_con_off(tabs + D.tab, D.n_expr);
+        const uint8_t* f = flags + D.exprs;
+        uint32_t k = 0;
+        for (uint32_t e = __ldg(con_off + c), end = __ldg(con_off + c + 1); e < end; e++) k += f[e] ? 0u : 1u;
+        dependent[i] = (uint8_t)k;
+    }
+}
+
+// out[i] = constraint_residual of the chunk's constraint i on its drawing's rows.
+__global__ void __launch_bounds__(256)
+fk_systems_residuals_kernel(uint32_t n, uint64_t total, const uint64_t* __restrict__ con_base, const SysAnJob* __restrict__ drawings,
+                            const uint32_t* __restrict__ tabs, const double* __restrict__ vars, const double* __restrict__ params,
+                            double* __restrict__ out) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < total; i += stride) {
+        const uint32_t d = systems_drawing_of(con_base, n, i);
+        const SysAnJob D = drawings[d];
+        const uint32_t c = (uint32_t)(i - __ldg(con_base + d));
+        const uint32_t* slot_var = tabs + D.tab;
+        const uint32_t* con_off = sys_an_con_off(slot_var, D.n_expr);
+        out[i] = constraint_residual(sys_an_kinds(slot_var, D.n_expr), slot_var, __ldg(con_off + c), __ldg(con_off + c + 1), vars + D.vars,
+                                     params + D.exprs);
     }
 }
 
@@ -360,6 +413,20 @@ int launch_system_residuals(uint32_t n, uint32_t n_vars, uint32_t n_expr, uint32
     if (total == 0) return 0;
     fk_system_residuals_kernel<<<grid_for(total), 256, 0, (cudaStream_t)stream>>>(n, n_vars, n_expr, n_constraints, kinds, slot_var, con_off,
                                                                                   vt, pt, out);
+    return (int)cudaGetLastError();
+}
+
+int launch_systems_an_reduce(uint32_t n, uint64_t total, const uint64_t* con_base, const SysAnJob* drawings, const uint32_t* tabs,
+                             const uint8_t* flags, uint8_t* dependent, void* stream) {
+    if (total == 0) return 0;
+    fk_systems_an_reduce_kernel<<<grid_for(total), 256, 0, (cudaStream_t)stream>>>(n, total, con_base, drawings, tabs, flags, dependent);
+    return (int)cudaGetLastError();
+}
+
+int launch_systems_residuals(uint32_t n, uint64_t total, const uint64_t* con_base, const SysAnJob* drawings, const uint32_t* tabs,
+                             const double* vars, const double* params, double* out, void* stream) {
+    if (total == 0) return 0;
+    fk_systems_residuals_kernel<<<grid_for(total), 256, 0, (cudaStream_t)stream>>>(n, total, con_base, drawings, tabs, vars, params, out);
     return (int)cudaGetLastError();
 }
 

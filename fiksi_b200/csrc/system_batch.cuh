@@ -144,6 +144,15 @@ int launch_system_an_reduce(uint32_t n, uint32_t n_expr, uint32_t n_constraints,
 // out[v][c] = fk_system_residuals of variant v (rows vt[v][n_vars], pt[v][n_expr]).
 int launch_system_residuals(uint32_t n, uint32_t n_vars, uint32_t n_expr, uint32_t n_constraints, const uint8_t* kinds, const uint32_t* slot_var,
                             const uint32_t* con_off, const double* vt, const double* pt, double* out, void* stream);
+// fk_systems_analyze / fk_systems_residuals over the chunk's n drawings (SysAnJob, lm_kernels.cuh: its tables in `tabs`, its rows
+// and flags), the chunk's constraints in drawing order: drawing d owns constraints [con_base[d], con_base[d + 1]), total =
+// con_base[n].  dependent[i] = the dependent expressions of constraint i (zero flags); out[i] = its residual, as
+// launch_system_residuals evaluates it.
+struct SysAnJob;
+int launch_systems_an_reduce(uint32_t n, uint64_t total, const uint64_t* con_base, const SysAnJob* drawings, const uint32_t* tabs,
+                             const uint8_t* flags, uint8_t* dependent, void* stream);
+int launch_systems_residuals(uint32_t n, uint64_t total, const uint64_t* con_base, const SysAnJob* drawings, const uint32_t* tabs,
+                             const double* vars, const double* params, double* out, void* stream);
 struct SystemAnBatch;
 int system_an_batch_create(SystemAnLayout&& layout, std::shared_ptr<SystemAnBatch>* out);
 struct SystemAnCall {
@@ -158,6 +167,21 @@ struct SystemAnCall {
 };
 // Refusals (analyze: choose_analyze's size limit) before any device work, then the chunks on every device.
 int system_an_batch_run(SystemAnBatch& b, const SystemAnCall& call);
+
+// fk_systems_analyze / fk_systems_residuals: System::analyze and calculate_residual over n different drawings, each with its own
+// SystemAnBatch plan.  capi.cu merges equal plans into structures, runs chunks of drawings and returns every drawing's counts or
+// residuals (drawing after drawing, constraint order); system.cpp validates the call.
+struct SystemsAnDrawing {
+    const SystemAnBatch* plan;
+    const double* vars;   // [plan n_vars]
+    const double* param;  // [plan n_expr]
+};
+// Host-only: per distinct structure (order of first appearance) its instances and analyze launch kind (0 heterogeneous warp
+// launch, 1 one launch of the kernel choose_analyze picks).
+void systems_an_layout(const std::vector<SystemsAnDrawing>& d, std::vector<uint32_t>* instances, std::vector<uint32_t>* launch_kind);
+// Exactly one of dependent / residuals is set, with room for every constraint of every drawing.  Refusals (analyze: a drawing
+// beyond choose_analyze's limit) before any device work.
+int systems_an_run(const std::vector<SystemsAnDrawing>& d, uint8_t* dependent, double* residuals, int n_gpus);
 
 // fk_systems_solve: System::solve over n different drawings, each with its own SystemBatch plan (its components, grouped by
 // structure inside the drawing).  capi.cu merges the structures of all drawings, runs chunks of drawings and returns every

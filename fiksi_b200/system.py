@@ -293,3 +293,44 @@ def solve_systems(systems, optimizer="lm", perturb=True, n_gpus=1):
                                  int(n_gpus)))
     ends = np.cumsum(solved[:n])
     return [reps[e - k:e].copy() for e, k in zip(ends.tolist(), solved[:n].tolist())]
+
+
+def _handles(systems):
+    return (C.c_void_p * max(len(systems), 1))(*[s._h for s in systems])
+
+
+def systems_analyze_layout(systems):
+    """(distinct analyze structures across the drawings, [instances per structure], [launch kind per structure: 0 heterogeneous
+    warp launch, 1 one launch of the kernel choose_analyze picks]) of analyze_systems' plan (host only,
+    fk_systems_analyze_layout)."""
+    handles = _handles(systems)
+    ns = C.c_uint32(0)
+    check(lib().fk_systems_analyze_layout(len(systems), handles, C.byref(ns), None, None))
+    inst = np.zeros(max(ns.value, 1), np.uint32)
+    kind = np.zeros(max(ns.value, 1), np.uint32)
+    check(lib().fk_systems_analyze_layout(len(systems), handles, C.byref(ns), ptr(inst, C.c_uint32), ptr(kind, C.c_uint32)))
+    return int(ns.value), inst[:ns.value].tolist(), kind[:ns.value].tolist()
+
+
+def _ragged(systems, out):
+    ends = np.cumsum([s.num_constraints() for s in systems], dtype=np.int64)
+    return [out[e - s.num_constraints():e].copy() for e, s in zip(ends.tolist(), systems)]
+
+
+def analyze_systems(systems, n_gpus=1):
+    """System.analyze() of every system in `systems` (different drawings) in one call (fk_systems_analyze).  Returns one uint8
+    array per system: how many of each constraint's expressions were found dependent, so that system i's analyze() is
+    np.repeat(np.arange(num_constraints), counts[i]).  No system is modified; the same system may appear more than once."""
+    total = sum(s.num_constraints() for s in systems)
+    out = np.zeros(max(total, 1), np.uint8)
+    check(lib().fk_systems_analyze(len(systems), _handles(systems), ptr(out, C.c_uint8), total, int(n_gpus)))
+    return _ragged(systems, out)
+
+
+def systems_residuals(systems, n_gpus=1):
+    """System.residuals() of every system in `systems` (different drawings) in one call (fk_systems_residuals).  Returns one
+    float64 array per system.  No system is modified; the same system may appear more than once."""
+    total = sum(s.num_constraints() for s in systems)
+    out = np.zeros(max(total, 1))
+    check(lib().fk_systems_residuals(len(systems), _handles(systems), ptr(out, C.c_double), total, int(n_gpus)))
+    return _ragged(systems, out)

@@ -585,6 +585,37 @@ FK_API int fk_system_batch_analyze(const fk_system* s, uint32_t n, const double*
  * fk_system_residuals combines a coincidence).  Every drawing size is taken: no topology, batch plan or front limit. */
 FK_API int fk_system_batch_residuals(const fk_system* s, uint32_t n, const double* vars, const double* params,
                                      double* out /* [n][n_constraints] */, int n_gpus);
+/* == System::analyze on each of n different drawings in one call.  dependent[]: the constraints of systems[0] in constraint
+ * order, then those of systems[1], ... (sum of fk_system_num_constraints entries); entry = how many of that constraint's
+ * expressions were found dependent.  For drawing i, every constraint c ascending, repeated its entry times, is exactly the
+ * list fk_system_analyze(systems[i]) returns: bit for bit, quirks included (rows beyond min(n_expressions, n_variables) are
+ * never examined and count as dependent; every variable is a column, fixed or not).  NaN and inf stay inside their own
+ * drawing.  No system is modified, so the same system may appear more than once.
+ * Each drawing keeps fk_system_batch_analyze's plan.  Per call, drawings with equal plans (variables, expression kinds, slot
+ * tables, constraint ranges: fixing an element changes none of them) are one structure.  A structure of fewer than 64
+ * drawings whose matrix fits one warp (200 KiB of shared memory) joins the heterogeneous warp launch of its chunk (one warp per
+ * drawing, one launch per footprint class: the warp's bytes rounded up to a power of two); any other gets one launch of the
+ * kernel choose_analyze picks for its drawings in the chunk (FK_ANALYZE_KERNEL honoured: cta or group sends every structure
+ * there).  On the device, per chunk of
+ * drawings on one stream per device: one copy up of the descriptors, tables and rows, the analyze launches, one kernel counts
+ * each constraint's dependent expressions, one copy down.  Drawings go in order in chunks of about 1 GiB of device buffers
+ * (FK_SYSTEM_BATCH_CHUNK caps the drawings per chunk), sharded by count over n_gpus devices (0 == all visible).
+ * Refusals come before any device work and leave `dependent` untouched: FK_ERR_INVALID for null `systems` with n > 0, a null
+ * entry (the message names its index), a null `dependent` with a non-empty total, or `cap` below the total (the message names
+ * it); FK_ERR_TOO_LARGE for a drawing beyond choose_analyze's limit, with "drawing i: " and choose_analyze's message.  n == 0
+ * and drawings without constraints return FK_OK. */
+FK_API int fk_systems_analyze(uint32_t n, const fk_system* const* systems, uint8_t* dependent, uint64_t cap, int n_gpus);
+/* == calculate_residual of every constraint of each of n different drawings in one call, in fk_systems_analyze's ragged
+ * layout: out[] holds bit for bit what fk_system_residuals(systems[i]) writes, on both of its paths.  Plan, chunks, devices,
+ * no modification and FK_ERR_INVALID as fk_systems_analyze; one kernel evaluates every constraint of the chunk (q += r * r in
+ * expression order, then sqrt, as fk_system_batch_residuals).  Every drawing size is taken. */
+FK_API int fk_systems_residuals(uint32_t n, const fk_system* const* systems, double* out, uint64_t cap, int n_gpus);
+/* Host-only probe of fk_systems_analyze's plan (no device needed): distinct analyze structures across the drawings, and per
+ * structure (order of first appearance) its instance count and launch kind (0 heterogeneous warp launch, 1 one launch of the
+ * kernel choose_analyze picks).  instances[n_structures] and launch_kind[n_structures] may be NULL; refusals as
+ * fk_systems_analyze's for null systems. */
+FK_API int fk_systems_analyze_layout(uint32_t n, const fk_system* const* systems, uint32_t* n_structures, uint32_t* instances,
+                                     uint32_t* launch_kind);
 FK_API uint32_t fk_system_num_components(const fk_system* s);
 FK_API int fk_system_component(const fk_system* s, uint32_t index, uint32_t* n_elements, uint32_t* elements,
                                uint32_t* n_constraints, uint32_t* constraints);

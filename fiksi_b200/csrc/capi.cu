@@ -46,6 +46,60 @@ int cuda_fail(cudaError_t e, const char* what) {
         if (e_ != cudaSuccess) return cuda_fail(e_, #call); \
     } while (0)
 
+// Grow-only buffer of T on one device: device memory, or pinned host memory.  reserve(need, alloc) replaces it (the contents are
+// lost) by one of `alloc` elements (default `need`, at least one) when it holds fewer than `need` or nothing yet.  Freed on its
+// device with its owner.
+template <class T>
+class GrowBuf {
+public:
+    explicit GrowBuf(bool pinned = false) : pinned_(pinned) {}
+    GrowBuf(const GrowBuf&) = delete;
+    GrowBuf& operator=(const GrowBuf&) = delete;
+    ~GrowBuf() {
+        if (!p_) return;
+        cudaSetDevice(device_);
+        release();
+    }
+    bool holds(size_t need) const { return p_ && cap_ >= need; }
+    int reserve(size_t need, size_t alloc = 0) {
+        if (holds(need)) return FK_OK;
+        release();
+        const size_t count = std::max<size_t>({need, alloc, 1});
+        const cudaError_t e = pinned_ ? cudaMallocHost((void**)&p_, sizeof(T) * count) : cudaMalloc((void**)&p_, sizeof(T) * count);
+        if (e != cudaSuccess) {
+            p_ = nullptr;
+            return cuda_fail(e, pinned_ ? "cudaMallocHost" : "cudaMalloc");
+        }
+        cudaGetDevice(&device_);
+        cap_ = count;
+        return FK_OK;
+    }
+    T* get() const { return p_; }
+    operator T*() const { return p_; }
+
+private:
+    void release() {
+        if (p_) pinned_ ? cudaFreeHost(p_) : cudaFree(p_);
+        p_ = nullptr;
+        cap_ = 0;
+    }
+    T* p_ = nullptr;
+    size_t cap_ = 0;
+    int device_ = 0;
+    bool pinned_;
+};
+
+// Regions of a staging block one after the other, each at a 256-byte boundary and at least one byte long: put(bytes) returns a
+// region's offset, `end` is the size of the block so far.
+struct BlockLayout {
+    size_t end = 0;
+    size_t put(size_t bytes) {
+        const size_t o = end;
+        end = (end + std::max<size_t>(bytes, 1) + 255) & ~size_t(255);
+        return o;
+    }
+};
+
 int usable_devices() {
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess) {
@@ -194,24 +248,76 @@ int upload_program(const fk::Topology& t, int device, DeviceProgram& out) {
     return FK_OK;
 }
 
-// The batched LM kernel of a topology, chosen in this one place: on the global sparse path the one-CTA-per-sketch kernel
-// over the supernodal tree (workspace `ws` with room for `ws_ctas` CTAs, see alloc_lm_workspace), launch_batch_lm's
-// tile / sketch-per-thread kernels otherwise.
-int launch_lm(const DeviceProgram& full, uint32_t n, const double* vars, const double* params, double* out, fk_report* reps,
-              double* ws, uint32_t ws_ctas, cudaStream_t st) {
-    if (full.sparse_batch) return full.sparse_batch->launch(n, vars, params, out, reps, ws, ws_ctas, st);
-    return fk::launch_batch_lm(full.view, n, vars, params, out, reps, st);
+// The batched solve kernels (solve_kernel picks one for a topology and an optimizer): LM -- on the global sparse path the
+// one-CTA-per-sketch kernel over the supernodal tree, launch_batch_lm's tile / sketch-per-thread kernels otherwise --, the L-BFGS
+// tile kernel (state in shared memory) and the L-BFGS CTA kernel (state in global memory).
+enum SolveKernel { kSolveLm, kSolveLbfgsTile, kSolveLbfgsCta };
+
+// The grow-only workspaces of the solve kernels that need one: the sparse batch LM kernel and the L-BFGS CTA kernel.  A workspace
+// serves one stream: two launches that may run at the same time need two.
+struct SolveWorkspace {
+    GrowBuf<double> lm, lbfgs;
+    // Room for one launch of `kernel` over n sketches of `full`: per-CTA workspaces for min(n, resident CTAs) CTAs, within the
+    // kernel's workspace limit (*ctas: that CTA count).  Nothing when it already has the room, or for a kernel without workspace.
+    int reserve(const DeviceProgram& full, SolveKernel kernel, uint32_t n, uint32_t* ctas = nullptr) {
+        if (kernel == kSolveLm && full.sparse_batch) {
+            const uint32_t c = full.sparse_batch->workspace_ctas(n);
+            if (ctas) *ctas = c;
+            return lm.reserve(full.sparse_batch->workspace_doubles(c));
+        }
+        if (kernel == kSolveLbfgsCta) {
+            const uint32_t c = fk::lbfgs_workspace_ctas(full.view, n);
+            if (c == 0) return fail(FK_ERR_CUDA, "occupancy query of fk_lbfgs_cta_kernel failed");
+            if (ctas) *ctas = c;
+            return lbfgs.reserve(fk::lbfgs_workspace_doubles(full.view, c));
+        }
+        return FK_OK;
+    }
+};
+
+// One launch of `kernel` over n sketches of `full` (vars[n][n_vars], params[n][n_expr] -> out[n][n_free], reps[n]) on st, its
+// workspace reserved in ws first.
+int solve_launch(const DeviceProgram& full, SolveKernel kernel, uint32_t n, const double* vars, const double* params, double* out,
+                 fk_report* reps, SolveWorkspace& ws, cudaStream_t st) {
+    if (kernel == kSolveLbfgsCta && n == 0) return FK_OK;
+    uint32_t ctas = 0;
+    const int rc = ws.reserve(full, kernel, n, &ctas);
+    if (rc != FK_OK) return rc;
+    int e;
+    switch (kernel) {
+        case kSolveLm:
+            e = full.sparse_batch ? full.sparse_batch->launch(n, vars, params, out, reps, ws.lm, ctas, st)
+                                  : fk::launch_batch_lm(full.view, n, vars, params, out, reps, st);
+            return e != 0 ? cuda_fail((cudaError_t)e, "launch batched LM kernel") : FK_OK;
+        case kSolveLbfgsTile:
+            e = fk::launch_batch_lbfgs(full.view, full.jcolptr, full.jrow, n, vars, params, out, reps, st);
+            if (e == (int)cudaErrorInvalidConfiguration) return fail(FK_ERR_TOO_LARGE, "the L-BFGS state of one sketch does not fit the tile path");
+            return e != 0 ? cuda_fail((cudaError_t)e, "launch fk_batch_lbfgs_kernel") : FK_OK;
+        default:
+            e = fk::launch_lbfgs_cta(full.view, full.jcolptr, full.jrow, n, vars, params, out, reps, ws.lbfgs, ctas, st);
+            if (e == (int)cudaErrorInvalidConfiguration) return fail(FK_ERR_TOO_LARGE, "more than 2^24 Jacobian entries");
+            return e != 0 ? cuda_fail((cudaError_t)e, "launch fk_lbfgs_cta_kernel") : FK_OK;
+    }
 }
 
-// Workspace of launch_lm for launches of up to `capacity` sketches (nothing off the global sparse path): per-CTA workspaces
-// for min(capacity, resident CTAs) CTAs, within fk::kSbWorkspaceBytes.  Two launches that may run at the same time need two
-// workspaces.
-int alloc_lm_workspace(const DeviceProgram& full, uint32_t capacity, double** ws, uint32_t* ws_ctas) {
-    if (!full.sparse_batch) return FK_OK;
-    const uint32_t ctas = full.sparse_batch->workspace_ctas(capacity);
-    CU(cudaMalloc(ws, sizeof(double) * full.sparse_batch->workspace_doubles(ctas)));
-    *ws_ctas = ctas;
-    return FK_OK;
+// One analyze launch over n sketches (kinds, slot table, vars[n][n_vars], params[n][n_expr] -> out[n][n_expr]) on `device`'s
+// stream st: the kernel choose_analyze picks for n, with its workspace in the grow-only ws.  The stream is synchronised before a
+// smaller workspace is freed, since an earlier launch on it may still use that one.
+int analyze_launch(uint32_t n_vars, uint32_t n_expr, const uint8_t* kinds, const uint32_t* slot, uint32_t n, const double* vars,
+                   const double* params, uint8_t* out, int device, GrowBuf<double>& ws, cudaStream_t st) {
+    fk::AnalyzePlan plan;
+    std::string err;
+    int rc = fk::choose_analyze(n_vars, n_expr, n, device, &plan, &err);
+    if (rc != FK_OK) return fail(rc, err);
+    const size_t need = plan.workspace_bytes() / sizeof(double);  // (within fk::kAnWorkspaceBytes)
+    if (need && !ws.holds(need)) {
+        CU(cudaStreamSynchronize(st));
+        if ((rc = ws.reserve(need)) != FK_OK) return rc;
+    }
+    const bool warp = plan.kernel == fk::kAnWarp;
+    const int e = warp ? fk::launch_batch_analyze(n_vars, n_expr, kinds, slot, n, vars, params, out, st)
+                       : fk::launch_analyze(plan, n_vars, n_expr, kinds, slot, n, vars, params, out, ws, st);
+    return e != 0 ? cuda_fail((cudaError_t)e, warp ? "launch fk_batch_analyze_kernel" : "launch fk_analyze_cta_kernel") : FK_OK;
 }
 
 }  // namespace
@@ -234,13 +340,9 @@ struct DevicePipeline {
     cudaStream_t streams[kStreams] = {};
     // small requests (one sketch, a handful): one pinned staging block, one device block, one copy each way
     static constexpr size_t kSmallBytes = 64 * 1024;
-    unsigned char* small_h = nullptr;
-    unsigned char* small_d = nullptr;
+    GrowBuf<unsigned char> small_h{true}, small_d;
     cudaStream_t small_stream = nullptr;
-    double* small_ws = nullptr;  // launch_lm workspace of the small requests (global sparse path)
-    uint32_t small_ws_ctas = 0;
-    double* small_lb_ws = nullptr;  // L-BFGS CTA kernel workspace of the small requests
-    uint32_t small_lb_ws_ctas = 0;
+    SolveWorkspace small_ws;
     bool plans_lm = false;  // the plans were created for LM too
     cudaEvent_t shared_param_ev = nullptr;  // fk_batch_system_solve with one parameter row for all sketches: its upload, once per call
     // Every call on the chunk pipeline takes a token.  Its parity picks the call's copy of the shared parameter row and the events
@@ -260,15 +362,13 @@ struct AnalyzePool {
     void* d_tables = nullptr;
     const uint8_t* d_kind = nullptr;
     const uint32_t* d_slot = nullptr;
-    double *d_vars = nullptr, *d_param = nullptr;
-    uint8_t* d_out = nullptr;
-    uint32_t capacity = 0;
-    double* d_ws = nullptr;  // workspace of the global-memory kernels, at most fk::kAnWorkspaceBytes
-    uint64_t ws_bytes = 0;
+    GrowBuf<double> d_vars, d_param;
+    GrowBuf<uint8_t> d_out;
+    GrowBuf<double> ws;  // workspace of the global-memory kernels
     cudaStream_t stream = nullptr;
     ~AnalyzePool() {
         if (device >= 0) cudaSetDevice(device);
-        cudaFree(d_tables); cudaFree(d_vars); cudaFree(d_param); cudaFree(d_out); cudaFree(d_ws);
+        cudaFree(d_tables);
         if (stream) cudaStreamDestroy(stream);
     }
 };
@@ -396,17 +496,14 @@ struct fk_batch_plan {
     const DeviceProgram* full = nullptr;
     double *d_vars = nullptr, *d_params = nullptr, *d_out = nullptr, *d_er = nullptr, *d_ej = nullptr;
     fk_report* d_rep = nullptr;
-    double* d_ws = nullptr;  // launch_lm workspace (global sparse path)
-    uint32_t ws_ctas = 0;
+    SolveWorkspace ws;
     bool lm = true;          // LM may run on the plan (false: the L-BFGS calls' internal plans, which skip its tables)
-    double* d_lb_ws = nullptr;  // L-BFGS CTA kernel workspace, grown on first use
-    uint32_t lb_ws_ctas = 0;
     double *d_raw_vars = nullptr, *d_raw_param = nullptr, *d_scales = nullptr;  // fk_batch_system_solve: unscaled input, scale per sketch
     uint64_t launches = 0;
     ~fk_batch_plan() {
         cudaSetDevice(device);
         cudaFree(d_vars); cudaFree(d_params); cudaFree(d_out); cudaFree(d_er); cudaFree(d_ej); cudaFree(d_rep);
-        cudaFree(d_raw_vars); cudaFree(d_raw_param); cudaFree(d_scales); cudaFree(d_ws); cudaFree(d_lb_ws);
+        cudaFree(d_raw_vars); cudaFree(d_raw_param); cudaFree(d_scales);
     }
 };
 
@@ -423,17 +520,8 @@ void DevicePipeline::release() {
         plans[s] = nullptr;
     }
     chunk = 0;
-    if (small_h) cudaFreeHost(small_h);
-    if (small_d) cudaFree(small_d);
     if (small_stream) cudaStreamDestroy(small_stream);
-    if (small_ws) cudaFree(small_ws);
-    if (small_lb_ws) cudaFree(small_lb_ws);
-    small_h = small_d = nullptr;
     small_stream = nullptr;
-    small_ws = nullptr;
-    small_ws_ctas = 0;
-    small_lb_ws = nullptr;
-    small_lb_ws_ctas = 0;
     plans_lm = false;
     if (shared_param_ev) cudaEventDestroy(shared_param_ev);
     shared_param_ev = nullptr;
@@ -579,54 +667,46 @@ static int single_pass_device_range(fk_topology* topo, const std::vector<fk_topo
     const size_t steps = subs.size();
     uint32_t max_free = 1;
     for (const fk_topology* s : subs) max_free = std::max(max_free, s->t.n_free);
-    int rc = FK_OK;
-    double *d_vars = nullptr, *d_params = nullptr, *d_out = nullptr;
-    fk_report *d_rep = nullptr, *d_rep_t = nullptr;
-    cudaStream_t stream = nullptr;
-    auto done = [&](int code) {
-        if (stream) cudaStreamDestroy(stream);
-        cudaFree(d_vars); cudaFree(d_params); cudaFree(d_out); cudaFree(d_rep); cudaFree(d_rep_t);
-        return code;
-    };
-#define SP_CU(call)                                              \
-    do {                                                         \
-        cudaError_t e_ = (call);                                 \
-        if (e_ != cudaSuccess) return done(cuda_fail(e_, #call)); \
-    } while (0)
-    SP_CU(cudaSetDevice(device));
+    CU(cudaSetDevice(device));
     // bound the resident set of one chunk to ~8 GiB
     const size_t per_sketch = sizeof(double) * ((size_t)t.n_vars + t.n_expr + max_free) + 2 * sizeof(fk_report) * std::max<size_t>(1, steps);
     const uint32_t chunk = (uint32_t)std::min<uint64_t>(hi - lo, std::max<uint64_t>(1, (8ull << 30) / per_sketch));
-    SP_CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-    SP_CU(cudaMalloc(&d_vars, sizeof(double) * std::max<size_t>(1, (size_t)chunk * t.n_vars)));
-    SP_CU(cudaMalloc(&d_params, sizeof(double) * std::max<size_t>(1, (size_t)chunk * t.n_expr)));
-    SP_CU(cudaMalloc(&d_out, sizeof(double) * (size_t)chunk * max_free));
-    SP_CU(cudaMalloc(&d_rep, sizeof(fk_report) * std::max<size_t>(1, (size_t)chunk * steps)));
-    if (reports) SP_CU(cudaMalloc(&d_rep_t, sizeof(fk_report) * std::max<size_t>(1, (size_t)chunk * steps)));
-    std::vector<const fk::DevProgram*> progs(steps, nullptr);
-    for (size_t st = 0; st < steps; st++) {
-        rc = subs[st]->program_for(device, &progs[st]);
-        if (rc != FK_OK) return done(rc);
+    cudaStream_t stream = nullptr;
+    CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+    const std::unique_ptr<CUstream_st, cudaError_t (*)(cudaStream_t)> own_stream(stream, cudaStreamDestroy);
+    GrowBuf<double> d_vars, d_params, d_out;
+    GrowBuf<fk_report> d_rep, d_rep_t;
+    SolveWorkspace ws;
+    int rc = d_vars.reserve((size_t)chunk * t.n_vars);
+    if (rc == FK_OK) rc = d_params.reserve((size_t)chunk * t.n_expr);
+    if (rc == FK_OK) rc = d_out.reserve((size_t)chunk * max_free);
+    if (rc == FK_OK) rc = d_rep.reserve((size_t)chunk * steps);
+    if (rc == FK_OK && reports) rc = d_rep_t.reserve((size_t)chunk * steps);
+    std::vector<const DeviceProgram*> full(steps, nullptr);
+    for (size_t st = 0; st < steps && rc == FK_OK; st++) {
+        const fk::DevProgram* v = nullptr;
+        rc = subs[st]->program_for(device, &v, &full[st]);
     }
+    if (rc != FK_OK) return rc;
     for (uint32_t at = lo; at < hi; at += chunk) {
         const uint32_t cnt = std::min(chunk, hi - at);
-        SP_CU(cudaMemcpyAsync(d_vars, vars + (size_t)at * t.n_vars, sizeof(double) * (size_t)cnt * t.n_vars, cudaMemcpyHostToDevice, stream));
-        if (t.n_expr) SP_CU(cudaMemcpyAsync(d_params, param + (size_t)at * t.n_expr, sizeof(double) * (size_t)cnt * t.n_expr, cudaMemcpyHostToDevice, stream));
+        CU(cudaMemcpyAsync(d_vars, vars + (size_t)at * t.n_vars, sizeof(double) * (size_t)cnt * t.n_vars, cudaMemcpyHostToDevice, stream));
+        if (t.n_expr) CU(cudaMemcpyAsync(d_params, param + (size_t)at * t.n_expr, sizeof(double) * (size_t)cnt * t.n_expr, cudaMemcpyHostToDevice, stream));
         for (size_t st = 0; st < steps; st++) {
-            int e = fk::launch_batch_lm(*progs[st], cnt, d_vars, d_params, d_out, d_rep + st * (size_t)cnt, stream);
-            if (e == 0) e = fk::launch_scatter_free(progs[st]->free_vars, progs[st]->n, t.n_vars, cnt, d_out, d_vars, stream);
-            if (e != 0) return done(cuda_fail((cudaError_t)e, "launch SinglePass set"));
+            const fk::DevProgram& v = full[st]->view;
+            if ((rc = solve_launch(*full[st], kSolveLm, cnt, d_vars, d_params, d_out, d_rep + st * (size_t)cnt, ws, stream)) != FK_OK) return rc;
+            const int e = fk::launch_scatter_free(v.free_vars, v.n, t.n_vars, cnt, d_out, d_vars, stream);
+            if (e != 0) return cuda_fail((cudaError_t)e, "launch SinglePass set");
         }
-        SP_CU(cudaMemcpyAsync(vars + (size_t)at * t.n_vars, d_vars, sizeof(double) * (size_t)cnt * t.n_vars, cudaMemcpyDeviceToHost, stream));
+        CU(cudaMemcpyAsync(vars + (size_t)at * t.n_vars, d_vars, sizeof(double) * (size_t)cnt * t.n_vars, cudaMemcpyDeviceToHost, stream));
         if (reports && steps) {
             const int e = fk::launch_transpose_reports(d_rep, d_rep_t, cnt, (uint32_t)steps, stream);
-            if (e != 0) return done(cuda_fail((cudaError_t)e, "launch fk_transpose_reports_kernel"));
-            SP_CU(cudaMemcpyAsync(reports + (size_t)at * steps, d_rep_t, sizeof(fk_report) * (size_t)cnt * steps, cudaMemcpyDeviceToHost, stream));
+            if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_transpose_reports_kernel");
+            CU(cudaMemcpyAsync(reports + (size_t)at * steps, d_rep_t, sizeof(fk_report) * (size_t)cnt * steps, cudaMemcpyDeviceToHost, stream));
         }
-        SP_CU(cudaStreamSynchronize(stream));
+        CU(cudaStreamSynchronize(stream));
     }
-#undef SP_CU
-    return done(FK_OK);
+    return FK_OK;
 }
 
 int fk_batch_solve_single_pass(const fk_topology* topo_c, uint32_t n, double* vars, const double* param, fk_report* reports,
@@ -654,6 +734,11 @@ static int choose_lbfgs(const fk_topology* topo, uint32_t n_sketches) {
     (void)n_sketches;  // (the choice depends on the topology alone)
     const fk::Topology& t = topo->t;
     return t.path == 0 && fk::batch_lbfgs_tile_fits(t.n_free, t.n_rows, t.jac_nnz, t.tile) ? 0 : 1;
+}
+
+// The batched solve kernel of n sketches of a topology: optimizer 0 LM, 1 L-BFGS with the kernel of choose_lbfgs.
+static SolveKernel solve_kernel(const fk_topology* topo, int optimizer, uint32_t n) {
+    return optimizer == 0 ? kSolveLm : choose_lbfgs(topo, n) == 0 ? kSolveLbfgsTile : kSolveLbfgsCta;
 }
 
 int fk_batch_solve_lbfgs(const fk_topology* topo_c, int device, uint32_t n, const double* vars, const double* param, double* free_out,
@@ -700,28 +785,15 @@ int fk_batch_analyze(const fk_topology* topo_c, int device, uint32_t n, const do
         pool->d_kind = pk.at<uint8_t>(o_kind);
         pool->d_slot = pk.at<uint32_t>(o_slot);
     }
-    if (pool->capacity < n) {  // grow-only
-        cudaFree(pool->d_vars); cudaFree(pool->d_param); cudaFree(pool->d_out);
-        pool->d_vars = pool->d_param = nullptr; pool->d_out = nullptr; pool->capacity = 0;
-        const uint32_t cap = std::max<uint32_t>(n, 1024);
-        CU(cudaMalloc(&pool->d_vars, sizeof(double) * (size_t)cap * std::max<uint32_t>(t.n_vars, 1)));
-        CU(cudaMalloc(&pool->d_param, sizeof(double) * (size_t)cap * t.n_expr));
-        CU(cudaMalloc(&pool->d_out, (size_t)cap * t.n_expr));
-        pool->capacity = cap;
-    }
-    if (pool->ws_bytes < plan.workspace_bytes()) {  // grow-only, within fk::kAnWorkspaceBytes
-        cudaFree(pool->d_ws);
-        pool->d_ws = nullptr; pool->ws_bytes = 0;
-        CU(cudaMalloc(&pool->d_ws, plan.workspace_bytes()));
-        pool->ws_bytes = plan.workspace_bytes();
-    }
+    const size_t cap = std::max<uint32_t>(n, 1024), nv = std::max<uint32_t>(t.n_vars, 1);  // (grow-only: rows for at least cap sketches)
+    int grc = pool->d_vars.reserve(n * nv, cap * nv);
+    if (grc == FK_OK) grc = pool->d_param.reserve((size_t)n * t.n_expr, cap * t.n_expr);
+    if (grc == FK_OK) grc = pool->d_out.reserve((size_t)n * t.n_expr, cap * t.n_expr);
+    if (grc != FK_OK) return grc;
     CU(cudaMemcpyAsync(pool->d_vars, vars, sizeof(double) * (size_t)n * t.n_vars, cudaMemcpyHostToDevice, pool->stream));
     CU(cudaMemcpyAsync(pool->d_param, param, sizeof(double) * (size_t)n * t.n_expr, cudaMemcpyHostToDevice, pool->stream));
-    const int e = plan.kernel == fk::kAnWarp
-                      ? fk::launch_batch_analyze(t.n_vars, t.n_expr, pool->d_kind, pool->d_slot, n, pool->d_vars, pool->d_param, pool->d_out, pool->stream)
-                      : fk::launch_analyze(plan, t.n_vars, t.n_expr, pool->d_kind, pool->d_slot, n, pool->d_vars, pool->d_param, pool->d_out,
-                                           pool->d_ws, pool->stream);
-    if (e != 0) return cuda_fail((cudaError_t)e, plan.kernel == fk::kAnWarp ? "launch fk_batch_analyze_kernel" : "launch fk_analyze_cta_kernel");
+    grc = analyze_launch(t.n_vars, t.n_expr, pool->d_kind, pool->d_slot, n, pool->d_vars, pool->d_param, pool->d_out, device, pool->ws, pool->stream);
+    if (grc != FK_OK) return grc;
     CU(cudaMemcpyAsync(independent, pool->d_out, (size_t)n * t.n_expr, cudaMemcpyDeviceToHost, pool->stream));
     CU(cudaStreamSynchronize(pool->stream));
     return FK_OK;
@@ -747,7 +819,7 @@ static int plan_create(fk_topology* topo, uint32_t capacity, int device, bool lm
     CU(cudaMalloc(&p->d_params, sizeof(double) * std::max<size_t>(1, (size_t)capacity * t.n_expr)));
     CU(cudaMalloc(&p->d_out, sizeof(double) * std::max<size_t>(1, (size_t)capacity * t.n_free)));
     CU(cudaMalloc(&p->d_rep, sizeof(fk_report) * (size_t)capacity));
-    if (lm && (rc = alloc_lm_workspace(*p->full, capacity, &p->d_ws, &p->ws_ctas)) != FK_OK) return rc;
+    if (lm && (rc = p->ws.reserve(*p->full, kSolveLm, capacity)) != FK_OK) return rc;  // (out of memory surfaces here)
     *out = p.release();
     return FK_OK;
 }
@@ -769,59 +841,24 @@ int fk_batch_plan_upload(fk_batch_plan* plan, uint32_t n, const double* vars, co
     return FK_OK;
 }
 
-int fk_batch_plan_run(fk_batch_plan* plan, void* stream) {
+// A solve of the plan's n sketches with `kernel` on `stream`.
+static int plan_solve(fk_batch_plan* plan, SolveKernel kernel, void* stream) {
     if (!plan) return fail(FK_ERR_INVALID, "null plan");
     CU(cudaSetDevice(plan->device));
-    const int e = launch_lm(*plan->full, plan->n, plan->d_vars, plan->d_params, plan->d_out, plan->d_rep, plan->d_ws, plan->ws_ctas,
-                            (cudaStream_t)stream);
-    if (e != 0) return cuda_fail((cudaError_t)e, "launch batched LM kernel");
-    if (plan->n) plan->launches++;
-    return FK_OK;
-}
-
-// Grow-only L-BFGS CTA workspace with room for `ctas` CTAs (*buf, *have: its current size).
-static int grow_lbfgs_workspace(const fk::DevProgram& prog, uint32_t ctas, double** buf, uint32_t* have) {
-    if (*have >= ctas) return FK_OK;
-    if (*buf) cudaFree(*buf);
-    *buf = nullptr;
-    *have = 0;
-    CU(cudaMalloc(buf, sizeof(double) * fk::lbfgs_workspace_doubles(prog, ctas)));
-    *have = ctas;
-    return FK_OK;
-}
-
-static int run_lbfgs_cta(const DeviceProgram& full, uint32_t n, const double* vars, const double* params, double* out, fk_report* reps,
-                         double** ws, uint32_t* ws_ctas, cudaStream_t st) {
-    if (n == 0) return FK_OK;
-    const uint32_t ctas = fk::lbfgs_workspace_ctas(full.view, n);
-    if (ctas == 0) return fail(FK_ERR_CUDA, "occupancy query of fk_lbfgs_cta_kernel failed");
-    const int rc = grow_lbfgs_workspace(full.view, ctas, ws, ws_ctas);
-    if (rc != FK_OK) return rc;
-    const int e = fk::launch_lbfgs_cta(full.view, full.jcolptr, full.jrow, n, vars, params, out, reps, *ws, ctas, st);
-    if (e == (int)cudaErrorInvalidConfiguration) return fail(FK_ERR_TOO_LARGE, "more than 2^24 Jacobian entries");
-    if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_lbfgs_cta_kernel");
-    return FK_OK;
-}
-
-int fk_batch_plan_run_lbfgs_global(fk_batch_plan* plan, void* stream) {
-    if (!plan) return fail(FK_ERR_INVALID, "null plan");
-    CU(cudaSetDevice(plan->device));
-    const int rc = run_lbfgs_cta(*plan->full, plan->n, plan->d_vars, plan->d_params, plan->d_out, plan->d_rep, &plan->d_lb_ws,
-                                 &plan->lb_ws_ctas, (cudaStream_t)stream);
+    const int rc = solve_launch(*plan->full, kernel, plan->n, plan->d_vars, plan->d_params, plan->d_out, plan->d_rep, plan->ws,
+                                (cudaStream_t)stream);
     if (rc == FK_OK && plan->n) plan->launches++;
     return rc;
 }
 
+int fk_batch_plan_run(fk_batch_plan* plan, void* stream) { return plan_solve(plan, kSolveLm, stream); }
+
+int fk_batch_plan_run_lbfgs_global(fk_batch_plan* plan, void* stream) { return plan_solve(plan, kSolveLbfgsCta, stream); }
+
 int fk_batch_plan_run_lbfgs(fk_batch_plan* plan, void* stream) {
     if (!plan) return fail(FK_ERR_INVALID, "null plan");
     if (plan->topo->t.path != 0) return fail(FK_ERR_TOO_LARGE, "L-BFGS is built for the shared-memory tile paths only");
-    CU(cudaSetDevice(plan->device));
-    const int e = fk::launch_batch_lbfgs(*plan->prog, plan->full->jcolptr, plan->full->jrow, plan->n, plan->d_vars, plan->d_params,
-                                         plan->d_out, plan->d_rep, stream);
-    if (e == (int)cudaErrorInvalidConfiguration) return fail(FK_ERR_TOO_LARGE, "the L-BFGS state of one sketch does not fit the tile path");
-    if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_batch_lbfgs_kernel");
-    if (plan->n) plan->launches++;
-    return FK_OK;
+    return plan_solve(plan, kSolveLbfgsTile, stream);
 }
 
 int fk_batch_plan_download(fk_batch_plan* plan, double* free_out, fk_report* reports, void* stream) {
@@ -1088,31 +1125,13 @@ static int small_solve(fk_topology* topo, int device, uint32_t lo, uint32_t hi, 
     const DeviceProgram* full = nullptr;
     int rc = topo->program_for(device, &prog, &full, optimizer == 0);
     if (rc != FK_OK) return rc;
-    const bool lbfgs_cta = optimizer == 1 && choose_lbfgs(topo, total) == 1;
     cudaError_t e = cudaSetDevice(device);
     if (e != cudaSuccess) return cuda_fail(e, "cudaSetDevice");
-    if (!pl->small_h || !pl->small_d || !pl->small_stream) {
-        // all three or none: a half-initialised block would poison every later call on this topology
-        if (pl->small_h) cudaFreeHost(pl->small_h);
-        if (pl->small_d) cudaFree(pl->small_d);
-        if (pl->small_stream) cudaStreamDestroy(pl->small_stream);
-        pl->small_h = pl->small_d = nullptr;
+    if ((rc = pl->small_h.reserve(DevicePipeline::kSmallBytes)) != FK_OK || (rc = pl->small_d.reserve(DevicePipeline::kSmallBytes)) != FK_OK)
+        return rc;
+    if (!pl->small_stream && (e = cudaStreamCreateWithFlags(&pl->small_stream, cudaStreamNonBlocking)) != cudaSuccess) {
         pl->small_stream = nullptr;
-        if ((e = cudaMallocHost((void**)&pl->small_h, DevicePipeline::kSmallBytes)) != cudaSuccess) { pl->small_h = nullptr; return cuda_fail(e, "cudaMallocHost"); }
-        if ((e = cudaMalloc((void**)&pl->small_d, DevicePipeline::kSmallBytes)) != cudaSuccess) {
-            cudaFreeHost(pl->small_h); pl->small_h = pl->small_d = nullptr;
-            return cuda_fail(e, "cudaMalloc");
-        }
-        if ((e = cudaStreamCreateWithFlags(&pl->small_stream, cudaStreamNonBlocking)) != cudaSuccess) {
-            cudaFreeHost(pl->small_h); cudaFree(pl->small_d); pl->small_h = pl->small_d = nullptr; pl->small_stream = nullptr;
-            return cuda_fail(e, "cudaStreamCreate");
-        }
-    }
-    if (optimizer == 0 && full->sparse_batch && pl->small_ws_ctas < full->sparse_batch->workspace_ctas(total)) {  // grow-only
-        if (pl->small_ws) cudaFree(pl->small_ws);
-        pl->small_ws = nullptr;
-        pl->small_ws_ctas = 0;
-        if ((rc = alloc_lm_workspace(*full, total, &pl->small_ws, &pl->small_ws_ctas)) != FK_OK) return rc;
+        return cuda_fail(e, "cudaStreamCreate");
     }
     std::memcpy(pl->small_h, vars + (size_t)lo * t.n_vars, in_v);
     if (in_p) std::memcpy(pl->small_h + in_v, param + (size_t)lo * t.n_expr, in_p);
@@ -1132,14 +1151,8 @@ static int small_solve(fk_topology* topo, int device, uint32_t lo, uint32_t hi, 
     const double *d_vars = (const double*)base, *d_param = (const double*)(base + in_v);
     double* d_out = (double*)(base + in_al);
     fk_report* d_rep = (fk_report*)(base + in_al + out_x);
-    if (lbfgs_cta) {
-        if ((rc = run_lbfgs_cta(*full, total, d_vars, d_param, d_out, d_rep, &pl->small_lb_ws, &pl->small_lb_ws_ctas, pl->small_stream)) != FK_OK)
-            return rc;
-    } else {
-        const int le = optimizer == 1 ? fk::launch_batch_lbfgs(full->view, full->jcolptr, full->jrow, total, d_vars, d_param, d_out, d_rep, pl->small_stream)
-                                      : launch_lm(*full, total, d_vars, d_param, d_out, d_rep, pl->small_ws, pl->small_ws_ctas, pl->small_stream);
-        if (le != 0) return cuda_fail((cudaError_t)le, optimizer == 1 ? "launch fk_batch_lbfgs_kernel" : "launch batched solve kernel");
-    }
+    rc = solve_launch(*full, solve_kernel(topo, optimizer, total), total, d_vars, d_param, d_out, d_rep, pl->small_ws, pl->small_stream);
+    if (rc != FK_OK) return rc;
     if (!zero_copy && (e = cudaMemcpyAsync(pl->small_h + in_al, pl->small_d + in_al, out_x + out_r, cudaMemcpyDeviceToHost, pl->small_stream)) != cudaSuccess) return cuda_fail(e, "cudaMemcpyAsync");
     if ((e = cudaStreamSynchronize(pl->small_stream)) != cudaSuccess) return cuda_fail(e, "batch kernel / copy failed");
     std::memcpy(free_out + (size_t)lo * t.n_free, pl->small_h + in_al, out_x);
@@ -1157,13 +1170,13 @@ static int run_device_range(fk_topology* topo, int device, uint32_t lo, uint32_t
     if (small_fits(t, hi - lo)) return small_solve(topo, device, lo, hi, vars, param, free_out, reports, optimizer);
     // (the L-BFGS kernel is not the sketch-per-thread kernel: its chunks are not rounded to that kernel's waves)
     const uint32_t chunk = pipeline_chunk(topo, device, hi - lo, 8, optimizer == 0);
-    const bool lbfgs_cta = optimizer == 1 && choose_lbfgs(topo, hi - lo) == 1;
+    const SolveKernel kernel = solve_kernel(topo, optimizer, hi - lo);
     return run_pipeline(topo, device, lo, hi, chunk, token, nullptr,
                         [&](fk_batch_plan* p, cudaStream_t st, uint32_t at, uint32_t cnt, const std::function<void()>& mark) {
                             int rc = fk_batch_plan_upload(p, cnt, vars + (size_t)at * t.n_vars, param ? param + (size_t)at * t.n_expr : nullptr, st);
                             if (rc != FK_OK) return rc;
                             mark();
-                            rc = optimizer == 0 ? fk_batch_plan_run(p, st) : lbfgs_cta ? fk_batch_plan_run_lbfgs_global(p, st) : fk_batch_plan_run_lbfgs(p, st);
+                            rc = plan_solve(p, kernel, st);
                             if (rc != FK_OK) return rc;
                             mark();
                             return fk_batch_plan_download(p, free_out + (size_t)at * t.n_free, reports ? reports + at : nullptr, st);
@@ -1271,11 +1284,14 @@ static int batch_system_solve(const fk_topology* topo_c, int device, uint32_t n,
             e = fk::launch_batch_lm_sketch(*p->prog->sketch_prog, cnt, nullptr, nullptr, p->d_out, p->d_rep, st, &raw);
             p->launches += 1;
         } else {
+            p->launches += 3;
             e = fk::launch_batch_prepare(cnt, t.n_vars, t.n_expr, pt->d_kind, shared, (uint32_t)pt->perturb_vars.size(), pt->d_perturb, pt->d_draws,
                                          p->d_raw_vars, d_param, p->d_vars, p->d_params, p->d_scales, st);
-            if (e == 0) e = launch_lm(*p->full, cnt, p->d_vars, p->d_params, p->d_out, p->d_rep, p->d_ws, p->ws_ctas, st);
-            if (e == 0) e = fk::launch_batch_unscale(cnt, t.n_free, p->d_scales, p->d_out, st);
-            p->launches += 3;
+            if (e == 0) {
+                const int rc = solve_launch(*p->full, kSolveLm, cnt, p->d_vars, p->d_params, p->d_out, p->d_rep, p->ws, st);
+                if (rc != FK_OK) return rc;
+                e = fk::launch_batch_unscale(cnt, t.n_free, p->d_scales, p->d_out, st);
+            }
         }
         if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_batch_system_solve kernels");
         mark();
@@ -1543,8 +1559,7 @@ void fk_topology_cache_stats(uint64_t* hits, uint64_t* misses, uint32_t* entries
 struct HeteroPool {
     std::mutex mu;
     int device = -1;
-    unsigned char *h = nullptr, *d = nullptr;
-    size_t cap = 0;
+    GrowBuf<unsigned char> h{true}, d;
     cudaStream_t stream = nullptr;
 };
 static HeteroPool* hetero_pool_for(int device) {
@@ -1561,9 +1576,18 @@ static HeteroPool* hetero_pool_for(int device) {
 
 // Whether a structure of `instances` systems goes to fk_hetero_lm_kernel (one warp per system) rather than a uniform batch
 // launch: path 0, fewer than 64 systems (from there the sketch-per-thread kernel is the faster one) and an LM state within
-// 48 KiB.  The caller also needs the topology's 32-lane tables (fk_topology::lanes32).
+// 48 KiB.  The launch also needs the topology's 32-lane tables (hetero_topology).
 static bool hetero_fits(const fk::Topology& t, size_t instances) {
     return t.path == 0 && instances < 64 && fk::lm_smem_doubles(t.n_free, t.n_rows, t.jac_nnz, (uint32_t)t.l_rowidx.size()) * 8 <= 48 * 1024;
+}
+
+// The topology with 32-lane tables (fk_topology::lanes32) through which a structure of `instances` systems goes to
+// fk_hetero_lm_kernel, or null when it keeps a uniform batch launch: hetero_fits fails, or there are no 32-lane tables
+// (FK_NO_LATENCY_TWIN).
+static fk_topology* hetero_topology(fk_topology* topo, size_t instances) {
+    if (!hetero_fits(topo->t, instances)) return nullptr;
+    fk_topology* t32 = topo->lanes32();
+    return t32->t.tile == 32 ? t32 : nullptr;
 }
 
 // The programs of fk_hetero_lm_kernel on `device` (32-lane tables, no sketch-kernel block) and the largest LM state among them.
@@ -1601,7 +1625,6 @@ static int hetero_solve(int device, const std::vector<fk_topology*>& topos32, co
     uint32_t max_state = 1;
     if (const int rc = hetero_programs(device, topos32, progs, &max_state); rc != FK_OK) return rc;
     // layout of the staging block: [programs][jobs][inputs: vars row + param row per job] | [outputs][reports]
-    auto align = [](size_t x) { return (x + 255) & ~size_t(255); };
     std::vector<fk::HeteroJob> jobs(nj);
     size_t in_doubles = 0, out_doubles = 0;
     for (size_t k = 0; k < nj; k++) {
@@ -1611,19 +1634,13 @@ static int hetero_solve(int device, const std::vector<fk_topology*>& topos32, co
         jobs[k].param_off = in_doubles; in_doubles += t.n_expr;
         jobs[k].out_off = out_doubles; out_doubles += t.n_free;
     }
-    const size_t o_progs = 0, o_jobs = align(o_progs + ng * sizeof(fk::DevProgram)), o_in = align(o_jobs + nj * sizeof(fk::HeteroJob));
-    const size_t o_out = align(o_in + in_doubles * sizeof(double)), o_rep = align(o_out + out_doubles * sizeof(double));
-    const size_t total = align(o_rep + nj * sizeof(fk_report));
-    if (pool->cap < total) {
-        if (pool->h) cudaFreeHost(pool->h);
-        if (pool->d) cudaFree(pool->d);
-        pool->h = pool->d = nullptr; pool->cap = 0;
-        const size_t cap = std::max<size_t>(total + total / 2, 1 << 20);
-        CU(cudaMallocHost((void**)&pool->h, cap));
-        cudaError_t e = cudaMalloc((void**)&pool->d, cap);
-        if (e != cudaSuccess) { cudaFreeHost(pool->h); pool->h = nullptr; return cuda_fail(e, "cudaMalloc"); }
-        pool->cap = cap;
-    }
+    BlockLayout blk;
+    const size_t o_progs = blk.put(ng * sizeof(fk::DevProgram)), o_jobs = blk.put(nj * sizeof(fk::HeteroJob));
+    const size_t o_in = blk.put(in_doubles * sizeof(double)), o_out = blk.put(out_doubles * sizeof(double)), o_rep = blk.put(nj * sizeof(fk_report));
+    const size_t total = blk.end, alloc = std::max<size_t>(total + total / 2, 1 << 20);
+    int grc = pool->h.reserve(total, alloc);
+    if (grc == FK_OK) grc = pool->d.reserve(total, alloc);
+    if (grc != FK_OK) return grc;
     if (!pool->stream) CU(cudaStreamCreateWithFlags(&pool->stream, cudaStreamNonBlocking));
     std::memcpy(pool->h + o_progs, progs.data(), ng * sizeof(fk::DevProgram));
     std::memcpy(pool->h + o_jobs, jobs.data(), nj * sizeof(fk::HeteroJob));
@@ -1778,8 +1795,8 @@ int fk_lm_solve_batch(uint32_t n, const fk_problem* const* problems, double* con
             std::vector<HeteroItem> items;
             for (size_t q = 0; q < small.size(); q++) {
                 BatchGroup& gr = groups[small[q]];
-                fk_topology* t32 = gr.topo->lanes32();
-                if (t32->t.tile != 32) continue;  // no 32-lane tables (FK_NO_LATENCY_TWIN): the group keeps the uniform kernel
+                fk_topology* t32 = hetero_topology(gr.topo.get(), gr.members.size());
+                if (!t32) continue;
                 for (uint32_t i : gr.members) items.push_back({(uint32_t)topos32.size(), i});
                 topos32.push_back(t32);
                 gr.done = true;
@@ -1896,47 +1913,17 @@ static uint32_t system_batch_chunk(uint32_t n, uint64_t bytes, uint64_t sketches
     return (uint32_t)std::min<uint64_t>(chunk, n);
 }
 
-// The state of a system batch call on one device, all on one stream: the layout's tables, the template rows and the chunk buffers
-// (grow / release_buffers).  d_vt / d_pt: the variants' scaled variables and parameters where the call keeps them resident (not
+// The state of a system batch call on one device, all on one stream: the layout's tables, the template rows and the grow-only chunk
+// buffers.  d_vt / d_pt: the variants' scaled variables and parameters where the call keeps them resident (not
 // fk_system_batch_solve).  The caller holds mu.
 struct SystemDevice {
     std::mutex mu;
     int device = -1;
     cudaStream_t stream = nullptr;
     bool ready = false;  // tables uploaded
-    uint32_t chunk = 0;  // variants the chunk buffers hold
     void* d_tables = nullptr;
     double *d_tmpl_vars = nullptr, *d_tmpl_param = nullptr;
-    double *d_raw_param = nullptr, *d_vt = nullptr, *d_pt = nullptr;
-    // What grow has allocated: the member it set and the buffer (the destructor frees the buffers of members that derived
-    // classes own after those members are gone).
-    struct Grown { void** member; void* buf; };
-    std::vector<Grown> grown;
-
-    // *ptr = a new buffer of `count` elements (at least one), freed by release_buffers; frees the one grow put there before.
-    template <class T>
-    int grow(T** ptr, size_t count) {
-        void** member = (void**)ptr;
-        auto it = std::find_if(grown.begin(), grown.end(), [&](const Grown& g) { return g.member == member; });
-        if (it != grown.end()) {
-            cudaFree(it->buf);
-            grown.erase(it);
-        }
-        *member = nullptr;
-        void* buf = nullptr;
-        CU(cudaMalloc(&buf, sizeof(T) * std::max<size_t>(count, 1)));
-        grown.push_back({member, buf});
-        *member = buf;
-        return FK_OK;
-    }
-    void release_buffers() {
-        for (const Grown& g : grown) {
-            cudaFree(g.buf);
-            *g.member = nullptr;
-        }
-        grown.clear();
-        chunk = 0;
-    }
+    GrowBuf<double> d_raw_param, d_vt, d_pt;
     // Once per device: the stream, the tables of `pk` and the template rows (an earlier failed attempt's are freed first).
     int upload_tables(int dev, TablePack& pk, uint32_t n_vars, uint32_t n_expr) {
         device = dev;
@@ -1953,7 +1940,6 @@ struct SystemDevice {
     ~SystemDevice() {
         if (device < 0) return;
         cudaSetDevice(device);
-        for (const Grown& g : grown) cudaFree(g.buf);
         cudaFree(d_tables); cudaFree(d_tmpl_vars); cudaFree(d_tmpl_param);
         if (stream) cudaStreamDestroy(stream);
     }
@@ -1983,38 +1969,38 @@ static int run_chunks(SystemDevice* d, uint32_t n_vars, uint32_t n_expr, const d
 // The solve batches' device state: the prepare kernel's tables and descriptors (d_desc), the structures' batch plans, and the
 // chunk's raw, scale and output rows.  Plus, for fk_system_batch_solve, the scatter kernel's tables.
 struct SystemBatchDevice : SystemDevice {
+    uint32_t chunk = 0;  // variants the plans and chunk buffers hold
     bool lm = false;  // the plans were made for LM (which on the global sparse path needs the sparse batch tables)
     std::vector<std::unique_ptr<fk_batch_plan>> plans;
     const uint8_t* d_kind = nullptr;
     const uint32_t *d_expr_con = nullptr, *d_var_struct = nullptr, *d_var_off = nullptr, *d_comp_struct = nullptr, *d_comp_member = nullptr;
     const double* d_draws = nullptr;
     std::vector<SbStructure> desc;  // (host copy; the buffer pointers change with the plans)
-    SbStructure* d_desc = nullptr;
-    double *d_raw_vars = nullptr, *d_scales = nullptr, *d_vars_out = nullptr;
-    fk_report* d_rep_out = nullptr;
+    GrowBuf<SbStructure> d_desc;
+    GrowBuf<double> d_raw_vars, d_scales, d_vars_out;
+    GrowBuf<fk_report> d_rep_out;
 
-    // The chunk buffers of `cap` variants, everything released first and again after a failure: per structure s a plan of
+    // The plans and chunk buffers of `cap` variants, the plans made again (and dropped after a failure): per structure s a plan of
     // cap * st[s].mult sketches, the raw, scale and output rows with n_rep reports per variant, and with `resident` vt and pt.
     template <class Structure>
     int grow_chunk(const SystemBatchLayout& L, const std::vector<Structure>& st, uint32_t cap, bool lm_plans, uint32_t n_rep, bool resident) {
         plans.clear();
-        release_buffers();
+        chunk = 0;
         int rc = FK_OK;
         for (size_t s = 0; s < st.size() && rc == FK_OK; s++) {
             fk_batch_plan* p = nullptr;
             if ((rc = plan_create(st[s].topo.get(), cap * st[s].mult, device, lm_plans, &p)) == FK_OK) plans.emplace_back(p);
         }
-        if (rc == FK_OK) rc = grow(&d_raw_vars, (size_t)cap * L.n_vars);
-        if (rc == FK_OK) rc = grow(&d_raw_param, (size_t)cap * L.n_constraints);
-        if (rc == FK_OK) rc = grow(&d_scales, cap);
-        if (rc == FK_OK) rc = grow(&d_vars_out, (size_t)cap * L.n_vars);
-        if (rc == FK_OK) rc = grow(&d_rep_out, (size_t)cap * n_rep);
-        if (rc == FK_OK && resident) rc = grow(&d_vt, (size_t)cap * L.n_vars);
-        if (rc == FK_OK && resident) rc = grow(&d_pt, (size_t)cap * L.kind.size());
-        if (rc == FK_OK) rc = grow(&d_desc, desc.size());
+        if (rc == FK_OK) rc = d_raw_vars.reserve((size_t)cap * L.n_vars);
+        if (rc == FK_OK) rc = d_raw_param.reserve((size_t)cap * L.n_constraints);
+        if (rc == FK_OK) rc = d_scales.reserve(cap);
+        if (rc == FK_OK) rc = d_vars_out.reserve((size_t)cap * L.n_vars);
+        if (rc == FK_OK) rc = d_rep_out.reserve((size_t)cap * n_rep);
+        if (rc == FK_OK && resident) rc = d_vt.reserve((size_t)cap * L.n_vars);
+        if (rc == FK_OK && resident) rc = d_pt.reserve((size_t)cap * L.kind.size());
+        if (rc == FK_OK) rc = d_desc.reserve(desc.size());
         if (rc != FK_OK) {
             plans.clear();
-            release_buffers();
             return rc;
         }
         chunk = cap;
@@ -2057,7 +2043,7 @@ static int solve_chunks(SystemBatchDevice* d, const SystemBatchLayout& L, const 
             CU(cudaMemcpyAsync(d->d_raw_param, c.params + (size_t)at * L.n_constraints, sizeof(double) * (size_t)cnt * L.n_constraints,
                                cudaMemcpyHostToDevice, st));
         const int e = launch_system_batch_prepare(cnt, L.n_vars, n_expr, L.n_constraints, d->d_kind, d->d_expr_con, d->d_draws, c.perturb, raw,
-                                                  raw_stride, c.params ? d->d_raw_param : nullptr, d->d_tmpl_param, n_desc, d->d_desc, d->d_scales, st);
+                                                  raw_stride, c.params ? d->d_raw_param.get() : nullptr, d->d_tmpl_param, n_desc, d->d_desc, d->d_scales, st);
         if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_batch_prepare_kernel");
         const int rc = step(cnt, raw, raw_stride);
         if (rc != FK_OK) return rc;
@@ -2195,9 +2181,7 @@ static int system_batch_range(SystemBatch& b, const SystemBatchCall& c, int devi
                             for (uint32_t s = 0; s < ns; s++) {
                                 fk_batch_plan* p = d->plans[s].get();
                                 p->n = cnt * b.st[s].mult;
-                                const int r = c.optimizer == 0                    ? fk_batch_plan_run(p, d->stream)
-                                              : choose_lbfgs(p->topo, p->n) == 1 ? fk_batch_plan_run_lbfgs_global(p, d->stream)
-                                                                                 : fk_batch_plan_run_lbfgs(p, d->stream);
+                                const int r = plan_solve(p, solve_kernel(p->topo, c.optimizer, p->n), d->stream);
                                 if (r != FK_OK) return r;
                             }
                             const int e = launch_system_batch_scatter(cnt, L.n_vars, raw, raw_stride, d->d_scales, d->d_var_struct, d->d_var_off, n_rep,
@@ -2230,7 +2214,7 @@ struct SystemSpDevice : SystemBatchDevice {
     std::vector<uint32_t> pert_off;                        // [n_waves + 1]
     std::vector<SpGroup> groups;                           // (host copy) every wave's groups, wave after wave
     std::vector<uint32_t> group_off;                       // [n_waves + 1]
-    SpGroup* d_groups = nullptr;
+    GrowBuf<SpGroup> d_groups;
 };
 
 struct SystemSpBatch {
@@ -2374,10 +2358,10 @@ static int system_sp_device(SystemSpBatch& b, SystemSpDevice* d, int device, uin
     *chunk = system_batch_chunk(n, bytes, mult, std::max({L.n_vars, L.n_constraints, n_expr, n_sets}));
     if (d->chunk >= *chunk && d->plans.size() == ns) return FK_OK;
     int rc = d->grow_chunk(L, b.st, std::max(*chunk, d->chunk), true, n_sets, true);
-    if (rc == FK_OK) rc = d->grow(&d->d_groups, d->groups.size());
+    if (rc == FK_OK) rc = d->d_groups.reserve(d->groups.size());
     if (rc != FK_OK) {
         d->plans.clear();
-        d->release_buffers();
+        d->chunk = 0;
         return rc;
     }
     d->desc[0].vars = d->d_vt;
@@ -2416,7 +2400,7 @@ static int system_sp_range(SystemSpBatch& b, const SystemBatchCall& c, int devic
                                 const int e = launch_system_sp_gather_scatter(
                                     cnt, L.n_vars, n_expr, d->d_vt, d->d_pt, s_hi - s_lo, d->d_groups + s_lo, n_rep, d->d_rep_out, p_hi - p_lo,
                                     d->d_pvar + p_lo, d->d_pdraw + p_lo, d->d_draws, g_hi - g_lo, d->d_groups + g_lo, d->d_solved, raw, raw_stride,
-                                    d->d_scales, w == nw ? d->d_vars_out : nullptr, d->stream);
+                                    d->d_scales, w == nw ? d->d_vars_out.get() : nullptr, d->stream);
                                 if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_sp_gather_scatter_kernel");
                                 if (w == nw) break;
                                 for (const SystemSpBatch::Group& g : b.waves[w]) {  // LM under SinglePass / RecursiveAssembly whatever the optimizer (assemble/mod.rs:191, :224)
@@ -2449,15 +2433,13 @@ int system_sp_batch_solve(SystemSpBatch& b, const SystemBatchCall& c) {
 // ---- fk_system_batch_analyze / fk_system_batch_residuals: System::analyze and calculate_residual over n variants -----------
 // Per device: the layout's tables, the template rows, the chunk buffers (variables vt and expanded parameters pt are what the
 // analyze kernels and fk_system_residuals_kernel read), the outputs of each operation (grown on its first call) and the analyze
-// workspace, grow-only within fk::kAnWorkspaceBytes.
+// workspace.
 struct SystemAnDevice : SystemDevice {
     const uint8_t* d_kind = nullptr;
     const uint32_t *d_slot = nullptr, *d_expr_con = nullptr, *d_con_off = nullptr;
-    uint32_t an_chunk = 0, res_chunk = 0;  // variants the analyze outputs, the residual outputs hold
-    double* d_res = nullptr;
-    uint8_t *d_indep = nullptr, *d_dep = nullptr;
-    double* d_ws = nullptr;
-    uint64_t ws_bytes = 0;
+    GrowBuf<double> d_res;
+    GrowBuf<uint8_t> d_indep, d_dep;
+    GrowBuf<double> d_ws;
 };
 
 struct SystemAnBatch {
@@ -2507,26 +2489,14 @@ static int system_an_device(const SystemAnBatch& b, SystemAnDevice* d, int devic
     // per variant: the raw parameters, vt and pt, and the operation's outputs
     const uint64_t bytes = sizeof(double) * ((uint64_t)L.n_vars + ncon + ne) + (analyze ? (uint64_t)ne + ncon : sizeof(double) * ncon);
     *chunk = system_batch_chunk(n, bytes, 1, std::max({L.n_vars, ncon, ne}));
-    const uint32_t cap = *chunk;
-    int rc = FK_OK;
-    if (d->chunk < cap) {
-        d->chunk = 0;
-        if ((rc = d->grow(&d->d_raw_param, (size_t)cap * ncon)) != FK_OK || (rc = d->grow(&d->d_vt, (size_t)cap * L.n_vars)) != FK_OK ||
-            (rc = d->grow(&d->d_pt, (size_t)cap * ne)) != FK_OK)
-            return rc;
-        d->chunk = cap;
-    }
-    if (analyze && d->an_chunk < cap) {
-        d->an_chunk = 0;
-        if ((rc = d->grow(&d->d_indep, (size_t)cap * ne)) != FK_OK || (rc = d->grow(&d->d_dep, (size_t)cap * ncon)) != FK_OK) return rc;
-        d->an_chunk = cap;
-    }
-    if (!analyze && d->res_chunk < cap) {
-        d->res_chunk = 0;
-        if ((rc = d->grow(&d->d_res, (size_t)cap * ncon)) != FK_OK) return rc;
-        d->res_chunk = cap;
-    }
-    return FK_OK;
+    const size_t cap = *chunk;
+    int rc = d->d_raw_param.reserve(cap * ncon);
+    if (rc == FK_OK) rc = d->d_vt.reserve(cap * L.n_vars);
+    if (rc == FK_OK) rc = d->d_pt.reserve(cap * ne);
+    if (rc == FK_OK && analyze) rc = d->d_indep.reserve(cap * ne);
+    if (rc == FK_OK && analyze) rc = d->d_dep.reserve(cap * ncon);
+    if (rc == FK_OK && !analyze) rc = d->d_res.reserve(cap * ncon);
+    return rc;
 }
 
 // Variants [lo, hi) on one device, per chunk: upload (or broadcast the template), expand the parameters, then analyze + reduce or
@@ -2548,7 +2518,7 @@ static int system_an_range(SystemAnBatch& b, const SystemAnCall& c, int device, 
         if (c.params)
             CU(cudaMemcpyAsync(d->d_raw_param, c.params + (size_t)at * ncon, sizeof(double) * (size_t)cnt * ncon, cudaMemcpyHostToDevice, st));
         int e = launch_system_an_expand(cnt, L.n_vars, ne, ncon, c.vars ? nullptr : d->d_tmpl_vars, d->d_vt, d->d_expr_con,
-                                        c.params ? d->d_raw_param : nullptr, d->d_tmpl_param, d->d_pt, st);
+                                        c.params ? d->d_raw_param.get() : nullptr, d->d_tmpl_param, d->d_pt, st);
         if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_an_expand_kernel");
         if (!analyze) {
             e = launch_system_residuals(cnt, L.n_vars, ne, ncon, d->d_kind, d->d_slot, d->d_con_off, d->d_vt, d->d_pt, d->d_res, st);
@@ -2556,20 +2526,8 @@ static int system_an_range(SystemAnBatch& b, const SystemAnCall& c, int device, 
             CU(cudaMemcpyAsync(c.residuals + (size_t)at * ncon, d->d_res, sizeof(double) * (size_t)cnt * ncon, cudaMemcpyDeviceToHost, st));
             return FK_OK;
         }
-        AnalyzePlan plan;  // the kernel for this chunk's size
-        std::string err;
-        const int prc = choose_analyze(L.n_vars, ne, cnt, device, &plan, &err);
-        if (prc != FK_OK) return fail(prc, err);
-        if (d->ws_bytes < plan.workspace_bytes()) {  // grow-only, within fk::kAnWorkspaceBytes
-            CU(cudaStreamSynchronize(st));  // (an earlier chunk's launch may still use the old workspace)
-            d->ws_bytes = 0;
-            const int grc = d->grow(&d->d_ws, plan.workspace_bytes() / sizeof(double));
-            if (grc != FK_OK) return grc;
-            d->ws_bytes = plan.workspace_bytes();
-        }
-        e = plan.kernel == kAnWarp ? launch_batch_analyze(L.n_vars, ne, d->d_kind, d->d_slot, cnt, d->d_vt, d->d_pt, d->d_indep, st)
-                                   : launch_analyze(plan, L.n_vars, ne, d->d_kind, d->d_slot, cnt, d->d_vt, d->d_pt, d->d_indep, d->d_ws, st);
-        if (e != 0) return cuda_fail((cudaError_t)e, plan.kernel == kAnWarp ? "launch fk_batch_analyze_kernel" : "launch fk_analyze_cta_kernel");
+        const int rc = analyze_launch(L.n_vars, ne, d->d_kind, d->d_slot, cnt, d->d_vt, d->d_pt, d->d_indep, device, d->d_ws, st);
+        if (rc != FK_OK) return rc;
         e = launch_system_an_reduce(cnt, ne, ncon, d->d_indep, d->d_con_off, d->d_dep, st);
         if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_system_an_reduce_kernel");
         CU(cudaMemcpyAsync(c.dependent + (size_t)at * ncon, d->d_dep, (size_t)cnt * ncon, cudaMemcpyDeviceToHost, st));
@@ -2657,13 +2615,11 @@ static void systems_plan_create(const std::vector<SystemsDrawing>& d, int optimi
     for (SystemsPlan::Structure& S : P.st) {
         const fk::Topology& t = S.topo->t;
         S.kind = optimizer == 0 && t.path == 2 ? 2 : 1;
-        if (optimizer == 0 && hetero_fits(t, S.instances)) {
-            fk_topology* t32 = S.topo->lanes32();
-            if (t32->t.tile != 32) continue;  // no 32-lane tables (FK_NO_LATENCY_TWIN): a uniform batch
-            S.kind = 0;
-            S.hetero = (uint32_t)P.topos32.size();
-            P.topos32.push_back(t32);
-        }
+        fk_topology* t32 = optimizer == 0 ? hetero_topology(S.topo.get(), S.instances) : nullptr;
+        if (!t32) continue;
+        S.kind = 0;
+        S.hetero = (uint32_t)P.topos32.size();
+        P.topos32.push_back(t32);
     }
 }
 
@@ -2681,16 +2637,15 @@ void systems_layout(const std::vector<SystemsDrawing>& d, int optimizer, uint32_
 }
 
 // Per device, reused across calls (never destroyed: CUDA may be gone at static-destruction time): one stream, a grow-only
-// pinned staging block and device arena, and the grow-only workspaces of the sparse batch LM kernel, the L-BFGS CTA kernel and
-// the global-memory analyze kernels (launches on the one stream run one after the other, so one workspace serves them all).
-// fk_systems_solve, fk_systems_analyze and fk_systems_residuals share it.
+// pinned staging block and device arena, and the grow-only workspaces of the solve kernels and of the global-memory analyze
+// kernels (launches on the one stream run one after the other, so one workspace serves them all).  fk_systems_solve,
+// fk_systems_analyze and fk_systems_residuals share it.
 struct SystemsDevice {
     std::mutex mu;
     cudaStream_t stream = nullptr;
-    unsigned char *h = nullptr, *d = nullptr;
-    size_t h_cap = 0, d_cap = 0;
-    double *lm_ws = nullptr, *lb_ws = nullptr, *an_ws = nullptr;
-    uint64_t lm_ws_doubles = 0, lb_ws_doubles = 0, an_ws_bytes = 0;
+    GrowBuf<unsigned char> h{true}, d;
+    SolveWorkspace ws;
+    GrowBuf<double> an_ws;
 };
 static SystemsDevice* systems_device_for(int device) {
     static std::mutex m;
@@ -2699,6 +2654,50 @@ static SystemsDevice* systems_device_for(int device) {
     SystemsDevice*& p = devs[device];
     if (!p) p = new SystemsDevice();
     return p;
+}
+
+// Drawings [lo, hi) of a many-drawing call on one device, chunk after chunk on its SystemsDevice's stream.  The cut: drawings in
+// order, at least one per chunk, closed at about 1 GiB of bytes(a, b) -- the device bytes drawing b adds to a chunk that starts at
+// drawing a --, at FK_SYSTEM_BATCH_CHUNK drawings and, given inst_off (the instances before each drawing), at INT32_MAX instances,
+// so that every launch stays within INT32_MAX sketches.  layout(c) places the rows of chunk c (c.a, c.b set): the pinned staging
+// block takes its first c.o_work bytes and the device arena its c.end bytes, both reserved for the largest chunk.  Then
+// prepare(D, chunks) once and body(D, c) for every chunk; after a failure the stream is synchronised, so that nothing of the failed
+// chunk still runs when the staging is reused.
+template <class Chunk, class Bytes, class Layout, class Prepare, class Body>
+static int run_drawing_chunks(int device, uint32_t lo, uint32_t hi, const size_t* inst_off, const Bytes& bytes, const Layout& layout,
+                              const Prepare& prepare, const Body& body) {
+    CU(cudaSetDevice(device));
+    SystemsDevice* D = systems_device_for(device);
+    std::lock_guard<std::mutex> lock(D->mu);
+    if (!D->stream) CU(cudaStreamCreateWithFlags(&D->stream, cudaStreamNonBlocking));
+    std::vector<Chunk> chunks;
+    size_t h_need = 0, d_need = 0;
+    const uint32_t cap = system_batch_chunk_env();
+    for (uint32_t a = lo; a < hi;) {
+        uint32_t b = a;
+        uint64_t total = 0;
+        while (b < hi) {
+            const uint64_t db = bytes(a, b);
+            if (b > a && (total + db > (1ull << 30) || (cap && b - a >= cap) || (inst_off && inst_off[b + 1] - inst_off[a] > (uint64_t)INT32_MAX)))
+                break;
+            total += db;
+            b++;
+        }
+        chunks.emplace_back();
+        Chunk& c = chunks.back();
+        c.a = a;
+        c.b = b;
+        layout(c);
+        h_need = std::max(h_need, c.o_work);
+        d_need = std::max(d_need, c.end);
+        a = b;
+    }
+    int rc = D->h.reserve(h_need, h_need + h_need / 4);
+    if (rc == FK_OK) rc = D->d.reserve(d_need, d_need + d_need / 4);
+    if (rc == FK_OK) rc = prepare(*D, chunks);
+    for (size_t k = 0; k < chunks.size() && rc == FK_OK; k++)
+        if ((rc = body(*D, chunks[k])) != FK_OK) cudaStreamSynchronize(D->stream);
+    return rc;
 }
 
 // One chunk of drawings [a, b) on one device and where its rows live in the arena: [0, o_output) the input the host stages in
@@ -2736,43 +2735,38 @@ static void systems_chunk_layout(const std::vector<SystemsDrawing>& d, const Sys
             }
         }
     }
-    size_t at = 0;
-    auto put = [&](size_t bytes) {
-        const size_t o = at;
-        at = (at + std::max<size_t>(bytes, 1) + 255) & ~size_t(255);
-        return o;
-    };
+    BlockLayout blk;
     const size_t ni = c.i1 - c.i0;
-    c.o_draws = put(sizeof(double) * P.draws->size());
-    c.o_progs = put(sizeof(fk::DevProgram) * P.topos32.size());
-    c.o_jobs = put(sizeof(fk::HeteroJob) * c.nj);
-    c.o_inst = put(sizeof(SysInst) * ni);
-    c.o_ioff = put(sizeof(uint32_t) * (n + 1));
-    c.o_voff = put(sizeof(uint64_t) * (n + 1));
-    c.o_eoff = put(sizeof(uint64_t) * (n + 1));
-    c.o_tabs = put(sizeof(uint32_t) * c.tab_words);
-    c.o_rawv = put(sizeof(double) * c.nvars);
-    c.o_rawp = put(sizeof(double) * c.nexpr);
-    c.o_kinds = put(c.nexpr);
-    c.o_output = at;
-    c.o_outv = put(sizeof(double) * c.nvars);
-    c.o_outr = put(sizeof(fk_report) * ni);
-    c.o_work = at;
-    c.o_scales = put(sizeof(double) * n);
-    c.o_hin = put(sizeof(double) * c.hin);
-    c.o_hout = put(sizeof(double) * c.hout);
-    c.o_hrep = put(sizeof(fk_report) * c.nj);
+    c.o_draws = blk.put(sizeof(double) * P.draws->size());
+    c.o_progs = blk.put(sizeof(fk::DevProgram) * P.topos32.size());
+    c.o_jobs = blk.put(sizeof(fk::HeteroJob) * c.nj);
+    c.o_inst = blk.put(sizeof(SysInst) * ni);
+    c.o_ioff = blk.put(sizeof(uint32_t) * (n + 1));
+    c.o_voff = blk.put(sizeof(uint64_t) * (n + 1));
+    c.o_eoff = blk.put(sizeof(uint64_t) * (n + 1));
+    c.o_tabs = blk.put(sizeof(uint32_t) * c.tab_words);
+    c.o_rawv = blk.put(sizeof(double) * c.nvars);
+    c.o_rawp = blk.put(sizeof(double) * c.nexpr);
+    c.o_kinds = blk.put(c.nexpr);
+    c.o_output = blk.end;
+    c.o_outv = blk.put(sizeof(double) * c.nvars);
+    c.o_outr = blk.put(sizeof(fk_report) * ni);
+    c.o_work = blk.end;
+    c.o_scales = blk.put(sizeof(double) * n);
+    c.o_hin = blk.put(sizeof(double) * c.hin);
+    c.o_hout = blk.put(sizeof(double) * c.hout);
+    c.o_hrep = blk.put(sizeof(fk_report) * c.nj);
     c.rows.assign(ns, SystemsChunk::Rows{});
     for (size_t s = 0; s < ns; s++) {
         if (P.st[s].kind == 0 || c.count[s] == 0) continue;
         const fk::Topology& t = P.st[s].topo->t;
         SystemsChunk::Rows& r = c.rows[s];
-        r.vars = put(sizeof(double) * c.count[s] * t.n_vars);
-        r.params = put(sizeof(double) * c.count[s] * t.n_expr);
-        r.out = put(sizeof(double) * c.count[s] * t.n_free);
-        r.reps = put(sizeof(fk_report) * c.count[s]);
+        r.vars = blk.put(sizeof(double) * c.count[s] * t.n_vars);
+        r.params = blk.put(sizeof(double) * c.count[s] * t.n_expr);
+        r.out = blk.put(sizeof(double) * c.count[s] * t.n_free);
+        r.reps = blk.put(sizeof(fk_report) * c.count[s]);
     }
-    c.end = at;
+    c.end = blk.end;
 }
 
 // Device bytes one drawing adds to a chunk (the budget of system_batch_chunk: about 1 GiB per chunk).
@@ -2787,97 +2781,33 @@ static uint64_t systems_drawing_bytes(const std::vector<SystemsDrawing>& d, cons
     return bytes;
 }
 
-// Grow-only device buffer of at least `bytes` (the stream is idle: every call ends with a synchronise).
-template <class T>
-static int systems_grow(T** buf, uint64_t* have, uint64_t need) {
-    if (*have >= need) return FK_OK;
-    cudaFree(*buf);
-    *buf = nullptr;
-    *have = 0;
-    CU(cudaMalloc((void**)buf, std::max<uint64_t>(need, 1)));
-    *have = need;
-    return FK_OK;
-}
-
 // Drawings [lo, hi) on one device, chunk after chunk on its stream: stage and upload, fk_systems_prepare_kernel, one
 // heterogeneous launch, one launch per uniform or sparse structure, fk_systems_scatter_kernel, download; then the chunk's
 // variables and reports into the call's rows (vars_out, reports).
 static int systems_range(const std::vector<SystemsDrawing>& d, const SystemsPlan& P, int optimizer, int perturb, int device, uint32_t lo,
                          uint32_t hi, double* vars_out, fk_report* reports) {
-    CU(cudaSetDevice(device));
-    SystemsDevice* D = systems_device_for(device);
-    std::lock_guard<std::mutex> lock(D->mu);
-    if (!D->stream) CU(cudaStreamCreateWithFlags(&D->stream, cudaStreamNonBlocking));
-    const cudaStream_t st = D->stream;
-    const bool lm = optimizer == 0;
     const size_t ns = P.st.size();
-    // ---- chunks: drawings in order, closed at about 1 GiB (FK_SYSTEM_BATCH_CHUNK caps the drawings), at least one drawing,
-    // at most INT32_MAX instances (so every launch stays within INT32_MAX sketches)
-    std::vector<SystemsChunk> chunks;
-    std::vector<uint32_t> max_count(ns, 0);
-    size_t h_need = 0, d_need = 0;
-    const uint32_t cap = system_batch_chunk_env();
-    for (uint32_t a = lo; a < hi;) {
-        uint32_t b = a;
-        uint64_t bytes = 0, inst = 0;
-        while (b < hi) {
-            const uint64_t db = systems_drawing_bytes(d, P, b), di = P.inst_off[b + 1] - P.inst_off[b];
-            if (b > a && (bytes + db > (1ull << 30) || (cap && b - a >= cap) || inst + di > (uint64_t)INT32_MAX)) break;
-            bytes += db;
-            inst += di;
-            b++;
-        }
-        chunks.emplace_back();
-        SystemsChunk& c = chunks.back();
-        c.a = a;
-        c.b = b;
-        systems_chunk_layout(d, P, c);
-        for (size_t s = 0; s < ns; s++) max_count[s] = std::max(max_count[s], c.count[s]);
-        h_need = std::max(h_need, c.o_work);
-        d_need = std::max(d_need, c.end);
-        a = b;
-    }
-    // ---- programs of the structures present and the workspaces of their largest launch
     std::vector<const DeviceProgram*> full(ns, nullptr);
-    uint64_t lm_ws = 0, lb_ws = 0;
-    for (size_t s = 0; s < ns; s++) {
-        if (P.st[s].kind == 0 || max_count[s] == 0) continue;
-        const fk::DevProgram* v = nullptr;
-        const int rc = P.st[s].topo->program_for(device, &v, &full[s], lm);
-        if (rc != FK_OK) return rc;
-        if (lm && full[s]->sparse_batch) {
-            const fk::SparseBatchProgram& sb = *full[s]->sparse_batch;
-            lm_ws = std::max(lm_ws, sb.workspace_doubles(sb.workspace_ctas(max_count[s])));
-        } else if (!lm && choose_lbfgs(P.st[s].topo.get(), max_count[s]) == 1) {
-            const uint32_t ctas = fk::lbfgs_workspace_ctas(*v, max_count[s]);
-            if (ctas == 0) return fail(FK_ERR_CUDA, "occupancy query of fk_lbfgs_cta_kernel failed");
-            lb_ws = std::max(lb_ws, fk::lbfgs_workspace_doubles(*v, ctas));
-        }
-    }
     std::vector<fk::DevProgram> progs;
     uint32_t max_state = 1;
-    if (!P.topos32.empty())
-        if (const int rc = hetero_programs(device, P.topos32, progs, &max_state); rc != FK_OK) return rc;
-    if (D->h_cap < h_need) {
-        if (D->h) cudaFreeHost(D->h);
-        D->h = nullptr;
-        D->h_cap = 0;
-        const size_t want = h_need + h_need / 4;
-        CU(cudaMallocHost((void**)&D->h, want));
-        D->h_cap = want;
-    }
-    uint64_t d_cap = D->d_cap, lm_have = D->lm_ws_doubles * sizeof(double), lb_have = D->lb_ws_doubles * sizeof(double);
-    int grc = systems_grow(&D->d, &d_cap, d_need + d_need / 4);
-    D->d_cap = d_cap;
-    if (grc == FK_OK) grc = systems_grow(&D->lm_ws, &lm_have, lm_ws * sizeof(double));
-    D->lm_ws_doubles = lm_have / sizeof(double);
-    if (grc == FK_OK) grc = systems_grow(&D->lb_ws, &lb_have, lb_ws * sizeof(double));
-    D->lb_ws_doubles = lb_have / sizeof(double);
-    if (grc != FK_OK) return grc;
-
-    auto run = [&](const SystemsChunk& c) -> int {
-        unsigned char* H = D->h;
-        unsigned char* G = D->d;
+    // the programs of the structures present, the workspaces of their largest launch, the programs of the heterogeneous launch
+    auto prepare = [&](SystemsDevice& D, const std::vector<SystemsChunk>& chunks) -> int {
+        std::vector<uint32_t> max_count(ns, 0);
+        for (const SystemsChunk& c : chunks)
+            for (size_t s = 0; s < ns; s++) max_count[s] = std::max(max_count[s], c.count[s]);
+        for (size_t s = 0; s < ns; s++) {
+            if (P.st[s].kind == 0 || max_count[s] == 0) continue;
+            const fk::DevProgram* v = nullptr;
+            int rc = P.st[s].topo->program_for(device, &v, &full[s], optimizer == 0);
+            if (rc == FK_OK) rc = D.ws.reserve(*full[s], solve_kernel(P.st[s].topo.get(), optimizer, max_count[s]), max_count[s]);
+            if (rc != FK_OK) return rc;
+        }
+        return P.topos32.empty() ? FK_OK : hetero_programs(device, P.topos32, progs, &max_state);
+    };
+    auto run = [&](SystemsDevice& D, const SystemsChunk& c) -> int {
+        const cudaStream_t st = D.stream;
+        unsigned char* H = D.h;
+        unsigned char* G = D.d;
         const uint32_t n = c.b - c.a;
         if (!P.draws->empty()) std::memcpy(H + c.o_draws, P.draws->data(), sizeof(double) * P.draws->size());
         if (!progs.empty()) std::memcpy(H + c.o_progs, progs.data(), sizeof(fk::DevProgram) * progs.size());
@@ -2969,24 +2899,10 @@ static int systems_range(const std::vector<SystemsDrawing>& d, const SystemsPlan
         for (size_t s = 0; s < ns; s++) {
             const uint32_t cnt = c.count[s];
             if (P.st[s].kind == 0 || cnt == 0) continue;
-            const DeviceProgram& F = *full[s];
             const SystemsChunk::Rows& r = c.rows[s];
-            const double* v = (const double*)(G + r.vars);
-            const double* q = (const double*)(G + r.params);
-            double* o = (double*)(G + r.out);
-            fk_report* rp = (fk_report*)(G + r.reps);
-            if (lm) {
-                const uint32_t ws_ctas = F.sparse_batch ? F.sparse_batch->workspace_ctas(cnt) : 0;
-                e = launch_lm(F, cnt, v, q, o, rp, D->lm_ws, ws_ctas, st);
-                if (e != 0) return cuda_fail((cudaError_t)e, "launch batched LM kernel");
-            } else if (choose_lbfgs(P.st[s].topo.get(), cnt) == 1) {
-                e = fk::launch_lbfgs_cta(F.view, F.jcolptr, F.jrow, cnt, v, q, o, rp, D->lb_ws, fk::lbfgs_workspace_ctas(F.view, cnt), st);
-                if (e == (int)cudaErrorInvalidConfiguration) return fail(FK_ERR_TOO_LARGE, "more than 2^24 Jacobian entries");
-                if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_lbfgs_cta_kernel");
-            } else {
-                e = fk::launch_batch_lbfgs(F.view, F.jcolptr, F.jrow, cnt, v, q, o, rp, st);
-                if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_batch_lbfgs_kernel");
-            }
+            const int rc = solve_launch(*full[s], solve_kernel(P.st[s].topo.get(), optimizer, cnt), cnt, (const double*)(G + r.vars),
+                                        (const double*)(G + r.params), (double*)(G + r.out), (fk_report*)(G + r.reps), D.ws, st);
+            if (rc != FK_OK) return rc;
         }
         e = launch_systems_scatter(n, d_voff, d_ioff, d_rawv, d_scales, d_inst, d_tabs, (double*)(G + c.o_outv), (fk_report*)(G + c.o_outr), st);
         if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_systems_scatter_kernel");
@@ -2996,14 +2912,9 @@ static int systems_range(const std::vector<SystemsDrawing>& d, const SystemsPlan
         if (c.i1 > c.i0) std::memcpy(reports + c.i0, H + c.o_outr, sizeof(fk_report) * (c.i1 - c.i0));
         return FK_OK;
     };
-    for (const SystemsChunk& c : chunks) {
-        const int rc = run(c);
-        if (rc != FK_OK) {
-            cudaStreamSynchronize(st);  // (nothing of a failed chunk may still run when the staging is reused)
-            return rc;
-        }
-    }
-    return FK_OK;
+    return run_drawing_chunks<SystemsChunk>(
+        device, lo, hi, P.inst_off.data(), [&](uint32_t, uint32_t b) { return systems_drawing_bytes(d, P, b); },
+        [&](SystemsChunk& c) { systems_chunk_layout(d, P, c); }, prepare, run);
 }
 
 int systems_solve(const std::vector<SystemsDrawing>& d, int optimizer, int perturb, int n_gpus, double* vars_out, fk_report* reports) {
@@ -3131,23 +3042,17 @@ static void systems_an_chunk_layout(const std::vector<SystemsAnDrawing>& d, cons
         c.nexpr += (size_t)c.count[s] * P.st[s].b->n_expr;
     }
     c.ncon = P.con_off[c.b] - P.con_off[c.a];
-    size_t at = 0;
-    auto put = [&](size_t bytes) {
-        const size_t o = at;
-        at = (at + std::max<size_t>(bytes, 1) + 255) & ~size_t(255);
-        return o;
-    };
-    c.o_desc = put(sizeof(SysAnJob) * n);
-    c.o_base = put(sizeof(uint64_t) * (n + 1));
-    c.o_jobs = put(sizeof(SysAnJob) * c.nj);
-    c.o_tabs = put(sizeof(uint32_t) * c.tab_words);
-    c.o_vars = put(sizeof(double) * c.nvars);
-    c.o_params = put(sizeof(double) * c.nexpr);
-    c.o_output = at;
-    put(analyze ? c.ncon : sizeof(double) * c.ncon);
-    c.o_work = at;
-    if (analyze) put(c.nexpr);
-    c.end = at;
+    BlockLayout blk;
+    c.o_desc = blk.put(sizeof(SysAnJob) * n);
+    c.o_base = blk.put(sizeof(uint64_t) * (n + 1));
+    c.o_jobs = blk.put(sizeof(SysAnJob) * c.nj);
+    c.o_tabs = blk.put(sizeof(uint32_t) * c.tab_words);
+    c.o_vars = blk.put(sizeof(double) * c.nvars);
+    c.o_params = blk.put(sizeof(double) * c.nexpr);
+    c.o_output = blk.put(analyze ? c.ncon : sizeof(double) * c.ncon);
+    c.o_work = blk.end;
+    if (analyze) blk.put(c.nexpr);
+    c.end = blk.end;
 }
 
 // The warp footprint class of a drawing: its batch_analyze_warp_bytes rounded up to a power of two, at most 200 KiB.  One
@@ -3165,57 +3070,22 @@ static size_t an_footprint_class(uint32_t n_vars, uint32_t n_expr) {
 // download, then the chunk's counts or residuals into the call's output.
 static int systems_an_range(const std::vector<SystemsAnDrawing>& d, const SystemsAnPlan& P, int device, uint32_t lo, uint32_t hi,
                             uint8_t* dependent, double* residuals) {
-    CU(cudaSetDevice(device));
-    SystemsDevice* D = systems_device_for(device);
-    std::lock_guard<std::mutex> lock(D->mu);
-    if (!D->stream) CU(cudaStreamCreateWithFlags(&D->stream, cudaStreamNonBlocking));
-    const cudaStream_t st = D->stream;
     const bool analyze = dependent != nullptr;
     const size_t ns = P.st.size();
-    // ---- chunks: drawings in order, closed at about 1 GiB (FK_SYSTEM_BATCH_CHUNK caps the drawings), at least one drawing
-    std::vector<SystemsAnChunk> chunks;
     std::vector<uint32_t> seen(ns, kSbNone);  // the chunk that last counted a structure's tables
-    size_t h_need = 0, d_need = 0;
-    const uint32_t cap = system_batch_chunk_env();
-    for (uint32_t a = lo; a < hi;) {
-        uint32_t b = a;
-        uint64_t bytes = 0;
-        while (b < hi) {
-            const uint32_t s = P.drawing_struct[b];
-            const SystemAnBatch& B = *d[b].plan;
-            uint64_t db = sizeof(double) * ((uint64_t)B.L.n_vars + B.n_expr) + B.n_expr + 2 * sizeof(SysAnJob) + sizeof(uint64_t) +
-                          (analyze ? 1 : sizeof(double)) * (uint64_t)B.n_constraints;
-            if (seen[s] != a) db += sizeof(uint32_t) * P.st[s].tab_words;
-            if (b > a && (bytes + db > (1ull << 30) || (cap && b - a >= cap))) break;
-            seen[s] = a;
-            bytes += db;
-            b++;
-        }
-        chunks.emplace_back();
-        SystemsAnChunk& c = chunks.back();
-        c.a = a;
-        c.b = b;
-        systems_an_chunk_layout(d, P, analyze, c);
-        h_need = std::max(h_need, c.o_work);
-        d_need = std::max(d_need, c.end);
-        a = b;
-    }
-    if (D->h_cap < h_need) {
-        if (D->h) cudaFreeHost(D->h);
-        D->h = nullptr;
-        D->h_cap = 0;
-        const size_t want = h_need + h_need / 4;
-        CU(cudaMallocHost((void**)&D->h, want));
-        D->h_cap = want;
-    }
-    uint64_t d_cap = D->d_cap;
-    const int grc = systems_grow(&D->d, &d_cap, d_need + d_need / 4);
-    D->d_cap = d_cap;
-    if (grc != FK_OK) return grc;
-
-    auto run = [&](const SystemsAnChunk& c) -> int {
-        unsigned char* H = D->h;
-        unsigned char* G = D->d;
+    auto bytes = [&](uint32_t a, uint32_t b) -> uint64_t {
+        const uint32_t s = P.drawing_struct[b];
+        const SystemAnBatch& B = *d[b].plan;
+        uint64_t db = sizeof(double) * ((uint64_t)B.L.n_vars + B.n_expr) + B.n_expr + 2 * sizeof(SysAnJob) + sizeof(uint64_t) +
+                      (analyze ? 1 : sizeof(double)) * (uint64_t)B.n_constraints;
+        if (seen[s] != a) db += sizeof(uint32_t) * P.st[s].tab_words;
+        seen[s] = a;  // (a drawing the cut leaves out starts the next chunk, which counts the tables again)
+        return db;
+    };
+    auto run = [&](SystemsDevice& D, const SystemsAnChunk& c) -> int {
+        const cudaStream_t st = D.stream;
+        unsigned char* H = D.h;
+        unsigned char* G = D.d;
         const uint32_t n = c.b - c.a;
         SysAnJob* desc = (SysAnJob*)(H + c.o_desc);
         uint64_t* base = (uint64_t*)(H + c.o_base);
@@ -3284,25 +3154,10 @@ static int systems_an_range(const std::vector<SystemsAnDrawing>& d, const System
             for (size_t s = 0; s < ns; s++) {
                 if (P.st[s].kind == 0 || c.count[s] == 0) continue;
                 const SystemAnBatch& B = *P.st[s].b;
-                AnalyzePlan plan;
-                std::string err;
-                const int prc = choose_analyze(B.L.n_vars, B.n_expr, c.count[s], device, &plan, &err);
-                if (prc != FK_OK) return fail(prc, err);
-                if (D->an_ws_bytes < plan.workspace_bytes()) {  // grow-only, within fk::kAnWorkspaceBytes
-                    CU(cudaStreamSynchronize(st));  // (an earlier launch may still use the old workspace)
-                    uint64_t have = D->an_ws_bytes;
-                    const int rc = systems_grow(&D->an_ws, &have, plan.workspace_bytes());
-                    D->an_ws_bytes = have;
-                    if (rc != FK_OK) return rc;
-                }
                 const uint32_t* slot = d_tabs + c.tab[s];
-                const uint8_t* kinds = sys_an_kinds(slot, B.n_expr);
-                const double* v = d_vars + c.vblk[s];
-                const double* q = d_params + c.eblk[s];
-                e = plan.kernel == kAnWarp ? launch_batch_analyze(B.L.n_vars, B.n_expr, kinds, slot, c.count[s], v, q, d_flags + c.eblk[s], st)
-                                           : launch_analyze(plan, B.L.n_vars, B.n_expr, kinds, slot, c.count[s], v, q, d_flags + c.eblk[s],
-                                                            D->an_ws, st);
-                if (e != 0) return cuda_fail((cudaError_t)e, plan.kernel == kAnWarp ? "launch fk_batch_analyze_kernel" : "launch fk_analyze_cta_kernel");
+                const int rc = analyze_launch(B.L.n_vars, B.n_expr, sys_an_kinds(slot, B.n_expr), slot, c.count[s], d_vars + c.vblk[s],
+                                              d_params + c.eblk[s], d_flags + c.eblk[s], device, D.an_ws, st);
+                if (rc != FK_OK) return rc;
             }
             e = launch_systems_an_reduce(n, c.ncon, d_base, d_desc, d_tabs, d_flags, G + c.o_output, st);
             if (e != 0) return cuda_fail((cudaError_t)e, "launch fk_systems_an_reduce_kernel");
@@ -3316,14 +3171,9 @@ static int systems_an_range(const std::vector<SystemsAnDrawing>& d, const System
         }
         return FK_OK;
     };
-    for (const SystemsAnChunk& c : chunks) {
-        const int rc = run(c);
-        if (rc != FK_OK) {
-            cudaStreamSynchronize(st);  // (nothing of a failed chunk may still run when the staging is reused)
-            return rc;
-        }
-    }
-    return FK_OK;
+    return run_drawing_chunks<SystemsAnChunk>(
+        device, lo, hi, nullptr, bytes, [&](SystemsAnChunk& c) { systems_an_chunk_layout(d, P, analyze, c); },
+        [](SystemsDevice&, const std::vector<SystemsAnChunk>&) { return FK_OK; }, run);
 }
 
 int systems_an_run(const std::vector<SystemsAnDrawing>& d, uint8_t* dependent, double* residuals, int n_gpus) {
